@@ -57,7 +57,14 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-verify", action="store_true")
     ap.add_argument("--cpu-seconds", type=float, default=12.0)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="one GPU: write the timed solve's value and policy tables to DIR/*.npy (see dump_outputs)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU solve's tables; the reference arm solves a sub-grid only")
+    return args
 
 
 def make_spec(S, name, n_gpus, states_per_gpu):
@@ -319,6 +326,30 @@ def sample_check(spec, solver, n=32, seed=5):
     return True
 
 
+DUMP_BYTES = 56 << 20  # V, Q and the state index together: the whole dump stays under 64 MB
+
+
+def dump_outputs(out_dir, solver, init, seed=0):
+    """What a caller of the timed solve receives, as float64 .npy files, for comparing two builds output for output:
+    V.npy / Q.npy [T, k]: the value and order-quantity tables of every period (sdpb_period_tables) at the k flattened
+    state indices in state_index.npy -- every state when that fits in DUMP_BYTES, else a fixed sample drawn with
+    `seed` (the same states in every run of the same workload); V1_init.npy / Q1_init.npy: sdpb_value at the
+    workload's initial state."""
+    import numpy as np
+    n, T = solver.n_states, solver.T
+    k = min(n, DUMP_BYTES // (16 * T + 8))
+    idx = np.arange(n) if k == n else np.sort(np.random.default_rng(seed).choice(n, size=k, replace=False))
+    V, Q = np.empty((T, k)), np.empty((T, k))
+    Vt, Qt = np.empty(n), np.empty(n)
+    for t in range(1, T + 1):
+        solver.period_tables(t, out_v=Vt, out_q=Qt)
+        V[t - 1], Q[t - 1] = Vt[idx], Qt[idx]
+    v1, q1 = solver.value(1, init)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in (("V", V), ("Q", Q), ("state_index", idx.astype(np.float64)), ("V1_init", v1), ("Q1_init", q1)):
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def verify_vs_unsharded(S, torch, dist, sp, sharded, local, dedup):
     """Multi-GPU result check (outside every timed region): each rank re-solves the WHOLE grid by itself and compares
     its own block of V_1 and Q_1, bit for bit, with what the sharded solve (real peer exchange) left in its tables."""
@@ -419,6 +450,8 @@ def run_gpu(args):
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if not torch.cuda.is_available():
         raise SystemExit("bench.py needs a CUDA device: libsdpb200 has no CPU path")
+    if args.dump_outputs and world > 1:
+        raise SystemExit("--dump-outputs needs --gpus 1: a shard holds only its block of the tables")
     torch.cuda.set_device(local)
     dist = None
     if world > 1:
@@ -474,6 +507,8 @@ def run_gpu(args):
             [ms, ev_step * args.steps, fp_step * args.steps, launches_step * args.steps])
         value = ev_total / (ms * 1e-3)
         dev_bytes = sh.solver.grid.device_bytes
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, sh.solver, INIT[name])
         bytes_out, bytes_in = sh.bytes_out, sh.bytes_in
 
         # ---- verification of the timed workload's result (outside every timed region) ----
