@@ -207,10 +207,11 @@ typedef struct sdpb_model {
 typedef enum sdpb_kernel_choice {
     SDPB_KERNEL_AUTO = 0,     /* fastest bit-exact kernel available for the model */
     SDPB_KERNEL_GENERIC = 1,  /* always the generic per-(s,a,d) kernel */
-    SDPB_KERNEL_TILED = 2,    /* shared-memory kernel (tiled for lead_time 0, staged warp-per-state
-                                 for backorder lead-time models); error if the model has none */
+    SDPB_KERNEL_TILED = 2,    /* shared-memory kernel: tiled for lead_time 0; for backorder lead-time models the
+                                 column kernel (else slab, else staged); for integer-exact cash models the
+                                 integer cash kernels; error if the model has none */
     SDPB_KERNEL_STAGED = 3,   /* warp-per-state staged kernel for backorder lead-time models (as a request:
-                                 skip the slab kernel) */
+                                 skip the all-actions-in-thread, column and slab kernels) */
     SDPB_KERNEL_CASH_INT = 4, /* integer-exact cash kernel (as a request: skip the diagonal-window variant) */
     SDPB_KERNEL_CASH_DIAG = 8,/* reported only: integer-exact cash kernel with a register window along the
                                  (1, -price) diagonal; the last period runs on SDPB_KERNEL_CASH_INT */
@@ -233,8 +234,9 @@ typedef enum sdpb_kernel_choice {
                                  SDPB_F_NO_ORDER_LAST; sdpb_create fails with SDPB_ERR_ARG otherwise */
     SDPB_KERNEL_TWO_PRODUCT_ROW = 10, /* reported only: two-product kernel that shares the cash-independent terms
                                          of an (action, demand) pair across a row of cash levels (integer prices) */
-    SDPB_KERNEL_CASH_ROW = 12,/* reported only: cash-constraint kind on any cash grid; a CTA is one inventory level x 128
-                                 cash levels and shares the cash-independent terms of each (action, demand) */
+    SDPB_KERNEL_CASH_ROW = 12,/* cash-constraint kind on any cash grid; a CTA is one inventory level x 128 cash levels and
+                                 shares the cash-independent terms of each (action, demand).  As a request: skip
+                                 SDPB_KERNEL_CASH_TAIL (integer-exact models still run the integer cash kernels) */
     SDPB_KERNEL_CASH_TAIL = 13,/* reported only: cash-constraint and overdraft kinds on any rounding cash grid; row-shared terms as
                                  SDPB_KERNEL_CASH_ROW, with the cash clamp applied to the rounded integer (as a request,
                                  SDPB_KERNEL_CASH_ROW skips it) */

@@ -281,19 +281,17 @@ inline CashIntShape cash_int_shape(const sdpb_model& m, const DevModel& dm, int 
     const long long tiles = (long long)rows * ((dm.nW + s.tile - 1) / s.tile);
     s.parts = parts_for(tiles);
     if (s.wide && tiles16 >= 3LL * sm_count) s.parts = 1;  // measured on C3 (1002 CTAs): 103.9 ms unsliced, 104.6 in 10 slices
-    static const int env_split = [] { const char* e = std::getenv("SDPB_CASH_INT_SPLIT"); return e ? std::atoi(e) : 0; }();
-    if (env_split) s.parts = std::max(1, std::min(env_split, 32));  // tuning knob, read once per process
     s.grid = dim3((unsigned)rows, (unsigned)((dm.nW + s.tile - 1) / s.tile), (unsigned)s.parts);
     return s;
 }
 
-// SDPB_OK, SDPB_ERR_STATE (no plan for this period: use the generic kernel), SDPB_ERR_NOMEM (slice scratch too small:
-// the caller sizes it with cash_int_shape) or SDPB_ERR_CUDA.
-inline int launch_cash(const CashPlan& P, const sdpb_model& m, const DevModel& dm, int t, int D, int pmf_off,
-                       const double* Vn, double* Vt, int* Qt, long long lo, long long hi, cudaStream_t stream,
-                       double* fp64_ops, double evals, int sm_count, const DevPeer* d_peers = nullptr, int n_peers = 0,
-                       bool* pushed = nullptr) {
-    if (!P.available || !P.period[t - 1].ok) return SDPB_ERR_STATE;
+inline size_t cash_int_smem(int D) { return (size_t)D * 28 + 16; }
+
+// For a period with a plan and cash_int_smem(D) <= 200 KB.  SDPB_OK, SDPB_ERR_NOMEM (slice scratch too small: the caller
+// sizes it with sh = cash_int_shape) or SDPB_ERR_CUDA.
+inline int launch_cash(const CashPlan& P, const CashIntShape& sh, const sdpb_model& m, const DevModel& dm, int t, int D,
+                       int pmf_off, const double* Vn, double* Vt, int* Qt, long long lo, long long hi, cudaStream_t stream,
+                       const DevPeer* d_peers, int n_peers) {
     if (hi <= lo) return SDPB_OK;
     const CashPeriod& cp = P.period[t - 1];
     CashArgs a;
@@ -301,7 +299,6 @@ inline int launch_cash(const CashPlan& P, const sdpb_model& m, const DevModel& d
     a.ix0 = (int)(lo / dm.nW);
     a.price = cp.price; a.v = cp.v; a.K = P.K; a.ovh = cp.ovh; a.d0 = cp.d0; a.inv_min_i = (int)m.inv_min;
     const bool surv = m.recursion == SDPB_REC_SURVIVAL;
-    const CashIntShape sh = cash_int_shape(m, dm, t, lo, hi, sm_count);
     const bool wide = sh.wide;
     const dim3 grid = sh.grid;
     const long long n_local = hi - lo;
@@ -309,8 +306,7 @@ inline int launch_cash(const CashPlan& P, const sdpb_model& m, const DevModel& d
         if ((size_t)sh.parts * (size_t)n_local > P.slice_cap) return SDPB_ERR_NOMEM;
         a.slice_v = P.slice_v; a.slice_a = P.slice_a;
     } else { a.slice_v = nullptr; a.slice_a = nullptr; }
-    const size_t smem = (size_t)D * 28 + 16;
-    if (smem > 200 * 1024) return SDPB_ERR_STATE;  // demand support too long for the shared-memory tables: general path
+    const size_t smem = cash_int_smem(D);
     if (smem > 48 * 1024) {
         cudaFuncSetAttribute(bi_cash_int<true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         cudaFuncSetAttribute(bi_cash_int<false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
@@ -341,11 +337,6 @@ inline int launch_cash(const CashPlan& P, const sdpb_model& m, const DevModel& d
         if (dm.is_min && !surv) merge_action_slices<true><<<mb, 256, 0, stream>>>(P.slice_v, P.slice_a, sh.parts, n_local, Vt + lo, Qt + lo, lo, d_peers, n_peers, t);
         else merge_action_slices<false><<<mb, 256, 0, stream>>>(P.slice_v, P.slice_a, sh.parts, n_local, Vt + lo, Qt + lo, lo, d_peers, n_peers, t);
         if (cudaGetLastError() != cudaSuccess) return SDPB_ERR_CUDA;
-        if (pushed && n_peers > 0) *pushed = true;
-    }
-    if (fp64_ops) {
-        if (t == m.T) *fp64_ops += evals * (surv ? 2.0 + 3.0 / kCashR : 1.0 + 4.0 / (wide ? kCashRLast : kCashR));
-        else *fp64_ops += evals * (surv ? 2.0 : 3.0 + 2.0 / kCashR);
     }
     return SDPB_OK;
 }
@@ -370,11 +361,11 @@ inline int launch_cash(const CashPlan& P, const sdpb_model& m, const DevModel& d
 constexpr int kDiagYT = 8;
 constexpr int kDiagCols = 64;  // state columns (cash levels of slot 0) per CTA
 
-template <bool SURVIVAL, bool IS_MIN, int PF = 2>
+template <bool SURVIVAL, bool IS_MIN>
 __global__ void __launch_bounds__(kDiagCols, 512 / kDiagCols)
 bi_cash_diag(const __grid_constant__ DevModel M, const __grid_constant__ CashArgs a) {
     constexpr int kDiagThreads = kDiagCols;
-    constexpr int YT = kDiagYT;
+    constexpr int YT = kDiagYT, PF = 2;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     double2* PP = reinterpret_cast<double2*>(smem_raw);                    // (p, p*gamma)
     double* PRd = reinterpret_cast<double*>(smem_raw + (size_t)a.D * 16);  // price * d_j
@@ -494,7 +485,7 @@ bi_cash_diag(const __grid_constant__ DevModel M, const __grid_constant__ CashArg
             j += 1;                                                                                  \
         }
         while (j + W <= jy0) {
-            const int ro_last = ro_run - (W - 1) * M.nW, c_last = c_run + (W - 1) * price;  // (price > 0: checked by the launcher)
+            const int ro_last = ro_run - (W - 1) * M.nW, c_last = c_run + (W - 1) * price;  // (price > 0: cash_diag_ok)
             const bool rows_in = ro_last >= 0 && ro_run <= row_max;
             const bool cash_in = c_run >= 0 && c_last <= nW1, cash_hi = c_run >= nW1;
             if (!SURVIVAL && rows_in && (cash_in || cash_hi)) {
@@ -579,21 +570,24 @@ inline int cash_diag_parts(const sdpb_model& m, const DevModel& dm, const CashPe
     int parts = 1;
     if (tiles < want) parts = (int)std::min<long long>((want + tiles - 1) / tiles, 16);
     parts = std::max(1, std::min(parts, (m.max_order_idx + 1) / 12));
-    static const int env_split = [] { const char* e = std::getenv("SDPB_DIAG_SPLIT"); return e ? std::atoi(e) : 0; }();
-    if (env_split) parts = std::max(1, std::min(env_split, 32));  // tuning knob, read once per process
     return parts;
 }
 
-inline int launch_cash_diag(const CashPlan& P, const sdpb_model& m, const DevModel& dm, int t, int D, int pmf_off,
+inline size_t cash_diag_smem(int D) { return (((size_t)D * 24 + 15) & ~(size_t)15) + 16; }
+
+// Whether bi_cash_diag can solve a period (t < T) whose integer plan is cp.
+inline bool cash_diag_ok(const CashPeriod& cp, const sdpb_model& m, const DevModel& dm, int D) {
+    return cp.price > 0 && cp.price * (kDiagYT - 1) <= dm.nW &&  // the diagonal must stay on the cash axis
+           (long long)(dm.nI + D + std::abs(cp.d0) + 2 * kDiagYT + m.max_order_idx) * dm.nW < 0x7fffffffLL &&  // 32-bit row offsets
+           cash_diag_smem(D) <= 200 * 1024;
+}
+
+// For a period t < T with a plan and cash_diag_ok; `parts` = cash_diag_parts.  SDPB_OK, SDPB_ERR_NOMEM or SDPB_ERR_CUDA.
+inline int launch_cash_diag(const CashPlan& P, int parts, const sdpb_model& m, const DevModel& dm, int t, int D, int pmf_off,
                             const double* Vn, double* Vt, int* Qt, long long lo, long long hi, cudaStream_t stream,
-                            double* fp64_ops, double evals, int sm_count, const DevPeer* d_peers = nullptr, int n_peers = 0,
-                            bool* pushed = nullptr) {
-    if (!P.available || t >= m.T || !P.period[t - 1].ok) return SDPB_ERR_STATE;
+                            const DevPeer* d_peers, int n_peers) {
     if (hi <= lo) return SDPB_OK;
     const CashPeriod& cp = P.period[t - 1];
-    if (cp.price <= 0 || cp.price * (kDiagYT - 1) > dm.nW) return SDPB_ERR_STATE;  // diagonal must stay on the cash axis
-    if ((long long)(dm.nI + D + std::abs(cp.d0) + 2 * kDiagYT + m.max_order_idx) * dm.nW >= 0x7fffffffLL)
-        return SDPB_ERR_STATE;  // running 32-bit row offsets
     CashArgs a;
     a.t = t; a.D = D; a.pmf_off = pmf_off; a.Vn = Vn; a.Vt = Vt; a.Qt = Qt; a.lo = lo; a.hi = hi;
     a.ix0 = (int)(lo / dm.nW);
@@ -601,23 +595,20 @@ inline int launch_cash_diag(const CashPlan& P, const sdpb_model& m, const DevMod
     a.price = cp.price; a.v = cp.v; a.K = P.K; a.ovh = cp.ovh; a.d0 = cp.d0; a.inv_min_i = (int)m.inv_min;
     const int span_w = dm.nW + cp.price * (kDiagYT - 1);  // slot 0's cash index runs past the axis so slot 7 covers it
     const unsigned gx = (unsigned)((span_w + kDiagCols - 1) / kDiagCols), gy = (unsigned)((ix1 - a.ix0 + 1 + kDiagYT - 1) / kDiagYT);
-    const int parts = cash_diag_parts(m, dm, cp, lo, hi, sm_count);
     const long long n_local = hi - lo;
     if (parts > 1) {
         const size_t need = (size_t)parts * (size_t)n_local;
-        if (need > P.slice_cap) return SDPB_ERR_NOMEM;  // (the caller sizes the scratch: see cash_diag_scratch)
+        if (need > P.slice_cap) return SDPB_ERR_NOMEM;  // (the caller sizes the scratch)
         a.slice_v = P.slice_v; a.slice_a = P.slice_a;
         // (every slice writes every state of [lo, hi): a valid state has at least one action, so its thread never exits early)
     } else { a.slice_v = nullptr; a.slice_a = nullptr; }
     const dim3 grid(gx, gy, (unsigned)parts);
-    const size_t smem = (((size_t)D * 24 + 15) & ~(size_t)15) + 16;
+    const size_t smem = cash_diag_smem(D);
     const bool surv = m.recursion == SDPB_REC_SURVIVAL;
-    if (smem > 200 * 1024) return SDPB_ERR_STATE;  // demand support too long for the shared-memory tables: general path
     cudaError_t e = cudaSuccess;
-    static const int env_pf = [] { const char* e2 = std::getenv("SDPB_DIAG_PF"); return e2 ? std::atoi(e2) : 0; }();
 #define SDPB_DIAG_LAUNCH(SV, MN)                                                                              \
     {                                                                                                         \
-        auto k = env_pf == 4 ? bi_cash_diag<SV, MN, 4> : env_pf == 3 ? bi_cash_diag<SV, MN, 3> : bi_cash_diag<SV, MN>; \
+        auto k = bi_cash_diag<SV, MN>;                                                                        \
         if (smem > 48 * 1024) e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
         if (e == cudaSuccess) k<<<grid, kDiagCols, smem, stream>>>(dm, a);                                   \
     }
@@ -629,9 +620,7 @@ inline int launch_cash_diag(const CashPlan& P, const sdpb_model& m, const DevMod
         if (dm.is_min && !surv) merge_action_slices<true><<<mb, 256, 0, stream>>>(P.slice_v, P.slice_a, parts, n_local, Vt + lo, Qt + lo, lo, d_peers, n_peers, t);
         else merge_action_slices<false><<<mb, 256, 0, stream>>>(P.slice_v, P.slice_a, parts, n_local, Vt + lo, Qt + lo, lo, d_peers, n_peers, t);
         if (cudaGetLastError() != cudaSuccess) return SDPB_ERR_CUDA;
-        if (pushed && n_peers > 0) *pushed = true;
     }
-    if (fp64_ops) *fp64_ops += evals * (surv ? 2.0 : 3.0 + 2.0 / kDiagYT);
     return SDPB_OK;
 }
 

@@ -97,9 +97,9 @@ inline int launch_collapsed(const DevModel& dm, int t, int D, int pmf_off, const
                             long long il0, double* G, double* Vt, int* Qt, cudaStream_t stream) {
     const int nY = dm.nI + dm.max_order_idx;
     const unsigned gb = (unsigned)((nY + 255) / 256), sb = (unsigned)((dm.S + 255) / 256);
+    // both below 48 KB: sdpb_create refuses max_order_idx >= 6000 and demand rows longer than 2000 for this kernel
     const size_t smem_l = (size_t)D * 20 + 16;
     const size_t smem = (size_t)(dm.max_order_idx + 1) * sizeof(double);
-    if (smem > 48 * 1024 || smem_l > 48 * 1024) return SDPB_ERR_STATE;  // (sdpb_create refuses such a model for this kernel)
     if (Vn) collapsed_levels<false><<<gb, 256, smem_l, stream>>>(dm, D, pmf_off, Vn, Lc, il0, G, nY);
     else collapsed_levels<true><<<gb, 256, smem_l, stream>>>(dm, D, pmf_off, Vn, Lc, il0, G, nY);
     if (dm.is_min) collapsed_actions<true><<<sb, 256, smem, stream>>>(dm, t, G, Vt, Qt, dm.S);

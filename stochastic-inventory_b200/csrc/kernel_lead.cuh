@@ -294,7 +294,7 @@ inline int launch_lead(const LeadPlan& P, const DevModel& dm, int t, int D, int 
 // staging, no per-tile set-up.  A CTA is NQB whole preQ2 values x all actions (505 of 512 threads
 // busy for C4), so the argopt over a stays inside the CTA: after each chunk the 8 x NQB states are
 // reduced through shared memory with the lexicographic (value, action) rule.
-constexpr int kColYT = 8;  // default levels per chunk; a 4-level instantiation exists for the tuning knob
+constexpr int kColYT = 8;  // levels per chunk
 
 struct ColArgs {
     int t, D, pmf_off;
@@ -309,9 +309,10 @@ struct ColArgs {
     int nthreads;
 };
 
-template <bool IS_MIN, bool LAST, bool DEDUP, int YT>
-__global__ void __launch_bounds__(512, (YT == 4 ? 2 : 1))
+template <bool IS_MIN, bool LAST, bool DEDUP>
+__global__ void __launch_bounds__(512, 1)
 bi_lead_col(const __grid_constant__ DevModel M, const __grid_constant__ ColArgs a) {
+    constexpr int YT = kColYT;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int D = a.D, A = a.A;
     // layout: [ red 2 x YT*nthreads doubles (double-buffered) ][ Lw NRW doubles ][ RO NRW int64 row offsets ][ PP D double2 ]
@@ -443,7 +444,6 @@ bi_lead_col(const __grid_constant__ DevModel M, const __grid_constant__ ColArgs 
 
 struct ColPlan {
     bool ok = false;
-    int YT = kColYT;
     int NQB = 1, nthreads = 0, LT = 0, di_max = 0, span = 0, NRW = 0;
     size_t smem = 0;
 };
@@ -459,20 +459,16 @@ inline ColPlan plan_col(const sdpb_model& m, const DevModel& d, int D, const int
     }
     const int A = d.max_order_idx + 1;
     if (A > 512) return P;
-    int max_threads = 512;  // measured best on C4 (512: 238 ms, 128: 244, 224: 270, 320: 317)
-    static const int env_threads = [] { const char* e = std::getenv("SDPB_COL_THREADS"); return e ? std::atoi(e) : 0; }();
-    if (env_threads) max_threads = std::max(32, std::min(512, env_threads));  // tuning knob, read once per process
+    const int max_threads = 512;  // measured best on C4 (512: 238 ms, 128: 244, 224: 270, 320: 317)
     P.NQB = m.lead_time == 2 ? std::max(1, std::min(max_threads / A, d.nQ)) : 1;
     P.nthreads = ((P.NQB * A + 31) / 32) * 32;
-    static const int env_yt = [] { const char* e = std::getenv("SDPB_COL_YT"); return e ? std::atoi(e) : 0; }();
-    if (env_yt) P.YT = env_yt == 4 ? 4 : 8;  // tuning knob, read once per process
     const int n_levels = dedup ? d.nI + d.nQ - 1 : d.nQ;
     // real grid: one CTA walks the whole preQ1 axis; folded grid: 64 levels per CTA for parallelism
-    P.LT = dedup ? 64 : ((n_levels + P.YT - 1) / P.YT) * P.YT;
+    P.LT = dedup ? 64 : ((n_levels + kColYT - 1) / kColYT) * kColYT;
     P.di_max = hi;
     P.span = hi - lo;
     P.NRW = P.LT + P.span;
-    P.smem = ((((size_t)2 * P.YT * P.nthreads + 2 * (size_t)P.NRW) * 8 + 15) & ~(size_t)15) + (size_t)D * 16 + 16;
+    P.smem = ((((size_t)2 * kColYT * P.nthreads + 2 * (size_t)P.NRW) * 8 + 15) & ~(size_t)15) + (size_t)D * 16 + 16;
     P.ok = P.smem <= 100 * 1024;
     return P;
 }
@@ -499,12 +495,8 @@ inline int launch_col(const ColPlan& P, const DevModel& dm, int t, int D, int pm
     const bool last = (Vn == nullptr), mn = dm.is_min != 0;  // period T without a terminal table
     cudaError_t e = cudaSuccess;
 #define SDPB_COL_LAUNCH(MN, LS)                                                                        \
-    if (P.YT == 4) {                                                                                   \
-        auto k = bi_lead_col<MN, LS, DEDUP, 4>;                                                        \
-        if (P.smem > 48 * 1024) e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)P.smem); \
-        if (e == cudaSuccess) k<<<(unsigned)blocks, P.nthreads, P.smem, stream>>>(dm, a);              \
-    } else {                                                                                           \
-        auto k = bi_lead_col<MN, LS, DEDUP, 8>;                                                        \
+    {                                                                                                  \
+        auto k = bi_lead_col<MN, LS, DEDUP>;                                                           \
         if (P.smem > 48 * 1024) e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)P.smem); \
         if (e == cudaSuccess) k<<<(unsigned)blocks, P.nthreads, P.smem, stream>>>(dm, a);              \
     }
@@ -762,30 +754,28 @@ constexpr int kQ2mNC = 2;  // preQ2 columns per thread
 
 struct Q2mLayout { int NG; unsigned off_rg, off_gb, off_bv, off_ba, off_mt; size_t smem; };
 
-__host__ __device__ inline Q2mLayout q2m_layout(int NRW, int D, int NT, int parts, int half) {
+__host__ __device__ inline Q2mLayout q2m_layout(int NRW, int D, int NT, int half) {
     Q2mLayout L;
-    const int cols = NT / parts;
-    L.NG = (cols - 1) / half + 2;                                // distinct (x, chunk) groups among `cols` consecutive threads
+    L.NG = (NT - 1) / half + 2;                                  // distinct (x, chunk) groups among NT consecutive threads
     unsigned o = (unsigned)(NRW + D) * 16u;                      // WR, PP
     L.off_rg = o; o += (unsigned)(L.NG * D) * 16u;               // R[group][j] = (p_j*gamma, refill row offset)
     L.off_gb = o; o += ((unsigned)L.NG * 4u + 15u) & ~15u;       // window base row of each group
     L.off_bv = o; o += (unsigned)(kQ2mNC * kQ2YT * NT) * 8u;     // running optimum per state: value ...
     L.off_ba = o; o += (unsigned)(kQ2mNC * kQ2YT * NT) * 4u;     // ... and action
-    L.off_mt = o; o += 2u * (unsigned)(parts * L.NG * D) * 64u;  // M[buffer][slice][group][j][8]
+    L.off_mt = o; o += 2u * (unsigned)(L.NG * D) * 64u;          // M[buffer][group][j][8]
     L.smem = o;
     return L;
 }
 
-template <bool IS_MIN, bool LAST, int NT, int PARTS>
+template <bool IS_MIN, bool LAST, int NT>
 __global__ void __launch_bounds__(NT, 512 / NT)
 bi_lead_q2m(const __grid_constant__ DevModel M, const __grid_constant__ Q2Args a) {
     constexpr int YT = kQ2YT, PF = kQ2PF, W = YT + PF, PAD = kQ2PAD, NC = kQ2mNC;
     static_assert(W == 10, "the demand loop below is written out for W = 10");
-    static_assert(NT % 8 == 0 && (NT / PARTS) % 8 == 0, "the table builder keeps the slot index fixed per thread");
+    static_assert(NT % 8 == 0, "the table builder keeps the slot index fixed per thread");
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int D = a.D, nQ = M.nQ, half = a.half, tid = threadIdx.x;
-    constexpr int cols = NT / PARTS;
-    const Q2mLayout L = q2m_layout(a.NRW, D, NT, PARTS, half);
+    const Q2mLayout L = q2m_layout(a.NRW, D, NT, half);
     double2* WR = reinterpret_cast<double2*>(smem_raw);  // (level cost, successor row offset in the low word)
     double2* PP = WR + a.NRW;                            // (p, p*gamma)
     double2* RG = reinterpret_cast<double2*>(smem_raw + L.off_rg);
@@ -794,8 +784,7 @@ bi_lead_q2m(const __grid_constant__ DevModel M, const __grid_constant__ Q2Args a
     int* BA = reinterpret_cast<int*>(smem_raw + L.off_ba);
     double* MT = reinterpret_cast<double*>(smem_raw + L.off_mt);
     const int NG = L.NG;
-    const int part = tid / cols, col = tid - part * cols;
-    const long long F0 = a.f_begin + (long long)blockIdx.x * cols;
+    const long long F0 = a.f_begin + (long long)blockIdx.x * NT;
     const long long x_first = F0 / a.tpx;
     const long long G0 = F0 / half;                      // first (x, chunk) group of the CTA: G = x * n_chunks + chunk
     const bool lost = (M.flags & SDPB_F_LOST_SALES) != 0;
@@ -828,7 +817,7 @@ bi_lead_q2m(const __grid_constant__ DevModel M, const __grid_constant__ Q2Args a
         RG[e] = make_double2(PP[j].y, w.y);
     }
 
-    const long long F = min(F0 + col, a.f_end - 1);
+    const long long F = min(F0 + tid, a.f_end - 1);
     const long long x = F / a.tpx;
     const int f = (int)(F - x * a.tpx);
     const int chunk = f / half, c0 = f - chunk * half, l0 = chunk * YT;
@@ -841,43 +830,40 @@ bi_lead_q2m(const __grid_constant__ DevModel M, const __grid_constant__ Q2Args a
         const long long i0 = idx0 + (long long)k * nQ;
         any |= (l0 + k < nQ) && ((i0 >= a.lo && i0 < a.hi) || (has_b && i0 + half >= a.lo && i0 + half < a.hi));
     }
-    any = any && F0 + col < a.f_end;
+    any = any && F0 + tid < a.f_end;
 
     const unsigned wr0 = (unsigned)__cvta_generic_to_shared(WR) + (unsigned)((int)(x - x_first) + l0 + (D - 1) + PAD) * 16u;
     const unsigned rg0 = (unsigned)__cvta_generic_to_shared(RG) + (unsigned)(g_own * D) * 16u;
-    const unsigned mt0 = (unsigned)__cvta_generic_to_shared(MT) + (unsigned)((part * NG + g_own) * D) * 64u;
-    const unsigned mt_buf = (unsigned)(PARTS * NG * D) * 64u;  // bytes between the two buffers
+    const unsigned mt0 = (unsigned)__cvta_generic_to_shared(MT) + (unsigned)(g_own * D) * 64u;
+    const unsigned mt_buf = (unsigned)(NG * D) * 64u;  // bytes between the two buffers
     const unsigned bv_s = (unsigned)__cvta_generic_to_shared(BV) + (unsigned)tid * 8u;
     const unsigned ba_s = (unsigned)__cvta_generic_to_shared(BA) + (unsigned)tid * 4u;
     const double* __restrict__ cb = LAST ? nullptr : a.VnT + c0;
     const int colb = has_b ? half : 0;                   // a thread without a second column gathers the first one twice
     const double vt = M.v_t[a.t - 1];
 
-    // the action range: first cut over gridDim.y (separate CTAs, merged by merge_action_slices: small grids need more
-    // CTAs than their states give), then over the PARTS thread groups of the CTA
+    // the action range, cut over gridDim.y (separate CTAs, merged by merge_action_slices: small grids need more CTAs
+    // than their states give)
     const int n_sl = (int)gridDim.y, sl = (int)blockIdx.y;
     const int per_sl = (M.max_order_idx + n_sl) / n_sl;      // ceil(A / n_sl)
-    const int sl_begin = sl * per_sl, sl_end = min(M.max_order_idx + 1, sl_begin + per_sl);
-    const int per_part = (sl_end - sl_begin + PARTS - 1) / PARTS;
-    const int ai_begin = sl_begin + part * per_part;
-    const int ai_end = min(sl_end, ai_begin + per_part);
+    const int ai_begin = sl * per_sl, ai_end = min(M.max_order_idx + 1, ai_begin + per_sl);
     if (!LAST) cb += (long long)ai_begin * nQ;
-    double* MTp = MT + (size_t)(part * NG) * D * YT;
-    // the builder's entries e = col, col + cols, ...: slot k = e & 7 is fixed, (group, demand) advance by cols / 8
-    const int k_b = col & (YT - 1);
-    const int gj_b = col >> 3;
-    for (int it = 0; it < per_part; it++) {  // every slice runs per_part rounds: the barrier below is CTA-wide
+    // the builder's entries e = tid, tid + NT, ...: slot k = e & 7 is fixed, (group, demand) advance by NT / 8
+    const int k_b = tid & (YT - 1);
+    const int gj_b = tid >> 3;
+    // (the two `ai < ai_end` tests always hold; without them ptxas allocates registers differently and spills more)
+    for (int it = 0; it < ai_end - ai_begin; it++) {
         const int ai = ai_begin + it;
         const unsigned buf = (unsigned)(it & 1);
-        if (ai < ai_end) {  // ---- tabulate p_j * (fv_a + L) for this slice's groups ----
+        if (ai < ai_end) {  // ---- tabulate p_j * (fv_a + L) for the CTA's groups ----
             const double av = (double)ai * M.step;
             const double fv = (av > 0.0 ? M.K : 0.0) + vt * av;  // Leadtime.java:73-74,79
-            double* Mb = MTp + (size_t)buf * (PARTS * NG) * D * YT;
+            double* Mb = MT + (size_t)buf * NG * D * YT;
             int g = gj_b / D, j = gj_b - g * D;
-            for (int e = col; e < NG * D * YT; e += cols) {
+            for (int e = tid; e < NG * D * YT; e += NT) {
                 const double cst = fv + WR[GB[g] + k_b - j].x;
                 Mb[e] = PP[j].x * cst;                           // LeadtimeRecursion.java:59
-                j += cols / YT;
+                j += NT / YT;
                 while (j >= D) { j -= D; g++; }
             }
         }
@@ -947,8 +933,7 @@ bi_lead_q2m(const __grid_constant__ DevModel M, const __grid_constant__ Q2Args a
         }
         if (!LAST) cb += nQ;
     }
-    if (PARTS > 1) __syncthreads();
-    if (part > 0 || !any) return;
+    if (!any) return;
 #pragma unroll
     for (int c2 = 0; c2 < NC; c2++) {
         if (c2 == 1 && !has_b) break;
@@ -956,13 +941,8 @@ bi_lead_q2m(const __grid_constant__ DevModel M, const __grid_constant__ Q2Args a
         for (int k = 0; k < YT; k++) {
             const long long idx = idx0 + (long long)k * nQ + (c2 ? half : 0);
             if (!(l0 + k < nQ && idx >= a.lo && idx < a.hi)) continue;
-            double best = BV[(c2 * YT + k) * NT + tid];
-            int arg = BA[(c2 * YT + k) * NT + tid];
-            for (int q = 1; q < PARTS; q++) {  // ascending slices hold ascending actions: strict compare = first wins
-                const double v = BV[(c2 * YT + k) * NT + q * cols + col];
-                const int av = BA[(c2 * YT + k) * NT + q * cols + col];
-                if (av != kNoAction && (IS_MIN ? (v < best) : (v > best))) { best = v; arg = av; }
-            }
+            const double best = BV[(c2 * YT + k) * NT + tid];
+            const int arg = BA[(c2 * YT + k) * NT + tid];
             if (n_sl > 1) {  // this CTA saw one slice of the actions only
                 a.slice_v[(long long)sl * (a.hi - a.lo) + (idx - a.lo)] = best;
                 a.slice_a[(long long)sl * (a.hi - a.lo) + (idx - a.lo)] = arg;
@@ -1002,9 +982,10 @@ inline Q2Plan plan_q2(const sdpb_model& m, const DevModel& d, int D, const int* 
 // [row0, row1): inventory rows of V_{t+1} the range [lo, hi) can read (sdpb_shard_reads); only those are transposed.
 constexpr int kQ2MaxPeers = 2;
 
-// How a launch over [lo, hi) is shaped.  Enough warps for ~6 waves: nothing to do.  Otherwise the action range is cut:
-// with the shared-product kernel over separate CTAs (gridDim.y slices, merged by merge_action_slices -- the per-action
-// product table is then still built by a full CTA), else over 2 or 4 thread groups inside a CTA of bi_lead_q2.
+// How a launch over [lo, hi) is shaped.  bi_lead_q2m (shared products) whenever its tables leave four CTAs per SM, with
+// the action range cut over separate CTAs (gridDim.y slices, merged by merge_action_slices -- the per-action product
+// table is then still built by a full CTA) when the grid is short of ~8 waves; else bi_lead_q2, with the action range cut
+// over 2 or 4 thread groups inside a CTA when the grid is short of ~6 waves.
 struct Q2Shape { bool shared; int parts, slices, half, tpx, NRW; long long f_begin, f_end; Q2mLayout L; };
 
 inline Q2Shape q2_shape(const Q2Plan& P, const DevModel& dm, int D, long long lo, long long hi, int sm_count) {
@@ -1013,33 +994,32 @@ inline Q2Shape q2_shape(const Q2Plan& P, const DevModel& dm, int D, long long lo
     const long long rows = (hi - 1) / per_x - lo / per_x + 1;
     const double waves = (double)(rows * P.tpx) / 32.0 / (16.0 * sm_count);
     S.parts = waves >= 6.0 ? 1 : (waves >= 3.0 ? 2 : 4);
-    static const int env_split = [] { const char* e2 = std::getenv("SDPB_Q2_SPLIT"); return e2 ? std::atoi(e2) : 0; }();
-    if (env_split) S.parts = env_split == 1 ? 1 : env_split == 2 ? 2 : 4;  // tuning knobs, read once per process
-    static const bool no_share = std::getenv("SDPB_Q2_NOSHARE") != nullptr;
-    static const bool force_share = std::getenv("SDPB_Q2_SHARE") != nullptr;
-    static const int env_slices = [] { const char* e2 = std::getenv("SDPB_Q2_SLICES"); return e2 ? std::atoi(e2) : 0; }();
     S.half = (dm.nQ + 1) / 2;
     const int tpx2 = P.n_chunks * S.half;
     const int NRW2 = P.n_chunks * kQ2YT + D + kQ2PAD + (P.NT + tpx2 - 1) / tpx2 + 1;
     S.slices = 1;
-    // bi_lead_q2m whenever its tables leave four CTAs per SM; its threads are numbered over (x, chunk, column pair).
-    // Measured on C4 (ms, bi_lead_q2m vs bi_lead_q2): whole grid 131.0 vs 140.3.  Shards: with the action range cut over
-    // thread groups INSIDE a CTA the per-action tables and the barrier cost more than they save (a quarter of the grid
-    // 37.8 vs 36.7, an eighth 20.8 vs 18.7); cut over SEPARATE CTAs they do not (34.1 and 17.7; 2 / 4 / 8 / 16 slices on
-    // the eighth: 18.4 / 17.5 / 17.7 / 18.0), so that is the shape every launch takes when the tables fit.
-    const Q2mLayout L1 = q2m_layout(NRW2, D, P.NT, 1, S.half);
-    if (!no_share && !force_share && !env_split && L1.smem <= 56 * 1024) {
-        S.shared = true; S.parts = 1; S.L = L1;
+    // bi_lead_q2m's threads are numbered over (x, chunk, column pair).  Measured on C4 (ms, bi_lead_q2m vs bi_lead_q2):
+    // whole grid 131.0 vs 140.3.  Shards: with the action range cut over thread groups INSIDE a CTA the per-action tables
+    // and the barrier cost more than they save (a quarter of the grid 37.8 vs 36.7, an eighth 20.8 vs 18.7); cut over
+    // SEPARATE CTAs they do not (34.1 and 17.7; 2 / 4 / 8 / 16 slices on the eighth: 18.4 / 17.5 / 17.7 / 18.0), so that
+    // is the shape every launch takes when the tables fit.
+    S.L = q2m_layout(NRW2, D, P.NT, S.half);
+    // Test hooks, read once per process: they force shapes that small instances do not take by themselves.
+    //   SDPB_Q2_SHARE=1      bi_lead_q2m with no action slices wherever its tables fit: the epilogue with peer stores
+    //                        that large shards take
+    //   SDPB_Q2_SPLIT=2 | 4  bi_lead_q2 with 2 or 4 thread groups, no shared products
+    static const bool force_share = std::getenv("SDPB_Q2_SHARE") != nullptr;
+    static const int force_split = [] { const char* e = std::getenv("SDPB_Q2_SPLIT"); return e ? std::atoi(e) : 0; }();
+    if (force_split) {
+        S.parts = force_split == 2 ? 2 : 4;
+    } else if (S.L.smem <= 56 * 1024) {
+        S.shared = true; S.parts = 1;
         const double ctas = (double)(rows * tpx2) / P.NT;
         const double w = ctas / (4.0 * sm_count);                // CTA waves at four CTAs per SM
-        if (w < 8.0) S.slices = (int)std::min(8.0, std::ceil(8.0 / std::max(w, 0.01)));
-        if (env_slices) S.slices = env_slices;
+        if (w < 8.0 && !force_share) S.slices = (int)std::min(8.0, std::ceil(8.0 / std::max(w, 0.01)));
         S.slices = std::max(1, std::min(S.slices, (dm.max_order_idx + 1) / 8));
         const int per = (dm.max_order_idx + S.slices) / S.slices;  // as the kernel cuts: no empty slice
         S.slices = (dm.max_order_idx + per) / per;
-    } else {
-        S.L = q2m_layout(NRW2, D, P.NT, S.parts, S.half);
-        S.shared = !no_share && (S.parts == 1 || force_share) && S.L.smem <= 56 * 1024;
     }
     S.tpx = S.shared ? tpx2 : P.tpx;
     S.NRW = S.shared ? NRW2 : P.NRW;
@@ -1048,20 +1028,17 @@ inline Q2Shape q2_shape(const Q2Plan& P, const DevModel& dm, int D, long long lo
     return S;
 }
 
-inline int launch_q2(const Q2Plan& P, const DevModel& dm, int t, int D, int pmf_off, const double* Vn, double* VnT,
-                     double* Vt, int* Qt, long long lo, long long hi, int row0, int row1, cudaStream_t stream,
-                     const PeerStore* peers = nullptr, int n_peers = 0, bool* shared_products = nullptr,
-                     double* slice_v = nullptr, int* slice_a = nullptr, size_t slice_cap = 0,
-                     const DevPeer* d_peers = nullptr, int n_dev_peers = 0, int* slices_used = nullptr) {
+// S = q2_shape(P, ..., lo, hi, ...).  SDPB_OK, SDPB_ERR_NOMEM (slice scratch too small) or SDPB_ERR_CUDA.
+inline int launch_q2(const Q2Plan& P, const Q2Shape& S, const DevModel& dm, int t, int D, int pmf_off, const double* Vn,
+                     double* VnT, double* Vt, int* Qt, long long lo, long long hi, int row0, int row1, cudaStream_t stream,
+                     const PeerStore* peers, int n_peers, double* slice_v, int* slice_a, size_t slice_cap,
+                     const DevPeer* d_peers, int n_dev_peers) {
     if (hi <= lo) return SDPB_OK;
     const bool last = (Vn == nullptr), mn = dm.is_min != 0;  // period T without a terminal table
     if (!last) {
         const unsigned tiles = (unsigned)((dm.nQ + 31) / 32);
         transpose_q2a<<<dim3((unsigned)(row1 - row0), tiles, tiles), dim3(32, 8), 0, stream>>>(Vn, VnT, dm.nQ, row0);
     }
-    int sm_count = 148, dev = 0;
-    if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sm_count, cudaDevAttrMultiProcessorCount, dev);
-    const Q2Shape S = q2_shape(P, dm, D, lo, hi, sm_count);
     const long long n_local = hi - lo;
     if (S.slices > 1 && (size_t)S.slices * (size_t)n_local > slice_cap) return SDPB_ERR_NOMEM;  // the caller sizes it: q2_shape
     Q2Args a;
@@ -1076,29 +1053,22 @@ inline int launch_q2(const Q2Plan& P, const DevModel& dm, int t, int D, int pmf_
             a.peer_v[p] = peers[p].v; a.peer_lo[p] = peers[p].lo; a.peer_hi[p] = peers[p].hi;
             a.n_peer = p + 1;
         }
-    if (shared_products) *shared_products = S.shared;
-    if (slices_used) *slices_used = S.slices;
     const int cols = P.NT / a.parts;
     const Q2mLayout L = S.L;
     const bool shared = S.shared;
     cudaError_t e = cudaSuccess;
     const dim3 grid((unsigned)((a.f_end - a.f_begin + cols - 1) / cols), (unsigned)S.slices);
-#define SDPB_Q2_LAUNCH(MN, LS, PT)                                                                     \
-    if (shared) {                                                                                      \
-        auto k = bi_lead_q2m<MN, LS, 128, PT>;                                                         \
-        if (L.smem > 48 * 1024) e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L.smem); \
-        if (e == cudaSuccess) k<<<grid, 128, L.smem, stream>>>(dm, a);                                 \
-    } else {                                                                                           \
-        auto k = bi_lead_q2<MN, LS, 128, PT>;                                                          \
-        if (P.smem > 48 * 1024) e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)P.smem); \
-        if (e == cudaSuccess) k<<<grid.x, 128, P.smem, stream>>>(dm, a);                               \
+#define SDPB_Q2_LAUNCH(K, SMEM, GRID)                                                                  \
+    {                                                                                                  \
+        auto k = K;                                                                                    \
+        if (SMEM > 48 * 1024) e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM); \
+        if (e == cudaSuccess) k<<<GRID, 128, SMEM, stream>>>(dm, a);                                   \
     }
 #define SDPB_Q2_NT(MN, LS)                                                                             \
-    switch (a.parts) {                                                                                 \
-    case 1: SDPB_Q2_LAUNCH(MN, LS, 1) break;                                                           \
-    case 2: SDPB_Q2_LAUNCH(MN, LS, 2) break;                                                           \
-    default: SDPB_Q2_LAUNCH(MN, LS, 4) break;                                                          \
-    }
+    if (shared) SDPB_Q2_LAUNCH((bi_lead_q2m<MN, LS, 128>), L.smem, grid)                               \
+    else if (a.parts == 1) SDPB_Q2_LAUNCH((bi_lead_q2<MN, LS, 128, 1>), P.smem, grid.x)                \
+    else if (a.parts == 2) SDPB_Q2_LAUNCH((bi_lead_q2<MN, LS, 128, 2>), P.smem, grid.x)                \
+    else SDPB_Q2_LAUNCH((bi_lead_q2<MN, LS, 128, 4>), P.smem, grid.x)
     if (mn) { if (last) SDPB_Q2_NT(true, true) else SDPB_Q2_NT(true, false) }
     else    { if (last) SDPB_Q2_NT(false, true) else SDPB_Q2_NT(false, false) }
 #undef SDPB_Q2_NT

@@ -512,19 +512,16 @@ inline cudaError_t launch_tiled2_inst(const DevModel& dm, const TiledArgs& a, di
     return cudaGetLastError();
 }
 
-// Returns SDPB_OK, or SDPB_ERR_STATE when this period has no tiled plan (caller falls back to the
-// generic kernel), or SDPB_ERR_CUDA / SDPB_ERR_NOMEM.  *variant_used: 1 = bi_inv_tiled, 2 = bi_inv_tiled2.
+// For a period whose plan has tp.ok or tp.ok2.  Returns SDPB_OK, SDPB_ERR_CUDA or SDPB_ERR_NOMEM.
+// *variant_used: 1 = bi_inv_tiled, 2 = bi_inv_tiled2.
 inline int launch_tiled(TiledPlan& P, const DevModel& dm, int t, int D, int pmf_off, const double* Vn,
-                        double* Vt, int* Qt, long long lo, long long hi, cudaStream_t stream,
-                        double* fp64_ops, int* variant_used = nullptr) {
+                        double* Vt, int* Qt, long long lo, long long hi, cudaStream_t stream, int* variant_used) {
     const TiledPeriod& tp = P.period[t - 1];
-    if (!tp.ok && !tp.ok2) return SDPB_ERR_STATE;
     const long long n = hi - lo;
     if (n <= 0) return SDPB_OK;
     const bool last = (Vn == nullptr);  // period T without a terminal table (Recursion.java:140)
     const bool mn = dm.is_min != 0;
     const long long target = std::max(1LL, 4LL * P.sm_count / P.batch);  // about 4 CTAs per SM (of this instance's share)
-    const double evals = (double)n * (dm.max_order_idx + 1) * D;
     TiledArgs a;
     a.t = t; a.D = D; a.pmf_off = pmf_off; a.Vn = Vn; a.Vt = Vt; a.Qt = Qt; a.lo = lo; a.hi = hi;
     a.di_max = tp.di_max;
@@ -539,10 +536,8 @@ inline int launch_tiled(TiledPlan& P, const DevModel& dm, int t, int D, int pmf_
         int nsplit = 1;
         // enough CTAs for ~8 waves of 2 CTAs per SM: a grid of a few waves loses its last, partial one
         // (measured, C5: S = 1e6 32.9 -> 30.0 ms, S = 1e5 3.36 -> 3.17 ms; no change at 3e5 and 3e6)
-        static const int env_waves = [] { const char* e = std::getenv("SDPB_T2_WAVES"); return e ? std::max(1, std::atoi(e)) : 0; }();
         // (one instance of a batch: 3 waves of its share -- measured 64 x C2: 8 waves 3.15 ms, 4: 3.08, 3: 3.06, 1: 3.26)
-        long long want = P.batch > 1 ? std::max(1LL, 6LL * P.sm_count / P.batch) : 16LL * P.sm_count;
-        if (env_waves) want = std::max(1LL, env_waves * 2LL * P.sm_count / P.batch);  // tuning knob, read once per process
+        const long long want = P.batch > 1 ? std::max(1LL, 6LL * P.sm_count / P.batch) : 16LL * P.sm_count;
         if (tiles2 < want) nsplit = (int)std::min<long long>(P.n_chunks2, (want + tiles2 - 1) / tiles2);
         const int cps = (P.n_chunks2 + nsplit - 1) / nsplit;
         nsplit = (P.n_chunks2 + cps - 1) / cps;
@@ -557,9 +552,7 @@ inline int launch_tiled(TiledPlan& P, const DevModel& dm, int t, int D, int pmf_
         else e = last ? launch_tiled2_inst<false, true>(dm, a, grid, tp.smem2, stream)
                       : launch_tiled2_inst<false, false>(dm, a, grid, tp.smem2, stream);
         if (e != cudaSuccess) return SDPB_ERR_CUDA;
-        // per 16 evaluations: 4 new costs + 4 products + 16 * (mul, add, add); last period: 4 + 16 * 2
-        if (fp64_ops) *fp64_ops += last ? evals * 2.25 : evals * 3.5;
-        if (variant_used) *variant_used = 2;
+        *variant_used = 2;
         return SDPB_OK;
     }
 
@@ -585,9 +578,7 @@ inline int launch_tiled(TiledPlan& P, const DevModel& dm, int t, int D, int pmf_
     }
 #undef SDPB_TILED_CASE
     if (e != cudaSuccess) return SDPB_ERR_CUDA;
-    // useful fp64 instructions: per evaluation add+mul+add(+add), plus one mul per R evaluations
-    if (fp64_ops) *fp64_ops += last ? evals * 3.0 : evals * 4.0 + evals / kTiledR;
-    if (variant_used) *variant_used = 1;
+    *variant_used = 1;
     return SDPB_OK;
 }
 

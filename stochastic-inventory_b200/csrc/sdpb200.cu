@@ -144,6 +144,7 @@ struct sdpb_handle {
     unsigned long long* dCounters = nullptr;  // [4] dense-grid artefacts seen by sdpb_reach
     double reach_cnt[3] = {0, 0, 0};
     PeerLink peer;
+    std::vector<sdpb_kernel_choice> period_kernel;  // [T] choose_period_kernel
     bool push_fused = false;   // the period's kernel already stored the peers' rows into their tables (bi_lead_q2)
     double* q2_slice_v = nullptr;  // bi_lead_q2m with action slices over separate CTAs: per slice and state the slice's optimum
     int* q2_slice_a = nullptr;
@@ -427,6 +428,7 @@ void launch_generic(sdpb_handle* h, int t, const double* Vn, double* Vt, int* Qt
         h->dm, t, h->pmf_len[t - 1], h->pmf_off[t - 1], Vn, Vt, Qt, lo, hi);
 }
 
+// The general kernel for every cost kind.  Only kinds with a lead time (backorder, deposit, overdraft) are ever folded.
 template <bool DEDUP>
 int dispatch_generic_d(sdpb_handle* h, int t, const double* Vn, double* Vt, int* Qt, long long lo, long long hi) {
     const sdpb_model& m = h->m;
@@ -447,62 +449,26 @@ int dispatch_generic_d(sdpb_handle* h, int t, const double* Vn, double* Vt, int*
         else if (mn) launch_generic<SDPB_COST_CASH_OVERDRAFT, false, true, 1, DEDUP>(h, t, Vn, Vt, Qt, lo, hi);
         else launch_generic<SDPB_COST_CASH_OVERDRAFT, false, false, 1, DEDUP>(h, t, Vn, Vt, Qt, lo, hi);
         break;
-    case SDPB_COST_CASH_XR:
-        if (DEDUP) { h->err = "XR kind has no lead time to fold"; return SDPB_ERR_ARG; }
-        if (mn) launch_generic<SDPB_COST_CASH_XR, false, true, 1, false>(h, t, Vn, Vt, Qt, lo, hi);
-        else launch_generic<SDPB_COST_CASH_XR, false, false, 1, false>(h, t, Vn, Vt, Qt, lo, hi);
-        break;
     case SDPB_COST_STAFF: {
-        if (DEDUP) { h->err = "no lead time to fold"; return SDPB_ERR_ARG; }
         const long long nst = hi - lo;
-        if (nst > 0) {
-            const unsigned blocks = (unsigned)((nst + 7) / 8);
-            const bool last = Vn == nullptr;
-            if (mn) { if (last) bi_staff<true, true><<<blocks, 256, 0, h->stream>>>(h->dm, t, Vn, Vt, Qt, lo, hi);
-                      else bi_staff<true, false><<<blocks, 256, 0, h->stream>>>(h->dm, t, Vn, Vt, Qt, lo, hi); }
-            else    { if (last) bi_staff<false, true><<<blocks, 256, 0, h->stream>>>(h->dm, t, Vn, Vt, Qt, lo, hi);
-                      else bi_staff<false, false><<<blocks, 256, 0, h->stream>>>(h->dm, t, Vn, Vt, Qt, lo, hi); }
-        }
+        const bool last = Vn == nullptr;
+        auto k = mn ? (last ? bi_staff<true, true> : bi_staff<true, false>) : (last ? bi_staff<false, true> : bi_staff<false, false>);
+        if (nst > 0) k<<<(unsigned)((nst + 7) / 8), 256, 0, h->stream>>>(h->dm, t, Vn, Vt, Qt, lo, hi);
         break;
     }
     case SDPB_COST_CASH_TWO_PRODUCT: {
-        if (DEDUP) { h->err = "no lead time to fold"; return SDPB_ERR_ARG; }
         const long long nst = hi - lo;
-        const int Dt = h->pmf_len[t - 1];
-        const bool term_T = t == h->m.T && Vn != nullptr;  // boundary table: the row kernel folds LAST and 'no continuation'
-        if (nst > 0 && !term_T && h->opt.kernel != SDPB_KERNEL_GENERIC && plan_two_product_row(h->m, h->dm, t, Dt)) {
-            // CTA = one (inv1, inv2) pair x 128 cash levels; cash-independent terms shared through shared memory
-            const int segs = (h->dm.nW + 127) / 128;
-            const long long pair0 = lo / h->dm.nW, pair1 = (hi - 1) / h->dm.nW;
-            const unsigned blocks = (unsigned)((pair1 - pair0 + 1) * segs);
-            const size_t smem = (size_t)Dt * sizeof(TwoProductRowTables);
-            cudaError_t e = cudaSuccess;
-            if (t == h->m.T) {
-                auto k = bi_two_product_row<true>;
-                if (smem > 48 * 1024) e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-                if (e == cudaSuccess) k<<<blocks, 128, smem, h->stream>>>(h->dm, t, Dt, h->pmf_off[t - 1], Vn, Vt, Qt, lo, hi, pair0, segs);
-            } else {
-                auto k = bi_two_product_row<false>;
-                if (smem > 48 * 1024) e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-                if (e == cudaSuccess) k<<<blocks, 128, smem, h->stream>>>(h->dm, t, Dt, h->pmf_off[t - 1], Vn, Vt, Qt, lo, hi, pair0, segs);
-            }
-            if (e != cudaSuccess) { h->err = cudaGetErrorString(e); return SDPB_ERR_CUDA; }
-            h->stats.kernel_used = SDPB_KERNEL_TWO_PRODUCT_ROW;
-            h->stats.fp64_ops += count_evals_period(h, t) * (t == h->m.T ? 1.0 : 3.0);
-        } else if (nst > 0) {
-            const unsigned blocks = (unsigned)((nst + 127) / 128);
-            if (term_T) bi_two_product<true, true><<<blocks, 128, 0, h->stream>>>(h->dm, t, h->pmf_len[t - 1], h->pmf_off[t - 1], Vn, Vt, Qt, lo, hi);
-            else if (t == h->m.T) bi_two_product<true, false><<<blocks, 128, 0, h->stream>>>(h->dm, t, h->pmf_len[t - 1], h->pmf_off[t - 1], Vn, Vt, Qt, lo, hi);
-            else bi_two_product<false, true><<<blocks, 128, 0, h->stream>>>(h->dm, t, h->pmf_len[t - 1], h->pmf_off[t - 1], Vn, Vt, Qt, lo, hi);
-        }
+        const bool term_T = t == h->m.T && Vn != nullptr;  // boundary table: the kernel folds LAST and 'no continuation'
+        auto k = term_T ? bi_two_product<true, true> : t == h->m.T ? bi_two_product<true, false> : bi_two_product<false, true>;
+        if (nst > 0) k<<<(unsigned)((nst + 127) / 128), 128, 0, h->stream>>>(h->dm, t, h->pmf_len[t - 1], h->pmf_off[t - 1], Vn, Vt, Qt, lo, hi);
         break;
     }
 #define SDPB_PLAIN_KIND(K)                                                                    \
     case K:                                                                                   \
-        if (DEDUP) { h->err = "no lead time to fold"; return SDPB_ERR_ARG; }                  \
         if (mn) launch_generic<K, false, true, 1, false>(h, t, Vn, Vt, Qt, lo, hi);           \
         else launch_generic<K, false, false, 1, false>(h, t, Vn, Vt, Qt, lo, hi);             \
         break;
+    SDPB_PLAIN_KIND(SDPB_COST_CASH_XR)
     SDPB_PLAIN_KIND(SDPB_COST_CASH_OD_LIMIT)
     SDPB_PLAIN_KIND(SDPB_COST_CASH_OD_TESTING)
     SDPB_PLAIN_KIND(SDPB_COST_CASH_LOAN)
@@ -514,13 +480,31 @@ int dispatch_generic_d(sdpb_handle* h, int t, const double* Vn, double* Vt, int*
     return SDPB_OK;
 }
 
+// Two-product kind, plan_two_product_row: a CTA = one (inv1, inv2) pair x 128 cash levels; cash-independent terms shared
+// through shared memory.
+int launch_two_product_row(sdpb_handle* h, int t, const double* Vn, double* Vt, int* Qt, long long lo, long long hi) {
+    const int Dt = h->pmf_len[t - 1];
+    const int segs = (h->dm.nW + 127) / 128;
+    const long long pair0 = lo / h->dm.nW, pair1 = (hi - 1) / h->dm.nW;
+    const unsigned blocks = (unsigned)((pair1 - pair0 + 1) * segs);
+    const size_t smem = (size_t)Dt * sizeof(TwoProductRowTables);
+    cudaError_t e = cudaSuccess;
+    auto k = t == h->m.T ? bi_two_product_row<true> : bi_two_product_row<false>;
+    if (smem > 48 * 1024) e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e == cudaSuccess) k<<<blocks, 128, smem, h->stream>>>(h->dm, t, Dt, h->pmf_off[t - 1], Vn, Vt, Qt, lo, hi, pair0, segs);
+    if (e != cudaSuccess) { h->err = cudaGetErrorString(e); return SDPB_ERR_CUDA; }
+    return SDPB_OK;
+}
+
+size_t staged_smem(int D) { return (size_t)D * 16 + (size_t)8 * D * sizeof(StagedRow); }
+
 // Staged warp-per-state kernel for backorder lead-time models.
 template <bool DEDUP>
 int launch_staged(sdpb_handle* h, int t, const double* Vn, double* Vt, int* Qt, long long lo, long long hi) {
     const long long n = hi - lo;
     if (n <= 0) return SDPB_OK;
     const int D = h->pmf_len[t - 1];
-    const size_t smem = (size_t)D * 16 + (size_t)8 * D * sizeof(StagedRow);
+    const size_t smem = staged_smem(D);
     long long blocks = (n + 7) / 8;
     if (h->dm.lead == 2 && !DEDUP) {  // CTA = 8 consecutive preQ1 of one (x, preQ2): see the kernel
         const long long per_x = (long long)h->dm.nQ * h->dm.nQ;
@@ -528,141 +512,11 @@ int launch_staged(sdpb_handle* h, int t, const double* Vn, double* Vt, int* Qt, 
         blocks = rows * ((h->dm.nQ + 7) / 8) * h->dm.nQ;
     }
     cudaError_t e = cudaSuccess;
-    if (h->dm.is_min) {
-        auto k = bi_backorder_staged<true, DEDUP>;
-        if (smem > 48 * 1024) e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e == cudaSuccess) k<<<(unsigned)blocks, 256, smem, h->stream>>>(h->dm, t, D, h->pmf_off[t - 1], Vn, Vt, Qt, lo, hi);
-    } else {
-        auto k = bi_backorder_staged<false, DEDUP>;
-        if (smem > 48 * 1024) e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e == cudaSuccess) k<<<(unsigned)blocks, 256, smem, h->stream>>>(h->dm, t, D, h->pmf_off[t - 1], Vn, Vt, Qt, lo, hi);
-    }
+    auto k = h->dm.is_min ? bi_backorder_staged<true, DEDUP> : bi_backorder_staged<false, DEDUP>;
+    if (smem > 48 * 1024) e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e == cudaSuccess) k<<<(unsigned)blocks, 256, smem, h->stream>>>(h->dm, t, D, h->pmf_off[t - 1], Vn, Vt, Qt, lo, hi);
     if (e != cudaSuccess) { h->err = cudaGetErrorString(e); return SDPB_ERR_CUDA; }
     return SDPB_OK;
-}
-
-bool staged_ok(const sdpb_handle* h, int t) {
-    const size_t smem = (size_t)h->pmf_len[t - 1] * (16 + 8 * sizeof(StagedRow));
-    return h->m.cost_kind == SDPB_COST_BACKORDER && h->m.lead_time >= 1 && smem <= 200 * 1024;
-}
-
-double count_evals_virtual(const sdpb_handle* h, int t);
-
-// Solve [lo, hi) of the real grid (or of the virtual grid when DEDUP) with the best kernel allowed.
-template <bool DEDUP>
-int run_period_kernel(sdpb_handle* h, int t, const double* Vn, double* Vt, int* Qt, long long lo, long long hi,
-                      bool plain) {
-    const bool last = Vn == nullptr;  // no continuation: period T of a model without a boundary table
-    if (!plain && !DEDUP && h->dVT && (h->opt.kernel == SDPB_KERNEL_AUTO || h->opt.kernel == SDPB_KERNEL_LEAD_Q2)) {
-        const Q2Plan qp = plan_q2(h->m, h->dm, h->pmf_len[t - 1], h->pmf_di.data() + h->pmf_off[t - 1]);
-        if (qp.ok) {
-            h->stats.kernel_used = SDPB_KERNEL_LEAD_Q2;
-            const double ev = (double)(hi - lo) * (h->m.max_order_idx + 1) * h->pmf_len[t - 1];
-            if (!last) h->stats.launches++;  // the transposition pass
-            int64_t rlo = 0, rhi = h->S;
-            sdpb_shard_reads(h, &rlo, &rhi);
-            const long long per_x = (long long)h->dm.nQ * h->dm.nQ;
-            // multi-GPU: the kernel's epilogue stores the rows its (at most two) neighbours read straight into their
-            // tables; enqueue_period_sharded then skips the copies
-            PeerStore ps[kQ2MaxPeers];
-            int nps = 0;
-            h->push_fused = false;
-            const bool pushing = h->peer.attached && t > 1 && !h->peer.sends.empty();
-            // a launch whose action range is cut over separate CTAs needs one (value, action) entry per slice and state
-            const Q2Shape shape = q2_shape(qp, h->dm, h->pmf_len[t - 1], lo, hi, h->sm_count);
-            if (shape.slices > 1) {
-                const size_t need = (size_t)shape.slices * (size_t)(hi - lo);
-                if (need > h->q2_slice_cap) {
-                    void* p = nullptr;
-                    CU(dev_alloc(h, &p, need * sizeof(double)));
-                    h->q2_slice_v = (double*)p;
-                    CU(dev_alloc(h, &p, need * sizeof(int)));
-                    h->q2_slice_a = (int*)p;
-                    h->q2_slice_cap = need;
-                }
-                if (pushing) h->push_fused = true;  // merge_action_slices stores the peers' rows
-            } else if (pushing && h->peer.sends.size() <= (size_t)kQ2MaxPeers) {
-                for (const PeerSend& sd : h->peer.sends) {
-                    const PeerInfo& pi = h->peer.info[sd.rank];
-                    char* base = h->peer.mapped[sd.rank] + pi.v_off0 + (size_t)(t - 1) * pi.v_stride;
-                    ps[nps++] = PeerStore{reinterpret_cast<double*>(base) - pi.vlo, sd.a, sd.b};
-                }
-                h->push_fused = true;
-            }
-            bool shared_products = false;
-            int slices_used = 1;
-            const bool merge_pushes = pushing && shape.slices > 1;
-            const int rc = launch_q2(qp, h->dm, t, h->pmf_len[t - 1], h->pmf_off[t - 1], Vn, h->dVT, Vt, Qt, lo, hi,
-                                     (int)(rlo / per_x), (int)(rhi / per_x), h->stream, ps, nps, &shared_products,
-                                     h->q2_slice_v, h->q2_slice_a, h->q2_slice_cap,
-                                     merge_pushes ? (const DevPeer*)h->peer.d_peers : nullptr,
-                                     merge_pushes ? (int)h->peer.sends.size() : 0, &slices_used);
-            if (rc == SDPB_OK && slices_used > 1) h->stats.launches++;  // merge_action_slices
-            // per evaluation: (mul, add, mul, add) + one cost per 8 -- or, with the products p*(fv + L) shared by the
-            // CTA (bi_lead_q2m), (add, mul, add); the last period has no continuation term
-            if (shared_products) { h->stats.fp64_ops += ev * (last ? 1.0 : 3.0); h->stats.kernel_used = SDPB_KERNEL_LEAD_Q2M; }
-            else h->stats.fp64_ops += ev * (last ? (1.0 + 2.0 * kQ2YT) / kQ2YT : (1.0 + 4.0 * kQ2YT) / kQ2YT);
-            return rc;
-        }
-    }
-    if (!plain && h->opt.kernel != SDPB_KERNEL_GENERIC && h->opt.kernel != SDPB_KERNEL_STAGED && h->m.lead_time >= 1 &&
-        h->m.cost_kind == SDPB_COST_BACKORDER) {
-        const ColPlan cp = plan_col(h->m, h->dm, h->pmf_len[t - 1], h->pmf_di.data() + h->pmf_off[t - 1], DEDUP);
-        if (cp.ok && h->opt.kernel != SDPB_KERNEL_LEAD_SLAB) {
-            h->stats.kernel_used = SDPB_KERNEL_LEAD_COL;
-            const double ev = (double)(hi - lo) * (h->m.max_order_idx + 1) * h->pmf_len[t - 1];
-            // per YT evaluations: 1 new cost + YT (p*c) + YT adds (+ YT (p*gamma*V) + YT adds)
-            h->stats.fp64_ops += ev * (last ? (1.0 + 2.0 * cp.YT) / cp.YT : (1.0 + 4.0 * cp.YT) / cp.YT);
-            return launch_col<DEDUP>(cp, h->dm, t, h->pmf_len[t - 1], h->pmf_off[t - 1], Vn, Vt, Qt, lo, hi, h->stream);
-        }
-        const LeadPlan lp = plan_lead(h->m, h->dm, h->pmf_len[t - 1], h->pmf_di.data() + h->pmf_off[t - 1]);
-        if (lp.ok) {
-            h->stats.kernel_used = SDPB_KERNEL_LEAD_SLAB;
-            const double ev = (double)(hi - lo) * (h->m.max_order_idx + 1) * h->pmf_len[t - 1];
-            const double q = 4.0 * lp.RQ;  // evaluations per thread per demand point
-            h->stats.fp64_ops += ev * (last ? (5.0 + q) / q : (5.0 + 3.0 * q) / q);
-            return launch_lead<DEDUP>(lp, h->dm, t, h->pmf_len[t - 1], h->pmf_off[t - 1], Vn, Vt, Qt, lo, hi, h->stream);
-        }
-    }
-    if (h->opt.kernel != SDPB_KERNEL_GENERIC && staged_ok(h, t)) {
-        h->stats.kernel_used = SDPB_KERNEL_STAGED;
-        // per evaluation: add, mul, add (+ mul, add when a continuation exists)
-        h->stats.fp64_ops += (double)(hi - lo) * (plain ? 1 : h->m.max_order_idx + 1) * h->pmf_len[t - 1] * (last ? 3.0 : 5.0);
-        return launch_staged<DEDUP>(h, t, Vn, Vt, Qt, lo, hi);
-    }
-    if (!DEDUP && h->opt.kernel != SDPB_KERNEL_GENERIC && h->opt.kernel != SDPB_KERNEL_CASH_ROW) {
-        // row-shared kernel with the minimal per-lane tail: cash-constraint and overdraft lambdas
-        const CashTailPlan tp = plan_cash_tail(h->m, h->dm, h->pmf_len[t - 1], h->pmf_d.data(), (int)h->pmf_d.size());
-        if (tp.ok) {
-            h->stats.kernel_used = SDPB_KERNEL_CASH_TAIL;
-            // DADD + DMUL per evaluation as counted by ncu (profiles/r02_fp64_audit.md)
-            const int kd = h->m.cost_kind;  // (overdraft-limit / -testing: a few more for the two interest products)
-            const double body = kd == SDPB_COST_CASH_DEPOSIT ? 4.0 : kd == SDPB_COST_CASH_OVERDRAFT ? 2.0 : kd == SDPB_COST_CASH_OD_LIMIT ? 9.0 : 7.0;
-            h->stats.fp64_ops += count_evals_period(h, t) * (last ? body + 3.0 : body + 8.0);
-            return launch_cash_tail(tp, h->m, h->dm, t, h->pmf_len[t - 1], h->pmf_off[t - 1], Vn, Vt, Qt, lo, hi, h->stream);
-        }
-    }
-    if (!DEDUP && h->opt.kernel != SDPB_KERNEL_GENERIC && cash_row_ok(h->m, h->dm, h->pmf_len[t - 1])) {
-        h->stats.kernel_used = SDPB_KERNEL_CASH_ROW;
-        // cash-dependent tail per evaluation: deposit chain 4, salvage 1, end cash 1, p*c 2 (+ clamp / quantiser /
-        // continuation 5 when a successor exists); compares and selects not counted
-        h->stats.fp64_ops += count_evals_period(h, t) * (last ? 8.0 : 13.0);
-        return launch_cash_row(h->m, h->dm, t, h->pmf_len[t - 1], h->pmf_off[t - 1], Vn, Vt, Qt, lo, hi, h->stream);
-    }
-    if (h->stats.kernel_used == 0) h->stats.kernel_used = SDPB_KERNEL_GENERIC;
-    {   // bi_generic evaluates the lambdas as written: its fp64 count per evaluation is MEASURED (ncu DADD + DMUL thread
-        // instructions, profiles/r02_fp64_audit.md), not derived; kinds that were not measured report nothing
-        double per_eval = 0.0;
-        switch (h->m.cost_kind) {
-        case SDPB_COST_BACKORDER: per_eval = 8.4; break;
-        case SDPB_COST_CASH_DEPOSIT: per_eval = 18.4; break;
-        case SDPB_COST_CASH_OVERDRAFT: per_eval = 11.5; break;
-        case SDPB_COST_STAFF: per_eval = 7.4; break;
-        default: break;
-        }
-        h->stats.fp64_ops += per_eval * (DEDUP ? count_evals_virtual(h, t) : count_evals_period(h, t));
-    }
-    return dispatch_generic_d<DEDUP>(h, t, Vn, Vt, Qt, lo, hi);
 }
 
 template <int KIND>
@@ -672,9 +526,6 @@ void launch_expand(sdpb_handle* h, double* Vt, int* Qt) {
     expand_dedup<KIND><<<(unsigned)((n + 255) / 256), 256, 0, h->stream>>>(h->dm, h->dHv, h->dHa, Vt, Qt, h->lo, h->hi);
 }
 
-// Evaluations actually executed for one period in dedup mode (virtual states only).
-double count_evals_virtual(const sdpb_handle* h, int t);
-
 template <int KIND, bool SURV>
 void launch_reach(sdpb_handle* h, int t) {
     const long long blocks = (h->S + 255) / 256;
@@ -683,6 +534,7 @@ void launch_reach(sdpb_handle* h, int t) {
         h->dCounters);
 }
 
+// Evaluations actually executed for one period in dedup mode (virtual states only).
 double count_evals_virtual(const sdpb_handle* h, int t) {
     const sdpb_model& m = h->m;
     const DevModel& d = h->dm;
@@ -843,6 +695,19 @@ int finish_sharded(sdpb_handle* h) {
     return SDPB_OK;
 }
 
+// Scratch for action slices: a (value, action) entry per slice and state (a smaller earlier one stays in dev_allocs).
+int grow_slice_scratch(sdpb_handle* h, size_t need, double*& v, int*& a, size_t& cap) {
+    if (need <= cap) return SDPB_OK;
+    void* p = nullptr;
+    CU(dev_alloc(h, &p, need * sizeof(double)));
+    v = (double*)p;
+    CU(dev_alloc(h, &p, need * sizeof(int)));
+    a = (int*)p;
+    cap = need;
+    return SDPB_OK;
+}
+
+// Runs the kernel family choose_period_kernel picked for period t, and counts it in h->stats.
 int solve_period(sdpb_handle* h, int t) {
     const sdpb_model& m = h->m;
     if (t < 1 || t > m.T) { h->err = "period out of range"; return SDPB_ERR_ARG; }
@@ -850,99 +715,230 @@ int solve_period(sdpb_handle* h, int t) {
     // V_{t+1}: the next period's table, or in period T the boundary table when the model has one
     // (CashRecursionV.java:125-128), else nothing (Recursion.java:140)
     const double* Vn = t < m.T ? h->dV[t] : h->dTerm;
-    int rc = SDPB_ERR_STATE;
-    const int D = h->pmf_len[t - 1];
-    // A(s) = {0} in period T (SingleProductLeadtime.java:74-75): only decode_state() knows that rule, so the
-    // period runs on the kernels that call it (generic, staged, cash_row) -- one period of T, one action per state
-    const bool plain = (m.flags & SDPB_F_NO_ORDER_LAST) && t == m.T;
-    // a boundary table in period T: the integer-exact cash kernels fold "last period" and "no continuation" into one
-    // template flag, so that one period takes the general path
-    const bool term_T = t == m.T && h->dTerm != nullptr;
-    if (h->opt.kernel == SDPB_KERNEL_COLLAPSED) {  // opt-in, not bit-identical (kernel_collapsed.cuh); validated by sdpb_create
-        rc = launch_collapsed(h->dm, t, D, h->pmf_off[t - 1], Vn, h->dLc, h->lc_il0, h->dG, h->dV[t - 1], h->dQ[t - 1], h->stream);
+    const bool last = Vn == nullptr;
+    const int D = h->pmf_len[t - 1], off = h->pmf_off[t - 1];
+    const bool plain = (m.flags & SDPB_F_NO_ORDER_LAST) && t == m.T;  // A(s) = {0}: see choose_period_kernel
+    const bool surv = m.recursion == SDPB_REC_SURVIVAL;
+    // dedup (lead-time models): solve each distinct (x + preQ, ...) of the virtual grid once, then broadcast (exact)
+    double* Vt = h->dedup ? h->dHv : h->dV[t - 1];
+    int* Qt = h->dedup ? h->dHa : h->dQ[t - 1];
+    const long long lo = h->dedup ? 0 : h->lo, hi = h->dedup ? h->vS : h->hi;
+    const double ev_range = (double)(hi - lo) * (m.max_order_idx + 1) * D;  // every action of every state of [lo, hi)
+    double executed = h->dedup ? count_evals_virtual(h, t) : count_evals_period(h, t);
+    const bool push = h->peer.attached && t > 1 && !h->peer.sends.empty();  // a peer reads rows of this period
+    const sdpb_kernel_choice kind = h->period_kernel[t - 1];
+    sdpb_kernel_choice used = kind;
+    int rc = SDPB_OK;
+    switch (kind) {
+    case SDPB_KERNEL_COLLAPSED: {  // opt-in, not bit-identical (kernel_collapsed.cuh)
+        rc = launch_collapsed(h->dm, t, D, off, Vn, h->dLc, h->lc_il0, h->dG, Vt, Qt, h->stream);
         if (rc != SDPB_OK) { h->err = "collapsed kernel launch failed"; return rc; }
         const double nY = (double)h->dm.nI + m.max_order_idx, nA = m.max_order_idx + 1.0;
-        h->solved[t - 1] = 1;
-        h->stats.kernel_used = SDPB_KERNEL_COLLAPSED;
-        h->stats.launches += 2;
-        h->stats.evals += count_evals_period(h, t);            // what the reference evaluates
-        h->stats.evals_executed += nY * D + (double)h->S * nA;  // level-demand pairs + state-action pairs
+        h->stats.launches++;                     // (two kernels)
+        executed = nY * D + (double)h->S * nA;   // level-demand pairs + state-action pairs
         h->stats.fp64_ops += nY * D * (Vn ? 7.0 : 5.0) + (double)h->S * nA * 3.0;
-        return SDPB_OK;
+        break;
     }
-    if (h->dedup) {
-        // lead-time models: solve each distinct (x + preQ, ...) once, then broadcast (exact)
-        rc = run_period_kernel<true>(h, t, Vn, h->dHv, h->dHa, 0, h->vS, plain);
+    case SDPB_KERNEL_TILED: {
+        int variant = 1;
+        rc = launch_tiled(h->tiled, h->dm, t, D, off, Vn, Vt, Qt, lo, hi, h->stream, &variant);
+        if (rc != SDPB_OK) { h->err = "tiled kernel launch failed"; return rc; }
+        if (variant == 2) {
+            used = SDPB_KERNEL_TILED2;
+            // per 16 evaluations: 4 new costs + 4 products + 16 * (mul, add, add); last period: 4 + 16 * 2
+            h->stats.fp64_ops += last ? ev_range * 2.25 : ev_range * 3.5;
+        } else {
+            // per evaluation add+mul+add(+add), plus one mul per R evaluations
+            h->stats.fp64_ops += last ? ev_range * 3.0 : ev_range * 4.0 + ev_range / kTiledR;
+        }
+        break;
+    }
+    case SDPB_KERNEL_CASH_DIAG:
+    case SDPB_KERNEL_CASH_INT: {
+        const bool diag = kind == SDPB_KERNEL_CASH_DIAG;
+        const CashIntShape sh = cash_int_shape(m, h->dm, t, lo, hi, h->sm_count);
+        const int parts = diag ? cash_diag_parts(m, h->dm, h->cash.period[t - 1], lo, hi, h->sm_count) : sh.parts;
+        if (int e = grow_slice_scratch(h, parts > 1 ? (size_t)parts * (size_t)(hi - lo) : 0, h->cash.slice_v,
+                                       h->cash.slice_a, h->cash.slice_cap))
+            return e;
+        // a sliced launch: merge_action_slices also stores the rows the peers read
+        const DevPeer* d_peers = push ? (const DevPeer*)h->peer.d_peers : nullptr;
+        const int n_peers = push ? (int)h->peer.sends.size() : 0;
+        rc = diag ? launch_cash_diag(h->cash, parts, m, h->dm, t, D, off, Vn, Vt, Qt, lo, hi, h->stream, d_peers, n_peers)
+                  : launch_cash(h->cash, sh, m, h->dm, t, D, off, Vn, Vt, Qt, lo, hi, h->stream, d_peers, n_peers);
+        if (rc != SDPB_OK) { h->err = "cash kernel launch failed"; return rc; }
+        if (parts > 1) {
+            h->stats.launches++;  // merge_action_slices
+            if (push) h->push_fused = true;
+        }
+        if (diag) h->stats.fp64_ops += executed * (surv ? 2.0 : 3.0 + 2.0 / kDiagYT);
+        else if (t == m.T) h->stats.fp64_ops += executed * (surv ? 2.0 + 3.0 / kCashR : 1.0 + 4.0 / (sh.wide ? kCashRLast : kCashR));
+        else h->stats.fp64_ops += executed * (surv ? 2.0 : 3.0 + 2.0 / kCashR);
+        break;
+    }
+    case SDPB_KERNEL_LEAD_Q2: {
+        const Q2Plan qp = plan_q2(m, h->dm, D, h->pmf_di.data() + off);
+        const Q2Shape shape = q2_shape(qp, h->dm, D, lo, hi, h->sm_count);
+        int64_t rlo = 0, rhi = h->S;
+        sdpb_shard_reads(h, &rlo, &rhi);
+        const long long per_x = (long long)h->dm.nQ * h->dm.nQ;
+        // multi-GPU: the kernel's epilogue stores the rows its (at most two) neighbours read straight into their
+        // tables, or, when the action range is cut over separate CTAs, merge_action_slices does; enqueue_period_sharded
+        // then skips the copies
+        PeerStore ps[kQ2MaxPeers];
+        int nps = 0;
+        if (shape.slices > 1) {
+            if (int e = grow_slice_scratch(h, (size_t)shape.slices * (size_t)(hi - lo), h->q2_slice_v, h->q2_slice_a,
+                                           h->q2_slice_cap))
+                return e;
+            if (push) h->push_fused = true;
+        } else if (push && h->peer.sends.size() <= (size_t)kQ2MaxPeers) {
+            for (const PeerSend& sd : h->peer.sends) {
+                const PeerInfo& pi = h->peer.info[sd.rank];
+                char* base = h->peer.mapped[sd.rank] + pi.v_off0 + (size_t)(t - 1) * pi.v_stride;
+                ps[nps++] = PeerStore{reinterpret_cast<double*>(base) - pi.vlo, sd.a, sd.b};
+            }
+            h->push_fused = true;
+        }
+        const bool merge_pushes = push && shape.slices > 1;
+        rc = launch_q2(qp, shape, h->dm, t, D, off, Vn, h->dVT, Vt, Qt, lo, hi, (int)(rlo / per_x), (int)(rhi / per_x),
+                       h->stream, ps, nps, h->q2_slice_v, h->q2_slice_a, h->q2_slice_cap,
+                       merge_pushes ? (const DevPeer*)h->peer.d_peers : nullptr, merge_pushes ? (int)h->peer.sends.size() : 0);
         if (rc != SDPB_OK) return rc;
+        const bool ran = hi > lo;  // (an empty shard launches nothing and reports bi_lead_q2)
+        if (!last) h->stats.launches++;                      // the transposition pass
+        if (ran && shape.slices > 1) h->stats.launches++;    // merge_action_slices
+        // per evaluation: (mul, add, mul, add) + one cost per 8 -- or, with the products p*(fv + L) shared by the CTA
+        // (bi_lead_q2m), (add, mul, add); the last period has no continuation term
+        if (ran && shape.shared) { used = SDPB_KERNEL_LEAD_Q2M; h->stats.fp64_ops += ev_range * (last ? 1.0 : 3.0); }
+        else h->stats.fp64_ops += ev_range * (last ? (1.0 + 2.0 * kQ2YT) / kQ2YT : (1.0 + 4.0 * kQ2YT) / kQ2YT);
+        break;
+    }
+    case SDPB_KERNEL_LEAD_COL: {
+        const ColPlan cp = plan_col(m, h->dm, D, h->pmf_di.data() + off, h->dedup);
+        rc = h->dedup ? launch_col<true>(cp, h->dm, t, D, off, Vn, Vt, Qt, lo, hi, h->stream)
+                      : launch_col<false>(cp, h->dm, t, D, off, Vn, Vt, Qt, lo, hi, h->stream);
+        // per YT evaluations: 1 new cost + YT (p*c) + YT adds (+ YT (p*gamma*V) + YT adds)
+        h->stats.fp64_ops += ev_range * (last ? (1.0 + 2.0 * kColYT) / kColYT : (1.0 + 4.0 * kColYT) / kColYT);
+        break;
+    }
+    case SDPB_KERNEL_LEAD_SLAB: {
+        const LeadPlan lp = plan_lead(m, h->dm, D, h->pmf_di.data() + off);
+        rc = h->dedup ? launch_lead<true>(lp, h->dm, t, D, off, Vn, Vt, Qt, lo, hi, h->stream)
+                      : launch_lead<false>(lp, h->dm, t, D, off, Vn, Vt, Qt, lo, hi, h->stream);
+        const double q = 4.0 * lp.RQ;  // evaluations per thread per demand point
+        h->stats.fp64_ops += ev_range * (last ? (5.0 + q) / q : (5.0 + 3.0 * q) / q);
+        break;
+    }
+    case SDPB_KERNEL_STAGED:
+        rc = h->dedup ? launch_staged<true>(h, t, Vn, Vt, Qt, lo, hi) : launch_staged<false>(h, t, Vn, Vt, Qt, lo, hi);
+        // per evaluation: add, mul, add (+ mul, add when a continuation exists)
+        h->stats.fp64_ops += (double)(hi - lo) * (plain ? 1 : m.max_order_idx + 1) * D * (last ? 3.0 : 5.0);
+        break;
+    case SDPB_KERNEL_CASH_TAIL: {
+        const CashTailPlan tp = plan_cash_tail(m, h->dm, D, h->pmf_d.data(), (int)h->pmf_d.size());
+        rc = launch_cash_tail(tp, m, h->dm, t, D, off, Vn, Vt, Qt, lo, hi, h->stream);
+        // DADD + DMUL per evaluation as counted by ncu (profiles/r02_fp64_audit.md)
+        const int kd = m.cost_kind;  // (overdraft-limit / -testing: a few more for the two interest products)
+        const double body = kd == SDPB_COST_CASH_DEPOSIT ? 4.0 : kd == SDPB_COST_CASH_OVERDRAFT ? 2.0 : kd == SDPB_COST_CASH_OD_LIMIT ? 9.0 : 7.0;
+        h->stats.fp64_ops += executed * (last ? body + 3.0 : body + 8.0);
+        break;
+    }
+    case SDPB_KERNEL_CASH_ROW:
+        rc = launch_cash_row(m, h->dm, t, D, off, Vn, Vt, Qt, lo, hi, h->stream);
+        // cash-dependent tail per evaluation: deposit chain 4, salvage 1, end cash 1, p*c 2 (+ clamp / quantiser /
+        // continuation 5 when a successor exists); compares and selects not counted
+        h->stats.fp64_ops += executed * (last ? 8.0 : 13.0);
+        break;
+    case SDPB_KERNEL_TWO_PRODUCT_ROW:
+        rc = launch_two_product_row(h, t, Vn, Vt, Qt, lo, hi);
+        h->stats.fp64_ops += executed * (t == m.T ? 1.0 : 3.0);
+        break;
+    default: {  // SDPB_KERNEL_GENERIC
+        rc = h->dedup ? dispatch_generic_d<true>(h, t, Vn, Vt, Qt, lo, hi) : dispatch_generic_d<false>(h, t, Vn, Vt, Qt, lo, hi);
+        // bi_generic evaluates the lambdas as written: its fp64 count per evaluation is MEASURED (ncu DADD + DMUL thread
+        // instructions, profiles/r02_fp64_audit.md), not derived; kinds that were not measured report nothing
+        double per_eval = 0.0;
+        switch (m.cost_kind) {
+        case SDPB_COST_BACKORDER: per_eval = 8.4; break;
+        case SDPB_COST_CASH_DEPOSIT: per_eval = 18.4; break;
+        case SDPB_COST_CASH_OVERDRAFT: per_eval = 11.5; break;
+        case SDPB_COST_STAFF: per_eval = 7.4; break;
+        default: break;
+        }
+        h->stats.fp64_ops += per_eval * executed;
+        break;
+    }
+    }
+    if (rc != SDPB_OK) return rc;
+    if (h->dedup) {
         switch (m.cost_kind) {
         case SDPB_COST_BACKORDER: launch_expand<SDPB_COST_BACKORDER>(h, h->dV[t - 1], h->dQ[t - 1]); break;
         case SDPB_COST_CASH_DEPOSIT: launch_expand<SDPB_COST_CASH_DEPOSIT>(h, h->dV[t - 1], h->dQ[t - 1]); break;
         default: launch_expand<SDPB_COST_CASH_OVERDRAFT>(h, h->dV[t - 1], h->dQ[t - 1]); break;
         }
-        CU(cudaGetLastError());
-        h->solved[t - 1] = 1;
-        h->stats.launches += 2;
-        h->stats.evals += count_evals_period(h, t);
-        h->stats.evals_executed += count_evals_virtual(h, t);
-        return SDPB_OK;
+        h->stats.launches++;
     }
-    if (h->tiled.available && h->opt.kernel != SDPB_KERNEL_GENERIC && !plain) {
-        int variant = 1;
-        rc = launch_tiled(h->tiled, h->dm, t, h->pmf_len[t - 1], h->pmf_off[t - 1], Vn, h->dV[t - 1],
-                          h->dQ[t - 1], h->lo, h->hi, h->stream, &h->stats.fp64_ops, &variant);
-        if (rc == SDPB_OK) h->stats.kernel_used = variant == 2 ? SDPB_KERNEL_TILED2 : SDPB_KERNEL_TILED;
-        else if (rc != SDPB_ERR_STATE) { h->err = "tiled kernel launch failed"; return rc; }
-    }
-    if (rc == SDPB_ERR_STATE && h->opt.kernel != SDPB_KERNEL_GENERIC && !plain && !term_T) {  // integer cash models
-        rc = SDPB_ERR_STATE;
-        // scratch for the action slices: one (value, action) entry per slice and state of the shard
-        auto slice_scratch = [&](int parts) -> int {
-            const size_t need = parts > 1 ? (size_t)parts * (size_t)(h->hi - h->lo) : 0;
-            if (need > h->cash.slice_cap) {
-                void* p = nullptr;
-                CU(dev_alloc(h, &p, need * sizeof(double)));
-                h->cash.slice_v = (double*)p;
-                CU(dev_alloc(h, &p, need * sizeof(int)));
-                h->cash.slice_a = (int*)p;
-                h->cash.slice_cap = need;  // (an earlier, smaller scratch stays in dev_allocs until the handle goes)
-            }
-            return SDPB_OK;
-        };
-        static const bool no_fused = std::getenv("SDPB_NO_FUSED_PUSH") != nullptr;  // A/B knob: copies after the kernel
-        const bool push = h->peer.attached && t > 1 && !h->peer.sends.empty() && !no_fused;
-        const DevPeer* d_peers = push ? (const DevPeer*)h->peer.d_peers : nullptr;
-        const int n_peers = push ? (int)h->peer.sends.size() : 0;
-        if (h->opt.kernel != SDPB_KERNEL_CASH_INT && h->cash.available && t < m.T && h->cash.period[t - 1].ok && h->hi > h->lo) {
-            // (as a request, SDPB_KERNEL_CASH_INT skips the diagonal-window variant)
-            const int parts = cash_diag_parts(m, h->dm, h->cash.period[t - 1], h->lo, h->hi, h->sm_count);
-            if (int e = slice_scratch(parts)) return e;
-            rc = launch_cash_diag(h->cash, m, h->dm, t, D, h->pmf_off[t - 1], Vn, h->dV[t - 1], h->dQ[t - 1], h->lo,
-                                  h->hi, h->stream, &h->stats.fp64_ops, count_evals_period(h, t), h->sm_count,
-                                  d_peers, n_peers, &h->push_fused);
-            if (rc == SDPB_OK && parts > 1) h->stats.launches++;  // merge_action_slices
-        }
-        if (rc == SDPB_OK) h->stats.kernel_used = SDPB_KERNEL_CASH_DIAG;
-        else if (rc == SDPB_ERR_STATE && h->cash.available && h->cash.period[t - 1].ok && h->hi > h->lo) {
-            const int parts = cash_int_shape(m, h->dm, t, h->lo, h->hi, h->sm_count).parts;
-            if (int e = slice_scratch(parts)) return e;
-            rc = launch_cash(h->cash, m, h->dm, t, D, h->pmf_off[t - 1], Vn, h->dV[t - 1], h->dQ[t - 1], h->lo, h->hi,
-                             h->stream, &h->stats.fp64_ops, count_evals_period(h, t), h->sm_count, d_peers, n_peers,
-                             &h->push_fused);
-            if (rc == SDPB_OK && parts > 1) h->stats.launches++;  // merge_action_slices
-            if (rc == SDPB_OK && h->stats.kernel_used != SDPB_KERNEL_CASH_DIAG) h->stats.kernel_used = SDPB_KERNEL_CASH_INT;
-        }
-        if (rc != SDPB_OK && rc != SDPB_ERR_STATE) { h->err = "cash kernel launch failed"; return rc; }
-    }
-    if (rc == SDPB_ERR_STATE)  // no specialised plan for this model / period
-        rc = run_period_kernel<false>(h, t, Vn, h->dV[t - 1], h->dQ[t - 1], h->lo, h->hi, plain);
-    if (rc != SDPB_OK) return rc;
     CU(cudaGetLastError());
     h->solved[t - 1] = 1;
     h->stats.launches++;
-    const double ev = count_evals_period(h, t);
-    h->stats.evals += ev;
-    h->stats.evals_executed += ev;
+    h->stats.evals += count_evals_period(h, t);  // what the reference evaluates
+    h->stats.evals_executed += executed;
+    // The kernel a solve reports: the last one that ran, except that GENERIC does not replace a specialised kernel of
+    // an earlier period, and CASH_INT (period T) does not replace CASH_DIAG.
+    const int prev = h->stats.kernel_used;
+    if (!(used == SDPB_KERNEL_GENERIC && prev != 0) && !(used == SDPB_KERNEL_CASH_INT && prev == SDPB_KERNEL_CASH_DIAG))
+        h->stats.kernel_used = used;
     return SDPB_OK;
+}
+
+// The kernel family that solves period t, fixed by sdpb_create from the model, the request (opt.kernel), dedup, the
+// per-period plans, the shard's range and whether dVT exists.  "plain": period T of an SDPB_F_NO_ORDER_LAST model (A(s)
+// = {0}, SingleProductLeadtime.java:74-75, a rule only decode_state() knows); "term_T": period T with a boundary table
+// (the integer cash kernels fold "last period" and "no continuation" into one flag).  The first rule that applies wins:
+//   request COLLAPSED or GENERIC: that kernel
+//   backorder, lead 0, clamp: TILED (tiled / tiled2 at launch) if the period has a plan and is not plain
+//   integer-exact deposit models, any request, periods with a plan, not plain or term_T, a non-empty shard:
+//     CASH_DIAG if t < T, the request is not CASH_INT and cash_diag_ok;  CASH_INT if its tables fit
+//   backorder, lead >= 1, not plain: LEAD_Q2 (q2 / q2m at launch) if dVT exists (lead 2, unfolded, request AUTO or
+//     LEAD_Q2) and plan_q2 holds;  LEAD_COL if the request is neither STAGED nor LEAD_SLAB and plan_col holds;
+//     LEAD_SLAB if the request is not STAGED and plan_lead holds
+//   backorder, lead >= 1: STAGED if its tables fit
+//   cash kinds with row-shared kernels, lead 0: CASH_TAIL if the request is not CASH_ROW and plan_cash_tail holds;
+//     CASH_ROW if cash_row_ok
+//   two-product: TWO_PRODUCT_ROW in a non-empty shard, not term_T, if plan_two_product_row holds
+//   otherwise GENERIC
+// So a CASH_ROW request on an integer-exact deposit model runs the integer cash kernels, and a TILED request on a
+// backorder lead-time model runs LEAD_COL.
+sdpb_kernel_choice choose_period_kernel(const sdpb_handle* h, int t) {
+    const sdpb_model& m = h->m;
+    const int K = h->opt.kernel;
+    if (K == SDPB_KERNEL_COLLAPSED || K == SDPB_KERNEL_GENERIC) return (sdpb_kernel_choice)K;
+    const int D = h->pmf_len[t - 1];
+    const int* di = h->pmf_di.data() + h->pmf_off[t - 1];
+    const bool plain = (m.flags & SDPB_F_NO_ORDER_LAST) && t == m.T;
+    const bool term_T = t == m.T && h->dTerm != nullptr;
+    const bool backorder_lead = m.cost_kind == SDPB_COST_BACKORDER && m.lead_time >= 1;
+    if (h->tiled.available && !plain && (h->tiled.period[t - 1].ok || h->tiled.period[t - 1].ok2))
+        return SDPB_KERNEL_TILED;
+    if (h->cash.available && h->cash.period[t - 1].ok && !plain && !term_T && h->hi > h->lo) {
+        if (K != SDPB_KERNEL_CASH_INT && t < m.T && cash_diag_ok(h->cash.period[t - 1], m, h->dm, D))
+            return SDPB_KERNEL_CASH_DIAG;
+        if (cash_int_smem(D) <= 200 * 1024) return SDPB_KERNEL_CASH_INT;
+    }
+    if (backorder_lead && !plain) {
+        if (h->dVT && plan_q2(m, h->dm, D, di).ok) return SDPB_KERNEL_LEAD_Q2;
+        if (K != SDPB_KERNEL_STAGED && K != SDPB_KERNEL_LEAD_SLAB && plan_col(m, h->dm, D, di, h->dedup).ok)
+            return SDPB_KERNEL_LEAD_COL;
+        if (K != SDPB_KERNEL_STAGED && plan_lead(m, h->dm, D, di).ok) return SDPB_KERNEL_LEAD_SLAB;
+    }
+    if (backorder_lead && staged_smem(D) <= 200 * 1024) return SDPB_KERNEL_STAGED;
+    if (K != SDPB_KERNEL_CASH_ROW && plan_cash_tail(m, h->dm, D, h->pmf_d.data(), (int)h->pmf_d.size()).ok)
+        return SDPB_KERNEL_CASH_TAIL;
+    if (cash_row_ok(m, h->dm, D)) return SDPB_KERNEL_CASH_ROW;
+    if (two_product(m) && h->hi > h->lo && !term_T && plan_two_product_row(m, h->dm, t, D))
+        return SDPB_KERNEL_TWO_PRODUCT_ROW;
+    return SDPB_KERNEL_GENERIC;
 }
 
 }  // namespace
@@ -1372,6 +1368,8 @@ int sdpb_create(const sdpb_model* m, const sdpb_options* opt, sdpb_handle** out)
         collapsed_level_costs<<<(unsigned)((n_lc + 255) / 256), 256, 0, h->stream>>>(h->dm, h->lc_il0, n_lc, h->dLc);
         if (cudaGetLastError() != cudaSuccess) return fail_create(h, SDPB_ERR_CUDA, "level-cost kernel launch failed");
     }
+    h->period_kernel.resize(T);
+    for (int t = 1; t <= T; t++) h->period_kernel[t - 1] = choose_period_kernel(h, t);
     mark("planned");
     *out = h;
     return SDPB_OK;

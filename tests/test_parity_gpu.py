@@ -720,22 +720,23 @@ def test_solve_batch_wide(S, oracle):
         s.close()
 
 
-@pytest.mark.parametrize("split", ["default", "1", "2", "4"])
-def test_lead_q2m_forced(split):
-    """bi_lead_q2m (products p*(fv + L) shared through shared memory, two preQ2 columns per thread) is chosen by itself
-    on 16 small random lead-time-2 instances, unsharded and as a three-shard group: as the library shapes the launch
-    by itself (action slices over separate CTAs + merge kernel), and forced to 1, 2 and 4 action slices inside a CTA.
-    The knobs are read once per process, hence the subprocess."""
+@pytest.mark.parametrize("mode", ["default", "share", "split2", "split4"])
+def test_lead_q2m_forced(mode):
+    """The lead-time-2 kernels on 16 small random instances, unsharded and as a three-shard group: as the library shapes
+    the launch by itself (bi_lead_q2m with action slices over separate CTAs + merge kernel), and forced by one test hook
+    each to bi_lead_q2m without action slices (share) and to bi_lead_q2 with 2 or 4 thread groups (split2, split4).
+    The hooks are read once per process, hence the subprocess."""
     import os
     import subprocess
     import sys
     env = dict(os.environ)
-    if split == "default":
-        # no knob: on these small grids the library cuts the action range over separate CTAs (gridDim.y) and merges
-        # with merge_action_slices -- the path the multi-GPU shards of C4 take
-        env.pop("SDPB_Q2_SHARE", None), env.pop("SDPB_Q2_SPLIT", None)
-    else:
-        env.update(SDPB_Q2_SHARE="1", SDPB_Q2_SPLIT=split)
+    env.pop("SDPB_Q2_SHARE", None), env.pop("SDPB_Q2_SPLIT", None)
+    # default: on these small grids the library cuts the action range over separate CTAs (gridDim.y) and merges with
+    # merge_action_slices -- the path the multi-GPU shards of C4 take
+    if mode == "share":
+        env["SDPB_Q2_SHARE"] = "1"
+    elif mode.startswith("split"):
+        env["SDPB_Q2_SPLIT"] = mode[len("split"):]
     worker = os.path.join(os.path.dirname(os.path.abspath(__file__)), "q2m_worker.py")
     r = subprocess.run([sys.executable, worker], env=env, capture_output=True, text=True, timeout=600)
     assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-4000:]
