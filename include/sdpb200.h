@@ -26,6 +26,9 @@
  *                                                                                  sdpb_solve + sdpb_value
  *   getAction(state)                   Recursion.java:165-167 (and siblings)       sdpb_value (q out)
  *   getOptTable()/getCacheActions()    Recursion.java:169-186 (and siblings)       sdpb_reach + sdpb_opt_table
+ *   the same at off-grid states, steps that are not powers of two, unclamped models without a hull
+ *                                      (the memo maps of Recursion.java:89-163)     sdpb_topdown_solve +
+ *                                                                                  sdpb_topdown_value / _opt_table
  *   the lambdas A, f, c                src/capacitated/CLSPTesting.java:78-106, src/leadtime/Leadtime.java:50-81,
  *                                      src/cash/singleItem/CashConstraint.java:95-133,
  *                                      src/cash/overdraft/CashOverdraft.java:72-118,
@@ -505,6 +508,53 @@ typedef struct sdpb_reached_model {
 int sdpb_reached_solve(const sdpb_reached_model* m, int device, const double* init_state, double* value,
                        double* action1, double* action2, int64_t* n_states, double* solve_ms);
 const char* sdpb_reached_last_error(void);
+
+/* ---- any single-product model, solved over the states its top-down recursion reaches ---------------------------------
+ * The reference answers getExpectedValue(state) for ANY state: it recurses top-down over real-valued states and memoises
+ * what it visits (Recursion.java:89-163).  sdpb_create needs a grid (every level, action and demand a multiple of a
+ * power-of-two step, initial states on it, an unclamped model sized with sdpb_reachable_hull); this engine needs none.
+ * From the period-1 states it builds, period by period, exactly the states the reference visits -- successors through
+ * feasible actions only, while t < T, and in the survival recursion not a successor whose cash is negative
+ * (RiskRecursion.java:87-95) -- then runs the backward induction over them on the GPU with the dense engine's
+ * arithmetic.  Two states are one iff their coordinates are == as doubles.
+ *   inv_min / inv_max, cash_min / cash_max  only the clamp bounds the lambdas apply (no grid is built)
+ *   step                                    only defines the actions a_i = i * step (exactness is not required)
+ * An XR state whose order-up-to range is longer than max_order_idx + 1 is counted in sdpb_stats.capped_action_sets; the
+ * solve fails with SDPB_ERR_OFFGRID unless SDPB_ALLOW_CAPPED_ACTIONS is set (the rule sdpb_reach applies).
+ * Refused with SDPB_ERR_ARG: SDPB_COST_CASH_TWO_PRODUCT and SDPB_COST_STAFF (their action pairs / pmf rows are tied to
+ * the grid), and a non-NULL terminal_value (tabulated on the grid: it has no value at an off-grid state).
+ * stats: evals = sum_t sum_{s reached} |A_t(s)| * D_t; solve_ms = time between CUDA events recorded on the engine's
+ * stream at the start and the end of the solve -- the forward pass synchronises with the host after every chunk and
+ * allocates as it goes, so this is close to the wall time of the solve, not kernel time alone; kernel_ms = the backward
+ * pass, which is kernels only; launches = backward launches. */
+typedef struct sdpb_topdown_options {
+    uint32_t struct_size;     /* = sizeof(sdpb_topdown_options) */
+    int32_t  device;          /* CUDA ordinal; -1 = current device */
+    uint32_t allow;           /* sdpb_allow bits (SDPB_ALLOW_CAPPED_ACTIONS) */
+    int32_t  reserved;
+    int64_t  scratch_bytes;   /* forward-expansion budget, a hard bound on the scratch the expansion allocates (three
+                                 buffers of 32-byte keys and the radix sort's temporary storage); 0 = half of the free
+                                 device memory.  A period whose candidate successors do not fit is expanded in chunks,
+                                 each holding at least as many candidates as the period has reached so far; a period
+                                 whose reached states pass half a buffer fails with SDPB_ERR_NOMEM naming the period.
+                                 The reached states and value tables of every period are kept outside the budget */
+} sdpb_topdown_options;
+typedef struct sdpb_topdown sdpb_topdown;
+/* new Recursion(...) / CashRecursion / LeadtimeRecursion / RiskRecursion / CashRecursionXR + getExpectedValue on each of
+ * the n period-1 states `init_states` (n * ndim API-order doubles, as sdpb_value): the memo maps the calls fill.
+ * opt may be NULL. */
+int  sdpb_topdown_solve(const sdpb_model* m, const sdpb_topdown_options* opt, const double* init_states, int n,
+                        sdpb_topdown** out);
+void sdpb_topdown_destroy(sdpb_topdown* h);
+const char* sdpb_topdown_last_error(const sdpb_topdown* h);   /* h may be NULL: last sdpb_topdown_solve error */
+/* getExpectedValue / getAction (Recursion.java:89-90,165-167): cacheValues / cacheActions of n reached states of one
+ * period; SDPB_ERR_UNSOLVED for a state that was not reached (Java: NullPointerException).  v, q may be NULL. */
+int  sdpb_topdown_value(sdpb_topdown* h, int period, const double* states, int n, double* v, double* q);
+/* getOptTable() / getCacheActions() (Recursion.java:169-186): rows [t, state dims (API order)..., Q*] of every reached
+ * state, sorted in memo-map order (t, x, preQ1, preQ2, cash), as sdpb_opt_table.  rows == NULL: *nrows = the count. */
+int  sdpb_topdown_opt_table(sdpb_topdown* h, double* rows, size_t* nrows);
+int  sdpb_topdown_states(const sdpb_topdown* h, int64_t* n_states /* T: reached states of each period */);
+int  sdpb_topdown_stats(const sdpb_topdown* h, sdpb_stats* s);
 
 /* Return the memory cached by the library's private stream-ordered pool on `device` to the driver (-1 = current). */
 int sdpb_trim_pool(int device);

@@ -11,10 +11,12 @@
 // names as the driver's local variables).  Header-only; link with -lsdpb200.  tests/cpp_driver.cpp reads like
 // CLSPTesting.main / CashConstraint.main / Leadtime.main and is checked against the oracle on a B200.
 #pragma once
+#include <algorithm>
 #include <array>
 #include <cmath>
 #include <cstdint>
 #include <cstring>
+#include <memory>
 #include <stdexcept>
 #include <string>
 #include <vector>
@@ -398,6 +400,101 @@ class RiskRecursion {  // RiskRecursion.java:31-108: getSurvProb instead of getE
 
  private:
     Engine e_;
+};
+
+// ---- no grid: the states the reference's recursion reaches from given period-1 states (sdpb_topdown_*) ----
+// States, steps and demands need not be multiples of a power of two; an unclamped model needs no hull.
+class TopDown {
+ public:
+    // `roots`: period-1 states in API order; scratchBytes = 0: the library's default expansion budget
+    TopDown(const Model& model, const std::vector<std::vector<double>>& roots, int device = -1, uint32_t allow = 0,
+            int64_t scratchBytes = 0) : model_(model) {
+        sdpb_topdown_options o;
+        std::memset(&o, 0, sizeof o);
+        o.struct_size = (uint32_t)sizeof o;
+        o.device = device; o.allow = allow; o.scratch_bytes = scratchBytes;
+        std::vector<double> flat;
+        for (const auto& r : roots) flat.insert(flat.end(), r.begin(), r.end());
+        const int rc = sdpb_topdown_solve(&model_.m, &o, flat.data(), (int)roots.size(), &h_);
+        if (rc != SDPB_OK) throw SdpbError(rc, std::string("sdpb_topdown_solve: ") + sdpb_topdown_last_error(nullptr));
+    }
+    TopDown(const TopDown&) = delete;
+    TopDown& operator=(const TopDown&) = delete;
+    ~TopDown() { sdpb_topdown_destroy(h_); }
+
+    // (V, Q*) of a reached state; SdpbError(SDPB_ERR_UNSOLVED) for one that was not reached
+    std::array<double, 2> valueAndAction(int period, const std::vector<double>& st) {
+        if (st.size() != ndim_plus2() - 2) throw SdpbError(SDPB_ERR_ARG, "state has the wrong number of components");
+        double v = 0.0, q = 0.0;
+        check(sdpb_topdown_value(h_, period, st.data(), 1, &v, &q));
+        return {v, q};
+    }
+    double value(int period, const std::vector<double>& st) { return valueAndAction(period, st)[0]; }
+    // rows [period, state..., Q*] of every reached state in memo-map order (Recursion.java:169-186)
+    std::vector<std::vector<double>> optTable() {
+        size_t n = 0;
+        check(sdpb_topdown_opt_table(h_, nullptr, &n));
+        std::vector<double> buf(n * ndim_plus2());
+        check(sdpb_topdown_opt_table(h_, buf.data(), &n));
+        const size_t w = ndim_plus2();
+        std::vector<std::vector<double>> rows(n, std::vector<double>(w));
+        for (size_t i = 0; i < n; i++) std::copy(buf.begin() + i * w, buf.begin() + (i + 1) * w, rows[i].begin());
+        return rows;
+    }
+    size_t nStates(int period) const {
+        std::vector<int64_t> n((size_t)model_.m.T);
+        check(sdpb_topdown_states(h_, n.data()));
+        return (size_t)n.at((size_t)period - 1);
+    }
+    sdpb_stats stats() const { sdpb_stats s; check(sdpb_topdown_stats(h_, &s)); return s; }
+
+ private:
+    size_t ndim_plus2() const { return 3 + (model_.m.cost_kind != SDPB_COST_BACKORDER ? 1 : 0) + (size_t)model_.m.lead_time; }
+    void check(int rc) const {
+        if (rc != SDPB_OK) throw SdpbError(rc, sdpb_topdown_last_error(h_));
+    }
+    Model model_;
+    sdpb_topdown* h_ = nullptr;
+};
+
+// Recursion / LeadtimeRecursion / CashRecursion / RiskRecursion access over TopDown, with states given as API-order
+// vectors: getExpectedValue on a new period-1 state solves again with that root added (the memo maps grow the same
+// way); getAction / getExpectedValue of a later-period state that was not reached throws SDPB_ERR_UNSOLVED.
+class TopDownRecursion {
+ public:
+    explicit TopDownRecursion(const Model& model, int device = -1, uint32_t allow = 0)
+        : model_(model), device_(device), allow_(allow) {}
+    double getExpectedValue(int period, const std::vector<double>& st) {
+        if (period == 1 && std::find(roots_.begin(), roots_.end(), st) == roots_.end()) {
+            // solve with the new root first: if that throws, the roots and the previous solve stay as they were
+            std::vector<std::vector<double>> roots = roots_;
+            roots.push_back(st);
+            std::unique_ptr<TopDown> td(new TopDown(model_, roots, device_, allow_));
+            roots_.swap(roots);
+            td_.swap(td);
+        }
+        return engine().value(period, st);
+    }
+    double getAction(int period, const std::vector<double>& st) { return engine().valueAndAction(period, st)[1]; }
+    double getExpectedValue(const State& s) { return getExpectedValue(s.period, {s.iniInventory}); }
+    double getAction(const State& s) { return getAction(s.period, {s.iniInventory}); }
+    double getExpectedValue(const LeadtimeState& s) { return getExpectedValue(s.period, {s.iniInventory, s.preQ}); }
+    double getAction(const LeadtimeState& s) { return getAction(s.period, {s.iniInventory, s.preQ}); }
+    double getExpectedValue(const CashState& s) { return getExpectedValue(s.period, {s.iniInventory, s.iniCash}); }
+    double getSurvProb(const CashState& s) { return getExpectedValue(s); }
+    double getAction(const CashState& s) { return getAction(s.period, {s.iniInventory, s.iniCash}); }
+    std::vector<std::vector<double>> getOptTable() { return engine().optTable(); }
+    TopDown& engine() {
+        if (!td_) throw SdpbError(SDPB_ERR_UNSOLVED, "no period-1 state has been solved");
+        return *td_;
+    }
+
+ private:
+    Model model_;
+    int device_;
+    uint32_t allow_;
+    std::vector<std::vector<double>> roots_;
+    std::unique_ptr<TopDown> td_;
 };
 
 }  // namespace sdpb200

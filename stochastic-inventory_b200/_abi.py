@@ -105,6 +105,13 @@ class SdpbReachedModel(C.Structure):
     ]
 
 
+class SdpbTopdownOptions(C.Structure):
+    _fields_ = [
+        ("struct_size", C.c_uint32), ("device", C.c_int32), ("allow", C.c_uint32), ("reserved", C.c_int32),
+        ("scratch_bytes", C.c_int64),
+    ]
+
+
 REACHED_MULTILEAD, REACHED_MULTI_XR, REACHED_MULTI_YR, REACHED_CASH_ROUNDED = 0, 1, 2, 3
 
 # every symbol include/sdpb200.h declares
@@ -117,6 +124,8 @@ EXPORTS = [
     "sdpb_peer_traffic", "sdpb_period_profile", "sdpb_shard_tables", "sdpb_group_create", "sdpb_group_destroy",
     "sdpb_group_last_error", "sdpb_group_solve", "sdpb_group_shard", "sdpb_group_value", "sdpb_group_period_tables",
     "sdpb_group_stats", "sdpb_solve_batch", "sdpb_trim_pool", "sdpb_reached_solve", "sdpb_reached_last_error",
+    "sdpb_topdown_solve", "sdpb_topdown_destroy", "sdpb_topdown_last_error", "sdpb_topdown_value",
+    "sdpb_topdown_opt_table", "sdpb_topdown_states", "sdpb_topdown_stats",
 ]
 
 _lib = None
@@ -197,6 +206,15 @@ def load():
     lib.sdpb_reached_solve.argtypes = [C.POINTER(SdpbReachedModel), C.c_int, _dp, _dp, _dp, _dp,
                                        C.POINTER(C.c_int64), _dp]
     lib.sdpb_reached_last_error.restype = C.c_char_p
+    lib.sdpb_topdown_solve.argtypes = [C.POINTER(SdpbModel), C.POINTER(SdpbTopdownOptions), _dp, C.c_int, C.POINTER(vp)]
+    lib.sdpb_topdown_destroy.argtypes = [vp]
+    lib.sdpb_topdown_destroy.restype = None
+    lib.sdpb_topdown_last_error.argtypes = [vp]
+    lib.sdpb_topdown_last_error.restype = C.c_char_p
+    lib.sdpb_topdown_value.argtypes = [vp, C.c_int, _dp, C.c_int, _dp, _dp]
+    lib.sdpb_topdown_opt_table.argtypes = [vp, _dp, C.POINTER(C.c_size_t)]
+    lib.sdpb_topdown_states.argtypes = [vp, C.POINTER(C.c_int64)]
+    lib.sdpb_topdown_stats.argtypes = [vp, C.POINTER(SdpbStats)]
     if (lib.sdpb_sizeof_model() != C.sizeof(SdpbModel) or lib.sdpb_sizeof_options() != C.sizeof(SdpbOptions)
             or lib.sdpb_sizeof_grid() != C.sizeof(SdpbGrid) or lib.sdpb_sizeof_stats() != C.sizeof(SdpbStats)
             or lib.sdpb_abi_version() != ABI_VERSION):

@@ -49,6 +49,30 @@ struct ActionCtx {
     long long pipe;   // successor's pipeline-slot offset
 };
 
+// |A(s)| (S.nA, S.capped) of a state whose t, x, w, v and last are set; shared by the grid kernels and the
+// top-down engine (topdown.cu), whose states are not grid points.
+template <int KIND>
+__device__ __forceinline__ void feasible_actions(const DevModel& M, StateCtx& S) {
+    int nA = M.max_order_idx + 1;
+    S.capped = false;
+    if (KIND == SDPB_COST_CASH_XR) {
+        // CashConstraintXR.java:71-75
+        const double rv = S.w / S.v;
+        const double maxY = rv < S.x ? S.x : rv;
+        const int length = (int)(maxY - S.x) + 1;
+        S.capped = length > nA;  // dense-grid artefact: the reference has no cap (sdpb_reach reports it)
+        nA = length < nA ? length : nA;
+    } else {
+        if (M.flags & SDPB_F_CASH_LIMITED_ACTIONS) {
+            // CashConstraint.java:96-99, cashSurvival.java:103-110
+            const double bound = fmax(0.0, ((S.w - M.reserve_t[S.t - 1]) - M.reserve2) / S.v);
+            nA = (int)fmin((double)M.max_order_idx, bound) + 1;
+        }
+        if ((M.flags & SDPB_F_NO_ORDER_LAST) && S.last) nA = 1;
+    }
+    S.nA = nA;
+}
+
 // `dedup`: idx addresses a VIRTUAL state (y = x + preQ, [preQ2], [cash]) with preQ folded into the
 // inventory index — lead-time models depend on (x, preQ) only through their sum, so every real
 // state with the same sum has the same value and policy (exactly, not approximately).
@@ -76,26 +100,7 @@ __device__ __forceinline__ StateCtx decode_state(const DevModel& M, int t, long 
     S.lost = (M.flags & SDPB_F_LOST_SALES) != 0;
     S.gy = (KIND == SDPB_COST_BACKORDER) && (M.flags & SDPB_F_GY_MODE) && t == 1;
     S.strideX = (long long)M.nW * (M.lead >= 1 ? M.nQ : 1) * (M.lead >= 2 ? M.nQ : 1);
-
-    // feasible actions
-    int nA = M.max_order_idx + 1;
-    S.capped = false;
-    if (KIND == SDPB_COST_CASH_XR) {
-        // CashConstraintXR.java:71-75
-        const double rv = S.w / S.v;
-        const double maxY = rv < S.x ? S.x : rv;
-        const int length = (int)(maxY - S.x) + 1;
-        S.capped = length > nA;  // dense-grid artefact: the reference has no cap (sdpb_reach reports it)
-        nA = length < nA ? length : nA;
-    } else {
-        if (M.flags & SDPB_F_CASH_LIMITED_ACTIONS) {
-            // CashConstraint.java:96-99, cashSurvival.java:103-110
-            const double bound = fmax(0.0, ((S.w - M.reserve_t[t - 1]) - M.reserve2) / S.v);
-            nA = (int)fmin((double)M.max_order_idx, bound) + 1;
-        }
-        if ((M.flags & SDPB_F_NO_ORDER_LAST) && S.last) nA = 1;
-    }
-    S.nA = nA;
+    feasible_actions<KIND>(M, S);
     return S;
 }
 

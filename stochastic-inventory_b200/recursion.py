@@ -31,7 +31,7 @@ import numpy as np
 
 from . import _abi as A
 from .models import ModelSpec
-from .solver import Solver
+from .solver import Solver, TopDown
 
 
 class OptDirection(Enum):
@@ -133,15 +133,35 @@ class _Engine:
 
     def __init__(self, spec: ModelSpec, getFeasibleAction=None, stateTransition=None, immediateValue=None,
                  device: int = -1, kernel: int = A.KERNEL_AUTO, dedup: bool = False, spot_checks: int = 200,
-                 boundFinalCash=None, allow: int = 0, devices=None):
+                 boundFinalCash=None, allow: int = 0, devices=None, topdown: bool = False):
         """`boundFinalCash`: a FinalCash.BoundaryFuncton (src/sdp/inventory/FinalCash.java:16-18) -- a function of the
         state dimensions in API order, evaluated on numpy arrays over the whole grid (ModelSpec.tabulate) -- that
         values the states of period T+1 (CashRecursionV.java:125-128).  `allow`: sdpb_allow bits.  `devices`: a list
         of CUDA ordinals to partition the state grid over (sdpb_group_*); value queries work as usual, the visited-state
-        tables (getOptTable) need a single-GPU engine."""
+        tables (getOptTable) need a single-GPU engine.
+
+        `topdown=True`: no grid.  The engine solves exactly the states the reference's recursion visits from the
+        period-1 states asked for so far (sdpb_topdown_*), so states, steps and demands need not be multiples of a
+        power of two and an unclamped model needs no hull; getExpectedValue on a new period-1 state solves again with
+        that root added.  A later-period state that was not reached raises KeyError, as getAction on an unsolved
+        state does.  The lambdas are kept but not spot-checked against the descriptor (that check evaluates them on
+        the dense grid), and there is no boundary function (it is tabulated on the grid) and no multi-GPU split."""
         if spec.cost_kind not in self._kinds or spec.lead_time != self._lead:
             raise ValueError(f"{type(self).__name__} does not take this descriptor "
                              f"(cost_kind={spec.cost_kind}, lead_time={spec.lead_time})")
+        self._topdown = topdown
+        self._td = None
+        if topdown:
+            if boundFinalCash is not None or (devices is not None and len(devices) > 1):
+                raise ValueError("topdown=True takes no boundFinalCash and runs on one GPU")
+            self.spec, self.pmf = spec, spec.pmf
+            self.getFeasibleActions, self.stateTransition, self.immediateValue = (getFeasibleAction, stateTransition,
+                                                                                  immediateValue)
+            self.boundFinalCash = None
+            self._device, self._allow = device, allow
+            self._queried = []
+            self._tree_map = False
+            return
         if boundFinalCash is not None:
             import copy
             spec = copy.copy(spec)
@@ -187,11 +207,30 @@ class _Engine:
             self._solved = True
 
     def _value(self, state):
+        if self._topdown:
+            if self._td is None:
+                raise KeyError(f"{state} was not reached: no period-1 state has been solved (Recursion.java:165-167)")
+            try:
+                v, q = self._td.value(state.getPeriod(), [state._vec()])
+            except A.SdpbError as e:
+                if e.code == A.SDPB_ERR_UNSOLVED:
+                    raise KeyError(f"{state} was not reached from {self._queried} (Recursion.java:165-167)") from None
+                raise
+            return float(v[0]), float(q[0])
         self._ensure_solved()
         v, q = (self._group or self._solver).value(state.getPeriod(), [state._vec()])
         return float(v[0]), float(q[0])
 
     def getExpectedValue(self, state):
+        if self._topdown:
+            if state.getPeriod() == 1 and state._vec() not in self._queried:
+                td = TopDown(self.spec, self._queried + [state._vec()], device=self._device,
+                             allow=self._allow | self.spec.allow)
+                if self._td is not None:
+                    self._td.close()
+                self._td = td
+                self._queried.append(state._vec())
+            return self._value(state)[0]
         val, _ = self._value(state)
         if state.getPeriod() == 1 and state._vec() not in self._queried:
             self._queried.append(state._vec())
@@ -202,6 +241,8 @@ class _Engine:
         return val
 
     def getAction(self, state):
+        if self._topdown:
+            return self._value(state)[1]
         if not self._solved:
             # Java: cacheActions.get(state) is null -> NullPointerException on unboxing
             raise KeyError("getAction on a state that was never solved (Recursion.java:165-167)")
@@ -209,6 +250,8 @@ class _Engine:
 
     def getOptTable(self):
         """Rows [t, state dims..., Q*] for the visited states only (Recursion.java:177-186)."""
+        if self._topdown:
+            return self._td.opt_table() if self._td is not None else np.empty((0, self._ndim() + 2))
         if not self._queried:
             return np.empty((0, self._solver.ndim + 2))
         if self._group is not None:
@@ -226,7 +269,10 @@ class _Engine:
         return out
 
     def stats(self):
-        return self._solver.stats()
+        return self._td.stats() if self._topdown else self._solver.stats()
+
+    def _ndim(self):
+        return 1 + (self.spec.cost_kind != A.COST_BACKORDER) + self.spec.lead_time
 
     # -- descriptor <-> lambda validation --
     def _spot_check(self, n):

@@ -209,6 +209,87 @@ class Solver:
                 "exchange_ms": s.exchange_ms}
 
 
+class TopDown:
+    """One sdpb_topdown handle: `spec` solved over the states its top-down recursion reaches from the period-1 states
+    `init_states` ([n, ndim], API order).  Needs no grid: states, steps and demands need not be multiples of a power of
+    two, and an unclamped model needs no hull.  `scratch_bytes` bounds the forward expansion (0 = a fraction of free
+    device memory).  Release the device memory with close() (or use it as a context manager)."""
+
+    def __init__(self, spec: ModelSpec, init_states, device=None, allow=None, scratch_bytes: int = 0):
+        self.lib = A.load()
+        self.spec = spec
+        self._model = spec.to_struct()
+        self.ndim = 1 + (spec.cost_kind != A.COST_BACKORDER) + spec.lead_time
+        self.T = spec.T
+        st = np.ascontiguousarray(np.atleast_2d(np.asarray(init_states, dtype=np.float64)))
+        if st.shape[1] != self.ndim:
+            raise ValueError(f"initial states must have {self.ndim} columns")
+        opt = A.SdpbTopdownOptions()
+        opt.struct_size = C.sizeof(A.SdpbTopdownOptions)
+        opt.device = -1 if device is None else device
+        opt.allow = spec.allow if allow is None else allow
+        opt.scratch_bytes = scratch_bytes
+        h = C.c_void_p()
+        rc = self.lib.sdpb_topdown_solve(C.byref(self._model), C.byref(opt), st.ctypes.data_as(C.POINTER(C.c_double)),
+                                         st.shape[0], C.byref(h))
+        if rc != A.SDPB_OK:
+            raise A.SdpbError(rc, self.lib.sdpb_topdown_last_error(None).decode())
+        self.h = h
+
+    def _check(self, rc):
+        if rc != A.SDPB_OK:
+            raise A.SdpbError(rc, self.lib.sdpb_topdown_last_error(self.h).decode())
+
+    def close(self):
+        if getattr(self, "h", None):
+            self.lib.sdpb_topdown_destroy(self.h)
+            self.h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *a):
+        self.close()
+
+    def value(self, period: int, states):
+        """(V, Q) of reached API-order states [n, ndim] of one period; SDPB_ERR_UNSOLVED for a state not reached."""
+        st = np.ascontiguousarray(np.atleast_2d(np.asarray(states, dtype=np.float64)))
+        if st.shape[1] != self.ndim:
+            raise ValueError(f"states must have {self.ndim} columns")
+        n = st.shape[0]
+        v, q = np.empty(n), np.empty(n)
+        dp = C.POINTER(C.c_double)
+        self._check(self.lib.sdpb_topdown_value(self.h, period, st.ctypes.data_as(dp), n, v.ctypes.data_as(dp),
+                                                q.ctypes.data_as(dp)))
+        return v, q
+
+    def opt_table(self):
+        """[rows, ndim + 2]: (t, state..., Q*) of every reached state in memo-map order."""
+        n = C.c_size_t(0)
+        self._check(self.lib.sdpb_topdown_opt_table(self.h, None, C.byref(n)))
+        rows = np.empty((n.value, self.ndim + 2))
+        self._check(self.lib.sdpb_topdown_opt_table(self.h, rows.ctypes.data_as(C.POINTER(C.c_double)), C.byref(n)))
+        return rows
+
+    def n_states(self):
+        """Reached states of each period (T entries)."""
+        out = (C.c_int64 * self.T)()
+        self._check(self.lib.sdpb_topdown_states(self.h, out))
+        return list(out)
+
+    def stats(self):
+        s = A.SdpbStats()
+        self._check(self.lib.sdpb_topdown_stats(self.h, C.byref(s)))
+        return {"evals": s.evals, "solve_ms": s.solve_ms, "kernel_ms": s.kernel_ms, "launches": s.launches,
+                "capped_action_sets": s.capped_action_sets}
+
+
 class Group:
     """`n` shards of one model on the given CUDA devices of THIS process (sdpb_group_*): the grid is cut into
     contiguous blocks, every shard holds only the window of V_t it reads, and rows travel between the shards' tables
