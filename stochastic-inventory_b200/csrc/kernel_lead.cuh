@@ -567,7 +567,7 @@ struct Q2Args {
     long long lo, hi;
     long long f_begin, f_end; // flat thread range: f = (x * n_chunks + chunk) * nQ + preQ2
     int n_chunks, tpx;        // chunks of 8 levels along preQ1; threads per inventory row
-    int half;                 // bi_lead_q2m: ceil(nQ / 2), the distance between a thread's two preQ2 columns
+    int cs;                   // bi_lead_q2m: ceil(nQ / 3), the distance between a thread's preQ2 columns
     double* slice_v;          // bi_lead_q2m with the action range cut over gridDim.y: [slice][hi - lo] optima, merged by
     int* slice_a;             // merge_action_slices (which also stores the peers' rows)
     int di_max, NRW;
@@ -727,22 +727,31 @@ bi_lead_q2(const __grid_constant__ DevModel M, const __grid_constant__ Q2Args a)
 }
 
 // ---------------------------------------------------------------------------------------------
-// bi_lead_q2m -- bi_lead_q2 with the products p_j * (fv_a + L(level)) shared by the threads of a CTA.
+// bi_lead_q2m -- bi_lead_q2 with the products p_j * (fv_a + L(level)) shared by the threads of a CTA, and the demand loop
+// walked along level diagonals.
 //
 // The immediate value of (x, preQ1, preQ2) under action a and demand d_j does not depend on preQ2
 // (Leadtime.java:72-80: fixed + variable + holding/penalty of x + preQ1 - d_j), and the lanes of a warp ARE consecutive
 // preQ2 of one (x, chunk of 8 preQ1 levels): all of them form the identical product m = p_j * cst for each of their 8
-// slots.  Here a CTA tabulates, once per action, M[group][j][slot] = p_j * (fv_a + L(...)) for the few (x, chunk)
-// groups its threads belong to (4 on C4) with exactly the operations a thread used to do itself, and a thread then
-// reads its 8 products and spends (add, mul, add) per evaluation instead of (mul, add, mul, add) + 1/8.
-// A warp's LDS.128 returns 512 bytes however many lanes share an address -- four cycles of the SM's one shared-memory
-// pipe -- so with one preQ2 per thread the four product loads per demand step cost as much as the multiplies they
-// replace (measured: 138 vs 140 ms on C4).  A thread therefore owns TWO preQ2 columns (c and c + ceil(nQ/2): lanes stay
-// consecutive, every gather a coalesced row segment): 16 states, 48 fp64 instructions per demand step against five
-// shared-memory loads.  The running optimum of the 16 states lives in shared memory (read-compare-conditional-store
-// once per action), which is what lets 16 accumulators and two 10-entry successor windows fit in 128 registers.
-// The successor row offset of the window refill and p_j*gamma come from a second small table R[group][j], built once
-// per CTA.  One barrier per action (M is double-buffered).  Values are bit-identical: same operands, same order.
+// slots.  A CTA tabulates these products once per action for the few (x, chunk) groups its threads belong to (5 on C4)
+// with exactly the operations a thread used to do itself, and a thread reads them back and spends (add, mul, add) per
+// evaluation instead of (mul, add, mul, add) + 1/8.
+//
+// Demands are consecutive (d_j = d_0 + j), so slot k at demand j reads the successor level x + l0 + k - d_0 - j.  The
+// demand loop runs over diagonals n = j - k + 7 (n = 0 .. D + 6) instead of over j: on diagonal n every slot k that has
+// a demand j = n - 7 + k in [0, D) reads the SAME level u_n = x + l0 - d_0 - n + 7.  So per diagonal a thread gathers one
+// successor value per column, and reads the 8 products M[group][n][k] = p_{n-7+k} * (fv_a + L(u_n)) with four LDS.128;
+// p*gamma for slot k is p_{n-7+k}*gamma, a sliding window that all columns share.  The first 7 and the last 7 diagonals
+// have fewer active slots, known at compile time; demand supports shorter than 7 take a plain loop that tests each slot.
+// Each state still adds its terms for j = 0, 1, ..., D-1 in order with the same operands: values are bit-identical.
+//
+// Registers: 8*NC accumulators, an 8-entry p*gamma window and 2*NC prefetched successor values, so a thread owns THREE
+// preQ2 columns (c, c + cs, c + 2*cs with cs = ceil(nQ/3): lanes stay consecutive, every gather a coalesced row segment)
+// -- 24 states, 72 fp64 instructions per diagonal against 4 + 1 LDS.128 and 3 gathers.  The running optimum of the 24
+// states lives in shared memory (read-compare-conditional-store once per action; the action as 16 bits, since plan_q2
+// keeps nQ below 46341).  The per-diagonal refill (p*gamma entering the window, successor row offset two diagonals
+// ahead) comes from a second table R[group][n], built once per CTA.  M is single-buffered -- two barriers per action --
+// which keeps the tables of C4 at 45 KB, four CTAs per SM.
 template <int IMM>
 __device__ __forceinline__ double2 lds_double2_o(unsigned shared_addr) {
     double2 v;
@@ -750,46 +759,87 @@ __device__ __forceinline__ double2 lds_double2_o(unsigned shared_addr) {
     return v;
 }
 
-constexpr int kQ2mNC = 2;  // preQ2 columns per thread
+constexpr int kQ2mNC = 3;   // preQ2 columns per thread
+constexpr int kQ2mPW = kQ2YT;  // p*gamma window: one entry per slot
+constexpr unsigned short kQ2mNoAction = 0xffff;
 
-struct Q2mLayout { int NG; unsigned off_rg, off_gb, off_bv, off_ba, off_mt; size_t smem; };
+struct Q2mLayout { int NG; unsigned off_rg, off_gb, off_pz, off_bv, off_ba, off_mt; size_t smem; };
 
-__host__ __device__ inline Q2mLayout q2m_layout(int NRW, int D, int NT, int half) {
+__host__ __device__ inline Q2mLayout q2m_layout(int NRW, int D, int NT, int cs) {
     Q2mLayout L;
-    L.NG = (NT - 1) / half + 2;                                  // distinct (x, chunk) groups among NT consecutive threads
+    L.NG = (NT - 1) / cs + 2;                                    // distinct (x, chunk) groups among NT consecutive threads
+    const unsigned R = (unsigned)(D + kQ2YT - 1);                // diagonals per group
     unsigned o = (unsigned)(NRW + D) * 16u;                      // WR, PP
-    L.off_rg = o; o += (unsigned)(L.NG * D) * 16u;               // R[group][j] = (p_j*gamma, refill row offset)
-    L.off_gb = o; o += ((unsigned)L.NG * 4u + 15u) & ~15u;       // window base row of each group
+    L.off_rg = o; o += (unsigned)L.NG * R * 16u;                 // R[group][n] = (p_{n+1}*gamma, row offset of u_{n+2})
+    L.off_gb = o; o += ((unsigned)L.NG * 4u + 15u) & ~15u;       // window row of each group's level u_7
+    L.off_pz = o; o += ((R + kQ2YT - 1) * 8u + 15u) & ~15u;      // p_j for j = -7 .. D+6, zero outside [0, D)
     L.off_bv = o; o += (unsigned)(kQ2mNC * kQ2YT * NT) * 8u;     // running optimum per state: value ...
-    L.off_ba = o; o += (unsigned)(kQ2mNC * kQ2YT * NT) * 4u;     // ... and action
-    L.off_mt = o; o += 2u * (unsigned)(L.NG * D) * 64u;          // M[buffer][group][j][8]
+    L.off_ba = o; o += ((unsigned)(kQ2mNC * kQ2YT * NT) * 2u + 15u) & ~15u;  // ... and action
+    L.off_mt = o; o += (unsigned)L.NG * R * 64u;                 // M[group][n][8]
     L.smem = o;
     return L;
+}
+
+// Diagonal n of one action: slots [KLO, KHI) add their term, p*gamma of slot k in pw[(PH + k) % kQ2mPW], the successor
+// value of column c in vb[c][VS], the products at mt + IMM.
+template <bool LAST, int KLO, int KHI, int PH, int VS, int IMM>
+__device__ __forceinline__ void q2m_diag(double (&acc)[kQ2mNC][kQ2YT], unsigned mt, const double (&pw)[kQ2mPW],
+                                         const double (&vb)[kQ2mNC][2]) {
+    double mm[kQ2YT];
+    if (KLO < 2 && KHI > 0) { const double2 t = lds_double2_o<IMM>(mt); mm[0] = t.x; mm[1] = t.y; }
+    if (KLO < 4 && KHI > 2) { const double2 t = lds_double2_o<IMM + 16>(mt); mm[2] = t.x; mm[3] = t.y; }
+    if (KLO < 6 && KHI > 4) { const double2 t = lds_double2_o<IMM + 32>(mt); mm[4] = t.x; mm[5] = t.y; }
+    if (KLO < 8 && KHI > 6) { const double2 t = lds_double2_o<IMM + 48>(mt); mm[6] = t.x; mm[7] = t.y; }
+#pragma unroll
+    for (int k = KLO; k < KHI; k++)
+#pragma unroll
+        for (int c = 0; c < kQ2mNC; c++) {
+            acc[c][k] += mm[k];                                            // LeadtimeRecursion.java:59
+            if (!LAST) acc[c][k] += pw[(PH + k) % kQ2mPW] * vb[c][VS];    // LeadtimeRecursion.java:62
+        }
+}
+
+// After diagonal n: R[group][n] at rg + IMM gives p_{n+1}*gamma (into pw[PS]; PS < 0 drops it) and the successor row
+// of diagonal n + 2, whose values go to vb[.][VS].
+template <int VS, int PS, int IMM>
+__device__ __forceinline__ void q2m_refill(double (&pw)[kQ2mPW], double (&vb)[kQ2mNC][2], unsigned rg,
+                                           const double* const (&cb)[kQ2mNC]) {
+    const double2 r = lds_double2_o<IMM>(rg);
+    if (PS >= 0) pw[PS < 0 ? 0 : PS] = r.x;
+    const unsigned off = (unsigned)__double2loint(r.y);
+#pragma unroll
+    for (int c = 0; c < kQ2mNC; c++) vb[c][VS] = __ldg(cb[c] + off);
 }
 
 template <bool IS_MIN, bool LAST, int NT>
 __global__ void __launch_bounds__(NT, 512 / NT)
 bi_lead_q2m(const __grid_constant__ DevModel M, const __grid_constant__ Q2Args a) {
-    constexpr int YT = kQ2YT, PF = kQ2PF, W = YT + PF, PAD = kQ2PAD, NC = kQ2mNC;
-    static_assert(W == 10, "the demand loop below is written out for W = 10");
+    constexpr int YT = kQ2YT, PAD = kQ2PAD, NC = kQ2mNC, PW = kQ2mPW;
+    static_assert(YT == 8 && NC == 3 && PW == 8, "the diagonals below are written out for these sizes");
     static_assert(NT % 8 == 0, "the table builder keeps the slot index fixed per thread");
     extern __shared__ __align__(16) unsigned char smem_raw[];
-    const int D = a.D, nQ = M.nQ, half = a.half, tid = threadIdx.x;
-    const Q2mLayout L = q2m_layout(a.NRW, D, NT, half);
+    const int D = a.D, nQ = M.nQ, cs = a.cs, tid = threadIdx.x;
+    const int R = D + YT - 1;                            // diagonals
+    const Q2mLayout L = q2m_layout(a.NRW, D, NT, cs);
     double2* WR = reinterpret_cast<double2*>(smem_raw);  // (level cost, successor row offset in the low word)
     double2* PP = WR + a.NRW;                            // (p, p*gamma)
     double2* RG = reinterpret_cast<double2*>(smem_raw + L.off_rg);
     int* GB = reinterpret_cast<int*>(smem_raw + L.off_gb);
+    double* PZ = reinterpret_cast<double*>(smem_raw + L.off_pz);  // PZ[n + k] = p_{n-7+k}: slot k on diagonal n
     double* BV = reinterpret_cast<double*>(smem_raw + L.off_bv);
-    int* BA = reinterpret_cast<int*>(smem_raw + L.off_ba);
+    unsigned short* BA = reinterpret_cast<unsigned short*>(smem_raw + L.off_ba);
     double* MT = reinterpret_cast<double*>(smem_raw + L.off_mt);
     const int NG = L.NG;
     const long long F0 = a.f_begin + (long long)blockIdx.x * NT;
     const long long x_first = F0 / a.tpx;
-    const long long G0 = F0 / half;                      // first (x, chunk) group of the CTA: G = x * n_chunks + chunk
+    const long long G0 = F0 / cs;                        // first (x, chunk) group of the CTA: G = x * n_chunks + chunk
     const bool lost = (M.flags & SDPB_F_LOST_SALES) != 0;
 
     for (int j = tid; j < D; j += NT) PP[j] = make_double2(M.pmf_p[a.pmf_off + j], M.pmf_pg[a.pmf_off + j]);
+    for (int j = tid; j < R + YT - 1; j += NT) {
+        const int jd = j - (YT - 1);
+        PZ[j] = jd >= 0 && jd < D ? M.pmf_p[a.pmf_off + jd] : 0.0;
+    }
     for (int wi = tid; wi < a.NRW; wi += NT) {
         const long long il = x_first - a.di_max - PAD + wi;
         const double lvl = M.inv_min + (double)il * M.step;
@@ -800,7 +850,7 @@ bi_lead_q2m(const __grid_constant__ DevModel M, const __grid_constant__ Q2Args a
         WR[wi] = make_double2(M.h * fmax(lvl, 0.0) + M.pen * fmax(-lvl, 0.0),
                               __hiloint2double(0, (int)(is * nQ * nQ)));
     }
-    // window row of slot 0 at demand D-1 for each group
+    // window row of u_7 (slot 0 at demand D-1) for each group; diagonal n reads row GB + 7 - n
     for (int g = tid; g < NG; g += NT) {
         const long long G = G0 + g;
         const long long xg = G / a.n_chunks;
@@ -809,37 +859,33 @@ bi_lead_q2m(const __grid_constant__ DevModel M, const __grid_constant__ Q2Args a
         GB[g] = min(wb, a.NRW - YT);  // groups past the end of the range are built but never read
     }
 #pragma unroll
-    for (int s2 = 0; s2 < NC * YT; s2++) { BV[s2 * NT + tid] = IS_MIN ? DBL_MAX : -DBL_MAX; BA[s2 * NT + tid] = kNoAction; }
+    for (int s2 = 0; s2 < NC * YT; s2++) { BV[s2 * NT + tid] = IS_MIN ? DBL_MAX : -DBL_MAX; BA[s2 * NT + tid] = kQ2mNoAction; }
     __syncthreads();
-    for (int e = tid; e < NG * D; e += NT) {
-        const int g = e / D, j = e - g * D;
-        const double2 w = WR[GB[g] - (PF + 1) - j];      // the level slot 0 reaches PF + 1 demand steps after j
-        RG[e] = make_double2(PP[j].y, w.y);
+    for (int e = tid; e < NG * R; e += NT) {
+        const int g = e / R, n = e - g * R;
+        RG[e] = make_double2(n + 1 < D ? PP[n + 1].y : 0.0, WR[GB[g] + 5 - n].y);
     }
 
     const long long F = min(F0 + tid, a.f_end - 1);
     const long long x = F / a.tpx;
     const int f = (int)(F - x * a.tpx);
-    const int chunk = f / half, c0 = f - chunk * half, l0 = chunk * YT;
-    const int g_own = (int)(F / half - G0);
-    const bool has_b = c0 + half < nQ;                   // the second column: preQ2 = c0 + half
-    const long long idx0 = (x * nQ + l0) * nQ + c0;      // column 0, slot k: idx0 + k * nQ; column 1: + half
-    bool any = false;
-#pragma unroll
-    for (int k = 0; k < YT; k++) {
-        const long long i0 = idx0 + (long long)k * nQ;
-        any |= (l0 + k < nQ) && ((i0 >= a.lo && i0 < a.hi) || (has_b && i0 + half >= a.lo && i0 + half < a.hi));
-    }
-    any = any && F0 + tid < a.f_end;
+    const int chunk = f / cs, c0 = f - chunk * cs, l0 = chunk * YT;
+    const int g_own = (int)(F / cs - G0);
+    const long long idx0 = (x * nQ + l0) * nQ + c0;      // column c, slot k: idx0 + k * nQ + c * cs
+    // the thread's states span [idx0, idx_end]; one in [lo, hi) makes it compute (the stores below test each state)
+    const long long idx_end = idx0 + (long long)(min(YT, nQ - l0) - 1) * nQ + (long long)((nQ - 1 - c0) / cs) * cs;
+    const bool any = F0 + tid < a.f_end && idx_end >= a.lo && idx0 < a.hi;
 
-    const unsigned wr0 = (unsigned)__cvta_generic_to_shared(WR) + (unsigned)((int)(x - x_first) + l0 + (D - 1) + PAD) * 16u;
-    const unsigned rg0 = (unsigned)__cvta_generic_to_shared(RG) + (unsigned)(g_own * D) * 16u;
-    const unsigned mt0 = (unsigned)__cvta_generic_to_shared(MT) + (unsigned)(g_own * D) * 64u;
-    const unsigned mt_buf = (unsigned)(NG * D) * 64u;  // bytes between the two buffers
+    const unsigned wr_s = (unsigned)__cvta_generic_to_shared(WR);
+    const unsigned pp_s = (unsigned)__cvta_generic_to_shared(PP);
+    const unsigned rg0 = (unsigned)__cvta_generic_to_shared(RG) + (unsigned)(g_own * R) * 16u;
+    const unsigned mt0 = (unsigned)__cvta_generic_to_shared(MT) + (unsigned)(g_own * R) * 64u;
     const unsigned bv_s = (unsigned)__cvta_generic_to_shared(BV) + (unsigned)tid * 8u;
-    const unsigned ba_s = (unsigned)__cvta_generic_to_shared(BA) + (unsigned)tid * 4u;
-    const double* __restrict__ cb = LAST ? nullptr : a.VnT + c0;
-    const int colb = has_b ? half : 0;                   // a thread without a second column gathers the first one twice
+    const unsigned ba_s = (unsigned)__cvta_generic_to_shared(BA) + (unsigned)tid * 2u;
+    const int gb = (int)(x - x_first) + l0 + (D - 1) + PAD;  // this thread's window row of u_7
+    const double* cb[NC];  // the successor row of each column under action ai; a missing column gathers the first one
+#pragma unroll
+    for (int c = 0; c < NC; c++) cb[c] = LAST ? nullptr : a.VnT + c0 + (c0 + c * cs < nQ ? c * cs : 0);
     const double vt = M.v_t[a.t - 1];
 
     // the action range, cut over gridDim.y (separate CTAs, merged by merge_action_slices: small grids need more CTAs
@@ -847,102 +893,148 @@ bi_lead_q2m(const __grid_constant__ DevModel M, const __grid_constant__ Q2Args a
     const int n_sl = (int)gridDim.y, sl = (int)blockIdx.y;
     const int per_sl = (M.max_order_idx + n_sl) / n_sl;      // ceil(A / n_sl)
     const int ai_begin = sl * per_sl, ai_end = min(M.max_order_idx + 1, ai_begin + per_sl);
-    if (!LAST) cb += (long long)ai_begin * nQ;
-    // the builder's entries e = tid, tid + NT, ...: slot k = e & 7 is fixed, (group, demand) advance by NT / 8
-    const int k_b = tid & (YT - 1);
-    const int gj_b = tid >> 3;
-    // (the two `ai < ai_end` tests always hold; without them ptxas allocates registers differently and spills more)
-    for (int it = 0; it < ai_end - ai_begin; it++) {
-        const int ai = ai_begin + it;
-        const unsigned buf = (unsigned)(it & 1);
-        if (ai < ai_end) {  // ---- tabulate p_j * (fv_a + L) for the CTA's groups ----
+#pragma unroll
+    for (int c = 0; c < NC; c++) if (!LAST) cb[c] += (long long)ai_begin * nQ;
+    for (int ai = ai_begin; ai < ai_end; ai++) {
+        {  // ---- tabulate p_j * (fv_a + L(u_n)) for the CTA's groups, j = n - 7 + k: a thread per (group, diagonal) ----
             const double av = (double)ai * M.step;
             const double fv = (av > 0.0 ? M.K : 0.0) + vt * av;  // Leadtime.java:73-74,79
-            double* Mb = MT + (size_t)buf * NG * D * YT;
-            int g = gj_b / D, j = gj_b - g * D;
-            for (int e = tid; e < NG * D * YT; e += NT) {
-                const double cst = fv + WR[GB[g] + k_b - j].x;
-                Mb[e] = PP[j].x * cst;                           // LeadtimeRecursion.java:59
-                j += NT / YT;
-                while (j >= D) { j -= D; g++; }
+            for (int r = tid; r < NG * R; r += NT) {
+                const int g = r / R, n = r - g * R;
+                const double cst = fv + WR[GB[g] + (YT - 1) - n].x;
+                double2* Mr = reinterpret_cast<double2*>(MT + (size_t)r * YT);
+#pragma unroll
+                for (int k = 0; k < YT; k += 2)                   // LeadtimeRecursion.java:59
+                    Mr[k / 2] = make_double2(PZ[n + k] * cst, PZ[n + k + 1] * cst);
             }
         }
         __syncthreads();
-        if (ai < ai_end && any) {
-            double acc[NC][YT], Vw[NC][W];
+        if (any) {
+            double acc[NC][YT];
 #pragma unroll
-            for (int k = 0; k < YT; k++) { acc[0][k] = 0.0; acc[1][k] = 0.0; }
-            if (!LAST) {
+            for (int c = 0; c < NC; c++)
 #pragma unroll
-                for (int k = 0; k < W; k++) {  // entries YT..W-1: the levels slot 0 reaches at demands PF..1
-                    const double2 e = lds_double2(wr0 + (unsigned)((k < YT ? k : k - W) * 16));
-                    const double* src = cb + __double2loint(e.y);
-                    Vw[0][k] = __ldg(src);
-                    Vw[1][k] = __ldg(src + colb);
+                for (int k = 0; k < YT; k++) acc[c][k] = 0.0;
+            if (D >= YT - 1) {
+                double pw[PW], vb[NC][2];
+                if (!LAST) {  // p_0 * gamma, and the successor values of diagonals 0 and 1
+                    pw[0] = lds_double(pp_s + 8u);
+#pragma unroll
+                    for (int n = 0; n < 2; n++) {
+                        const unsigned off = (unsigned)__double2loint(lds_double(wr_s + (unsigned)(gb + 7 - n) * 16u + 8u));
+#pragma unroll
+                        for (int c = 0; c < NC; c++) vb[c][n] = __ldg(cb[c] + off);
+                    }
+                }
+#define SDPB_Q2M_HEAD(N)                                                                              \
+                q2m_diag<LAST, YT - 1 - (N), YT, (N) + 1, (N) & 1, (N) * 64>(acc, mt0, pw, vb);           \
+                if (!LAST) q2m_refill<(N) & 1, (N) + 1, (N) * 16>(pw, vb, rg0, cb);
+                SDPB_Q2M_HEAD(0) SDPB_Q2M_HEAD(1) SDPB_Q2M_HEAD(2) SDPB_Q2M_HEAD(3)
+                SDPB_Q2M_HEAD(4) SDPB_Q2M_HEAD(5) SDPB_Q2M_HEAD(6)
+#undef SDPB_Q2M_HEAD
+                // all slots active: diagonals 7 .. D-1, in blocks of PW that start at an odd n, so the window position
+                // of step U of a block is U and its successor values sit in vb[.][(U + 1) & 1]
+#define SDPB_Q2M_FULL(U)                                                                              \
+                q2m_diag<LAST, 0, YT, (U), ((U) + 1) & 1, (U) * 64>(acc, mt_run, pw, vb);                 \
+                if (!LAST) q2m_refill<((U) + 1) & 1, (U), (U) * 16>(pw, vb, rg_run, cb);
+                int n = YT - 1;
+                unsigned mt_run = mt0 + (unsigned)n * 64u, rg_run = rg0 + (unsigned)n * 16u;
+                for (; n + PW <= D; n += PW, mt_run += PW * 64u, rg_run += PW * 16u) {
+                    SDPB_Q2M_FULL(0) SDPB_Q2M_FULL(1) SDPB_Q2M_FULL(2) SDPB_Q2M_FULL(3) SDPB_Q2M_FULL(4)
+                    SDPB_Q2M_FULL(5) SDPB_Q2M_FULL(6) SDPB_Q2M_FULL(7)
+                }
+                if (n + 0 < D) { SDPB_Q2M_FULL(0) }
+                if (n + 1 < D) { SDPB_Q2M_FULL(1) }
+                if (n + 2 < D) { SDPB_Q2M_FULL(2) }
+                if (n + 3 < D) { SDPB_Q2M_FULL(3) }
+                if (n + 4 < D) { SDPB_Q2M_FULL(4) }
+                if (n + 5 < D) { SDPB_Q2M_FULL(5) }
+                if (n + 6 < D) { SDPB_Q2M_FULL(6) }
+                if (n + 7 < D) { SDPB_Q2M_FULL(7) }
+#undef SDPB_Q2M_FULL
+                // diagonals D .. D+6, slots k < 7 - e on diagonal D + e.  Where the window stands now depends on D, so
+                // p_{D-7..D-1} * gamma are read again, and the values of diagonals D and D+1 picked by the parity of D.
+                double pe[PW], ve[NC][2];
+                if (!LAST) {
+#pragma unroll
+                    for (int m = 0; m < YT - 1; m++) pe[m] = lds_double(pp_s + (unsigned)(D - (YT - 1) + m) * 16u + 8u);
+                    const bool odd = (D & 1) != 0;
+#pragma unroll
+                    for (int c = 0; c < NC; c++) {
+                        ve[c][0] = odd ? vb[c][1] : vb[c][0];
+                        ve[c][1] = odd ? vb[c][0] : vb[c][1];
+                    }
+                }
+                const unsigned mt_d = mt0 + (unsigned)D * 64u, rg_d = rg0 + (unsigned)D * 16u;
+#define SDPB_Q2M_TAIL(E)                                                                              \
+                q2m_diag<LAST, 0, YT - 1 - (E), (E), (E) & 1, (E) * 64>(acc, mt_d, pe, ve);               \
+                if (!LAST && (E) + 2 < YT - 1) q2m_refill<(E) & 1, -1, (E) * 16>(pe, ve, rg_d, cb);
+                SDPB_Q2M_TAIL(0) SDPB_Q2M_TAIL(1) SDPB_Q2M_TAIL(2) SDPB_Q2M_TAIL(3)
+                SDPB_Q2M_TAIL(4) SDPB_Q2M_TAIL(5) SDPB_Q2M_TAIL(6)
+#undef SDPB_Q2M_TAIL
+            } else {  // D < 7: every diagonal has both ends cut; test each slot
+                for (int n = 0; n < R; n++) {
+                    double mm[YT], v[NC];
+                    if (!LAST) {
+                        const unsigned off = (unsigned)__double2loint(lds_double(wr_s + (unsigned)(gb + 7 - n) * 16u + 8u));
+#pragma unroll
+                        for (int c = 0; c < NC; c++) v[c] = __ldg(cb[c] + off);
+                    }
+#pragma unroll
+                    for (int p = 0; p < YT / 2; p++) {
+                        const double2 t = lds_double2(mt0 + (unsigned)n * 64u + (unsigned)p * 16u);
+                        mm[2 * p] = t.x; mm[2 * p + 1] = t.y;
+                    }
+#pragma unroll
+                    for (int k = 0; k < YT; k++) {
+                        const int j = n - (YT - 1) + k;
+                        if (j < 0 || j >= D) continue;
+                        const double pg = LAST ? 0.0 : lds_double(pp_s + (unsigned)j * 16u + 8u);
+#pragma unroll
+                        for (int c = 0; c < NC; c++) {
+                            acc[c][k] += mm[k];                             // LeadtimeRecursion.java:59
+                            if (!LAST) acc[c][k] += pg * v[c];              // LeadtimeRecursion.java:62
+                        }
+                    }
                 }
             }
-            unsigned mt_run = mt0 + buf * mt_buf, rg_run = rg0;
-#define SDPB_Q2M_STEP(JJ)                                                                             \
-            {                                                                                             \
-                const double2 m01 = lds_double2_o<(JJ) * 64>(mt_run), m23 = lds_double2_o<(JJ) * 64 + 16>(mt_run); \
-                const double2 m45 = lds_double2_o<(JJ) * 64 + 32>(mt_run), m67 = lds_double2_o<(JJ) * 64 + 48>(mt_run); \
-                const double mm[YT] = {m01.x, m01.y, m23.x, m23.y, m45.x, m45.y, m67.x, m67.y};           \
-                if (LAST) {                                                                               \
-                    _Pragma("unroll") for (int k = 0; k < YT; k++) { acc[0][k] += mm[k]; acc[1][k] += mm[k]; } \
-                } else {                                                                                  \
-                    const double2 rg = lds_double2_o<(JJ) * 16>(rg_run);                                  \
-                    _Pragma("unroll") for (int k = 0; k < YT; k++) {                                      \
-                        acc[0][k] += mm[k];                               /* LeadtimeRecursion.java:59 */ \
-                        acc[0][k] += rg.x * Vw[0][(k - (JJ) + W) % W];    /* LeadtimeRecursion.java:62 */ \
-                        acc[1][k] += mm[k];                                                               \
-                        acc[1][k] += rg.x * Vw[1][(k - (JJ) + W) % W];                                    \
-                    }                                                                                     \
-                    const double* src = cb + __double2loint(rg.y);                                        \
-                    Vw[0][(YT - 1 - (JJ) + W) % W] = __ldg(src);                                          \
-                    Vw[1][(YT - 1 - (JJ) + W) % W] = __ldg(src + colb);                                   \
-                }                                                                                         \
-            }
-            int j = 0;
-            while (j + W <= D) {
-                SDPB_Q2M_STEP(0) SDPB_Q2M_STEP(1) SDPB_Q2M_STEP(2) SDPB_Q2M_STEP(3) SDPB_Q2M_STEP(4)
-                SDPB_Q2M_STEP(5) SDPB_Q2M_STEP(6) SDPB_Q2M_STEP(7) SDPB_Q2M_STEP(8) SDPB_Q2M_STEP(9)
-                j += W; mt_run += W * 64u; rg_run += W * 16u;
-            }
-            if (j + 0 < D) SDPB_Q2M_STEP(0)
-            if (j + 1 < D) SDPB_Q2M_STEP(1)
-            if (j + 2 < D) SDPB_Q2M_STEP(2)
-            if (j + 3 < D) SDPB_Q2M_STEP(3)
-            if (j + 4 < D) SDPB_Q2M_STEP(4)
-            if (j + 5 < D) SDPB_Q2M_STEP(5)
-            if (j + 6 < D) SDPB_Q2M_STEP(6)
-            if (j + 7 < D) SDPB_Q2M_STEP(7)
-            if (j + 8 < D) SDPB_Q2M_STEP(8)
-#undef SDPB_Q2M_STEP
             // running optimum: strictly better wins, so the first (lowest) optimal action stays (Recursion.java:146-157)
 #pragma unroll
-            for (int c2 = 0; c2 < NC; c2++)
+            for (int c = 0; c < NC; c++)
 #pragma unroll
                 for (int k = 0; k < YT; k++) {
-                    const unsigned so = (unsigned)((c2 * YT + k) * NT);
+                    const unsigned so = (unsigned)((c * YT + k) * NT);
                     const double bv = lds_double(bv_s + so * 8u);
-                    if (IS_MIN ? (acc[c2][k] < bv) : (acc[c2][k] > bv)) {
-                        asm volatile("st.shared.f64 [%0], %1;" ::"r"(bv_s + so * 8u), "d"(acc[c2][k]) : "memory");
-                        asm volatile("st.shared.s32 [%0], %1;" ::"r"(ba_s + so * 4u), "r"(ai) : "memory");
+                    if (IS_MIN ? (acc[c][k] < bv) : (acc[c][k] > bv)) {
+                        asm volatile("st.shared.f64 [%0], %1;" ::"r"(bv_s + so * 8u), "d"(acc[c][k]) : "memory");
+                        asm volatile("st.shared.u16 [%0], %1;" ::"r"(ba_s + so * 2u), "h"((unsigned short)ai) : "memory");
                     }
                 }
         }
-        if (!LAST) cb += nQ;
+        __syncthreads();  // M is rebuilt for the next action
+#pragma unroll
+        for (int c = 0; c < NC; c++) if (!LAST) cb[c] += nQ;
     }
     if (!any) return;
+    // the thread's states again, from a fresh read of its index: kept from above, they would stay live through the
+    // action loop and push its registers into local memory
+    unsigned ts;
+    asm volatile("mov.u32 %0, %%tid.x;" : "=r"(ts));
+    const long long Fs = min(F0 + (long long)ts, a.f_end - 1);
+    const long long xs = Fs / a.tpx;
+    const int fs = (int)(Fs - xs * a.tpx);
+    const int cks = fs / cs, c0s = fs - cks * cs, l0s = cks * YT;
+    const long long idx0s = (xs * nQ + l0s) * nQ + c0s;
 #pragma unroll
-    for (int c2 = 0; c2 < NC; c2++) {
-        if (c2 == 1 && !has_b) break;
+    for (int c = 0; c < NC; c++) {
+        if (c0s + c * cs >= nQ) break;
 #pragma unroll
         for (int k = 0; k < YT; k++) {
-            const long long idx = idx0 + (long long)k * nQ + (c2 ? half : 0);
-            if (!(l0 + k < nQ && idx >= a.lo && idx < a.hi)) continue;
-            const double best = BV[(c2 * YT + k) * NT + tid];
-            const int arg = BA[(c2 * YT + k) * NT + tid];
+            const long long idx = idx0s + (long long)k * nQ + c * cs;
+            if (!(l0s + k < nQ && idx >= a.lo && idx < a.hi)) continue;
+            const double best = BV[(c * YT + k) * NT + ts];
+            const unsigned short ba = BA[(c * YT + k) * NT + ts];
+            const int arg = ba == kQ2mNoAction ? kNoAction : (int)ba;
             if (n_sl > 1) {  // this CTA saw one slice of the actions only
                 a.slice_v[(long long)sl * (a.hi - a.lo) + (idx - a.lo)] = best;
                 a.slice_a[(long long)sl * (a.hi - a.lo) + (idx - a.lo)] = arg;
@@ -982,11 +1074,12 @@ inline Q2Plan plan_q2(const sdpb_model& m, const DevModel& d, int D, const int* 
 // [row0, row1): inventory rows of V_{t+1} the range [lo, hi) can read (sdpb_shard_reads); only those are transposed.
 constexpr int kQ2MaxPeers = 2;
 
-// How a launch over [lo, hi) is shaped.  bi_lead_q2m (shared products) whenever its tables leave four CTAs per SM, with
+// How a launch over [lo, hi) is shaped.  bi_lead_q2m (shared products) whenever its tables leave four CTAs per SM (at
+// most 56 KB each: an SM has 228 KB of shared memory and keeps 1 KB of it per CTA), with
 // the action range cut over separate CTAs (gridDim.y slices, merged by merge_action_slices -- the per-action product
 // table is then still built by a full CTA) when the grid is short of ~8 waves; else bi_lead_q2, with the action range cut
 // over 2 or 4 thread groups inside a CTA when the grid is short of ~6 waves.
-struct Q2Shape { bool shared; int parts, slices, half, tpx, NRW; long long f_begin, f_end; Q2mLayout L; };
+struct Q2Shape { bool shared; int parts, slices, cs, tpx, NRW; long long f_begin, f_end; Q2mLayout L; };
 
 inline Q2Shape q2_shape(const Q2Plan& P, const DevModel& dm, int D, long long lo, long long hi, int sm_count) {
     Q2Shape S{};
@@ -994,16 +1087,18 @@ inline Q2Shape q2_shape(const Q2Plan& P, const DevModel& dm, int D, long long lo
     const long long rows = (hi - 1) / per_x - lo / per_x + 1;
     const double waves = (double)(rows * P.tpx) / 32.0 / (16.0 * sm_count);
     S.parts = waves >= 6.0 ? 1 : (waves >= 3.0 ? 2 : 4);
-    S.half = (dm.nQ + 1) / 2;
-    const int tpx2 = P.n_chunks * S.half;
+    S.cs = (dm.nQ + kQ2mNC - 1) / kQ2mNC;
+    const int tpx2 = P.n_chunks * S.cs;
     const int NRW2 = P.n_chunks * kQ2YT + D + kQ2PAD + (P.NT + tpx2 - 1) / tpx2 + 1;
     S.slices = 1;
-    // bi_lead_q2m's threads are numbered over (x, chunk, column pair).  Measured on C4 (ms, bi_lead_q2m vs bi_lead_q2):
-    // whole grid 131.0 vs 140.3.  Shards: with the action range cut over thread groups INSIDE a CTA the per-action tables
+    // bi_lead_q2m's threads are numbered over (x, chunk, column triple).  Measured on C4 with two columns
+    // per thread (ms, bi_lead_q2m vs bi_lead_q2): whole grid 131.0 vs 140.3.  Shards: with the action range cut over thread groups INSIDE a CTA the per-action tables
     // and the barrier cost more than they save (a quarter of the grid 37.8 vs 36.7, an eighth 20.8 vs 18.7); cut over
     // SEPARATE CTAs they do not (34.1 and 17.7; 2 / 4 / 8 / 16 slices on the eighth: 18.4 / 17.5 / 17.7 / 18.0), so that
-    // is the shape every launch takes when the tables fit.
-    S.L = q2m_layout(NRW2, D, P.NT, S.half);
+    // is the shape every launch takes when the tables fit.  With three columns (B200, 1000 W): whole grid 117.5 ms with
+    // the 2 slices this rule gives it (an earlier build of the kernel: 121.0 sliced, 123.1 unsliced); slowest shard of
+    // 2 / 4 / 8: 61.2 / 31.6 / 16.6 ms.
+    S.L = q2m_layout(NRW2, D, P.NT, S.cs);
     // Test hooks, read once per process: they force shapes that small instances do not take by themselves.
     //   SDPB_Q2_SHARE=1      bi_lead_q2m with no action slices wherever its tables fit: the epilogue with peer stores
     //                        that large shards take
@@ -1044,7 +1139,7 @@ inline int launch_q2(const Q2Plan& P, const Q2Shape& S, const DevModel& dm, int 
     Q2Args a;
     a.t = t; a.D = D; a.pmf_off = pmf_off; a.VnT = last ? nullptr : VnT; a.Vt = Vt; a.Qt = Qt; a.lo = lo; a.hi = hi;
     a.n_chunks = P.n_chunks; a.tpx = S.tpx; a.di_max = P.di_max; a.NRW = S.NRW;
-    a.f_begin = S.f_begin; a.f_end = S.f_end; a.parts = S.parts; a.half = S.half;
+    a.f_begin = S.f_begin; a.f_end = S.f_end; a.parts = S.parts; a.cs = S.cs;
     a.slice_v = slice_v; a.slice_a = slice_a;
     a.n_peer = 0;
     for (int p = 0; p < kQ2MaxPeers; p++) { a.peer_v[p] = nullptr; a.peer_lo[p] = a.peer_hi[p] = 0; }
