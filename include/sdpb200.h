@@ -29,6 +29,8 @@
  *   the same at off-grid states, steps that are not powers of two, unclamped models without a hull
  *                                      (the memo maps of Recursion.java:89-163)     sdpb_topdown_solve +
  *                                                                                  sdpb_topdown_value / _opt_table
+ *   getExpectedValue(state) of any period on those memo maps                      sdpb_topdown_extend
+ *   Simulation over them, solving the states a path meets (Simulation.java:62)    sdpb_topdown_simulate
  *   the lambdas A, f, c                src/capacitated/CLSPTesting.java:78-106, src/leadtime/Leadtime.java:50-81,
  *                                      src/cash/singleItem/CashConstraint.java:95-133,
  *                                      src/cash/overdraft/CashOverdraft.java:72-118,
@@ -523,10 +525,12 @@ const char* sdpb_reached_last_error(void);
  * solve fails with SDPB_ERR_OFFGRID unless SDPB_ALLOW_CAPPED_ACTIONS is set (the rule sdpb_reach applies).
  * Refused with SDPB_ERR_ARG: SDPB_COST_CASH_TWO_PRODUCT and SDPB_COST_STAFF (their action pairs / pmf rows are tied to
  * the grid), and a non-NULL terminal_value (tabulated on the grid: it has no value at an off-grid state).
- * stats: evals = sum_t sum_{s reached} |A_t(s)| * D_t; solve_ms = time between CUDA events recorded on the engine's
- * stream at the start and the end of the solve -- the forward pass synchronises with the host after every chunk and
- * allocates as it goes, so this is close to the wall time of the solve, not kernel time alone; kernel_ms = the backward
- * pass, which is kernels only; launches = backward launches. */
+ * stats: evals = sum_t sum_{s reached} |A_t(s)| * D_t, evals_executed = evals and capped_action_sets accumulate over
+ * the life of the handle (a solve, then every extension).  solve_ms, kernel_ms and launches describe the most recent
+ * call only: for a solve or an extension, solve_ms = time between CUDA events recorded on the engine's stream at its
+ * start and end -- the forward pass synchronises with the host after every chunk and allocates as it goes, so this is
+ * close to the wall time of the call, not kernel time alone; kernel_ms = the backward pass (its kernels and the merges
+ * of new states into the tables); launches = backward launches.  For sdpb_topdown_simulate see there. */
 typedef struct sdpb_topdown_options {
     uint32_t struct_size;     /* = sizeof(sdpb_topdown_options) */
     int32_t  device;          /* CUDA ordinal; -1 = current device */
@@ -546,7 +550,8 @@ typedef struct sdpb_topdown sdpb_topdown;
 int  sdpb_topdown_solve(const sdpb_model* m, const sdpb_topdown_options* opt, const double* init_states, int n,
                         sdpb_topdown** out);
 void sdpb_topdown_destroy(sdpb_topdown* h);
-const char* sdpb_topdown_last_error(const sdpb_topdown* h);   /* h may be NULL: last sdpb_topdown_solve error */
+const char* sdpb_topdown_last_error(const sdpb_topdown* h);   /* h may be NULL: last sdpb_topdown_solve error, or the
+                                                                 error of a call given a NULL handle */
 /* getExpectedValue / getAction (Recursion.java:89-90,165-167): cacheValues / cacheActions of n reached states of one
  * period; SDPB_ERR_UNSOLVED for a state that was not reached (Java: NullPointerException).  v, q may be NULL. */
 int  sdpb_topdown_value(sdpb_topdown* h, int period, const double* states, int n, double* v, double* q);
@@ -555,6 +560,33 @@ int  sdpb_topdown_value(sdpb_topdown* h, int period, const double* states, int n
 int  sdpb_topdown_opt_table(sdpb_topdown* h, double* rows, size_t* nrows);
 int  sdpb_topdown_states(const sdpb_topdown* h, int64_t* n_states /* T: reached states of each period */);
 int  sdpb_topdown_stats(const sdpb_topdown* h, sdpb_stats* s);
+/* getExpectedValue(state) on n states of one period (1..T) of a solved handle: the memo maps grow by exactly the states
+ * the reference's recursion reaches from them (Recursion.java:89-163).  States already reached cost nothing, and each
+ * state is evaluated once over the life of the handle, so extending with roots r2 after a solve from r1 leaves the
+ * same states, values and evals as a solve from {r1, r2}.  Only the new states are expanded and solved; their values
+ * do not change those already held.  Fails with SDPB_ERR_ARG (period outside 1..T, n < 0, a coordinate that is not
+ * finite), SDPB_ERR_NOMEM (the scratch rule of sdpb_topdown_options, applied to the states new in a period) or
+ * SDPB_ERR_OFFGRID (a new XR state with a capped action set, unless SDPB_ALLOW_CAPPED_ACTIONS); a failed call leaves
+ * the reached states, tables and stats as they were.  n == 0 does nothing. */
+int  sdpb_topdown_extend(sdpb_topdown* h, int period, const double* states, int n);
+/* Simulation.simulateSDPGivenSamplNum / CashSimulation over the memo maps, with the reference's lazy
+ * getExpectedValue(state) at every step (Simulation.java:62-63): the loop and arguments of sdpb_simulate,
+ *     for each path i:  state = init;  sum = 0
+ *         for t = 1..T:  getExpectedValue(state);  Q = getAction(state);  d = Math.round(samples[i][t-1])
+ *                        sum += Math.pow(discount, t-1) * immediateValue(state, Q, d)
+ *                        state = stateTransition(state, Q, d)
+ *     values[i] = sum
+ * over real-valued states: no grid, and any rounded demand.  A path that meets a state the handle has not reached
+ * stops there; the stalled states become the roots of one extension (sdpb_topdown_extend, over several periods at
+ * once) and the stalled paths go on from where they stopped, at least one period further each round, so there are at
+ * most T rounds.  Partial sums stay in fp64 between rounds: each path's sum is the reference's bit for bit, and
+ * the handle ends up with the memo the reference's roll-out leaves.  The transition is applied whatever the cash (a
+ * survival model's path goes on after a bankrupt period).  SDPB_ERR_ARG: n < 1, a null pointer, a sample or initial
+ * coordinate that is not finite.  An extension that fails returns its error and leaves the handle as that extension
+ * found it (states added by earlier rounds stay).  stats: solve_ms = host wall time of the call, kernel_ms = the
+ * roll-out kernels' device time, launches = roll-out rounds; evals grows by the evaluations of the added states. */
+int  sdpb_topdown_simulate(sdpb_topdown* h, const double* init_state, const double* samples, int n, double discount,
+                           double* values);
 
 /* Return the memory cached by the library's private stream-ordered pool on `device` to the driver (-1 = current). */
 int sdpb_trim_pool(int device);

@@ -447,6 +447,30 @@ class TopDown {
         return (size_t)n.at((size_t)period - 1);
     }
     sdpb_stats stats() const { sdpb_stats s; check(sdpb_topdown_stats(h_, &s)); return s; }
+    // getExpectedValue on API-order states of one period: solves only what no earlier call reached; a failure leaves
+    // the handle as it was
+    void extend(int period, const std::vector<std::vector<double>>& states) {
+        std::vector<double> flat;
+        for (const auto& r : states) {
+            if (r.size() != ndim_plus2() - 2) throw SdpbError(SDPB_ERR_ARG, "state has the wrong number of components");
+            flat.insert(flat.end(), r.begin(), r.end());
+        }
+        check(sdpb_topdown_extend(h_, period, flat.data(), (int)states.size()));
+    }
+    // Simulation.java:59-70 over demand sample paths (one row of T samples per path) -> per-path sums; every state a
+    // path meets that was not reached is solved on the way and stays in the handle
+    std::vector<double> simulate(const std::vector<double>& initState, const std::vector<std::vector<double>>& samples,
+                                 double discount = 1.0) {
+        if (initState.size() != ndim_plus2() - 2) throw SdpbError(SDPB_ERR_ARG, "state has the wrong number of components");
+        std::vector<double> flat;
+        for (const auto& r : samples) {
+            if (r.size() != (size_t)model_.m.T) throw SdpbError(SDPB_ERR_ARG, "a sample path must have T demands");
+            flat.insert(flat.end(), r.begin(), r.end());
+        }
+        std::vector<double> values(samples.size());
+        check(sdpb_topdown_simulate(h_, initState.data(), flat.data(), (int)samples.size(), discount, values.data()));
+        return values;
+    }
 
  private:
     size_t ndim_plus2() const { return 3 + (model_.m.cost_kind != SDPB_COST_BACKORDER ? 1 : 0) + (size_t)model_.m.lead_time; }
@@ -458,20 +482,19 @@ class TopDown {
 };
 
 // Recursion / LeadtimeRecursion / CashRecursion / RiskRecursion access over TopDown, with states given as API-order
-// vectors: getExpectedValue on a new period-1 state solves again with that root added (the memo maps grow the same
-// way); getAction / getExpectedValue of a later-period state that was not reached throws SDPB_ERR_UNSOLVED.
+// vectors: getExpectedValue on a new period-1 state extends the solve with that root (the memo maps grow the same way;
+// states a roll-out over engine() added stay); getAction / getExpectedValue of a later-period state that was not
+// reached throws SDPB_ERR_UNSOLVED.
 class TopDownRecursion {
  public:
     explicit TopDownRecursion(const Model& model, int device = -1, uint32_t allow = 0)
         : model_(model), device_(device), allow_(allow) {}
     double getExpectedValue(int period, const std::vector<double>& st) {
         if (period == 1 && std::find(roots_.begin(), roots_.end(), st) == roots_.end()) {
-            // solve with the new root first: if that throws, the roots and the previous solve stay as they were
-            std::vector<std::vector<double>> roots = roots_;
-            roots.push_back(st);
-            std::unique_ptr<TopDown> td(new TopDown(model_, roots, device_, allow_));
-            roots_.swap(roots);
-            td_.swap(td);
+            // if this throws, the roots and the solve stay as they were
+            if (td_) td_->extend(1, {st});
+            else td_.reset(new TopDown(model_, {st}, device_, allow_));
+            roots_.push_back(st);
         }
         return engine().value(period, st);
     }

@@ -125,7 +125,8 @@ EXPORTS = [
     "sdpb_group_last_error", "sdpb_group_solve", "sdpb_group_shard", "sdpb_group_value", "sdpb_group_period_tables",
     "sdpb_group_stats", "sdpb_solve_batch", "sdpb_trim_pool", "sdpb_reached_solve", "sdpb_reached_last_error",
     "sdpb_topdown_solve", "sdpb_topdown_destroy", "sdpb_topdown_last_error", "sdpb_topdown_value",
-    "sdpb_topdown_opt_table", "sdpb_topdown_states", "sdpb_topdown_stats",
+    "sdpb_topdown_opt_table", "sdpb_topdown_states", "sdpb_topdown_stats", "sdpb_topdown_extend",
+    "sdpb_topdown_simulate",
 ]
 
 _lib = None
@@ -215,6 +216,8 @@ def load():
     lib.sdpb_topdown_opt_table.argtypes = [vp, _dp, C.POINTER(C.c_size_t)]
     lib.sdpb_topdown_states.argtypes = [vp, C.POINTER(C.c_int64)]
     lib.sdpb_topdown_stats.argtypes = [vp, C.POINTER(SdpbStats)]
+    lib.sdpb_topdown_extend.argtypes = [vp, C.c_int, _dp, C.c_int]
+    lib.sdpb_topdown_simulate.argtypes = [vp, _dp, _dp, C.c_int, C.c_double, _dp]
     if (lib.sdpb_sizeof_model() != C.sizeof(SdpbModel) or lib.sdpb_sizeof_options() != C.sizeof(SdpbOptions)
             or lib.sdpb_sizeof_grid() != C.sizeof(SdpbGrid) or lib.sdpb_sizeof_stats() != C.sizeof(SdpbStats)
             or lib.sdpb_abi_version() != ABI_VERSION):

@@ -13,6 +13,12 @@
 // stored as +0.0).  Each coordinate is stored as an order-preserving 64-bit integer, the active coordinates packed
 // first, so that a radix sort orders the keys as the reference's memo map does (t, x, q1, q2, w).
 //
+// A solved handle grows: getExpectedValue on states of any period (td_extend) expands only the states no earlier call
+// reached, N_t = (successors of N_{t-1} u roots of t) \ F_t, solves them against the merged F_{t+1}, and merges
+// (N_t, V, Q) into (F_t, V_t, Q_t) by key; V depends on the state alone, so nothing held changes.  A fresh solve is
+// the extension of an empty handle with period-1 roots.  The policy roll-out (td_simulate) runs on the same tables and
+// extends them with the states its paths meet, as the reference's getExpectedValue at every step does.
+//
 // The candidates of one period can be far more than memory holds (a cash model with ~1e6 states per period, 201
 // actions and 200 demand points has 4e10), so the (state, feasible action) pairs are expanded in chunks bounded by the
 // scratch budget; each chunk is compacted, sorted and uniqued, then merged into the running frontier.
@@ -25,11 +31,15 @@
 #include <thrust/execution_policy.h>
 #include <thrust/merge.h>
 #include <thrust/remove.h>
+#include <thrust/iterator/zip_iterator.h>
 #include <thrust/scan.h>
+#include <thrust/set_operations.h>
+#include <thrust/tuple.h>
 #include <thrust/unique.h>
 
 #include <algorithm>
 #include <cfloat>
+#include <chrono>
 #include <cmath>
 #include <cstdint>
 #include <cstring>
@@ -341,6 +351,55 @@ __global__ void td_query(const TDKey* __restrict__ F, const long long n, const d
     qi[i] = hit ? Q[at] : -2;
 }
 
+// One thread per path of act[0, na): Simulation.java:59-70 from where the path stands (period per[i], state key[i],
+// partial sum sum[i]) -- Q = getAction(state), d = Math.round(sample), sum += discount^(t-1) c, state = f(s, Q, d) --
+// until it ends (values[i] = sum) or meets a state the handle has not reached.  There it writes (path, t, state) to
+// the next slot of the stall list, keeps its period, state and partial sum, and stops; the host extends the handle
+// with the stalled states and relaunches the stalled paths.  f is applied whatever the cash: a survival model's
+// roll-out goes on after a bankrupt period, as the reference's does.
+template <int KIND>
+__global__ void __launch_bounds__(128) td_simulate(const __grid_constant__ TDModel P, const TDKey* const* __restrict__ tF,
+                                                   const int* const* __restrict__ tQ, const long long* __restrict__ tn,
+                                                   const double* __restrict__ samples, const double* __restrict__ pw,
+                                                   const int* __restrict__ act, const int na, TDKey* __restrict__ key,
+                                                   int* __restrict__ per, double* __restrict__ sum,
+                                                   double* __restrict__ values, int* __restrict__ stall_n,
+                                                   int* __restrict__ stall_path, int* __restrict__ stall_t,
+                                                   TDKey* __restrict__ stall_key) {
+    const int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= na) return;
+    const int i = act[k], T = P.M.T;
+    TDKey s = key[i];
+    double acc = sum[i];
+    for (int t = per[i]; t <= T; t++) {
+        const TDKey* __restrict__ F = tF[t - 1];
+        const long long n = tn[t - 1];
+        const long long at = td_lower(F, 0, n, s);
+        if (at >= n || !TDEq()(F[at], s)) {
+            key[i] = s;
+            per[i] = t;
+            sum[i] = acc;
+            const int slot = atomicAdd(stall_n, 1);
+            stall_path[slot] = i;
+            stall_t[slot] = t;
+            stall_key[slot] = s;
+            return;
+        }
+        int qi = tQ[t - 1][at];
+        if (qi < 0) qi = 0;  // bestOrderQty stayed 0
+        double q2;
+        const StateCtx S = td_state<KIND>(P, t, s, q2);
+        const ActionCtx A = prep_action<KIND>(P.M, S, qi);
+        const double d = (double)jround(samples[(size_t)i * T + (t - 1)]);  // Math.round(samples[i][t])
+        double after;
+        const double c = immediate<KIND>(P.M, S, A, d, after);
+        acc += pw[t - 1] * c;
+        bool bankrupt;
+        if (t < T) s = td_next<KIND>(P, S, q2, A, d, c, after, bankrupt);
+    }
+    values[i] = acc;
+}
+
 bool has_cash(const sdpb_model& m) { return m.cost_kind != SDPB_COST_BACKORDER; }
 
 thread_local std::string g_td_error;
@@ -397,40 +456,44 @@ cudaError_t td_sort_nd(int nd, void* tmp, size_t& tmp_bytes, cub::DoubleBuffer<T
 }
 
 template <int KIND>
-void launch_count(const sdpb_topdown* h, int t, long long* nA, unsigned long long* capped) {
-    const long long n = h->nF[t - 1];
-    if (n == 0) return;  // every successor of the previous period was bankrupt (survival recursion)
-    td_count_actions<KIND><<<(unsigned)((n + 255) / 256), 256, 0, h->stream>>>(h->P, t, h->F[t - 1], n, nA, capped);
+void launch_count(const sdpb_topdown* h, int t, const TDKey* F, long long n, long long* nA, unsigned long long* capped) {
+    if (n == 0) return;
+    td_count_actions<KIND><<<(unsigned)((n + 255) / 256), 256, 0, h->stream>>>(h->P, t, F, n, nA, capped);
 }
 template <int KIND>
-void launch_expand(const sdpb_topdown* h, int t, const long long* off, long long p0, long long np, TDKey* out) {
+void launch_expand(const sdpb_topdown* h, int t, const TDKey* F, long long n, const long long* off, long long p0,
+                   long long np, TDKey* out) {
     const int D = h->pmf_len[t - 1], po = h->pmf_off[t - 1];
     const unsigned blocks = (unsigned)((np + 255) / 256);
     if (h->m.recursion == SDPB_REC_SURVIVAL)
-        td_expand<KIND, true><<<blocks, 256, 0, h->stream>>>(h->P, t, D, po, h->F[t - 1], h->nF[t - 1], off, p0, np, out);
+        td_expand<KIND, true><<<blocks, 256, 0, h->stream>>>(h->P, t, D, po, F, n, off, p0, np, out);
     else
-        td_expand<KIND, false><<<blocks, 256, 0, h->stream>>>(h->P, t, D, po, h->F[t - 1], h->nF[t - 1], off, p0, np, out);
+        td_expand<KIND, false><<<blocks, 256, 0, h->stream>>>(h->P, t, D, po, F, n, off, p0, np, out);
 }
+// V, Q of the n states F of period t, against the sorted (Fn, Vn) of period t + 1 (nn states; none when t == T)
 template <int KIND>
-void launch_backward(const sdpb_topdown* h, int t) {
-    const long long n = h->nF[t - 1];
-    const int T = h->m.T, D = h->pmf_len[t - 1], po = h->pmf_off[t - 1];
-    const TDKey* Fn = t < T ? h->F[t] : nullptr;
-    const double* Vn = t < T ? h->V[t] : nullptr;
-    const long long nn = t < T ? h->nF[t] : 0;
-    if (n == 0) return;  // nothing reached in this period (survival recursion: every path went bankrupt before)
+void launch_backward(const sdpb_topdown* h, int t, const TDKey* F, long long n, const TDKey* Fn, const double* Vn,
+                     long long nn, double* V, int* Q) {
+    const int D = h->pmf_len[t - 1], po = h->pmf_off[t - 1];
+    if (n == 0) return;
     const unsigned blocks = (unsigned)((n + 7) / 8);
     if (h->m.recursion == SDPB_REC_SURVIVAL) {
         if constexpr (KIND == SDPB_COST_CASH_DEPOSIT || KIND == SDPB_COST_CASH_OVERDRAFT)
-            td_backward<KIND, true, false><<<blocks, 256, 0, h->stream>>>(h->P, t, D, po, h->F[t - 1], n, Fn, Vn, nn,
-                                                                        h->V[t - 1], h->Q[t - 1]);
+            td_backward<KIND, true, false><<<blocks, 256, 0, h->stream>>>(h->P, t, D, po, F, n, Fn, Vn, nn, V, Q);
     } else if (h->m.direction == SDPB_MIN) {
-        td_backward<KIND, false, true><<<blocks, 256, 0, h->stream>>>(h->P, t, D, po, h->F[t - 1], n, Fn, Vn, nn,
-                                                                    h->V[t - 1], h->Q[t - 1]);
+        td_backward<KIND, false, true><<<blocks, 256, 0, h->stream>>>(h->P, t, D, po, F, n, Fn, Vn, nn, V, Q);
     } else {
-        td_backward<KIND, false, false><<<blocks, 256, 0, h->stream>>>(h->P, t, D, po, h->F[t - 1], n, Fn, Vn, nn,
-                                                                     h->V[t - 1], h->Q[t - 1]);
+        td_backward<KIND, false, false><<<blocks, 256, 0, h->stream>>>(h->P, t, D, po, F, n, Fn, Vn, nn, V, Q);
     }
+}
+template <int KIND>
+void launch_simulate(const sdpb_topdown* h, const TDKey* const* tF, const int* const* tQ, const long long* tn,
+                     const double* samples, const double* pw,
+                     const int* act, int na, TDKey* key, int* per, double* sum, double* values, int* stall_n,
+                     int* stall_path, int* stall_t, TDKey* stall_key) {
+    td_simulate<KIND><<<(na + 127) / 128, 128, 0, h->stream>>>(h->P, tF, tQ, tn, samples, pw, act, na, key, per, sum,
+                                                               values,
+                                                               stall_n, stall_path, stall_t, stall_key);
 }
 
 #define TD_DISPATCH(fn, ...)                                                                  \
@@ -454,26 +517,155 @@ struct DevBuf {  // a scratch allocation released when it goes out of scope
     }
 };
 
-// The forward pass: F_2 .. F_T from F_1, and the evaluation count.
-int td_forward(sdpb_topdown* h) {
-    const int T = h->m.T, nd = h->P.nd();
+template <class P>
+bool td_alloc(P*& p, long long n) {
+    if (cudaMalloc((void**)&p, (size_t)std::max(n, 1ll) * sizeof(P)) == cudaSuccess) return true;
+    cudaGetLastError();
+    p = nullptr;
+    return false;
+}
+
+// What one extension builds, owned here until it is committed to the handle: per period the new states N_t with their
+// V / Q, and the merged tables F_t u N_t.  Whatever is still owned when the stage goes out of scope is freed, so an
+// extension that fails leaves the handle as it found it.
+struct TDStage {
+    std::vector<TDKey*> N, MF;
+    std::vector<double*> VN, MV;
+    std::vector<int*> QN, MQ;
+    std::vector<long long> nN, nM;
+    explicit TDStage(int T)
+        : N(T, nullptr), MF(T, nullptr), VN(T, nullptr), MV(T, nullptr), QN(T, nullptr), MQ(T, nullptr), nN(T, 0),
+          nM(T, 0) {}
+    ~TDStage() {
+        for (size_t k = 0; k < N.size(); k++) {
+            cudaFree(N[k]); cudaFree(MF[k]); cudaFree(VN[k]); cudaFree(MV[k]); cudaFree(QN[k]); cudaFree(MQ[k]);
+        }
+    }
+};
+
+// N_t: the roots of period t and the successors of the n_src states `src` of period t - 1 (`off`: their action offsets,
+// `pairs` (state, action) pairs), minus the states the handle already holds in period t; sorted, into *out.
+//
+// Scratch: three key buffers of `cap` keys (chunk candidates, sort output, merge output / new states) and the radix
+// sort's temporary storage, together at most `budget` bytes.  A chunk must hold at least as many candidates as the
+// period has new states so far (cap - nf >= nf), so the merges of a period cost at most twice its sorted candidates; a
+// period whose new states pass half a buffer fails with SDPB_ERR_NOMEM instead of crawling on.
+int td_new_states(sdpb_topdown* h, int t, const TDKey* src, long long n_src, const long long* off, long long pairs,
+                  const std::vector<TDKey>& roots, TDKey** out, long long* n_out) {
+    *out = nullptr;
+    *n_out = 0;
+    const long long nr = (long long)roots.size();
+    if (pairs == 0 && nr == 0) return SDPB_OK;
+    const int nd = h->P.nd(), D = t > 1 ? h->pmf_len[t - 2] : 1;
+    const TDKey* Fo = h->F[t - 1];
+    const long long no = h->nF[t - 1];
     cudaStream_t st = h->stream;
     auto par = thrust::cuda::par.on(st);
-    double capped_total = 0, evals = 0;
-    DevBuf cap_b;
+    const long long cand = pairs * D + nr, key3 = 3 * (long long)sizeof(TDKey);
+    const std::string per = "period " + std::to_string(t);
+    size_t free_b = 0, total_b = 0;
+    cudaMemGetInfo(&free_b, &total_b);
+    const long long budget = h->scratch_bytes > 0 ? h->scratch_bytes : (long long)(free_b / 2);
+    auto sort_temp = [&](long long items, size_t& bytes) {
+        cub::DoubleBuffer<TDKey> probe(nullptr, nullptr);
+        return td_sort_nd(nd, nullptr, bytes, probe, items, st) == cudaSuccess;
+    };
+    long long cap = std::max(1ll, std::min(cand, budget / key3));
+    size_t tmp_bytes = 0;
+    if (!sort_temp(cap, tmp_bytes)) return td_fail(h, SDPB_ERR_CUDA, "sizing the sort");
+    if (cap * key3 + (long long)tmp_bytes > budget) {  // the temporary storage shrinks with the item count
+        cap = (budget - (long long)tmp_bytes) / key3;
+        if (cap < 1 || !sort_temp(cap, tmp_bytes) || cap * key3 + (long long)tmp_bytes > budget)
+            return td_fail(h, SDPB_ERR_NOMEM, per + ": a scratch budget of " + std::to_string(budget) +
+                                                  " bytes does not hold the sort's temporary storage");
+    }
+    auto too_many = [&](long long nf) {
+        return td_fail(h, SDPB_ERR_NOMEM,
+                       per + " reaches at least " + std::to_string(nf) + " new states: more than a scratch budget of " +
+                           std::to_string(budget) + " bytes (" + std::to_string(cap) +
+                           " keys per buffer, at most half of them new states) can expand");
+    };
+    if (nr > cap) return too_many(nr);
+    DevBuf kb[3], tmp_b;
+    for (auto& b : kb)
+        if (!b.alloc((size_t)cap * sizeof(TDKey)))
+            return td_fail(h, SDPB_ERR_NOMEM, "allocation of the expansion scratch failed (" + per + ")");
+    if (!tmp_b.alloc(tmp_bytes)) return td_fail(h, SDPB_ERR_NOMEM, "allocation of the sort scratch failed (" + per + ")");
+    TDKey* front = (TDKey*)kb[0].p;
+    TDKey* x = (TDKey*)kb[1].p;
+    TDKey* y = (TDKey*)kb[2].p;
+    long long nf = 0;
+    try {
+        if (nr > 0) {  // the roots (sorted and unique) that period t does not hold yet
+            if (cudaMemcpyAsync(y, roots.data(), (size_t)nr * sizeof(TDKey), cudaMemcpyHostToDevice, st) != cudaSuccess)
+                return td_fail(h, SDPB_ERR_CUDA, "cudaMemcpyAsync failed");
+            nf = thrust::set_difference(par, y, y + nr, Fo, Fo + no, front, TDLess()) - front;
+        }
+        for (long long p = 0; p < pairs;) {
+            const long long room = cap - nf;
+            const long long np = std::min(pairs - p, room / D);
+            if (np < 1 || nf > room) return too_many(nf);
+            TD_DISPATCH(launch_expand, h, t - 1, src, n_src, off, p, np, x)
+            if (cudaGetLastError() != cudaSuccess) return td_fail(h, SDPB_ERR_CUDA, "td_expand launch failed");
+            long long m = thrust::remove_if(par, x, x + np * D, TDIsHole()) - x;
+            cub::DoubleBuffer<TDKey> db(x, y);
+            size_t tb = tmp_bytes;
+            if (td_sort_nd(nd, tmp_b.p, tb, db, m, st) != cudaSuccess) return td_fail(h, SDPB_ERR_CUDA, "radix sort failed");
+            TDKey* cur = db.Current();
+            TDKey* alt = db.Alternate();
+            m = thrust::unique(par, cur, cur + m, TDEq()) - cur;
+            thrust::merge(par, front, front + nf, cur, cur + m, alt, TDLess());
+            const long long nm = thrust::unique(par, alt, alt + nf + m, TDEq()) - alt;
+            TDKey* old = front;
+            if (no > 0) {  // keep only what period t does not hold yet
+                nf = thrust::set_difference(par, alt, alt + nm, Fo, Fo + no, cur, TDLess()) - cur;
+                front = cur;
+                y = alt;
+            } else {
+                nf = nm;
+                front = alt;
+                y = cur;
+            }
+            x = old;
+            p += np;
+        }
+    } catch (const std::exception& ex) {
+        return td_fail(h, SDPB_ERR_CUDA, std::string("sort / merge: ") + ex.what());
+    }
+    if (nf == 0) return cudaStreamSynchronize(st) == cudaSuccess ? SDPB_OK : td_fail(h, SDPB_ERR_CUDA, "forward pass");
+    if (!td_alloc(*out, nf)) return td_fail(h, SDPB_ERR_NOMEM, "allocation of the states of " + per + " failed");
+    *n_out = nf;
+    if (cudaMemcpyAsync(*out, front, (size_t)nf * sizeof(TDKey), cudaMemcpyDeviceToDevice, st) != cudaSuccess ||
+        cudaStreamSynchronize(st) != cudaSuccess)
+        return td_fail(h, SDPB_ERR_CUDA, std::string("forward pass: ") + cudaGetErrorString(cudaGetLastError()));
+    return SDPB_OK;
+}
+
+// The forward pass of an extension from period p: N_t for t = p .. T into the stage, and the evaluations and capped XR
+// action sets of the new states.
+int td_forward(sdpb_topdown* h, int p, const std::vector<std::vector<TDKey>>& roots, TDStage& sg, double& evals,
+               double& capped_total) {
+    const int T = h->m.T;
+    cudaStream_t st = h->stream;
+    auto par = thrust::cuda::par.on(st);
+    DevBuf cap_b, off_b;  // off_b: exclusive prefix sum of |A_t(s)| over N_t (n + 1 entries)
     if (!cap_b.alloc(sizeof(unsigned long long))) return td_fail(h, SDPB_ERR_NOMEM, "allocation failed");
     unsigned long long* d_capped = (unsigned long long*)cap_b.p;
-    for (int t = 1; t <= T; t++) {
-        const long long n = h->nF[t - 1];
-        const int D = h->pmf_len[t - 1];
-        DevBuf off_b;
+    long long pairs = 0;
+    for (int t = p; t <= T; t++) {
+        const int k = t - 1;
+        const int rc = td_new_states(h, t, t > p ? sg.N[k - 1] : nullptr, t > p ? sg.nN[k - 1] : 0,
+                                     (const long long*)off_b.p, pairs, roots[k], &sg.N[k], &sg.nN[k]);
+        if (rc != SDPB_OK) return rc;
+        const long long n = sg.nN[k];
+        pairs = 0;
+        if (n == 0) continue;
         if (!off_b.alloc((size_t)(n + 1) * sizeof(long long))) return td_fail(h, SDPB_ERR_NOMEM, "allocation of the action counts failed");
         long long* off = (long long*)off_b.p;
         if (cudaMemsetAsync(off, 0, sizeof(long long), st) != cudaSuccess ||
             cudaMemsetAsync(d_capped, 0, sizeof(unsigned long long), st) != cudaSuccess)
             return td_fail(h, SDPB_ERR_CUDA, "cudaMemsetAsync failed");
-        TD_DISPATCH(launch_count, h, t, off + 1, d_capped)
-        long long pairs = 0;
+        TD_DISPATCH(launch_count, h, t, sg.N[k], n, off + 1, d_capped)
         unsigned long long capped = 0;
         try {
             thrust::inclusive_scan(par, off + 1, off + 1 + n, off + 1);
@@ -485,138 +677,107 @@ int td_forward(sdpb_topdown* h) {
             cudaStreamSynchronize(st) != cudaSuccess)
             return td_fail(h, SDPB_ERR_CUDA, std::string("counting the actions: ") + cudaGetErrorString(cudaGetLastError()));
         capped_total += (double)capped;
-        evals += (double)pairs * D;
-        if (t == T) break;
-
-        // Scratch: three key buffers of `cap` keys (chunk candidates, sort output, merge output / frontier) and the radix
-        // sort's temporary storage, together at most `budget` bytes.  A chunk must hold at least as many candidates as
-        // the frontier has states (cap - nf >= nf), so the merges of a period cost at most twice its sorted candidates;
-        // a period whose reached states pass half a buffer fails with SDPB_ERR_NOMEM instead of crawling on.
-        const long long cand = pairs * D, key3 = 3 * (long long)sizeof(TDKey);
-        const std::string per = "period " + std::to_string(t + 1);
-        size_t free_b = 0, total_b = 0;
-        cudaMemGetInfo(&free_b, &total_b);
-        const long long budget = h->scratch_bytes > 0 ? h->scratch_bytes : (long long)(free_b / 2);
-        auto sort_temp = [&](long long items, size_t& bytes) {
-            cub::DoubleBuffer<TDKey> probe(nullptr, nullptr);
-            return td_sort_nd(nd, nullptr, bytes, probe, items, st) == cudaSuccess;
-        };
-        long long cap = std::max(1ll, std::min(cand, budget / key3));
-        size_t tmp_bytes = 0;
-        if (!sort_temp(cap, tmp_bytes)) return td_fail(h, SDPB_ERR_CUDA, "sizing the sort");
-        if (cap * key3 + (long long)tmp_bytes > budget) {  // the temporary storage shrinks with the item count
-            cap = (budget - (long long)tmp_bytes) / key3;
-            if (cap < 1 || !sort_temp(cap, tmp_bytes) || cap * key3 + (long long)tmp_bytes > budget)
-                return td_fail(h, SDPB_ERR_NOMEM, per + ": a scratch budget of " + std::to_string(budget) +
-                                                      " bytes does not hold the sort's temporary storage");
-        }
-        DevBuf kb[3], tmp_b;
-        for (auto& b : kb)
-            if (!b.alloc((size_t)cap * sizeof(TDKey)))
-                return td_fail(h, SDPB_ERR_NOMEM, "allocation of the expansion scratch failed (" + per + ")");
-        if (!tmp_b.alloc(tmp_bytes)) return td_fail(h, SDPB_ERR_NOMEM, "allocation of the sort scratch failed (" + per + ")");
-        TDKey* front = (TDKey*)kb[0].p;
-        TDKey* x = (TDKey*)kb[1].p;
-        TDKey* y = (TDKey*)kb[2].p;
-        long long nf = 0;
-        for (long long p = 0; p < pairs;) {
-            const long long room = cap - nf;
-            const long long np = std::min(pairs - p, room / D);
-            if (np < 1 || nf > room)
-                return td_fail(h, SDPB_ERR_NOMEM,
-                               per + " reaches at least " + std::to_string(nf) + " states: more than a scratch budget of " +
-                                   std::to_string(budget) + " bytes (" + std::to_string(cap) +
-                                   " keys per buffer, at most half of them reached states) can expand");
-            TD_DISPATCH(launch_expand, h, t, off, p, np, x)
-            if (cudaGetLastError() != cudaSuccess) return td_fail(h, SDPB_ERR_CUDA, "td_expand launch failed");
-            try {
-                long long m = thrust::remove_if(par, x, x + np * D, TDIsHole()) - x;
-                cub::DoubleBuffer<TDKey> db(x, y);
-                size_t tb = tmp_bytes;
-                if (td_sort_nd(nd, tmp_b.p, tb, db, m, st) != cudaSuccess) return td_fail(h, SDPB_ERR_CUDA, "radix sort failed");
-                TDKey* cur = db.Current();
-                TDKey* alt = db.Alternate();
-                m = thrust::unique(par, cur, cur + m, TDEq()) - cur;
-                thrust::merge(par, front, front + nf, cur, cur + m, alt, TDLess());
-                nf = thrust::unique(par, alt, alt + nf + m, TDEq()) - alt;
-                TDKey* old = front;
-                front = alt;
-                x = old;
-                y = cur;
-            } catch (const std::exception& ex) {
-                return td_fail(h, SDPB_ERR_CUDA, std::string("sort / merge: ") + ex.what());
-            }
-            p += np;
-        }
-        if (cudaMalloc(&h->F[t], (size_t)std::max(nf, 1ll) * sizeof(TDKey)) != cudaSuccess) {
-            cudaGetLastError();
-            h->F[t] = nullptr;
-            return td_fail(h, SDPB_ERR_NOMEM, "allocation of the states of period " + std::to_string(t + 1) + " failed");
-        }
-        if (cudaMemcpyAsync(h->F[t], front, (size_t)nf * sizeof(TDKey), cudaMemcpyDeviceToDevice, st) != cudaSuccess ||
-            cudaStreamSynchronize(st) != cudaSuccess)
-            return td_fail(h, SDPB_ERR_CUDA, std::string("forward pass: ") + cudaGetErrorString(cudaGetLastError()));
-        h->nF[t] = nf;
+        evals += (double)pairs * h->pmf_len[k];
     }
-    h->stats.evals = evals;
-    h->stats.evals_executed = evals;
-    h->stats.capped_action_sets = capped_total;
     return SDPB_OK;
 }
 
-// One solve from the period-1 states `init` (n * ndim API-order doubles).
-int td_solve(sdpb_topdown* h, const double* init, int n) {
+// getExpectedValue on the states roots[t - 1] of every period t >= p (each sorted and unique; roots[t - 1] empty for
+// t < p): the forward pass builds the states no earlier call reached, the backward pass solves only those against the
+// merged tables of the next period, and the merged tables of every touched period replace the handle's at the end.
+int td_extend(sdpb_topdown* h, int p, const std::vector<std::vector<TDKey>>& roots) {
     const int T = h->m.T;
-    td_free_tables(h);
-    std::vector<TDKey> k0((size_t)n);
-    for (int i = 0; i < n; i++) {
-        const double* s = init + (size_t)i * h->ndim;
-        int c = 1;
-        const double w = h->P.cash ? s[c++] : 0.0;
-        const double q1 = h->P.lead >= 1 ? s[c++] : 0.0;
-        const double q2 = h->P.lead >= 2 ? s[c++] : 0.0;
-        for (int k = 0; k < h->ndim; k++)
-            if (!std::isfinite(s[k])) return td_fail(h, SDPB_ERR_ARG, "an initial state is not finite");
-        k0[i] = td_pack(h->P, s[0], q1, q2, w);
-    }
-    std::sort(k0.begin(), k0.end(), TDLess());
-    k0.erase(std::unique(k0.begin(), k0.end(), TDEq()), k0.end());
     cudaStream_t st = h->stream;
+    auto par = thrust::cuda::par.on(st);
+    TDStage sg(T);
     if (cudaEventRecord(h->e0, st) != cudaSuccess) return td_fail(h, SDPB_ERR_CUDA, "cudaEventRecord failed");
-    if (cudaMalloc(&h->F[0], k0.size() * sizeof(TDKey)) != cudaSuccess) {
-        cudaGetLastError();
-        h->F[0] = nullptr;
-        return td_fail(h, SDPB_ERR_NOMEM, "allocation failed");
-    }
-    if (cudaMemcpyAsync(h->F[0], k0.data(), k0.size() * sizeof(TDKey), cudaMemcpyHostToDevice, st) != cudaSuccess)
-        return td_fail(h, SDPB_ERR_CUDA, "cudaMemcpyAsync failed");
-    h->nF[0] = (long long)k0.size();
-    int rc = td_forward(h);  // synchronises (k0 outlives the copy)
+    double evals = 0, capped = 0;
+    int rc = td_forward(h, p, roots, sg, evals, capped);
     if (rc != SDPB_OK) return rc;
-    if (h->stats.capped_action_sets > 0 && !(h->allow & SDPB_ALLOW_CAPPED_ACTIONS))
+    if (capped > 0 && !(h->allow & SDPB_ALLOW_CAPPED_ACTIONS))
         return td_fail(h, SDPB_ERR_OFFGRID,
-                       std::to_string((long long)h->stats.capped_action_sets) +
+                       std::to_string((long long)capped) +
                            " reached XR states have an order-up-to range longer than max_order_idx + 1 "
                            "(allow SDPB_ALLOW_CAPPED_ACTIONS to cut it there)");
-    for (int t = 1; t <= T; t++) {
-        const size_t nn = (size_t)std::max(h->nF[t - 1], 1ll);
-        if (cudaMalloc(&h->V[t - 1], nn * sizeof(double)) != cudaSuccess ||
-            cudaMalloc(&h->Q[t - 1], nn * sizeof(int)) != cudaSuccess) {
-            cudaGetLastError();
+    if (cudaEventRecord(h->e1, st) != cudaSuccess) return td_fail(h, SDPB_ERR_CUDA, "cudaEventRecord failed");
+    int launches = 0;
+    for (int t = T; t >= p; t--) {
+        const int k = t - 1;
+        const long long n = sg.nN[k], no = h->nF[k];
+        if (n == 0) continue;
+        if (!td_alloc(sg.VN[k], n) || !td_alloc(sg.QN[k], n))
             return td_fail(h, SDPB_ERR_NOMEM, "allocation of the value tables failed");
+        const bool nxt = t < T, nxt_new = nxt && sg.nN[k + 1] > 0;
+        TD_DISPATCH(launch_backward, h, t, sg.N[k], n, nxt ? (nxt_new ? sg.MF[k + 1] : h->F[k + 1]) : nullptr,
+                    nxt ? (nxt_new ? sg.MV[k + 1] : h->V[k + 1]) : nullptr,
+                    nxt ? (nxt_new ? sg.nM[k + 1] : h->nF[k + 1]) : 0, sg.VN[k], sg.QN[k])
+        launches++;
+        if (cudaGetLastError() != cudaSuccess) return td_fail(h, SDPB_ERR_CUDA, "td_backward launch failed");
+        sg.nM[k] = no + n;
+        if (no == 0) {  // nothing to merge with: the new tables are the merged ones
+            std::swap(sg.MF[k], sg.N[k]);
+            std::swap(sg.MV[k], sg.VN[k]);
+            std::swap(sg.MQ[k], sg.QN[k]);
+            continue;
+        }
+        if (!td_alloc(sg.MF[k], no + n) || !td_alloc(sg.MV[k], no + n) || !td_alloc(sg.MQ[k], no + n))
+            return td_fail(h, SDPB_ERR_NOMEM, "allocation of the merged tables of period " + std::to_string(t) + " failed");
+        try {  // the two key sets are disjoint: a merge by key keeps every row
+            thrust::merge_by_key(par, h->F[k], h->F[k] + no, sg.N[k], sg.N[k] + n,
+                                 thrust::make_zip_iterator(thrust::make_tuple(h->V[k], h->Q[k])),
+                                 thrust::make_zip_iterator(thrust::make_tuple(sg.VN[k], sg.QN[k])), sg.MF[k],
+                                 thrust::make_zip_iterator(thrust::make_tuple(sg.MV[k], sg.MQ[k])), TDLess());
+        } catch (const std::exception& ex) {
+            return td_fail(h, SDPB_ERR_CUDA, std::string("merge: ") + ex.what());
         }
     }
-    if (cudaEventRecord(h->e1, st) != cudaSuccess) return td_fail(h, SDPB_ERR_CUDA, "cudaEventRecord failed");
-    for (int t = T; t >= 1; t--) TD_DISPATCH(launch_backward, h, t)
-    if (cudaGetLastError() != cudaSuccess) return td_fail(h, SDPB_ERR_CUDA, "td_backward launch failed");
     if (cudaEventRecord(h->e2, st) != cudaSuccess || cudaEventSynchronize(h->e2) != cudaSuccess)
         return td_fail(h, SDPB_ERR_CUDA, std::string("backward pass: ") + cudaGetErrorString(cudaGetLastError()));
+    for (int k = p - 1; k < T; k++) {  // commit
+        if (sg.nN[k] == 0) continue;
+        cudaFree(h->F[k]);
+        cudaFree(h->V[k]);
+        cudaFree(h->Q[k]);
+        h->F[k] = sg.MF[k];
+        h->V[k] = sg.MV[k];
+        h->Q[k] = sg.MQ[k];
+        sg.MF[k] = nullptr;
+        sg.MV[k] = nullptr;
+        sg.MQ[k] = nullptr;
+        h->nF[k] = sg.nM[k];
+    }
     float solve = 0, kern = 0;
     cudaEventElapsedTime(&solve, h->e0, h->e2);
     cudaEventElapsedTime(&kern, h->e1, h->e2);
+    h->stats.evals += evals;
+    h->stats.evals_executed += evals;
+    h->stats.capped_action_sets += capped;
     h->stats.solve_ms = solve;
     h->stats.kernel_ms = kern;
-    h->stats.launches = T;
+    h->stats.launches = launches;
+    return SDPB_OK;
+}
+
+// The key of one API-order state
+TDKey td_key_of(const sdpb_topdown* h, const double* s) {
+    int c = 1;
+    const double w = h->P.cash ? s[c++] : 0.0;
+    const double q1 = h->P.lead >= 1 ? s[c++] : 0.0;
+    const double q2 = h->P.lead >= 2 ? s[c++] : 0.0;
+    return td_pack(h->P, s[0], q1, q2, w);
+}
+
+// n API-order states -> their keys, sorted and unique; SDPB_ERR_ARG when a coordinate is not finite
+int td_root_keys(sdpb_topdown* h, const double* states, int n, std::vector<TDKey>& out) {
+    out.resize((size_t)n);
+    for (int i = 0; i < n; i++) {
+        const double* s = states + (size_t)i * h->ndim;
+        for (int k = 0; k < h->ndim; k++)
+            if (!std::isfinite(s[k])) return td_fail(h, SDPB_ERR_ARG, "a state is not finite");
+        out[i] = td_key_of(h, s);
+    }
+    std::sort(out.begin(), out.end(), TDLess());
+    out.erase(std::unique(out.begin(), out.end(), TDEq()), out.end());
     return SDPB_OK;
 }
 
@@ -772,7 +933,9 @@ int sdpb_topdown_solve(const sdpb_model* m, const sdpb_topdown_options* opt, con
     h->P.lead = m->lead_time;
     h->P.cash = has_cash(*m) ? 1 : 0;
 
-    const int rc = td_solve(h, init_states, n);
+    std::vector<std::vector<TDKey>> roots((size_t)T);
+    int rc = td_root_keys(h, init_states, n, roots[0]);
+    if (rc == SDPB_OK) rc = td_extend(h, 1, roots);
     if (rc != SDPB_OK) {
         const std::string msg = h->err;
         return bail(rc, msg);
@@ -799,14 +962,7 @@ int sdpb_topdown_value(sdpb_topdown* h, int period, const double* states, int n,
     if (n == 0) return SDPB_OK;
     cudaSetDevice(h->device);
     std::vector<TDKey> keys((size_t)n);
-    for (int i = 0; i < n; i++) {
-        const double* s = states + (size_t)i * h->ndim;
-        int c = 1;
-        const double w = h->P.cash ? s[c++] : 0.0;
-        const double q1 = h->P.lead >= 1 ? s[c++] : 0.0;
-        const double q2 = h->P.lead >= 2 ? s[c++] : 0.0;
-        keys[i] = td_pack(h->P, s[0], q1, q2, w);
-    }
+    for (int i = 0; i < n; i++) keys[i] = td_key_of(h, states + (size_t)i * h->ndim);
     DevBuf kq, vq, aq;
     if (!kq.alloc(keys.size() * sizeof(TDKey)) || !vq.alloc((size_t)n * sizeof(double)) || !aq.alloc((size_t)n * sizeof(int)))
         return td_fail(h, SDPB_ERR_NOMEM, "allocation failed");
@@ -865,6 +1021,116 @@ int sdpb_topdown_opt_table(sdpb_topdown* h, double* rows, size_t* nrows) {
         }
     }
     *nrows = total;
+    return SDPB_OK;
+}
+
+int sdpb_topdown_extend(sdpb_topdown* h, int period, const double* states, int n) {
+    if (!h) return td_fail(nullptr, SDPB_ERR_ARG, "null handle");
+    if (period < 1 || period > h->m.T || n < 0 || (n > 0 && !states)) return td_fail(h, SDPB_ERR_ARG, "bad period or states");
+    if (n == 0) return SDPB_OK;
+    std::vector<std::vector<TDKey>> roots((size_t)h->m.T);
+    const int rc = td_root_keys(h, states, n, roots[period - 1]);
+    if (rc != SDPB_OK) return rc;
+    cudaSetDevice(h->device);
+    return td_extend(h, period, roots);
+}
+
+int sdpb_topdown_simulate(sdpb_topdown* h, const double* init_state, const double* samples, int n, double discount,
+                          double* values) {
+    if (!h) return td_fail(nullptr, SDPB_ERR_ARG, "null handle");
+    if (!init_state || !samples || !values || n < 1) return td_fail(h, SDPB_ERR_ARG, "null argument or n < 1");
+    const int T = h->m.T;
+    for (size_t i = 0; i < (size_t)n * T; i++)
+        if (!std::isfinite(samples[i])) return td_fail(h, SDPB_ERR_ARG, "a sample is not finite");
+    std::vector<std::vector<TDKey>> roots((size_t)T);
+    int rc = td_root_keys(h, init_state, 1, roots[0]);
+    if (rc != SDPB_OK) return rc;
+    const TDKey k0 = roots[0][0];
+    const auto w0 = std::chrono::steady_clock::now();
+    cudaSetDevice(h->device);
+    rc = td_extend(h, 1, roots);  // Simulation.java:62 asks for getExpectedValue(iniState) first
+    if (rc != SDPB_OK) return rc;
+
+    cudaStream_t st = h->stream;
+    std::vector<double> pw((size_t)T);
+    for (int t = 0; t < T; t++) pw[t] = std::pow(discount, (double)t);  // Math.pow(discountFactor, t)
+    std::vector<TDKey> key0((size_t)n, k0);
+    std::vector<int> per0((size_t)n, 1), act0((size_t)n);
+    for (int i = 0; i < n; i++) act0[i] = i;
+    DevBuf smp_b, pw_b, key_b, per_b, sum_b, val_b, act_b[2], st_b, sk_b, sn_b, tab_b;
+    const size_t N = (size_t)n;
+    if (!smp_b.alloc(N * T * sizeof(double)) || !pw_b.alloc(T * sizeof(double)) || !key_b.alloc(N * sizeof(TDKey)) ||
+        !per_b.alloc(N * sizeof(int)) || !sum_b.alloc(N * sizeof(double)) || !val_b.alloc(N * sizeof(double)) ||
+        !act_b[0].alloc(N * sizeof(int)) || !act_b[1].alloc(N * sizeof(int)) || !st_b.alloc(N * sizeof(int)) ||
+        !sk_b.alloc(N * sizeof(TDKey)) || !sn_b.alloc(sizeof(int)) || !tab_b.alloc((size_t)T * 3 * 8))
+        return td_fail(h, SDPB_ERR_NOMEM, "allocation of the roll-out buffers failed");
+    const TDKey** dF = (const TDKey**)tab_b.p;
+    const int** dQ = (const int**)(dF + T);
+    long long* dn = (long long*)(dQ + T);
+    if (cudaMemcpyAsync(smp_b.p, samples, N * T * sizeof(double), cudaMemcpyHostToDevice, st) != cudaSuccess ||
+        cudaMemcpyAsync(pw_b.p, pw.data(), T * sizeof(double), cudaMemcpyHostToDevice, st) != cudaSuccess ||
+        cudaMemcpyAsync(key_b.p, key0.data(), N * sizeof(TDKey), cudaMemcpyHostToDevice, st) != cudaSuccess ||
+        cudaMemcpyAsync(per_b.p, per0.data(), N * sizeof(int), cudaMemcpyHostToDevice, st) != cudaSuccess ||
+        cudaMemcpyAsync(act_b[0].p, act0.data(), N * sizeof(int), cudaMemcpyHostToDevice, st) != cudaSuccess ||
+        cudaMemsetAsync(sum_b.p, 0, N * sizeof(double), st) != cudaSuccess)
+        return td_fail(h, SDPB_ERR_CUDA, "cudaMemcpyAsync failed");
+    std::vector<const void*> tab((size_t)T * 3);
+    std::vector<int> stall_t;
+    std::vector<TDKey> stall_k;
+    float kern = 0;
+    int rounds = 0, na = n, cur = 0;
+    while (na > 0) {
+        // the tables move when an extension merges new states in: hand the kernel the current ones
+        for (int t = 0; t < T; t++) {
+            tab[t] = h->F[t];
+            tab[T + t] = h->Q[t];
+            std::memcpy(&tab[2 * T + t], &h->nF[t], sizeof(long long));
+        }
+        int ns = 0;
+        if (cudaMemcpyAsync(tab_b.p, tab.data(), tab.size() * 8, cudaMemcpyHostToDevice, st) != cudaSuccess ||
+            cudaMemsetAsync(sn_b.p, 0, sizeof(int), st) != cudaSuccess || cudaEventRecord(h->e1, st) != cudaSuccess)
+            return td_fail(h, SDPB_ERR_CUDA, "cudaMemcpyAsync failed");
+        TD_DISPATCH(launch_simulate, h, dF, dQ, dn, (const double*)smp_b.p, (const double*)pw_b.p,
+                    (const int*)act_b[cur].p, na, (TDKey*)key_b.p, (int*)per_b.p, (double*)sum_b.p, (double*)val_b.p,
+                    (int*)sn_b.p, (int*)act_b[1 - cur].p, (int*)st_b.p, (TDKey*)sk_b.p)
+        if (cudaGetLastError() != cudaSuccess) return td_fail(h, SDPB_ERR_CUDA, "td_simulate launch failed");
+        if (cudaEventRecord(h->e2, st) != cudaSuccess ||
+            cudaMemcpyAsync(&ns, sn_b.p, sizeof(int), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+            cudaStreamSynchronize(st) != cudaSuccess)
+            return td_fail(h, SDPB_ERR_CUDA, std::string("roll-out: ") + cudaGetErrorString(cudaGetLastError()));
+        float ms = 0;
+        cudaEventElapsedTime(&ms, h->e1, h->e2);
+        kern += ms;
+        rounds++;
+        if (ns == 0) break;
+        // the states the stalled paths stand on become roots of one extension (Simulation.java:62: getExpectedValue)
+        stall_t.resize((size_t)ns);
+        stall_k.resize((size_t)ns);
+        if (cudaMemcpyAsync(stall_t.data(), st_b.p, (size_t)ns * sizeof(int), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+            cudaMemcpyAsync(stall_k.data(), sk_b.p, (size_t)ns * sizeof(TDKey), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+            cudaStreamSynchronize(st) != cudaSuccess)
+            return td_fail(h, SDPB_ERR_CUDA, "cudaMemcpyAsync failed");
+        std::vector<std::vector<TDKey>> r((size_t)T);
+        int p = T;
+        for (int j = 0; j < ns; j++) {
+            r[stall_t[j] - 1].push_back(stall_k[j]);
+            p = std::min(p, stall_t[j]);
+        }
+        for (auto& v : r) {
+            std::sort(v.begin(), v.end(), TDLess());
+            v.erase(std::unique(v.begin(), v.end(), TDEq()), v.end());
+        }
+        rc = td_extend(h, p, r);
+        if (rc != SDPB_OK) return rc;
+        na = ns;
+        cur = 1 - cur;
+    }
+    if (cudaMemcpyAsync(values, val_b.p, N * sizeof(double), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+        cudaStreamSynchronize(st) != cudaSuccess)
+        return td_fail(h, SDPB_ERR_CUDA, "cudaMemcpyAsync failed");
+    h->stats.solve_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - w0).count();
+    h->stats.kernel_ms = kern;
+    h->stats.launches = rounds;
     return SDPB_OK;
 }
 

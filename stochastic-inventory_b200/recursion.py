@@ -142,9 +142,10 @@ class _Engine:
 
         `topdown=True`: no grid.  The engine solves exactly the states the reference's recursion visits from the
         period-1 states asked for so far (sdpb_topdown_*), so states, steps and demands need not be multiples of a
-        power of two and an unclamped model needs no hull; getExpectedValue on a new period-1 state solves again with
-        that root added.  A later-period state that was not reached raises KeyError, as getAction on an unsolved
-        state does.  The lambdas are kept but not spot-checked against the descriptor (that check evaluates them on
+        power of two and an unclamped model needs no hull; getExpectedValue on a new period-1 state solves only the
+        states it reaches that no earlier call did (sdpb_topdown_extend), and a Simulation over this recursion adds
+        the states its paths meet, as the reference's memo maps grow.  A later-period state that was not reached raises
+        KeyError, as getAction on an unsolved state does.  The lambdas are kept but not spot-checked against the descriptor (that check evaluates them on
         the dense grid), and there is no boundary function (it is tabulated on the grid) and no multi-GPU split."""
         if spec.cost_kind not in self._kinds or spec.lead_time != self._lead:
             raise ValueError(f"{type(self).__name__} does not take this descriptor "
@@ -224,11 +225,11 @@ class _Engine:
     def getExpectedValue(self, state):
         if self._topdown:
             if state.getPeriod() == 1 and state._vec() not in self._queried:
-                td = TopDown(self.spec, self._queried + [state._vec()], device=self._device,
-                             allow=self._allow | self.spec.allow)
-                if self._td is not None:
-                    self._td.close()
-                self._td = td
+                if self._td is None:
+                    self._td = TopDown(self.spec, [state._vec()], device=self._device,
+                                       allow=self._allow | self.spec.allow)
+                else:
+                    self._td.extend(1, [state._vec()])
                 self._queried.append(state._vec())
             return self._value(state)[0]
         val, _ = self._value(state)

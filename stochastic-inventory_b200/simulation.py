@@ -1,4 +1,5 @@
-"""Host-side mirror of the reference's policy roll-out classes, over sdpb_simulate.
+"""Host-side mirror of the reference's policy roll-out classes, over sdpb_simulate (a dense recursion) or
+sdpb_topdown_simulate (a recursion built with topdown=True).
 
     Simulation       src/sdp/inventory/Simulation.java:19-107
     CashSimulation   src/sdp/cash/CashSimulation.java:30-118
@@ -46,6 +47,9 @@ class Simulation:
         if samples is None:
             samples = generate_lh_samples(self.distributions, self.sampleNum)
         self.recursion.getExpectedValue(iniState)  # solves on first use, like the reference's lazy recursion
+        if getattr(self.recursion, "_topdown", False):
+            # no grid: the roll-out solves each state a path meets that was not reached yet (Simulation.java:62)
+            return self.recursion._td.simulate(iniState._vec(), samples, self.discountFactor)
         return self.recursion._solver.simulate(iniState._vec(), samples, self.discountFactor)
 
     def simulateSDPGivenSamplNum(self, iniState, samples=None):

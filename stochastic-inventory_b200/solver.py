@@ -269,6 +269,31 @@ class TopDown:
                                                 q.ctypes.data_as(dp)))
         return v, q
 
+    def extend(self, period: int, states):
+        """getExpectedValue on API-order states [n, ndim] of one period: solves only the states no earlier call reached
+        (sdpb_topdown_extend).  A failure leaves the handle as it was."""
+        st = np.ascontiguousarray(np.atleast_2d(np.asarray(states, dtype=np.float64)))
+        if st.shape[1] != self.ndim:
+            raise ValueError(f"states must have {self.ndim} columns")
+        self._check(self.lib.sdpb_topdown_extend(self.h, period, st.ctypes.data_as(C.POINTER(C.c_double)), st.shape[0]))
+        return self
+
+    def simulate(self, init_state, samples, discount: float = 1.0):
+        """Roll the policy over demand sample paths [n, T] -> per-path sums (Simulation.java:59-70), solving every state
+        a path meets that was not reached yet, as the reference's getExpectedValue at each step does
+        (sdpb_topdown_simulate).  The states it adds stay in the handle."""
+        st = np.ascontiguousarray(init_state, dtype=np.float64)
+        sm = np.ascontiguousarray(samples, dtype=np.float64)
+        if st.shape != (self.ndim,):
+            raise ValueError(f"init_state must have {self.ndim} components")
+        if sm.ndim != 2 or sm.shape[1] != self.T:
+            raise ValueError(f"samples must be [n, {self.T}]")
+        vals = np.empty(sm.shape[0])
+        dp = C.POINTER(C.c_double)
+        self._check(self.lib.sdpb_topdown_simulate(self.h, st.ctypes.data_as(dp), sm.ctypes.data_as(dp), sm.shape[0],
+                                                   float(discount), vals.ctypes.data_as(dp)))
+        return vals
+
     def opt_table(self):
         """[rows, ndim + 2]: (t, state..., Q*) of every reached state in memo-map order."""
         n = C.c_size_t(0)
