@@ -509,7 +509,59 @@ typedef struct sdpb_reached_model {
  * (may be NULL, T entries); solve_ms = device time.  Blocks.  No CPU fallback. */
 int sdpb_reached_solve(const sdpb_reached_model* m, int device, const double* init_state, double* value,
                        double* action1, double* action2, int64_t* n_states, double* solve_ms);
+/* The message of the last failed sdpb_reached_* call of this thread. */
 const char* sdpb_reached_last_error(void);
+
+/* A reached-state solve kept as a handle: the memo of getExpectedValue calls, every reached state queryable.
+ *   States      API order, as sdpb_reached_solve takes them: kind 0 (x1, x2, preQ1, preQ2, cash), kind 1 (x1, x2, R),
+ *               kind 2 (x1, x2, cash), kind 3 (x, cash).  A root (of open, extend, simulate) must have integer
+ *               inventories and pipeline quantities in [0, 65535] (kind 3: x = k / state_q with such a k), otherwise
+ *               SDPB_ERR_OFFGRID; a queried state that has no such form is simply not reached (SDPB_ERR_UNSOLVED).
+ *               A coordinate that is not finite is SDPB_ERR_ARG.
+ *   Actions     a1 / a2 as sdpb_reached_solve reports them, for every state: order quantities for kinds 0 and 3 (a2 = 0
+ *               for kind 3), order-up-to levels for kinds 1 and 2.  A state without any accepted action keeps the
+ *               reference's default: {0, 0} for kind 1, (x1, x2) for kind 2.
+ *   Order       memo-map order (t, x1, x2, preQ1, preQ2, cash) with cash compared numerically
+ *               (CashRecursionMultiLead.java:45-51); -0.0 is stored as +0.0.
+ *   Extension   only the states no earlier call reached are expanded and solved, each against the merged tables of the
+ *               next period, so a state's value never depends on the order of the calls.  The candidate successors of
+ *               the new states of one period are expanded at once: when candidates * 16 B * 2.2 exceed the budget --
+ *               the free device memory, or scratch_bytes when > 0 -- the call fails with SDPB_ERR_NOMEM naming the
+ *               period.  A failed call leaves states, tables and stats exactly as they were.
+ *   Stats       evals = sum_t sum_{s reached} |listed actions of s| * D_t over the life of the handle, evals_executed =
+ *               evals; solve_ms (device time between events at the start and end of the call), kernel_ms (its backward
+ *               pass) and launches (its backward launches) describe the latest call.  For simulate see there.
+ * The handle keeps, per period, the sorted keys (16 B), V (8 B) and action index (4 B) of the reached states; the
+ * candidate buffers of an extension are freed when it returns. */
+typedef struct sdpb_reached sdpb_reached;
+/* getExpectedValue on n >= 0 period-1 roots, one memo (the union of their visit sets); n == 0: an empty handle. */
+int  sdpb_reached_open(const sdpb_reached_model* m, int device, int64_t scratch_bytes, const double* init_states, int n,
+                       sdpb_reached** out);
+void sdpb_reached_destroy(sdpb_reached* h);
+/* value + action of n reached states of one period (v, a1, a2 may be NULL); SDPB_ERR_UNSOLVED for a state not reached */
+int  sdpb_reached_value(sdpb_reached* h, int period, const double* states, int n, double* v, double* a1, double* a2);
+/* getExpectedValue(state) on n states of one period 1..T; n == 0 does nothing */
+int  sdpb_reached_extend(sdpb_reached* h, int period, const double* states, int n);
+/* rows [t, state dims (API order)..., a1, a2] of every reached state in memo-map order; rows == NULL: *nrows = the count */
+int  sdpb_reached_opt_table(sdpb_reached* h, double* rows, size_t* nrows);
+int  sdpb_reached_states(const sdpb_reached* h, int64_t* n_states /* T: reached states of each period */);
+int  sdpb_reached_stats(const sdpb_reached* h, sdpb_stats* s);
+/* The policy rolled out over n demand sample paths, with a lazy getExpectedValue at every step (CashSimulation's loop,
+ * CashSimulation.java:85-118, over this engine's lambdas):
+ *     for each path i:  state = init;  sum = 0
+ *         for t = 1..T:  getExpectedValue(state);  (a1, a2) = getAction(state);  d = Math.round(samples[i][t-1][.])
+ *                        c = immediateValue(state, a, d)  (with the salvage term when t == T)
+ *                        sum += Math.pow(discount, t-1) * c;  state = stateTransition(state, a, d, c)
+ *     values[i] = sum
+ * `samples` is n * T * nd doubles, row-major: nd = 2 (one demand per product) for kinds 0-2, 1 for kind 3.  Kind 2, the
+ * V / Pi form, has no immediate value: a path is worth boundFinalCash (w + salvage . x) of the state reached after
+ * period T, and a discount other than 1 is SDPB_ERR_ARG.  A path that meets a state the handle has not reached stops
+ * there with its partial sum kept in fp64; the stalled states become the roots of one extension over several periods
+ * and the stalled paths go on, at least one period further each round: at most T rounds.  SDPB_ERR_ARG: n < 1, a null
+ * pointer, a sample or initial coordinate that is not finite.  stats: solve_ms = host wall time of the call, kernel_ms
+ * = the roll-out kernels' device time, launches = rounds; evals grows by the evaluations of the added states. */
+int  sdpb_reached_simulate(sdpb_reached* h, const double* init_state, const double* samples, int n, double discount,
+                           double* values);
 
 /* ---- any single-product model, solved over the states its top-down recursion reaches ---------------------------------
  * The reference answers getExpectedValue(state) for ANY state: it recurses top-down over real-valued states and memoises

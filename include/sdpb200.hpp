@@ -481,6 +481,87 @@ class TopDown {
     sdpb_topdown* h_ = nullptr;
 };
 
+// ---- the two-product recursions (and CashConstraintTest's), over the states they reach (sdpb_reached_*) ----
+// One memo for every call: every reached state can be queried, the handle extended with states of any period, and the
+// policy rolled out.  States in API order: (x1, x2, preQ1, preQ2, cash) | (x1, x2, R) | (x1, x2, cash) | (x, cash).
+class Reached {
+ public:
+    // `roots`: period-1 states (may be empty); the model's tables are copied.  scratchBytes > 0 replaces the free device
+    // memory as the expansion budget
+    Reached(const sdpb_reached_model& model, const std::vector<std::vector<double>>& roots, int device = -1,
+            int64_t scratchBytes = 0) : T_(model.T), kind_(model.kind) {
+        std::vector<double> flat = flatten(roots);
+        const int rc = sdpb_reached_open(&model, device, scratchBytes, flat.data(), (int)roots.size(), &h_);
+        if (rc != SDPB_OK) throw SdpbError(rc, std::string("sdpb_reached_open: ") + sdpb_reached_last_error());
+    }
+    Reached(const Reached&) = delete;
+    Reached& operator=(const Reached&) = delete;
+    ~Reached() { sdpb_reached_destroy(h_); }
+
+    // (V, a1, a2) of a reached state; SdpbError(SDPB_ERR_UNSOLVED) for one that was not reached
+    std::array<double, 3> valueAndAction(int period, const std::vector<double>& st) {
+        if (st.size() != ndim()) throw SdpbError(SDPB_ERR_ARG, "state has the wrong number of components");
+        std::array<double, 3> r{};
+        check(sdpb_reached_value(h_, period, st.data(), 1, &r[0], &r[1], &r[2]));
+        return r;
+    }
+    double value(int period, const std::vector<double>& st) { return valueAndAction(period, st)[0]; }
+    // rows [period, state..., a1, a2] of every reached state in memo-map order
+    std::vector<std::vector<double>> optTable() {
+        size_t n = 0;
+        check(sdpb_reached_opt_table(h_, nullptr, &n));
+        const size_t w = ndim() + 3;
+        std::vector<double> buf(n * w);
+        check(sdpb_reached_opt_table(h_, buf.data(), &n));
+        std::vector<std::vector<double>> rows(n, std::vector<double>(w));
+        for (size_t i = 0; i < n; i++) std::copy(buf.begin() + i * w, buf.begin() + (i + 1) * w, rows[i].begin());
+        return rows;
+    }
+    size_t nStates(int period) const {
+        std::vector<int64_t> n((size_t)T_);
+        check(sdpb_reached_states(h_, n.data()));
+        return (size_t)n.at((size_t)period - 1);
+    }
+    sdpb_stats stats() const { sdpb_stats s; check(sdpb_reached_stats(h_, &s)); return s; }
+    // getExpectedValue on API-order states of one period: solves only what no earlier call reached; a failure leaves
+    // the handle as it was
+    void extend(int period, const std::vector<std::vector<double>>& states) {
+        std::vector<double> flat = flatten(states);
+        check(sdpb_reached_extend(h_, period, flat.data(), (int)states.size()));
+    }
+    // the policy over demand sample paths (one row of T * nd samples per path, nd = 2 for two products, 1 for one) ->
+    // per-path values; every state a path meets that was not reached is solved on the way and stays in the handle
+    std::vector<double> simulate(const std::vector<double>& initState, const std::vector<std::vector<double>>& samples,
+                                 double discount = 1.0) {
+        if (initState.size() != ndim()) throw SdpbError(SDPB_ERR_ARG, "state has the wrong number of components");
+        const size_t per = (size_t)T_ * (kind_ == SDPB_REACHED_CASH_ROUNDED ? 1 : 2);
+        std::vector<double> flat;
+        for (const auto& r : samples) {
+            if (r.size() != per) throw SdpbError(SDPB_ERR_ARG, "a sample path must have T * nd demands");
+            flat.insert(flat.end(), r.begin(), r.end());
+        }
+        std::vector<double> values(samples.size());
+        check(sdpb_reached_simulate(h_, initState.data(), flat.data(), (int)samples.size(), discount, values.data()));
+        return values;
+    }
+
+ private:
+    size_t ndim() const { return kind_ == SDPB_REACHED_MULTILEAD ? 5 : kind_ == SDPB_REACHED_CASH_ROUNDED ? 2 : 3; }
+    std::vector<double> flatten(const std::vector<std::vector<double>>& states) const {
+        std::vector<double> flat;
+        for (const auto& r : states) {
+            if (r.size() != ndim()) throw SdpbError(SDPB_ERR_ARG, "state has the wrong number of components");
+            flat.insert(flat.end(), r.begin(), r.end());
+        }
+        return flat;
+    }
+    void check(int rc) const {
+        if (rc != SDPB_OK) throw SdpbError(rc, sdpb_reached_last_error());
+    }
+    int T_, kind_;
+    sdpb_reached* h_ = nullptr;
+};
+
 // Recursion / LeadtimeRecursion / CashRecursion / RiskRecursion access over TopDown, with states given as API-order
 // vectors: getExpectedValue on a new period-1 state extends the solve with that root (the memo maps grow the same way;
 // states a roll-out over engine() added stay); getAction / getExpectedValue of a later-period state that was not

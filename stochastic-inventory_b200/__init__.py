@@ -15,7 +15,7 @@ from .models import (workforce_model, two_product_cash_model, ModelSpec, cash_lo
 from .recursion import (CashRecursionMultiLead, CashRecursionMultiXR, CashRecursionRounded, CashRecursionV, CashStateMultiLead, CashStateMultiXR, StaffRecursion, StaffState, Actions, CashRecursionMulti, CashStateMulti, CashLeadtimeRecursion, CashLeadtimeState, CashRecursion, CashRecursionXR,
                         CashState, CashStateXR, LeadtimeRecursion, LeadtimeRecursion2, LeadtimeState,
                         OptDirection, Recursion, RiskRecursion, RiskState, State)
-from .solver import Group, Solver, TopDown, reachable_hull, solve_batch
+from .solver import Group, Reached, Solver, TopDown, reachable_hull, solve_batch
 from .simulation import CashSimulation, Simulation, generate_lh_samples
 from .sampling import MRG32k3a, Sampling
 from .write import WriteToCsv, WriteToExcelTxt, java_double

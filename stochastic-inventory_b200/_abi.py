@@ -126,7 +126,8 @@ EXPORTS = [
     "sdpb_group_stats", "sdpb_solve_batch", "sdpb_trim_pool", "sdpb_reached_solve", "sdpb_reached_last_error",
     "sdpb_topdown_solve", "sdpb_topdown_destroy", "sdpb_topdown_last_error", "sdpb_topdown_value",
     "sdpb_topdown_opt_table", "sdpb_topdown_states", "sdpb_topdown_stats", "sdpb_topdown_extend",
-    "sdpb_topdown_simulate",
+    "sdpb_topdown_simulate", "sdpb_reached_open", "sdpb_reached_destroy", "sdpb_reached_value", "sdpb_reached_extend",
+    "sdpb_reached_opt_table", "sdpb_reached_states", "sdpb_reached_stats", "sdpb_reached_simulate",
 ]
 
 _lib = None
@@ -207,6 +208,15 @@ def load():
     lib.sdpb_reached_solve.argtypes = [C.POINTER(SdpbReachedModel), C.c_int, _dp, _dp, _dp, _dp,
                                        C.POINTER(C.c_int64), _dp]
     lib.sdpb_reached_last_error.restype = C.c_char_p
+    lib.sdpb_reached_open.argtypes = [C.POINTER(SdpbReachedModel), C.c_int, C.c_int64, _dp, C.c_int, C.POINTER(vp)]
+    lib.sdpb_reached_destroy.argtypes = [vp]
+    lib.sdpb_reached_destroy.restype = None
+    lib.sdpb_reached_value.argtypes = [vp, C.c_int, _dp, C.c_int, _dp, _dp, _dp]
+    lib.sdpb_reached_extend.argtypes = [vp, C.c_int, _dp, C.c_int]
+    lib.sdpb_reached_opt_table.argtypes = [vp, _dp, C.POINTER(C.c_size_t)]
+    lib.sdpb_reached_states.argtypes = [vp, C.POINTER(C.c_int64)]
+    lib.sdpb_reached_stats.argtypes = [vp, C.POINTER(SdpbStats)]
+    lib.sdpb_reached_simulate.argtypes = [vp, _dp, _dp, C.c_int, C.c_double, _dp]
     lib.sdpb_topdown_solve.argtypes = [C.POINTER(SdpbModel), C.POINTER(SdpbTopdownOptions), _dp, C.c_int, C.POINTER(vp)]
     lib.sdpb_topdown_destroy.argtypes = [vp]
     lib.sdpb_topdown_destroy.restype = None

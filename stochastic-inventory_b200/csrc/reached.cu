@@ -19,6 +19,13 @@
 //   forward   F_1 = {initial state};  F_{t+1} = unique{ f(s, a, d) : s in F_t, a in A, d in D_t }   (expand, sort, unique)
 //   backward  V_T on F_T, then V_t on F_t with V_{t+1}(f(s,a,d)) found by binary search in the sorted F_{t+1}
 //
+// A solve is a handle (sdpb_reached_open) that keeps, per period, the sorted keys, V and the action index of the
+// reached states, so that every reached state can be queried (ml_query), the handle extended with states of any period
+// (ml_extend: only the states no earlier call reached are expanded -- N_t = (successors of N_{t-1} u roots of t) \ F_t,
+// membership by binary search (ml_known) -- and solved against the merged F_{t+1}, then merged into F_t by key), and
+// the policy rolled out over sample paths (ml_simulate), extending the handle with the states the paths meet.
+// sdpb_reached_solve is open -> read the root -> destroy.
+//
 // The arithmetic of every (s, a, d) is the reference's, operation for operation and in its order (no FMA: the file is
 // compiled with -fmad=false); the action scan is serial in the reference's i-major order because the acceptance rule
 // `value > best + 0.1` is order dependent.  Two thread mappings: a thread per state (large frontiers: the last
@@ -26,13 +33,21 @@
 // pair followed by a per-state scan (small frontiers, where a thread per state would leave the GPU empty).
 #include <cuda_runtime.h>
 #include <thrust/execution_policy.h>
+#include <thrust/iterator/zip_iterator.h>
+#include <thrust/merge.h>
+#include <thrust/remove.h>
 #include <thrust/sort.h>
+#include <thrust/tuple.h>
 #include <thrust/unique.h>
 
+#include <algorithm>
 #include <cfloat>
+#include <chrono>
 #include <cmath>
 #include <cstdint>
 #include <cstdio>
+#include <cstring>
+#include <exception>
 #include <string>
 #include <vector>
 
@@ -45,7 +60,10 @@ struct MLState {
     double cash;
 };
 
-// sort / search key: the four integers packed, then the cash bits (any total order will do; equality is exact)
+// sort / search key: the four integers packed, then the cash as an order-preserving word, so that the keys sort in the
+// reference's memo-map order (t, x1, x2, preQ1, preQ2, cash) with cash compared numerically (CashRecursionMultiLead.java:45-51).
+// The all-ones key marks a slot of an unlisted action: it sorts last and no state has it (q_bound <= 65535 keeps
+// preQ2 below 0xffff).
 struct MLKey {
     unsigned long long a, b;
 };
@@ -55,6 +73,24 @@ struct MLKeyLess {
 struct MLKeyEq {
     __host__ __device__ bool operator()(const MLKey& l, const MLKey& r) const { return l.a == r.a && l.b == r.b; }
 };
+struct MLFlagged {
+    __host__ __device__ bool operator()(unsigned char f) const { return f != 0; }
+};
+
+// order-preserving encoding of a double: set the sign bit of a non-negative value, flip every bit of a negative one
+__host__ __device__ inline unsigned long long ml_enc(double v) {
+    v += 0.0;  // -0.0 and +0.0 are one key in the reference's map (compared with ==)
+    unsigned long long b;
+    memcpy(&b, &v, sizeof b);
+    return b ^ ((unsigned long long)((long long)b >> 63) | 0x8000000000000000ull);  // branch-free: see ml_dec
+}
+__host__ __device__ inline double ml_dec(unsigned long long b) {
+    // branch-free (a select here costs the backward kernels 18 registers and 6 % more fp64 instructions)
+    b ^= (unsigned long long)((long long)~b >> 63) | 0x8000000000000000ull;
+    double v;
+    memcpy(&v, &b, sizeof v);
+    return v;
+}
 
 struct MLParams {
     int kind;  // sdpb_reached_kind
@@ -76,10 +112,7 @@ __host__ __device__ inline MLKey ml_key(const MLState& s) {
     MLKey k;
     k.a = ((unsigned long long)(unsigned)s.x1 << 48) | ((unsigned long long)(unsigned)s.x2 << 32) |
           ((unsigned long long)(unsigned)s.q1 << 16) | (unsigned long long)(unsigned)s.q2;
-    const double c = s.cash + 0.0;  // -0.0 and +0.0 are one key in the reference's map (compared with ==)
-    unsigned long long bits;
-    memcpy(&bits, &c, sizeof bits);
-    k.b = bits;
+    k.b = ml_enc(s.cash);
     return k;
 }
 
@@ -87,7 +120,7 @@ __host__ __device__ inline MLState ml_state(const MLKey& k) {
     MLState s;
     s.x1 = (int)((k.a >> 48) & 0xffff); s.x2 = (int)((k.a >> 32) & 0xffff);
     s.q1 = (int)((k.a >> 16) & 0xffff); s.q2 = (int)(k.a & 0xffff);
-    memcpy(&s.cash, &k.b, sizeof s.cash);
+    s.cash = ml_dec(k.b);
     return s;
 }
 
@@ -363,7 +396,376 @@ __global__ void ml_scan_pairs(MLParams P, const double* __restrict__ QV, long lo
     Qa[si] = best;
 }
 
+// the action getAction reports for a state with action index qi and value v: order quantities (i, j) for kinds 0 and 3,
+// order-up-to levels (x1 + i, x2 + j) for kinds 1 and 2; a state without any accepted action keeps the reference's
+// default, {0, 0} for kind 1 (new double[]{0, 0}) and (x1, x2) for kind 2 (bestYs = the offsets (0, 0))
+__host__ __device__ inline void ml_reported_action(int kind, int q2, const MLState& s, int qi, double v, double& a1,
+                                                   double& a2) {
+    const int ai = qi / q2, aj = qi % q2;
+    if (kind == 0 || kind == 3) { a1 = ai; a2 = aj; return; }
+    const bool none = v == -DBL_MAX;
+    a1 = kind == 1 && none ? 0.0 : (double)(s.x1 + ai);
+    a2 = kind == 1 && none ? 0.0 : (double)(s.x2 + aj);
+}
+
+// listed actions of each state summed into *total (kinds 2 and 3, whose lists depend on the state)
+__global__ void ml_count_actions(MLParams P, const MLKey* __restrict__ F, long long n, unsigned long long* __restrict__ total) {
+    const long long si = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (si >= n) return;
+    const MLState s = ml_state(F[si]);
+    unsigned long long c = 0;
+    for (int ai = 0; ai < P.Q * P.Q2; ai++) {
+        double a1, a2;
+        if (ml_action(P, s, ai, a1, a2)) c++;
+    }
+    atomicAdd(total, c);
+}
+
+// batched lookup: (V, action index) of each query key, action index -2 when the state is not in the sorted table F
+__global__ void ml_query(const MLKey* __restrict__ F, long long n, const double* __restrict__ V, const int* __restrict__ Qa,
+                         const MLKey* __restrict__ q, int nq, double* __restrict__ v, int* __restrict__ qi) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= nq) return;
+    const MLKey k = q[i];
+    const long long at = ml_find(F, n, k);
+    const bool hit = at < n && MLKeyEq()(F[at], k);
+    v[i] = hit ? V[at] : 0.0;
+    qi[i] = hit ? Qa[at] : -2;
+}
+
+// the filter of an extension: flag[i] = 1 when candidate i is already in the sorted table F
+__global__ void ml_known(const MLKey* __restrict__ F, long long n, const MLKey* __restrict__ c, long long m,
+                         unsigned char* __restrict__ flag) {
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= m) return;
+    const long long at = ml_find(F, n, c[i]);
+    flag[i] = at < n && MLKeyEq()(F[at], c[i]) ? 1 : 0;
+}
+
+// One thread per path of act[0, na): from where the path stands (period per[i], state key[i], partial sum sum[i]) --
+// (a1, a2) = getAction(state), d = Math.round(sample), sum += discount^(t-1) c(state, a, d) (salvage when t == T),
+// state = f(state, a, d, c) -- until it ends (values[i] = sum) or meets a state the handle has not reached.  There it
+// writes (path, t, state) to the next slot of the stall list, keeps its period, state and partial sum, and stops.
+// Kind 2 has no immediate value: a path is worth boundFinalCash of the state after period T.
+__global__ void __launch_bounds__(128) ml_simulate(MLParams P, const MLKey* const* __restrict__ tF,
+                                                   const double* const* __restrict__ tV, const int* const* __restrict__ tQ,
+                                                   const long long* __restrict__ tn, const double* __restrict__ samples,
+                                                   const int nd, const double* __restrict__ pw, const int* __restrict__ act,
+                                                   const int na, MLKey* __restrict__ key, int* __restrict__ per,
+                                                   double* __restrict__ sum, double* __restrict__ values,
+                                                   int* __restrict__ stall_n, int* __restrict__ stall_path,
+                                                   int* __restrict__ stall_t, MLKey* __restrict__ stall_key) {
+    const int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= na) return;
+    const int i = act[k], T = P.T;
+    MLKey s = key[i];
+    double acc = sum[i];
+    for (int t = per[i]; t <= T; t++) {
+        const MLKey* __restrict__ F = tF[t - 1];
+        const long long n = tn[t - 1];
+        const long long at = ml_find(F, n, s);
+        if (at >= n || !MLKeyEq()(F[at], s)) {
+            key[i] = s;
+            per[i] = t;
+            sum[i] = acc;
+            const int slot = atomicAdd(stall_n, 1);
+            stall_path[slot] = i;
+            stall_t[slot] = t;
+            stall_key[slot] = s;
+            return;
+        }
+        const MLState st = ml_state(s);
+        double a1, a2;
+        ml_reported_action(P.kind, P.Q2, st, tQ[t - 1][at], tV[t - 1][at], a1, a2);
+        const double* smp = samples + ((size_t)i * T + (t - 1)) * nd;
+        const double d1 = (double)ml_jround(smp[0]), d2 = nd > 1 ? (double)ml_jround(smp[1]) : 0.0;
+        const bool last = t == T;
+        if (P.kind == 2) {
+            const double iniR = (st.cash + P.v1 * (double)st.x1) + P.v2 * (double)st.x2;
+            const MLState nx = yr_transition(P, a1, a2, iniR, d1, d2);
+            if (last) acc = (nx.cash + P.sal1 * (double)nx.x1) + P.sal2 * (double)nx.x2;  // MultiItemYR.java:116-119
+            else s = ml_key(nx);
+            continue;
+        }
+        const double x3 = (double)st.x1 / P.sq;  // kind 3: the inventory value
+        const double c = P.kind == 0 ? ml_immediate(P, t, last, st, (int)a1, (int)a2, (int)d1, (int)d2)
+                       : P.kind == 1 ? xr_immediate(P, last, st, a1, a2, d1, d2)
+                                     : cct_immediate(P, last, x3, st.cash, a1, d1);
+        acc += pw[t - 1] * c;
+        if (!last)
+            s = ml_key(P.kind == 0 ? ml_transition(P, st, (int)a1, (int)a2, (int)d1, (int)d2, c)
+                       : P.kind == 1 ? xr_transition(P, st, a1, a2, d1, d2, c)
+                                     : cct_transition(P, x3, st.cash, a1, d1, c));
+    }
+    values[i] = acc;
+}
+
 thread_local std::string g_ml_error;
+
+int ml_fail(int rc, const std::string& msg) {
+    g_ml_error = msg;
+    return rc;
+}
+
+struct DevBuf {  // a scratch allocation released when it goes out of scope
+    void* p = nullptr;
+    ~DevBuf() { if (p) cudaFree(p); }
+    bool alloc(size_t bytes) {
+        if (p) { cudaFree(p); p = nullptr; }
+        if (cudaMalloc(&p, bytes > 0 ? bytes : 16) != cudaSuccess) { cudaGetLastError(); p = nullptr; return false; }
+        return true;
+    }
+};
+
+template <class T>
+bool ml_alloc(T*& p, long long n) {
+    if (cudaMalloc((void**)&p, (size_t)std::max(n, 1ll) * sizeof(T)) == cudaSuccess) return true;
+    cudaGetLastError();
+    p = nullptr;
+    return false;
+}
+
+}  // namespace
+
+struct sdpb_reached {
+    sdpb_reached_model m;  // scalars only: the caller's pointers are not kept
+    MLParams P{};
+    int device = 0;
+    int n_int = 4;  // API-order coordinates before the cash: 4 | 2 | 2 | 1
+    long long A = 0;
+    long long scratch_bytes = 0;
+    cudaStream_t stream = nullptr;
+    cudaEvent_t e0 = nullptr, e1 = nullptr, e2 = nullptr;
+    std::vector<int> lens;    // demand points of each period
+    std::vector<void*> owned; // model tables
+    std::vector<MLKey*> F;    // [T] reached states, sorted in memo-map order
+    std::vector<double*> V;   // [T]
+    std::vector<int*> Qa;     // [T] flat action index
+    std::vector<long long> nF;
+    sdpb_stats stats{};
+};
+
+namespace {
+
+// What one extension builds, owned here until it is committed to the handle: per period the new states N_t with their
+// V / Q, and the merged tables F_t u N_t.  Whatever is still owned when the stage goes out of scope is freed, so an
+// extension that fails leaves the handle as it found it.
+struct MLStage {
+    std::vector<MLKey*> N, MF;
+    std::vector<double*> VN, MV;
+    std::vector<int*> QN, MQ;
+    std::vector<long long> nN, nM;
+    explicit MLStage(int T)
+        : N(T, nullptr), MF(T, nullptr), VN(T, nullptr), MV(T, nullptr), QN(T, nullptr), MQ(T, nullptr), nN(T, 0), nM(T, 0) {}
+    ~MLStage() {
+        for (size_t k = 0; k < N.size(); k++) {
+            cudaFree(N[k]); cudaFree(MF[k]); cudaFree(VN[k]); cudaFree(MV[k]); cudaFree(QN[k]); cudaFree(MQ[k]);
+        }
+    }
+};
+
+// N_t: the sorted roots of period t and the successors of the n_src new states `src` of period t - 1, minus the states
+// the handle already holds in period t; sorted and unique, into a right-sized *out.  All candidates are expanded at
+// once: a period whose candidates, with the sort's scratch, would pass the budget fails with SDPB_ERR_NOMEM.
+int ml_new_states(sdpb_reached* h, int t, const MLKey* src, long long n_src, const std::vector<MLKey>& roots, MLKey** out,
+                  long long* n_out) {
+    *out = nullptr;
+    *n_out = 0;
+    const long long nr = (long long)roots.size(), pairs = n_src * h->A, cand = pairs * h->P.nD + nr;
+    if (cand == 0) return SDPB_OK;
+    cudaStream_t st = h->stream;
+    size_t free_b = 0, total_b = 0;
+    cudaMemGetInfo(&free_b, &total_b);
+    const double budget = h->scratch_bytes > 0 ? (double)h->scratch_bytes : (double)free_b;
+    if ((double)cand * sizeof(MLKey) * 2.2 > budget)
+        return ml_fail(SDPB_ERR_NOMEM, "period " + std::to_string(t) + " has " + std::to_string(cand) + " candidate states: more than " +
+                                           (h->scratch_bytes > 0 ? "a scratch budget of " + std::to_string(h->scratch_bytes) + " bytes"
+                                                                 : std::string("this GPU's memory")) + " holds");
+    DevBuf buf;
+    if (!buf.alloc((size_t)cand * sizeof(MLKey))) return ml_fail(SDPB_ERR_NOMEM, "allocation of the candidate states failed");
+    MLKey* c = (MLKey*)buf.p;
+    if (pairs > 0) {
+        ml_expand<<<(unsigned)((pairs + 127) / 128), 128, 0, st>>>(h->P, t - 1, src, n_src, c);
+        if (cudaGetLastError() != cudaSuccess) return ml_fail(SDPB_ERR_CUDA, "ml_expand launch failed");
+    }
+    if (nr > 0 && cudaMemcpyAsync(c + pairs * h->P.nD, roots.data(), (size_t)nr * sizeof(MLKey), cudaMemcpyHostToDevice, st) != cudaSuccess)
+        return ml_fail(SDPB_ERR_CUDA, "cudaMemcpyAsync failed");
+    long long m = 0;
+    const MLKey* Fo = h->F[t - 1];
+    const long long no = h->nF[t - 1];
+    try {
+        auto par = thrust::cuda::par.on(st);
+        thrust::sort(par, c, c + cand, MLKeyLess());
+        m = (long long)(thrust::unique(par, c, c + cand, MLKeyEq()) - c);
+        if (m > 0) {  // the slots of actions the reference's list does not contain sort last, as one key
+            MLKey tail;
+            if (cudaMemcpyAsync(&tail, c + m - 1, sizeof tail, cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+                cudaStreamSynchronize(st) != cudaSuccess)
+                return ml_fail(SDPB_ERR_CUDA, std::string("forward pass: ") + cudaGetErrorString(cudaGetLastError()));
+            if (tail.a == ~0ull && tail.b == ~0ull) m--;
+        }
+        if (m > 0 && no > 0) {  // keep what period t does not hold yet
+            DevBuf flag;
+            if (!flag.alloc((size_t)m)) return ml_fail(SDPB_ERR_NOMEM, "allocation of the filter flags failed");
+            ml_known<<<(unsigned)((m + 127) / 128), 128, 0, st>>>(Fo, no, c, m, (unsigned char*)flag.p);
+            if (cudaGetLastError() != cudaSuccess) return ml_fail(SDPB_ERR_CUDA, "ml_known launch failed");
+            m = (long long)(thrust::remove_if(par, c, c + m, (const unsigned char*)flag.p, MLFlagged()) - c);
+            if (cudaStreamSynchronize(st) != cudaSuccess) return ml_fail(SDPB_ERR_CUDA, "forward pass: filter");
+        }
+    } catch (const std::exception& ex) {
+        return ml_fail(SDPB_ERR_CUDA, std::string("sort / unique: ") + ex.what());
+    }
+    if (m == 0) return SDPB_OK;
+    if (!ml_alloc(*out, m)) return ml_fail(SDPB_ERR_NOMEM, "allocation of the states of period " + std::to_string(t) + " failed");
+    *n_out = m;
+    if (cudaMemcpyAsync(*out, c, (size_t)m * sizeof(MLKey), cudaMemcpyDeviceToDevice, st) != cudaSuccess ||
+        cudaStreamSynchronize(st) != cudaSuccess)
+        return ml_fail(SDPB_ERR_CUDA, std::string("forward pass: ") + cudaGetErrorString(cudaGetLastError()));
+    return SDPB_OK;
+}
+
+// sum over the n states F of period t of |listed actions| * D_t
+int ml_evals(sdpb_reached* h, int t, const MLKey* F, long long n, double& evals) {
+    const double D = h->lens[t - 1];
+    if (h->m.kind == SDPB_REACHED_MULTILEAD || h->m.kind == SDPB_REACHED_MULTI_XR) {  // every pair is listed
+        evals += (double)n * (double)h->A * D;
+        return SDPB_OK;
+    }
+    DevBuf tot;
+    unsigned long long listed = 0;
+    if (!tot.alloc(sizeof listed)) return ml_fail(SDPB_ERR_NOMEM, "allocation failed");
+    if (cudaMemsetAsync(tot.p, 0, sizeof listed, h->stream) != cudaSuccess) return ml_fail(SDPB_ERR_CUDA, "cudaMemsetAsync failed");
+    ml_count_actions<<<(unsigned)((n + 127) / 128), 128, 0, h->stream>>>(h->P, F, n, (unsigned long long*)tot.p);
+    if (cudaGetLastError() != cudaSuccess ||
+        cudaMemcpyAsync(&listed, tot.p, sizeof listed, cudaMemcpyDeviceToHost, h->stream) != cudaSuccess ||
+        cudaStreamSynchronize(h->stream) != cudaSuccess)
+        return ml_fail(SDPB_ERR_CUDA, std::string("counting the actions: ") + cudaGetErrorString(cudaGetLastError()));
+    evals += (double)listed * D;
+    return SDPB_OK;
+}
+
+// getExpectedValue on the states roots[t - 1] of every period t >= p (each sorted and unique; empty for t < p): the
+// forward pass builds the states no earlier call reached, the backward pass solves only those against the merged
+// tables of the next period, and the merged tables of every touched period replace the handle's at the end.
+int ml_extend(sdpb_reached* h, int p, const std::vector<std::vector<MLKey>>& roots) {
+    const int T = h->m.T;
+    const long long A = h->A;
+    cudaStream_t st = h->stream;
+    MLStage sg(T);
+    if (cudaEventRecord(h->e0, st) != cudaSuccess) return ml_fail(SDPB_ERR_CUDA, "cudaEventRecord failed");
+    double evals = 0;
+    for (int t = p; t <= T; t++) {
+        const int k = t - 1;
+        int rc = ml_new_states(h, t, t > p ? sg.N[k - 1] : nullptr, t > p ? sg.nN[k - 1] : 0, roots[k], &sg.N[k], &sg.nN[k]);
+        if (rc == SDPB_OK && sg.nN[k] > 0) rc = ml_evals(h, t, sg.N[k], sg.nN[k], evals);
+        if (rc != SDPB_OK) return rc;
+    }
+    if (cudaEventRecord(h->e1, st) != cudaSuccess) return ml_fail(SDPB_ERR_CUDA, "cudaEventRecord failed");
+    int launches = 0;
+    for (int t = T; t >= p; t--) {
+        const int k = t - 1;
+        const long long n = sg.nN[k], no = h->nF[k];
+        if (n == 0) continue;
+        if (!ml_alloc(sg.VN[k], n) || !ml_alloc(sg.QN[k], n)) return ml_fail(SDPB_ERR_NOMEM, "allocation of the value table failed");
+        const bool nxt = t < T, nxt_new = nxt && sg.nN[k + 1] > 0;
+        const MLKey* Fn = nxt ? (nxt_new ? sg.MF[k + 1] : h->F[k + 1]) : nullptr;
+        const double* Vn = nxt ? (nxt_new ? sg.MV[k + 1] : h->V[k + 1]) : nullptr;
+        const long long nFn = nxt ? (nxt_new ? sg.nM[k + 1] : h->nF[k + 1]) : 0;
+        DevBuf qv;
+        if (n * A <= 200000000LL && n < 50000) {  // few states: spread their actions over the GPU
+            if (!qv.alloc((size_t)(n * A) * sizeof(double))) return ml_fail(SDPB_ERR_NOMEM, "allocation of the action-value scratch failed");
+            ml_backward_pairs<<<(unsigned)((n * A + 127) / 128), 128, 0, st>>>(h->P, t, sg.N[k], n, Fn, Vn, nFn, (double*)qv.p);
+            ml_scan_pairs<<<(unsigned)((n + 127) / 128), 128, 0, st>>>(h->P, (const double*)qv.p, n, sg.VN[k], sg.QN[k]);
+            launches += 2;
+        } else {
+            ml_backward_state<<<(unsigned)((n + 127) / 128), 128, 0, st>>>(h->P, t, sg.N[k], n, Fn, Vn, nFn, sg.VN[k], sg.QN[k]);
+            launches++;
+        }
+        if (cudaGetLastError() != cudaSuccess) return ml_fail(SDPB_ERR_CUDA, "backward launch failed");
+        sg.nM[k] = no + n;
+        if (no == 0) {  // nothing to merge with: the new tables are the merged ones
+            std::swap(sg.MF[k], sg.N[k]);
+            std::swap(sg.MV[k], sg.VN[k]);
+            std::swap(sg.MQ[k], sg.QN[k]);
+            continue;
+        }
+        if (!ml_alloc(sg.MF[k], no + n) || !ml_alloc(sg.MV[k], no + n) || !ml_alloc(sg.MQ[k], no + n))
+            return ml_fail(SDPB_ERR_NOMEM, "allocation of the merged tables of period " + std::to_string(t) + " failed");
+        try {  // the two key sets are disjoint: a merge by key keeps every row
+            thrust::merge_by_key(thrust::cuda::par.on(st), h->F[k], h->F[k] + no, sg.N[k], sg.N[k] + n,
+                                 thrust::make_zip_iterator(thrust::make_tuple(h->V[k], h->Qa[k])),
+                                 thrust::make_zip_iterator(thrust::make_tuple(sg.VN[k], sg.QN[k])), sg.MF[k],
+                                 thrust::make_zip_iterator(thrust::make_tuple(sg.MV[k], sg.MQ[k])), MLKeyLess());
+        } catch (const std::exception& ex) {
+            return ml_fail(SDPB_ERR_CUDA, std::string("merge: ") + ex.what());
+        }
+    }
+    if (cudaEventRecord(h->e2, st) != cudaSuccess || cudaEventSynchronize(h->e2) != cudaSuccess)
+        return ml_fail(SDPB_ERR_CUDA, std::string("backward pass: ") + cudaGetErrorString(cudaGetLastError()));
+    for (int k = p - 1; k < T; k++) {  // commit
+        if (sg.nN[k] == 0) continue;
+        cudaFree(h->F[k]);
+        cudaFree(h->V[k]);
+        cudaFree(h->Qa[k]);
+        h->F[k] = sg.MF[k];
+        h->V[k] = sg.MV[k];
+        h->Qa[k] = sg.MQ[k];
+        sg.MF[k] = nullptr;
+        sg.MV[k] = nullptr;
+        sg.MQ[k] = nullptr;
+        h->nF[k] = sg.nM[k];
+    }
+    float solve = 0, kern = 0;
+    cudaEventElapsedTime(&solve, h->e0, h->e2);
+    cudaEventElapsedTime(&kern, h->e1, h->e2);
+    h->stats.evals += evals;
+    h->stats.evals_executed += evals;
+    h->stats.solve_ms = solve;
+    h->stats.kernel_ms = kern;
+    h->stats.launches = launches;
+    return SDPB_OK;
+}
+
+// The key of one API-order state: false when it has no key (an inventory or pipeline quantity that is not an integer
+// in [0, 65535], or for kind 3 not k / state_q with such a k).  Coordinates must be finite.
+bool ml_encode(const sdpb_reached* h, const double* s, MLKey& key) {
+    double k[4] = {0, 0, 0, 0};
+    for (int c = 0; c < h->n_int; c++) {
+        k[c] = s[c];
+        if (h->m.kind == SDPB_REACHED_CASH_ROUNDED) {  // the inventory is kept as k = round(x * q); x must be k / q exactly
+            k[c] = std::floor(s[c] * h->m.state_q + 0.5);
+            if (k[c] / h->m.state_q != s[c]) return false;
+        }
+        if (!(k[c] >= 0 && k[c] <= 65535) || k[c] != (double)(int)k[c]) return false;
+    }
+    MLState st;
+    st.x1 = (int)k[0]; st.x2 = (int)k[1]; st.q1 = (int)k[2]; st.q2 = (int)k[3];
+    st.cash = s[h->n_int];
+    key = ml_key(st);
+    return true;
+}
+
+bool ml_finite(const double* s, size_t n) {
+    for (size_t i = 0; i < n; i++)
+        if (!std::isfinite(s[i])) return false;
+    return true;
+}
+
+// n API-order roots -> their keys, sorted and unique: SDPB_ERR_ARG for a coordinate that is not finite,
+// SDPB_ERR_OFFGRID for a state without a key
+int ml_root_keys(const sdpb_reached* h, const double* states, int n, std::vector<MLKey>& out) {
+    const int nd = h->n_int + 1;
+    if (!ml_finite(states, (size_t)n * nd)) return ml_fail(SDPB_ERR_ARG, "a state coordinate is not finite");
+    out.resize((size_t)n);
+    for (int i = 0; i < n; i++)
+        if (!ml_encode(h, states + (size_t)i * nd, out[i]))
+            return ml_fail(SDPB_ERR_OFFGRID, h->m.kind == SDPB_REACHED_CASH_ROUNDED
+                                                 ? "the inventory of a state is not of the form k / state_q, k in [0, 65535]"
+                                                 : "inventories and pipeline quantities must be integers in [0, 65535]");
+    std::sort(out.begin(), out.end(), MLKeyLess());
+    out.erase(std::unique(out.begin(), out.end(), MLKeyEq()), out.end());
+    return SDPB_OK;
+}
 
 }  // namespace
 
@@ -371,64 +773,72 @@ extern "C" {
 
 const char* sdpb_reached_last_error(void) { return g_ml_error.c_str(); }
 
-int sdpb_reached_solve(const sdpb_reached_model* m, int device, const double* init_state, double* value, double* action1,
-                       double* action2, int64_t* n_states, double* solve_ms) {
-    g_ml_error.clear();
-    auto fail = [&](int rc, const std::string& msg) { g_ml_error = msg; return rc; };
-    if (!m || !init_state || m->struct_size != sizeof(sdpb_reached_model)) return fail(SDPB_ERR_ARG, "bad argument / struct_size");
-    if (m->kind < SDPB_REACHED_MULTILEAD || m->kind > SDPB_REACHED_CASH_ROUNDED) return fail(SDPB_ERR_ARG, "bad kind");
-    if (m->kind == SDPB_REACHED_CASH_ROUNDED && !(m->state_q > 0.0 && m->vari_cost[0] > 0.0)) return fail(SDPB_ERR_ARG, "CASH_ROUNDED needs state_q > 0 and a positive unit cost");
-    if (m->T < 1 || m->q_bound < 1 || m->q_bound > 65535 || m->n_demands < 1 || !m->d1 || !m->d2 || !m->p || !m->overhead_t)
-        return fail(SDPB_ERR_ARG, "T, q_bound, n_demands must be positive and the tables non-null");
-    // init_state: kind 0 (x1, x2, preQ1, preQ2, cash); kind 1 (x1, x2, R); kind 2 (x1, x2, cash)
-    const int n_int = m->kind == SDPB_REACHED_MULTILEAD ? 4 : (m->kind == SDPB_REACHED_CASH_ROUNDED ? 1 : 2);
-    double init_k[4] = {0, 0, 0, 0};
-    for (int k = 0; k < n_int; k++) {
-        init_k[k] = init_state[k];
-        if (m->kind == SDPB_REACHED_CASH_ROUNDED) {  // the inventory is kept as k = round(x * q); x must be k / q exactly
-            init_k[k] = std::floor(init_state[k] * m->state_q + 0.5);
-            if (init_k[k] / m->state_q != init_state[k]) return fail(SDPB_ERR_OFFGRID, "the initial inventory is not of the form k / state_q");
-        }
-        if (init_k[k] != (double)(int)init_k[k] || init_k[k] < 0 || init_k[k] > 65535)
-            return fail(SDPB_ERR_OFFGRID, "initial inventories and pipeline quantities must be integers in [0, 65535]");
-    }
-    if (!(m->max_inv <= 65535.0)) return fail(SDPB_ERR_ARG, "max_inv must fit 16 bits");
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) { cudaGetLastError(); return fail(SDPB_ERR_NO_DEVICE, "no CUDA device (libsdpb200 has no CPU path)"); }
-    if (device < 0) cudaGetDevice(&device);
-    if (device >= ndev || cudaSetDevice(device) != cudaSuccess) return fail(SDPB_ERR_NO_DEVICE, "cannot select the CUDA device");
+void sdpb_reached_destroy(sdpb_reached* h) {
+    if (!h) return;
+    cudaSetDevice(h->device);
+    for (MLKey* p : h->F) cudaFree(p);
+    for (double* p : h->V) cudaFree(p);
+    for (int* p : h->Qa) cudaFree(p);
+    for (void* p : h->owned) cudaFree(p);
+    if (h->e0) cudaEventDestroy(h->e0);
+    if (h->e1) cudaEventDestroy(h->e1);
+    if (h->e2) cudaEventDestroy(h->e2);
+    if (h->stream) cudaStreamDestroy(h->stream);
+    cudaGetLastError();
+    delete h;
+}
 
+int sdpb_reached_open(const sdpb_reached_model* m, int device, int64_t scratch_bytes, const double* init_states, int n,
+                      sdpb_reached** out) {
+    g_ml_error.clear();
+    if (!m || !out || n < 0 || (n > 0 && !init_states) || m->struct_size != sizeof(sdpb_reached_model))
+        return ml_fail(SDPB_ERR_ARG, "bad argument / struct_size");
+    *out = nullptr;
+    if (scratch_bytes < 0) return ml_fail(SDPB_ERR_ARG, "scratch_bytes < 0");
+    if (m->kind < SDPB_REACHED_MULTILEAD || m->kind > SDPB_REACHED_CASH_ROUNDED) return ml_fail(SDPB_ERR_ARG, "bad kind");
+    if (m->kind == SDPB_REACHED_CASH_ROUNDED && !(m->state_q > 0.0 && m->vari_cost[0] > 0.0)) return ml_fail(SDPB_ERR_ARG, "CASH_ROUNDED needs state_q > 0 and a positive unit cost");
+    if (m->T < 1 || m->q_bound < 1 || m->q_bound > 65535 || m->n_demands < 1 || !m->d1 || !m->d2 || !m->p || !m->overhead_t)
+        return ml_fail(SDPB_ERR_ARG, "T, q_bound, n_demands must be positive and the tables non-null");
+    if (!(m->max_inv <= 65535.0)) return ml_fail(SDPB_ERR_ARG, "max_inv must fit 16 bits");
     const int T = m->T, nD = m->n_demands;
+    std::vector<int> lens(T, nD);
+    if (m->n_demands_t)
+        for (int t = 0; t < T; t++) {
+            if (m->n_demands_t[t] < 1 || m->n_demands_t[t] > nD) return ml_fail(SDPB_ERR_ARG, "n_demands_t out of range");
+            lens[t] = m->n_demands_t[t];
+        }
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) { cudaGetLastError(); return ml_fail(SDPB_ERR_NO_DEVICE, "no CUDA device (libsdpb200 has no CPU path)"); }
+    if (device < 0) cudaGetDevice(&device);
+    if (device >= ndev || cudaSetDevice(device) != cudaSuccess) return ml_fail(SDPB_ERR_NO_DEVICE, "cannot select the CUDA device");
+
+    sdpb_reached* h = new (std::nothrow) sdpb_reached();
+    if (!h) return ml_fail(SDPB_ERR_NOMEM, "out of host memory");
+    h->m = *m;
+    h->device = device;
+    h->scratch_bytes = scratch_bytes;
+    h->lens = lens;
+    h->n_int = m->kind == SDPB_REACHED_MULTILEAD ? 4 : (m->kind == SDPB_REACHED_CASH_ROUNDED ? 1 : 2);
     const int q2 = m->kind == SDPB_REACHED_CASH_ROUNDED ? 1 : m->q_bound;
-    const long long A = (long long)m->q_bound * q2;
+    h->A = (long long)m->q_bound * q2;
+    h->F.assign(T, nullptr);
+    h->V.assign(T, nullptr);
+    h->Qa.assign(T, nullptr);
+    h->nF.assign(T, 0);
+    auto bail = [&](int rc, const std::string& msg) { sdpb_reached_destroy(h); return ml_fail(rc, msg); };
+    if (cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking) != cudaSuccess || cudaEventCreate(&h->e0) != cudaSuccess ||
+        cudaEventCreate(&h->e1) != cudaSuccess || cudaEventCreate(&h->e2) != cudaSuccess)
+        return bail(SDPB_ERR_CUDA, "stream / event creation failed");
     std::vector<double> pg((size_t)T * nD);
     for (size_t i = 0; i < pg.size(); i++) pg[i] = m->p[i] * m->gamma;  // first product of p * gamma * V
-    std::vector<void*> owned;
-    cudaStream_t stream = nullptr;
-    cudaEvent_t e0 = nullptr, e1 = nullptr;
-    auto cleanup = [&]() {
-        for (void* p : owned) cudaFree(p);
-        if (e0) cudaEventDestroy(e0);
-        if (e1) cudaEventDestroy(e1);
-        if (stream) cudaStreamDestroy(stream);
-        cudaGetLastError();
-    };
-    auto dalloc = [&](size_t bytes) -> void* {
+    auto upload = [&](const void* src, size_t bytes) -> void* {
         void* p = nullptr;
-        if (cudaMalloc(&p, bytes > 0 ? bytes : 16) != cudaSuccess) { cudaGetLastError(); return nullptr; }
-        owned.push_back(p);
+        if (cudaMalloc(&p, bytes) != cudaSuccess) { cudaGetLastError(); return nullptr; }
+        h->owned.push_back(p);
+        if (cudaMemcpyAsync(p, src, bytes, cudaMemcpyHostToDevice, h->stream) != cudaSuccess) return nullptr;
         return p;
     };
-#define ML_CU(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { const std::string msg_ = std::string(#call) + ": " + cudaGetErrorString(e_); cleanup(); return fail(SDPB_ERR_CUDA, msg_); } } while (0)
-    ML_CU(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking));
-    ML_CU(cudaEventCreate(&e0));
-    ML_CU(cudaEventCreate(&e1));
-    auto upload = [&](const double* src, size_t n) -> double* {
-        double* p = (double*)dalloc(n * sizeof(double));
-        if (p && cudaMemcpyAsync(p, src, n * sizeof(double), cudaMemcpyHostToDevice, stream) != cudaSuccess) return nullptr;
-        return p;
-    };
-    MLParams P;
+    MLParams& P = h->P;
     P.kind = m->kind; P.dr = m->deposit_rate;
     P.K = m->fixed_cost; P.h = m->hold_cost; P.min_cash_req = m->min_cash_required; P.sq = m->state_q > 0.0 ? m->state_q : 1.0;
     P.T = T; P.Q = m->q_bound; P.Q2 = q2; P.nD = nD;
@@ -437,110 +847,246 @@ int sdpb_reached_solve(const sdpb_reached_model* m, int device, const double* in
     P.r0 = m->r0; P.r1 = m->r1; P.r2 = m->r2; P.limit = m->limit; P.interest_free = m->interest_free;
     P.min_inv = m->min_inv; P.max_inv = m->max_inv; P.min_cash = m->min_cash; P.max_cash = m->max_cash;
     P.gamma = m->gamma; P.tie = m->tie_tolerance;
-    P.d1 = upload(m->d1, (size_t)T * nD); P.d2 = upload(m->d2, (size_t)T * nD); P.p = upload(m->p, (size_t)T * nD);
-    P.pg = upload(pg.data(), pg.size()); P.ovh = upload(m->overhead_t, (size_t)T);
-    {
-        std::vector<int> lens(T, nD);
-        if (m->n_demands_t)
-            for (int t = 0; t < T; t++) {
-                if (m->n_demands_t[t] < 1 || m->n_demands_t[t] > nD) { cleanup(); return fail(SDPB_ERR_ARG, "n_demands_t out of range"); }
-                lens[t] = m->n_demands_t[t];
-            }
-        int* dl = (int*)dalloc((size_t)T * sizeof(int));
-        if (dl && cudaMemcpyAsync(dl, lens.data(), (size_t)T * sizeof(int), cudaMemcpyHostToDevice, stream) != cudaSuccess) dl = nullptr;
-        if (dl) cudaStreamSynchronize(stream);  // (lens is a local)
-        P.nDt = dl;
-    }
-    if (!P.d1 || !P.d2 || !P.p || !P.pg || !P.ovh || !P.nDt) { cleanup(); return fail(SDPB_ERR_NOMEM, "allocation of the model tables failed"); }
-    ML_CU(cudaEventRecord(e0, stream));
+    const size_t tab = (size_t)T * nD * sizeof(double);
+    P.d1 = (const double*)upload(m->d1, tab); P.d2 = (const double*)upload(m->d2, tab); P.p = (const double*)upload(m->p, tab);
+    P.pg = (const double*)upload(pg.data(), tab); P.ovh = (const double*)upload(m->overhead_t, (size_t)T * sizeof(double));
+    P.nDt = (const int*)upload(lens.data(), (size_t)T * sizeof(int));
+    if (!P.d1 || !P.d2 || !P.p || !P.pg || !P.ovh || !P.nDt) return bail(SDPB_ERR_NOMEM, "allocation of the model tables failed");
+    if (cudaStreamSynchronize(h->stream) != cudaSuccess) return bail(SDPB_ERR_CUDA, "uploading the model tables failed");  // (pg, lens are locals)
 
-    // ---- forward: the states the reference's recursion visits, period by period ----
-    size_t free_b = 0, total_b = 0;
-    cudaMemGetInfo(&free_b, &total_b);
-    std::vector<MLKey*> F(T, nullptr);
-    std::vector<long long> nF(T, 0);
-    MLState s0;
-    s0.x1 = (int)init_k[0]; s0.x2 = n_int >= 2 ? (int)init_k[1] : 0;
-    s0.q1 = n_int == 4 ? (int)init_k[2] : 0; s0.q2 = n_int == 4 ? (int)init_k[3] : 0;
-    s0.cash = init_state[n_int];
-    const MLKey k0 = ml_key(s0);
-    F[0] = (MLKey*)dalloc(sizeof(MLKey));
-    if (!F[0]) { cleanup(); return fail(SDPB_ERR_NOMEM, "allocation failed"); }
-    ML_CU(cudaMemcpyAsync(F[0], &k0, sizeof k0, cudaMemcpyHostToDevice, stream));
-    nF[0] = 1;
-    for (int t = 1; t < T; t++) {
-        const long long cand = nF[t - 1] * A * nD;
-        if ((double)cand * sizeof(MLKey) * 2.2 > (double)free_b) {
-            cleanup();
-            return fail(SDPB_ERR_NOMEM, "period " + std::to_string(t + 1) + " has " + std::to_string(cand) +
-                                            " candidate states: more than this GPU's memory holds");
-        }
-        MLKey* buf = (MLKey*)dalloc((size_t)cand * sizeof(MLKey));
-        if (!buf) { cleanup(); return fail(SDPB_ERR_NOMEM, "allocation of the candidate states failed"); }
-        const long long pairs = nF[t - 1] * A;
-        ml_expand<<<(unsigned)((pairs + 127) / 128), 128, 0, stream>>>(P, t, F[t - 1], nF[t - 1], buf);
-        ML_CU(cudaGetLastError());
-        try {
-            thrust::sort(thrust::cuda::par.on(stream), buf, buf + cand, MLKeyLess());
-            MLKey* end = thrust::unique(thrust::cuda::par.on(stream), buf, buf + cand, MLKeyEq());
-            nF[t] = (long long)(end - buf);
-            if (nF[t] > 0) {  // the slots of actions the reference's list does not contain sort last, as one key
-                MLKey tail;
-                if (cudaMemcpyAsync(&tail, buf + nF[t] - 1, sizeof tail, cudaMemcpyDeviceToHost, stream) == cudaSuccess &&
-                    cudaStreamSynchronize(stream) == cudaSuccess && tail.a == ~0ull && tail.b == ~0ull)
-                    nF[t]--;
-            }
-        } catch (const std::exception& ex) {
-            const std::string msg = std::string("sort / unique: ") + ex.what();
-            cleanup();
-            return fail(SDPB_ERR_CUDA, msg);
-        }
-        F[t] = buf;
-        cudaMemGetInfo(&free_b, &total_b);
+    std::vector<std::vector<MLKey>> roots((size_t)T);
+    int rc = ml_root_keys(h, init_states, n, roots[0]);
+    if (rc == SDPB_OK && n > 0) rc = ml_extend(h, 1, roots);
+    if (rc != SDPB_OK) {
+        const std::string msg = g_ml_error;
+        return bail(rc, msg);
     }
-
-    // ---- backward ----
-    std::vector<double*> V(T, nullptr);
-    std::vector<int*> Qa(T, nullptr);
-    for (int t = T; t >= 1; t--) {
-        const long long n = nF[t - 1];
-        V[t - 1] = (double*)dalloc((size_t)n * sizeof(double));
-        Qa[t - 1] = (int*)dalloc((size_t)n * sizeof(int));
-        if (!V[t - 1] || !Qa[t - 1]) { cleanup(); return fail(SDPB_ERR_NOMEM, "allocation of the value table failed"); }
-        const MLKey* Fn = t < T ? F[t] : nullptr;
-        const double* Vn = t < T ? V[t] : nullptr;
-        const long long nFn = t < T ? nF[t] : 0;
-        if (n * A <= 200000000LL && n < 50000) {  // few states: spread their actions over the GPU
-            double* QV = (double*)dalloc((size_t)(n * A) * sizeof(double));
-            if (!QV) { cleanup(); return fail(SDPB_ERR_NOMEM, "allocation of the action-value scratch failed"); }
-            ml_backward_pairs<<<(unsigned)((n * A + 127) / 128), 128, 0, stream>>>(P, t, F[t - 1], n, Fn, Vn, nFn, QV);
-            ml_scan_pairs<<<(unsigned)((n + 127) / 128), 128, 0, stream>>>(P, QV, n, V[t - 1], Qa[t - 1]);
-        } else {
-            ml_backward_state<<<(unsigned)((n + 127) / 128), 128, 0, stream>>>(P, t, F[t - 1], n, Fn, Vn, nFn, V[t - 1], Qa[t - 1]);
-        }
-        ML_CU(cudaGetLastError());
-    }
-    ML_CU(cudaEventRecord(e1, stream));
-    double v0 = 0;
-    int a0 = 0;
-    ML_CU(cudaMemcpyAsync(&v0, V[0], sizeof v0, cudaMemcpyDeviceToHost, stream));
-    ML_CU(cudaMemcpyAsync(&a0, Qa[0], sizeof a0, cudaMemcpyDeviceToHost, stream));
-    ML_CU(cudaStreamSynchronize(stream));
-    float ms = 0;
-    cudaEventElapsedTime(&ms, e0, e1);
-#undef ML_CU
-    if (value) *value = v0;
-    // kind 0: order quantities (i, j); kinds 1, 2: order-up-to levels (x1 + i, x2 + j) (bestYs; the reference's default
-    // for a state without any accepted action is {0, 0} for kind 1 and (x1, x2) for kind 2)
-    const int ai = a0 / q2, aj = a0 % q2;
-    const bool none = v0 == -DBL_MAX;
-    const bool qty = m->kind == SDPB_REACHED_MULTILEAD || m->kind == SDPB_REACHED_CASH_ROUNDED;  // order quantities
-    if (action1) *action1 = qty ? ai : (m->kind == SDPB_REACHED_MULTI_XR && none ? 0.0 : s0.x1 + ai);
-    if (action2) *action2 = qty ? aj : (m->kind == SDPB_REACHED_MULTI_XR && none ? 0.0 : s0.x2 + aj);
-    if (n_states) for (int t = 0; t < T; t++) n_states[t] = nF[t];
-    if (solve_ms) *solve_ms = ms;
-    cleanup();
+    *out = h;
     return SDPB_OK;
+}
+
+int sdpb_reached_value(sdpb_reached* h, int period, const double* states, int n, double* v, double* a1, double* a2) {
+    g_ml_error.clear();
+    if (!h) return ml_fail(SDPB_ERR_ARG, "null handle");
+    if (period < 1 || period > h->m.T || n < 0 || (n > 0 && !states)) return ml_fail(SDPB_ERR_ARG, "bad period or states");
+    if (n == 0) return SDPB_OK;
+    const int nd = h->n_int + 1;
+    if (!ml_finite(states, (size_t)n * nd)) return ml_fail(SDPB_ERR_ARG, "a state coordinate is not finite");
+    std::vector<MLKey> keys((size_t)n);
+    for (int i = 0; i < n; i++)
+        if (!ml_encode(h, states + (size_t)i * nd, keys[i]))
+            return ml_fail(SDPB_ERR_UNSOLVED, "state " + std::to_string(i) + " was not reached in period " + std::to_string(period));
+    cudaSetDevice(h->device);
+    DevBuf kq, vq, aq;
+    if (!kq.alloc(keys.size() * sizeof(MLKey)) || !vq.alloc((size_t)n * sizeof(double)) || !aq.alloc((size_t)n * sizeof(int)))
+        return ml_fail(SDPB_ERR_NOMEM, "allocation failed");
+    std::vector<double> vv((size_t)n);
+    std::vector<int> qi((size_t)n);
+    cudaStream_t st = h->stream;
+    if (cudaMemcpyAsync(kq.p, keys.data(), keys.size() * sizeof(MLKey), cudaMemcpyHostToDevice, st) != cudaSuccess)
+        return ml_fail(SDPB_ERR_CUDA, "cudaMemcpyAsync failed");
+    ml_query<<<(n + 127) / 128, 128, 0, st>>>(h->F[period - 1], h->nF[period - 1], h->V[period - 1], h->Qa[period - 1],
+                                               (const MLKey*)kq.p, n, (double*)vq.p, (int*)aq.p);
+    if (cudaGetLastError() != cudaSuccess ||
+        cudaMemcpyAsync(vv.data(), vq.p, (size_t)n * sizeof(double), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+        cudaMemcpyAsync(qi.data(), aq.p, (size_t)n * sizeof(int), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+        cudaStreamSynchronize(st) != cudaSuccess)
+        return ml_fail(SDPB_ERR_CUDA, std::string("query: ") + cudaGetErrorString(cudaGetLastError()));
+    for (int i = 0; i < n; i++)
+        if (qi[i] == -2)
+            return ml_fail(SDPB_ERR_UNSOLVED, "state " + std::to_string(i) + " was not reached in period " + std::to_string(period));
+    for (int i = 0; i < n; i++) {
+        double b1, b2;
+        ml_reported_action(h->m.kind, h->P.Q2, ml_state(keys[i]), qi[i], vv[i], b1, b2);
+        if (v) v[i] = vv[i];
+        if (a1) a1[i] = b1;
+        if (a2) a2[i] = b2;
+    }
+    return SDPB_OK;
+}
+
+int sdpb_reached_extend(sdpb_reached* h, int period, const double* states, int n) {
+    g_ml_error.clear();
+    if (!h) return ml_fail(SDPB_ERR_ARG, "null handle");
+    if (period < 1 || period > h->m.T || n < 0 || (n > 0 && !states)) return ml_fail(SDPB_ERR_ARG, "bad period or states");
+    if (n == 0) return SDPB_OK;
+    std::vector<std::vector<MLKey>> roots((size_t)h->m.T);
+    const int rc = ml_root_keys(h, states, n, roots[period - 1]);
+    if (rc != SDPB_OK) return rc;
+    cudaSetDevice(h->device);
+    return ml_extend(h, period, roots);
+}
+
+int sdpb_reached_opt_table(sdpb_reached* h, double* rows, size_t* nrows) {
+    g_ml_error.clear();
+    if (!h || !nrows) return ml_fail(SDPB_ERR_ARG, "null argument");
+    size_t total = 0;
+    for (int t = 0; t < h->m.T; t++) total += (size_t)h->nF[t];
+    if (!rows) { *nrows = total; return SDPB_OK; }
+    if (*nrows < total) return ml_fail(SDPB_ERR_ARG, "rows holds fewer than the reached states");
+    cudaSetDevice(h->device);
+    const int nd = h->n_int + 1, w = nd + 3;
+    size_t r = 0;
+    for (int t = 1; t <= h->m.T; t++) {  // the device order is the memo-map order: a straight copy
+        const long long n = h->nF[t - 1];
+        std::vector<MLKey> k((size_t)n);
+        std::vector<double> v((size_t)n);
+        std::vector<int> qi((size_t)n);
+        if (cudaMemcpyAsync(k.data(), h->F[t - 1], (size_t)n * sizeof(MLKey), cudaMemcpyDeviceToHost, h->stream) != cudaSuccess ||
+            cudaMemcpyAsync(v.data(), h->V[t - 1], (size_t)n * sizeof(double), cudaMemcpyDeviceToHost, h->stream) != cudaSuccess ||
+            cudaMemcpyAsync(qi.data(), h->Qa[t - 1], (size_t)n * sizeof(int), cudaMemcpyDeviceToHost, h->stream) != cudaSuccess ||
+            cudaStreamSynchronize(h->stream) != cudaSuccess)
+            return ml_fail(SDPB_ERR_CUDA, "cudaMemcpyAsync failed");
+        for (long long i = 0; i < n; i++, r++) {
+            const MLState s = ml_state(k[i]);
+            double* row = rows + r * w;
+            int c = 0;
+            row[c++] = t;
+            if (h->m.kind == SDPB_REACHED_CASH_ROUNDED) {
+                row[c++] = (double)s.x1 / h->P.sq;
+            } else {
+                row[c++] = s.x1;
+                row[c++] = s.x2;
+                if (h->m.kind == SDPB_REACHED_MULTILEAD) { row[c++] = s.q1; row[c++] = s.q2; }
+            }
+            row[c++] = s.cash;
+            ml_reported_action(h->m.kind, h->P.Q2, s, qi[i], v[i], row[c], row[c + 1]);
+        }
+    }
+    *nrows = total;
+    return SDPB_OK;
+}
+
+int sdpb_reached_states(const sdpb_reached* h, int64_t* n_states) {
+    g_ml_error.clear();
+    if (!h || !n_states) return ml_fail(SDPB_ERR_ARG, "null argument");
+    for (int t = 0; t < h->m.T; t++) n_states[t] = h->nF[t];
+    return SDPB_OK;
+}
+
+int sdpb_reached_stats(const sdpb_reached* h, sdpb_stats* s) {
+    g_ml_error.clear();
+    if (!h || !s) return ml_fail(SDPB_ERR_ARG, "null argument");
+    *s = h->stats;
+    return SDPB_OK;
+}
+
+int sdpb_reached_simulate(sdpb_reached* h, const double* init_state, const double* samples, int n, double discount,
+                          double* values) {
+    g_ml_error.clear();
+    if (!h) return ml_fail(SDPB_ERR_ARG, "null handle");
+    if (!init_state || !samples || !values || n < 1) return ml_fail(SDPB_ERR_ARG, "null argument or n < 1");
+    if (h->m.kind == SDPB_REACHED_MULTI_YR && discount != 1.0)
+        return ml_fail(SDPB_ERR_ARG, "the V / Pi form values a path by boundFinalCash alone: discount must be 1");
+    if (!std::isfinite(discount)) return ml_fail(SDPB_ERR_ARG, "discount is not finite");
+    const int T = h->m.T, nd = h->m.kind == SDPB_REACHED_CASH_ROUNDED ? 1 : 2;
+    const size_t N = (size_t)n;
+    if (!ml_finite(samples, N * T * nd)) return ml_fail(SDPB_ERR_ARG, "a sample is not finite");
+    std::vector<std::vector<MLKey>> roots((size_t)T);
+    int rc = ml_root_keys(h, init_state, 1, roots[0]);
+    if (rc != SDPB_OK) return rc;
+    const MLKey k0 = roots[0][0];
+    const auto w0 = std::chrono::steady_clock::now();
+    cudaSetDevice(h->device);
+    rc = ml_extend(h, 1, roots);  // getExpectedValue(iniState) first
+    if (rc != SDPB_OK) return rc;
+
+    cudaStream_t st = h->stream;
+    std::vector<double> pw((size_t)T);
+    for (int t = 0; t < T; t++) pw[t] = std::pow(discount, (double)t);  // Math.pow(discountFactor, t)
+    std::vector<MLKey> key0(N, k0);
+    std::vector<int> per0(N, 1), act0(N);
+    for (int i = 0; i < n; i++) act0[i] = i;
+    DevBuf smp_b, pw_b, key_b, per_b, sum_b, val_b, act_b[2], st_b, sk_b, sn_b, tab_b;
+    if (!smp_b.alloc(N * T * nd * sizeof(double)) || !pw_b.alloc(T * sizeof(double)) || !key_b.alloc(N * sizeof(MLKey)) ||
+        !per_b.alloc(N * sizeof(int)) || !sum_b.alloc(N * sizeof(double)) || !val_b.alloc(N * sizeof(double)) ||
+        !act_b[0].alloc(N * sizeof(int)) || !act_b[1].alloc(N * sizeof(int)) || !st_b.alloc(N * sizeof(int)) ||
+        !sk_b.alloc(N * sizeof(MLKey)) || !sn_b.alloc(sizeof(int)) || !tab_b.alloc((size_t)T * 4 * 8))
+        return ml_fail(SDPB_ERR_NOMEM, "allocation of the roll-out buffers failed");
+    const MLKey** dF = (const MLKey**)tab_b.p;
+    const double** dV = (const double**)(dF + T);
+    const int** dQ = (const int**)(dV + T);
+    long long* dn = (long long*)(dQ + T);
+    if (cudaMemcpyAsync(smp_b.p, samples, N * T * nd * sizeof(double), cudaMemcpyHostToDevice, st) != cudaSuccess ||
+        cudaMemcpyAsync(pw_b.p, pw.data(), T * sizeof(double), cudaMemcpyHostToDevice, st) != cudaSuccess ||
+        cudaMemcpyAsync(key_b.p, key0.data(), N * sizeof(MLKey), cudaMemcpyHostToDevice, st) != cudaSuccess ||
+        cudaMemcpyAsync(per_b.p, per0.data(), N * sizeof(int), cudaMemcpyHostToDevice, st) != cudaSuccess ||
+        cudaMemcpyAsync(act_b[0].p, act0.data(), N * sizeof(int), cudaMemcpyHostToDevice, st) != cudaSuccess ||
+        cudaMemsetAsync(sum_b.p, 0, N * sizeof(double), st) != cudaSuccess)
+        return ml_fail(SDPB_ERR_CUDA, "cudaMemcpyAsync failed");
+    std::vector<const void*> tab((size_t)T * 4);
+    std::vector<int> stall_t;
+    std::vector<MLKey> stall_k;
+    float kern = 0;
+    int rounds = 0, na = n, cur = 0;
+    while (na > 0) {
+        // the tables move when an extension merges new states in: hand the kernel the current ones
+        for (int t = 0; t < T; t++) {
+            tab[t] = h->F[t];
+            tab[T + t] = h->V[t];
+            tab[2 * T + t] = h->Qa[t];
+            std::memcpy(&tab[3 * T + t], &h->nF[t], sizeof(long long));
+        }
+        int ns = 0;
+        if (cudaMemcpyAsync(tab_b.p, tab.data(), tab.size() * 8, cudaMemcpyHostToDevice, st) != cudaSuccess ||
+            cudaMemsetAsync(sn_b.p, 0, sizeof(int), st) != cudaSuccess || cudaEventRecord(h->e1, st) != cudaSuccess)
+            return ml_fail(SDPB_ERR_CUDA, "cudaMemcpyAsync failed");
+        ml_simulate<<<(na + 127) / 128, 128, 0, st>>>(h->P, dF, dV, dQ, dn, (const double*)smp_b.p, nd, (const double*)pw_b.p,
+                                                      (const int*)act_b[cur].p, na, (MLKey*)key_b.p, (int*)per_b.p,
+                                                      (double*)sum_b.p, (double*)val_b.p, (int*)sn_b.p,
+                                                      (int*)act_b[1 - cur].p, (int*)st_b.p, (MLKey*)sk_b.p);
+        if (cudaGetLastError() != cudaSuccess) return ml_fail(SDPB_ERR_CUDA, "ml_simulate launch failed");
+        if (cudaEventRecord(h->e2, st) != cudaSuccess ||
+            cudaMemcpyAsync(&ns, sn_b.p, sizeof(int), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+            cudaStreamSynchronize(st) != cudaSuccess)
+            return ml_fail(SDPB_ERR_CUDA, std::string("roll-out: ") + cudaGetErrorString(cudaGetLastError()));
+        float ms = 0;
+        cudaEventElapsedTime(&ms, h->e1, h->e2);
+        kern += ms;
+        rounds++;
+        if (ns == 0) break;
+        // the states the stalled paths stand on become the roots of one extension (getExpectedValue(state))
+        stall_t.resize((size_t)ns);
+        stall_k.resize((size_t)ns);
+        if (cudaMemcpyAsync(stall_t.data(), st_b.p, (size_t)ns * sizeof(int), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+            cudaMemcpyAsync(stall_k.data(), sk_b.p, (size_t)ns * sizeof(MLKey), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+            cudaStreamSynchronize(st) != cudaSuccess)
+            return ml_fail(SDPB_ERR_CUDA, "cudaMemcpyAsync failed");
+        std::vector<std::vector<MLKey>> r((size_t)T);
+        int p = T;
+        for (int j = 0; j < ns; j++) {
+            r[stall_t[j] - 1].push_back(stall_k[j]);
+            p = std::min(p, stall_t[j]);
+        }
+        for (auto& v : r) {
+            std::sort(v.begin(), v.end(), MLKeyLess());
+            v.erase(std::unique(v.begin(), v.end(), MLKeyEq()), v.end());
+        }
+        rc = ml_extend(h, p, r);
+        if (rc != SDPB_OK) return rc;
+        na = ns;
+        cur = 1 - cur;
+    }
+    if (cudaMemcpyAsync(values, val_b.p, N * sizeof(double), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+        cudaStreamSynchronize(st) != cudaSuccess)
+        return ml_fail(SDPB_ERR_CUDA, "cudaMemcpyAsync failed");
+    h->stats.solve_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - w0).count();
+    h->stats.kernel_ms = kern;
+    h->stats.launches = rounds;
+    return SDPB_OK;
+}
+
+int sdpb_reached_solve(const sdpb_reached_model* m, int device, const double* init_state, double* value, double* action1,
+                       double* action2, int64_t* n_states, double* solve_ms) {
+    if (!init_state) return ml_fail(SDPB_ERR_ARG, "bad argument / struct_size");
+    sdpb_reached* h = nullptr;
+    int rc = sdpb_reached_open(m, device, 0, init_state, 1, &h);
+    if (rc != SDPB_OK) return rc;
+    rc = sdpb_reached_value(h, 1, init_state, 1, value, action1, action2);
+    if (rc == SDPB_OK && n_states) sdpb_reached_states(h, n_states);
+    if (rc == SDPB_OK && solve_ms) *solve_ms = h->stats.solve_ms;
+    sdpb_reached_destroy(h);
+    return rc;
 }
 
 }  // extern "C"

@@ -31,7 +31,7 @@ import numpy as np
 
 from . import _abi as A
 from .models import ModelSpec
-from .solver import Solver, TopDown
+from .solver import Reached, Solver, TopDown
 
 
 class OptDirection(Enum):
@@ -470,7 +470,8 @@ class CashStateMultiLead:
 
 class _ReachedEngine:
     """The two-product engines whose states do not live on a grid: solved over the states the reference's recursion
-    reaches from the queried period-1 state (sdpb_reached_solve).  `pmf`: per period an array [D, 3] of
+    reaches from the states queried so far, kept in one handle (sdpb_reached_*): getAction answers every reached state,
+    and a Simulation / CashSimulation over the engine rolls its policy out.  `pmf`: per period an array [D, 3] of
     (demand1, demand2, prob) as GetPmfMulti.getPmf returns."""
     kind = A.REACHED_MULTILEAD
 
@@ -508,33 +509,37 @@ class _ReachedEngine:
         m.fixed_cost, m.hold_cost, m.min_cash_required, m.state_q = fixedCost, holdingCost, minCashRequired, stateQ
         m.n_demands_t = self._lens.ctypes.data_as(C.POINTER(C.c_int32))
         self._m, self.T, self.device = m, T, device
-        self._solved = {}
+        self._rh = None      # the Reached handle: one memo for every getExpectedValue call
+        self._asked = set()  # (period, state) pairs getExpectedValue has been called on
         self.n_states = None
         self.solve_ms = None
 
-    def _solve(self, state):
-        if state.getPeriod() != 1:
-            raise ValueError("the reached-state solve starts from a period-1 state")
-        key = state._vec()
-        if key not in self._solved:
-            st = np.ascontiguousarray(key, dtype=np.float64)
-            v, ms, a1, a2 = C.c_double(), C.c_double(), C.c_double(), C.c_double()
-            ns = (C.c_int64 * self.T)()
-            rc = self.lib.sdpb_reached_solve(C.byref(self._m), self.device, st.ctypes.data_as(C.POINTER(C.c_double)),
-                                             C.byref(v), C.byref(a1), C.byref(a2), ns, C.byref(ms))
-            if rc != A.SDPB_OK:
-                raise A.SdpbError(rc, self.lib.sdpb_reached_last_error().decode())
-            self._solved[key] = (v.value, (a1.value, a2.value))
-            self.n_states, self.solve_ms = list(ns), ms.value
-        return self._solved[key]
+    def _value(self, state):
+        if self._rh is None:
+            raise KeyError(f"{state._vec()} was not reached: getExpectedValue has not been called")
+        try:
+            v, a1, a2 = self._rh.value(state.getPeriod(), [state._vec()])
+        except A.SdpbError as e:
+            if e.code == A.SDPB_ERR_UNSOLVED:
+                raise KeyError(f"getAction on a state that was never reached: period {state.getPeriod()}, "
+                               f"{state._vec()}") from None
+            raise
+        return float(v[0]), (float(a1[0]), float(a2[0]))
 
     def getExpectedValue(self, state):
-        return self._solve(state)[0]
+        """A state of any period: the first call on it extends the one memo with the states it reaches (only those no
+        earlier call reached are solved); n_states / solve_ms then describe the memo and that call."""
+        key = (state.getPeriod(), state._vec())
+        if key not in self._asked:
+            if self._rh is None:
+                self._rh = Reached(self._m, [], device=self.device)
+            self._rh.extend(*key)
+            self._asked.add(key)
+            self.n_states, self.solve_ms = self._rh.n_states(), self._rh.stats()["solve_ms"]
+        return self._value(state)[0]
 
     def _action(self, state):
-        if state._vec() not in self._solved:
-            raise KeyError("getAction on a state that was never solved")
-        return self._solved[state._vec()][1]
+        return self._value(state)[1]
 
 
 class CashRecursionMultiLead(_ReachedEngine):
@@ -608,6 +613,16 @@ class CashRecursionRounded(_ReachedEngine):
 
     def getAction(self, state):
         return self._action(state)[0]
+
+    def getOptTable(self):
+        """CashRecursion.java:201-220: rows [t, x, w, Q] of every reached state in memo-map order."""
+        if self._rh is None:
+            return np.empty((0, 4))
+        return self._rh.opt_table()[:, :4]
+
+    def getCacheActions(self):
+        """Map CashState -> order quantity over the reached states."""
+        return {CashState(int(t), x, w): float(q) for t, x, w, q in self.getOptTable()}
 
 
 class CashRecursionV(_ReachedEngine):

@@ -1,5 +1,6 @@
-"""Host-side mirror of the reference's policy roll-out classes, over sdpb_simulate (a dense recursion) or
-sdpb_topdown_simulate (a recursion built with topdown=True).
+"""Host-side mirror of the reference's policy roll-out classes, over sdpb_simulate (a dense recursion),
+sdpb_topdown_simulate (a recursion built with topdown=True) or sdpb_reached_simulate (a reached-state engine:
+CashRecursionMultiLead, CashRecursionMultiXR, CashRecursionV, CashRecursionRounded).
 
     Simulation       src/sdp/inventory/Simulation.java:19-107
     CashSimulation   src/sdp/cash/CashSimulation.java:30-118
@@ -47,6 +48,9 @@ class Simulation:
         if samples is None:
             samples = generate_lh_samples(self.distributions, self.sampleNum)
         self.recursion.getExpectedValue(iniState)  # solves on first use, like the reference's lazy recursion
+        if getattr(self.recursion, "_rh", None) is not None:
+            # a two-product (reached-state) engine: samples are [n, T, 2] (one demand per product), or [n, T] for one
+            return self.recursion._rh.simulate(iniState._vec(), samples, self.discountFactor)
         if getattr(self.recursion, "_topdown", False):
             # no grid: the roll-out solves each state a path meets that was not reached yet (Simulation.java:62)
             return self.recursion._td.simulate(iniState._vec(), samples, self.discountFactor)

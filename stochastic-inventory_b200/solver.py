@@ -315,6 +315,106 @@ class TopDown:
                 "capped_action_sets": s.capped_action_sets}
 
 
+class Reached:
+    """One sdpb_reached handle: a two-product (or CashConstraintTest) model, an `SdpbReachedModel`, solved over the
+    states its recursion reaches from the period-1 states `init_states` ([n, ndim], API order; none gives an empty
+    handle).  Every reached state can be queried, the handle extended with states of any period, and the policy rolled
+    out over sample paths.  `scratch_bytes` > 0 replaces the free device memory as the expansion budget.  The model's
+    tables are copied at construction.  Release the device memory with close() (or use it as a context manager)."""
+    _NDIM = {A.REACHED_MULTILEAD: 5, A.REACHED_MULTI_XR: 3, A.REACHED_MULTI_YR: 3, A.REACHED_CASH_ROUNDED: 2}
+
+    def __init__(self, model, init_states=(), device: int = -1, scratch_bytes: int = 0):
+        self.lib = A.load()
+        self.ndim = self._NDIM[model.kind]
+        self.nd = 1 if model.kind == A.REACHED_CASH_ROUNDED else 2  # demands per period of a sample path
+        self.T = model.T
+        st = self._states(init_states)
+        h = C.c_void_p()
+        rc = self.lib.sdpb_reached_open(C.byref(model), device, scratch_bytes, st.ctypes.data_as(C.POINTER(C.c_double)),
+                                        st.shape[0], C.byref(h))
+        if rc != A.SDPB_OK:
+            raise A.SdpbError(rc, self.lib.sdpb_reached_last_error().decode())
+        self.h = h
+
+    def _states(self, states):
+        return np.ascontiguousarray(np.asarray(states, dtype=np.float64).reshape(-1, self.ndim))
+
+    def _check(self, rc):
+        if rc != A.SDPB_OK:
+            raise A.SdpbError(rc, self.lib.sdpb_reached_last_error().decode())
+
+    def close(self):
+        if getattr(self, "h", None):
+            self.lib.sdpb_reached_destroy(self.h)
+            self.h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *a):
+        self.close()
+
+    def value(self, period: int, states):
+        """(V, a1, a2) of reached API-order states [n, ndim] of one period; SDPB_ERR_UNSOLVED for a state not reached."""
+        st = self._states(states)
+        n = st.shape[0]
+        v, a1, a2 = np.empty(n), np.empty(n), np.empty(n)
+        dp = C.POINTER(C.c_double)
+        self._check(self.lib.sdpb_reached_value(self.h, period, st.ctypes.data_as(dp), n, v.ctypes.data_as(dp),
+                                                a1.ctypes.data_as(dp), a2.ctypes.data_as(dp)))
+        return v, a1, a2
+
+    def extend(self, period: int, states):
+        """getExpectedValue on API-order states [n, ndim] of one period: solves only the states no earlier call reached.
+        A failure leaves the handle as it was."""
+        st = self._states(states)
+        self._check(self.lib.sdpb_reached_extend(self.h, period, st.ctypes.data_as(C.POINTER(C.c_double)), st.shape[0]))
+        return self
+
+    def simulate(self, init_state, samples, discount: float = 1.0):
+        """Roll the policy over demand sample paths [n, T, nd] (nd = 2 for two products; [n, T] for one) -> per-path
+        sums, solving every state a path meets that was not reached yet.  The states it adds stay in the handle."""
+        st = np.ascontiguousarray(init_state, dtype=np.float64)
+        sm = np.ascontiguousarray(samples, dtype=np.float64)
+        if st.shape != (self.ndim,):
+            raise ValueError(f"init_state must have {self.ndim} components")
+        if self.nd == 1 and sm.ndim == 2:
+            sm = sm[:, :, None]
+        if sm.ndim != 3 or sm.shape[1:] != (self.T, self.nd):
+            raise ValueError(f"samples must be [n, {self.T}, {self.nd}]")
+        vals = np.empty(sm.shape[0])
+        dp = C.POINTER(C.c_double)
+        self._check(self.lib.sdpb_reached_simulate(self.h, st.ctypes.data_as(dp), sm.ctypes.data_as(dp), sm.shape[0],
+                                                   float(discount), vals.ctypes.data_as(dp)))
+        return vals
+
+    def opt_table(self):
+        """[rows, ndim + 3]: (t, state..., a1, a2) of every reached state in memo-map order."""
+        n = C.c_size_t(0)
+        self._check(self.lib.sdpb_reached_opt_table(self.h, None, C.byref(n)))
+        rows = np.empty((n.value, self.ndim + 3))
+        self._check(self.lib.sdpb_reached_opt_table(self.h, rows.ctypes.data_as(C.POINTER(C.c_double)), C.byref(n)))
+        return rows
+
+    def n_states(self):
+        """Reached states of each period (T entries)."""
+        out = (C.c_int64 * self.T)()
+        self._check(self.lib.sdpb_reached_states(self.h, out))
+        return list(out)
+
+    def stats(self):
+        s = A.SdpbStats()
+        self._check(self.lib.sdpb_reached_stats(self.h, C.byref(s)))
+        return {"evals": s.evals, "evals_executed": s.evals_executed, "solve_ms": s.solve_ms, "kernel_ms": s.kernel_ms,
+                "launches": s.launches}
+
+
 class Group:
     """`n` shards of one model on the given CUDA devices of THIS process (sdpb_group_*): the grid is cut into
     contiguous blocks, every shard holds only the window of V_t it reads, and rows travel between the shards' tables
