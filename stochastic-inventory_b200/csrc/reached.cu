@@ -33,16 +33,12 @@
 // pair followed by a per-state scan (small frontiers, where a thread per state would leave the GPU empty).
 #include <cuda_runtime.h>
 #include <thrust/execution_policy.h>
-#include <thrust/iterator/zip_iterator.h>
-#include <thrust/merge.h>
 #include <thrust/remove.h>
 #include <thrust/sort.h>
-#include <thrust/tuple.h>
 #include <thrust/unique.h>
 
 #include <algorithm>
 #include <cfloat>
-#include <chrono>
 #include <cmath>
 #include <cstdint>
 #include <cstdio>
@@ -52,6 +48,7 @@
 #include <vector>
 
 #include "../../include/sdpb200.h"
+#include "memo_tables.cuh"
 
 namespace {
 
@@ -78,6 +75,7 @@ struct MLFlagged {
 };
 
 // order-preserving encoding of a double: set the sign bit of a non-negative value, flip every bit of a negative one
+// (branch-free for the reason at ml_dec; topdown.cu's td_enc keeps a select: see there)
 __host__ __device__ inline unsigned long long ml_enc(double v) {
     v += 0.0;  // -0.0 and +0.0 are one key in the reference's map (compared with ==)
     unsigned long long b;
@@ -173,6 +171,15 @@ __device__ __forceinline__ long long ml_find(const MLKey* __restrict__ F, long l
     }
     return lo;  // the key is present by construction
 }
+
+struct MLTraits {  // the key of the memo tables (memo_tables.cuh)
+    typedef MLKey Key;
+    typedef MLKeyLess Less;
+    typedef MLKeyEq Eq;
+    static __device__ __forceinline__ long long lower(const MLKey* __restrict__ F, long long n, const MLKey& k) {
+        return ml_find(F, n, k);
+    }
+};
 
 // ---- kind 1: MultiItemCashXR.java:87-126 ----
 __device__ __forceinline__ double xr_immediate(const MLParams& P, bool last, const MLState& s, double action1, double action2,
@@ -421,18 +428,6 @@ __global__ void ml_count_actions(MLParams P, const MLKey* __restrict__ F, long l
     atomicAdd(total, c);
 }
 
-// batched lookup: (V, action index) of each query key, action index -2 when the state is not in the sorted table F
-__global__ void ml_query(const MLKey* __restrict__ F, long long n, const double* __restrict__ V, const int* __restrict__ Qa,
-                         const MLKey* __restrict__ q, int nq, double* __restrict__ v, int* __restrict__ qi) {
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= nq) return;
-    const MLKey k = q[i];
-    const long long at = ml_find(F, n, k);
-    const bool hit = at < n && MLKeyEq()(F[at], k);
-    v[i] = hit ? V[at] : 0.0;
-    qi[i] = hit ? Qa[at] : -2;
-}
-
 // the filter of an extension: flag[i] = 1 when candidate i is already in the sorted table F
 __global__ void ml_known(const MLKey* __restrict__ F, long long n, const MLKey* __restrict__ c, long long m,
                          unsigned char* __restrict__ flag) {
@@ -442,87 +437,41 @@ __global__ void ml_known(const MLKey* __restrict__ F, long long n, const MLKey* 
     flag[i] = at < n && MLKeyEq()(F[at], c[i]) ? 1 : 0;
 }
 
-// One thread per path of act[0, na): from where the path stands (period per[i], state key[i], partial sum sum[i]) --
-// (a1, a2) = getAction(state), d = Math.round(sample), sum += discount^(t-1) c(state, a, d) (salvage when t == T),
-// state = f(state, a, d, c) -- until it ends (values[i] = sum) or meets a state the handle has not reached.  There it
-// writes (path, t, state) to the next slot of the stall list, keeps its period, state and partial sum, and stops.
-// Kind 2 has no immediate value: a path is worth boundFinalCash of the state after period T.
-__global__ void __launch_bounds__(128) ml_simulate(MLParams P, const MLKey* const* __restrict__ tF,
-                                                   const double* const* __restrict__ tV, const int* const* __restrict__ tQ,
-                                                   const long long* __restrict__ tn, const double* __restrict__ samples,
-                                                   const int nd, const double* __restrict__ pw, const int* __restrict__ act,
-                                                   const int na, MLKey* __restrict__ key, int* __restrict__ per,
-                                                   double* __restrict__ sum, double* __restrict__ values,
-                                                   int* __restrict__ stall_n, int* __restrict__ stall_path,
-                                                   int* __restrict__ stall_t, MLKey* __restrict__ stall_key) {
-    const int k = blockIdx.x * blockDim.x + threadIdx.x;
-    if (k >= na) return;
-    const int i = act[k], T = P.T;
-    MLKey s = key[i];
-    double acc = sum[i];
-    for (int t = per[i]; t <= T; t++) {
-        const MLKey* __restrict__ F = tF[t - 1];
-        const long long n = tn[t - 1];
-        const long long at = ml_find(F, n, s);
-        if (at >= n || !MLKeyEq()(F[at], s)) {
-            key[i] = s;
-            per[i] = t;
-            sum[i] = acc;
-            const int slot = atomicAdd(stall_n, 1);
-            stall_path[slot] = i;
-            stall_t[slot] = t;
-            stall_key[slot] = s;
-            return;
-        }
+// One period of the roll-out for memo::memo_simulate: (a1, a2) = getAction(state), d = Math.round(sample),
+// c(state, a, d) (salvage when t == T), state = f(state, a, d, c).  Kind 2 has no immediate value: a path is worth
+// boundFinalCash of the state after period T.
+struct MLStep {
+    MLParams P;
+    __device__ __forceinline__ bool operator()(int t, MLKey& s, int qi, double v, const double* smp, double& c) const {
         const MLState st = ml_state(s);
         double a1, a2;
-        ml_reported_action(P.kind, P.Q2, st, tQ[t - 1][at], tV[t - 1][at], a1, a2);
-        const double* smp = samples + ((size_t)i * T + (t - 1)) * nd;
-        const double d1 = (double)ml_jround(smp[0]), d2 = nd > 1 ? (double)ml_jround(smp[1]) : 0.0;
-        const bool last = t == T;
+        ml_reported_action(P.kind, P.Q2, st, qi, v, a1, a2);
+        const double d1 = (double)ml_jround(smp[0]), d2 = P.kind != 3 ? (double)ml_jround(smp[1]) : 0.0;  // kind 3: one demand
+        const bool last = t == P.T;
         if (P.kind == 2) {
             const double iniR = (st.cash + P.v1 * (double)st.x1) + P.v2 * (double)st.x2;
             const MLState nx = yr_transition(P, a1, a2, iniR, d1, d2);
-            if (last) acc = (nx.cash + P.sal1 * (double)nx.x1) + P.sal2 * (double)nx.x2;  // MultiItemYR.java:116-119
-            else s = ml_key(nx);
-            continue;
+            c = last ? (nx.cash + P.sal1 * (double)nx.x1) + P.sal2 * (double)nx.x2 : 0.0;  // MultiItemYR.java:116-119
+            if (!last) s = ml_key(nx);
+            return last;
         }
         const double x3 = (double)st.x1 / P.sq;  // kind 3: the inventory value
-        const double c = P.kind == 0 ? ml_immediate(P, t, last, st, (int)a1, (int)a2, (int)d1, (int)d2)
-                       : P.kind == 1 ? xr_immediate(P, last, st, a1, a2, d1, d2)
-                                     : cct_immediate(P, last, x3, st.cash, a1, d1);
-        acc += pw[t - 1] * c;
+        c = P.kind == 0 ? ml_immediate(P, t, last, st, (int)a1, (int)a2, (int)d1, (int)d2)
+          : P.kind == 1 ? xr_immediate(P, last, st, a1, a2, d1, d2)
+                        : cct_immediate(P, last, x3, st.cash, a1, d1);
         if (!last)
             s = ml_key(P.kind == 0 ? ml_transition(P, st, (int)a1, (int)a2, (int)d1, (int)d2, c)
                        : P.kind == 1 ? xr_transition(P, st, a1, a2, d1, d2, c)
                                      : cct_transition(P, x3, st.cash, a1, d1, c));
+        return false;
     }
-    values[i] = acc;
-}
+};
 
 thread_local std::string g_ml_error;
 
 int ml_fail(int rc, const std::string& msg) {
     g_ml_error = msg;
     return rc;
-}
-
-struct DevBuf {  // a scratch allocation released when it goes out of scope
-    void* p = nullptr;
-    ~DevBuf() { if (p) cudaFree(p); }
-    bool alloc(size_t bytes) {
-        if (p) { cudaFree(p); p = nullptr; }
-        if (cudaMalloc(&p, bytes > 0 ? bytes : 16) != cudaSuccess) { cudaGetLastError(); p = nullptr; return false; }
-        return true;
-    }
-};
-
-template <class T>
-bool ml_alloc(T*& p, long long n) {
-    if (cudaMalloc((void**)&p, (size_t)std::max(n, 1ll) * sizeof(T)) == cudaSuccess) return true;
-    cudaGetLastError();
-    p = nullptr;
-    return false;
 }
 
 }  // namespace
@@ -534,35 +483,12 @@ struct sdpb_reached {
     int n_int = 4;  // API-order coordinates before the cash: 4 | 2 | 2 | 1
     long long A = 0;
     long long scratch_bytes = 0;
-    cudaStream_t stream = nullptr;
-    cudaEvent_t e0 = nullptr, e1 = nullptr, e2 = nullptr;
-    std::vector<int> lens;    // demand points of each period
-    std::vector<void*> owned; // model tables
-    std::vector<MLKey*> F;    // [T] reached states, sorted in memo-map order
-    std::vector<double*> V;   // [T]
-    std::vector<int*> Qa;     // [T] flat action index
-    std::vector<long long> nF;
-    sdpb_stats stats{};
+    std::vector<int> lens;      // demand points of each period
+    std::vector<void*> owned;   // model tables
+    memo::Tables<MLTraits> mt;  // sorted in memo-map order; Q: the flat action index
 };
 
 namespace {
-
-// What one extension builds, owned here until it is committed to the handle: per period the new states N_t with their
-// V / Q, and the merged tables F_t u N_t.  Whatever is still owned when the stage goes out of scope is freed, so an
-// extension that fails leaves the handle as it found it.
-struct MLStage {
-    std::vector<MLKey*> N, MF;
-    std::vector<double*> VN, MV;
-    std::vector<int*> QN, MQ;
-    std::vector<long long> nN, nM;
-    explicit MLStage(int T)
-        : N(T, nullptr), MF(T, nullptr), VN(T, nullptr), MV(T, nullptr), QN(T, nullptr), MQ(T, nullptr), nN(T, 0), nM(T, 0) {}
-    ~MLStage() {
-        for (size_t k = 0; k < N.size(); k++) {
-            cudaFree(N[k]); cudaFree(MF[k]); cudaFree(VN[k]); cudaFree(MV[k]); cudaFree(QN[k]); cudaFree(MQ[k]);
-        }
-    }
-};
 
 // N_t: the sorted roots of period t and the successors of the n_src new states `src` of period t - 1, minus the states
 // the handle already holds in period t; sorted and unique, into a right-sized *out.  All candidates are expanded at
@@ -573,7 +499,7 @@ int ml_new_states(sdpb_reached* h, int t, const MLKey* src, long long n_src, con
     *n_out = 0;
     const long long nr = (long long)roots.size(), pairs = n_src * h->A, cand = pairs * h->P.nD + nr;
     if (cand == 0) return SDPB_OK;
-    cudaStream_t st = h->stream;
+    cudaStream_t st = h->mt.stream;
     size_t free_b = 0, total_b = 0;
     cudaMemGetInfo(&free_b, &total_b);
     const double budget = h->scratch_bytes > 0 ? (double)h->scratch_bytes : (double)free_b;
@@ -581,7 +507,7 @@ int ml_new_states(sdpb_reached* h, int t, const MLKey* src, long long n_src, con
         return ml_fail(SDPB_ERR_NOMEM, "period " + std::to_string(t) + " has " + std::to_string(cand) + " candidate states: more than " +
                                            (h->scratch_bytes > 0 ? "a scratch budget of " + std::to_string(h->scratch_bytes) + " bytes"
                                                                  : std::string("this GPU's memory")) + " holds");
-    DevBuf buf;
+    memo::DevBuf buf;
     if (!buf.alloc((size_t)cand * sizeof(MLKey))) return ml_fail(SDPB_ERR_NOMEM, "allocation of the candidate states failed");
     MLKey* c = (MLKey*)buf.p;
     if (pairs > 0) {
@@ -591,8 +517,8 @@ int ml_new_states(sdpb_reached* h, int t, const MLKey* src, long long n_src, con
     if (nr > 0 && cudaMemcpyAsync(c + pairs * h->P.nD, roots.data(), (size_t)nr * sizeof(MLKey), cudaMemcpyHostToDevice, st) != cudaSuccess)
         return ml_fail(SDPB_ERR_CUDA, "cudaMemcpyAsync failed");
     long long m = 0;
-    const MLKey* Fo = h->F[t - 1];
-    const long long no = h->nF[t - 1];
+    const MLKey* Fo = h->mt.F[t - 1];
+    const long long no = h->mt.nF[t - 1];
     try {
         auto par = thrust::cuda::par.on(st);
         thrust::sort(par, c, c + cand, MLKeyLess());
@@ -605,7 +531,7 @@ int ml_new_states(sdpb_reached* h, int t, const MLKey* src, long long n_src, con
             if (tail.a == ~0ull && tail.b == ~0ull) m--;
         }
         if (m > 0 && no > 0) {  // keep what period t does not hold yet
-            DevBuf flag;
+            memo::DevBuf flag;
             if (!flag.alloc((size_t)m)) return ml_fail(SDPB_ERR_NOMEM, "allocation of the filter flags failed");
             ml_known<<<(unsigned)((m + 127) / 128), 128, 0, st>>>(Fo, no, c, m, (unsigned char*)flag.p);
             if (cudaGetLastError() != cudaSuccess) return ml_fail(SDPB_ERR_CUDA, "ml_known launch failed");
@@ -616,7 +542,7 @@ int ml_new_states(sdpb_reached* h, int t, const MLKey* src, long long n_src, con
         return ml_fail(SDPB_ERR_CUDA, std::string("sort / unique: ") + ex.what());
     }
     if (m == 0) return SDPB_OK;
-    if (!ml_alloc(*out, m)) return ml_fail(SDPB_ERR_NOMEM, "allocation of the states of period " + std::to_string(t) + " failed");
+    if (!memo::alloc(*out, m)) return ml_fail(SDPB_ERR_NOMEM, "allocation of the states of period " + std::to_string(t) + " failed");
     *n_out = m;
     if (cudaMemcpyAsync(*out, c, (size_t)m * sizeof(MLKey), cudaMemcpyDeviceToDevice, st) != cudaSuccess ||
         cudaStreamSynchronize(st) != cudaSuccess)
@@ -631,14 +557,14 @@ int ml_evals(sdpb_reached* h, int t, const MLKey* F, long long n, double& evals)
         evals += (double)n * (double)h->A * D;
         return SDPB_OK;
     }
-    DevBuf tot;
+    memo::DevBuf tot;
     unsigned long long listed = 0;
     if (!tot.alloc(sizeof listed)) return ml_fail(SDPB_ERR_NOMEM, "allocation failed");
-    if (cudaMemsetAsync(tot.p, 0, sizeof listed, h->stream) != cudaSuccess) return ml_fail(SDPB_ERR_CUDA, "cudaMemsetAsync failed");
-    ml_count_actions<<<(unsigned)((n + 127) / 128), 128, 0, h->stream>>>(h->P, F, n, (unsigned long long*)tot.p);
+    if (cudaMemsetAsync(tot.p, 0, sizeof listed, h->mt.stream) != cudaSuccess) return ml_fail(SDPB_ERR_CUDA, "cudaMemsetAsync failed");
+    ml_count_actions<<<(unsigned)((n + 127) / 128), 128, 0, h->mt.stream>>>(h->P, F, n, (unsigned long long*)tot.p);
     if (cudaGetLastError() != cudaSuccess ||
-        cudaMemcpyAsync(&listed, tot.p, sizeof listed, cudaMemcpyDeviceToHost, h->stream) != cudaSuccess ||
-        cudaStreamSynchronize(h->stream) != cudaSuccess)
+        cudaMemcpyAsync(&listed, tot.p, sizeof listed, cudaMemcpyDeviceToHost, h->mt.stream) != cudaSuccess ||
+        cudaStreamSynchronize(h->mt.stream) != cudaSuccess)
         return ml_fail(SDPB_ERR_CUDA, std::string("counting the actions: ") + cudaGetErrorString(cudaGetLastError()));
     evals += (double)listed * D;
     return SDPB_OK;
@@ -649,10 +575,8 @@ int ml_evals(sdpb_reached* h, int t, const MLKey* F, long long n, double& evals)
 // tables of the next period, and the merged tables of every touched period replace the handle's at the end.
 int ml_extend(sdpb_reached* h, int p, const std::vector<std::vector<MLKey>>& roots) {
     const int T = h->m.T;
-    const long long A = h->A;
-    cudaStream_t st = h->stream;
-    MLStage sg(T);
-    if (cudaEventRecord(h->e0, st) != cudaSuccess) return ml_fail(SDPB_ERR_CUDA, "cudaEventRecord failed");
+    memo::Stage<MLTraits> sg(T);
+    if (cudaEventRecord(h->mt.e0, h->mt.stream) != cudaSuccess) return ml_fail(SDPB_ERR_CUDA, "cudaEventRecord failed");
     double evals = 0;
     for (int t = p; t <= T; t++) {
         const int k = t - 1;
@@ -660,70 +584,21 @@ int ml_extend(sdpb_reached* h, int p, const std::vector<std::vector<MLKey>>& roo
         if (rc == SDPB_OK && sg.nN[k] > 0) rc = ml_evals(h, t, sg.N[k], sg.nN[k], evals);
         if (rc != SDPB_OK) return rc;
     }
-    if (cudaEventRecord(h->e1, st) != cudaSuccess) return ml_fail(SDPB_ERR_CUDA, "cudaEventRecord failed");
-    int launches = 0;
-    for (int t = T; t >= p; t--) {
-        const int k = t - 1;
-        const long long n = sg.nN[k], no = h->nF[k];
-        if (n == 0) continue;
-        if (!ml_alloc(sg.VN[k], n) || !ml_alloc(sg.QN[k], n)) return ml_fail(SDPB_ERR_NOMEM, "allocation of the value table failed");
-        const bool nxt = t < T, nxt_new = nxt && sg.nN[k + 1] > 0;
-        const MLKey* Fn = nxt ? (nxt_new ? sg.MF[k + 1] : h->F[k + 1]) : nullptr;
-        const double* Vn = nxt ? (nxt_new ? sg.MV[k + 1] : h->V[k + 1]) : nullptr;
-        const long long nFn = nxt ? (nxt_new ? sg.nM[k + 1] : h->nF[k + 1]) : 0;
-        DevBuf qv;
+    auto backward = [h](int t, const MLKey* F, long long n, const MLKey* Fn, const double* Vn, long long nFn, double* V,
+                        int* Q) {
+        const long long A = h->A;
+        cudaStream_t st = h->mt.stream;
         if (n * A <= 200000000LL && n < 50000) {  // few states: spread their actions over the GPU
+            memo::DevBuf qv;
             if (!qv.alloc((size_t)(n * A) * sizeof(double))) return ml_fail(SDPB_ERR_NOMEM, "allocation of the action-value scratch failed");
-            ml_backward_pairs<<<(unsigned)((n * A + 127) / 128), 128, 0, st>>>(h->P, t, sg.N[k], n, Fn, Vn, nFn, (double*)qv.p);
-            ml_scan_pairs<<<(unsigned)((n + 127) / 128), 128, 0, st>>>(h->P, (const double*)qv.p, n, sg.VN[k], sg.QN[k]);
-            launches += 2;
-        } else {
-            ml_backward_state<<<(unsigned)((n + 127) / 128), 128, 0, st>>>(h->P, t, sg.N[k], n, Fn, Vn, nFn, sg.VN[k], sg.QN[k]);
-            launches++;
+            ml_backward_pairs<<<(unsigned)((n * A + 127) / 128), 128, 0, st>>>(h->P, t, F, n, Fn, Vn, nFn, (double*)qv.p);
+            ml_scan_pairs<<<(unsigned)((n + 127) / 128), 128, 0, st>>>(h->P, (const double*)qv.p, n, V, Q);
+            return 2;
         }
-        if (cudaGetLastError() != cudaSuccess) return ml_fail(SDPB_ERR_CUDA, "backward launch failed");
-        sg.nM[k] = no + n;
-        if (no == 0) {  // nothing to merge with: the new tables are the merged ones
-            std::swap(sg.MF[k], sg.N[k]);
-            std::swap(sg.MV[k], sg.VN[k]);
-            std::swap(sg.MQ[k], sg.QN[k]);
-            continue;
-        }
-        if (!ml_alloc(sg.MF[k], no + n) || !ml_alloc(sg.MV[k], no + n) || !ml_alloc(sg.MQ[k], no + n))
-            return ml_fail(SDPB_ERR_NOMEM, "allocation of the merged tables of period " + std::to_string(t) + " failed");
-        try {  // the two key sets are disjoint: a merge by key keeps every row
-            thrust::merge_by_key(thrust::cuda::par.on(st), h->F[k], h->F[k] + no, sg.N[k], sg.N[k] + n,
-                                 thrust::make_zip_iterator(thrust::make_tuple(h->V[k], h->Qa[k])),
-                                 thrust::make_zip_iterator(thrust::make_tuple(sg.VN[k], sg.QN[k])), sg.MF[k],
-                                 thrust::make_zip_iterator(thrust::make_tuple(sg.MV[k], sg.MQ[k])), MLKeyLess());
-        } catch (const std::exception& ex) {
-            return ml_fail(SDPB_ERR_CUDA, std::string("merge: ") + ex.what());
-        }
-    }
-    if (cudaEventRecord(h->e2, st) != cudaSuccess || cudaEventSynchronize(h->e2) != cudaSuccess)
-        return ml_fail(SDPB_ERR_CUDA, std::string("backward pass: ") + cudaGetErrorString(cudaGetLastError()));
-    for (int k = p - 1; k < T; k++) {  // commit
-        if (sg.nN[k] == 0) continue;
-        cudaFree(h->F[k]);
-        cudaFree(h->V[k]);
-        cudaFree(h->Qa[k]);
-        h->F[k] = sg.MF[k];
-        h->V[k] = sg.MV[k];
-        h->Qa[k] = sg.MQ[k];
-        sg.MF[k] = nullptr;
-        sg.MV[k] = nullptr;
-        sg.MQ[k] = nullptr;
-        h->nF[k] = sg.nM[k];
-    }
-    float solve = 0, kern = 0;
-    cudaEventElapsedTime(&solve, h->e0, h->e2);
-    cudaEventElapsedTime(&kern, h->e1, h->e2);
-    h->stats.evals += evals;
-    h->stats.evals_executed += evals;
-    h->stats.solve_ms = solve;
-    h->stats.kernel_ms = kern;
-    h->stats.launches = launches;
-    return SDPB_OK;
+        ml_backward_state<<<(unsigned)((n + 127) / 128), 128, 0, st>>>(h->P, t, F, n, Fn, Vn, nFn, V, Q);
+        return 1;
+    };
+    return memo::commit(h->mt, sg, p, evals, 0.0, backward, g_ml_error);
 }
 
 // The key of one API-order state: false when it has no key (an inventory or pipeline quantity that is not an integer
@@ -762,8 +637,7 @@ int ml_root_keys(const sdpb_reached* h, const double* states, int n, std::vector
             return ml_fail(SDPB_ERR_OFFGRID, h->m.kind == SDPB_REACHED_CASH_ROUNDED
                                                  ? "the inventory of a state is not of the form k / state_q, k in [0, 65535]"
                                                  : "inventories and pipeline quantities must be integers in [0, 65535]");
-    std::sort(out.begin(), out.end(), MLKeyLess());
-    out.erase(std::unique(out.begin(), out.end(), MLKeyEq()), out.end());
+    memo::canonical<MLTraits>(out);
     return SDPB_OK;
 }
 
@@ -776,16 +650,8 @@ const char* sdpb_reached_last_error(void) { return g_ml_error.c_str(); }
 void sdpb_reached_destroy(sdpb_reached* h) {
     if (!h) return;
     cudaSetDevice(h->device);
-    for (MLKey* p : h->F) cudaFree(p);
-    for (double* p : h->V) cudaFree(p);
-    for (int* p : h->Qa) cudaFree(p);
     for (void* p : h->owned) cudaFree(p);
-    if (h->e0) cudaEventDestroy(h->e0);
-    if (h->e1) cudaEventDestroy(h->e1);
-    if (h->e2) cudaEventDestroy(h->e2);
-    if (h->stream) cudaStreamDestroy(h->stream);
-    cudaGetLastError();
-    delete h;
+    delete h;  // and its memo tables
 }
 
 int sdpb_reached_open(const sdpb_reached_model* m, int device, int64_t scratch_bytes, const double* init_states, int n,
@@ -821,21 +687,15 @@ int sdpb_reached_open(const sdpb_reached_model* m, int device, int64_t scratch_b
     h->n_int = m->kind == SDPB_REACHED_MULTILEAD ? 4 : (m->kind == SDPB_REACHED_CASH_ROUNDED ? 1 : 2);
     const int q2 = m->kind == SDPB_REACHED_CASH_ROUNDED ? 1 : m->q_bound;
     h->A = (long long)m->q_bound * q2;
-    h->F.assign(T, nullptr);
-    h->V.assign(T, nullptr);
-    h->Qa.assign(T, nullptr);
-    h->nF.assign(T, 0);
-    auto bail = [&](int rc, const std::string& msg) { sdpb_reached_destroy(h); return ml_fail(rc, msg); };
-    if (cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking) != cudaSuccess || cudaEventCreate(&h->e0) != cudaSuccess ||
-        cudaEventCreate(&h->e1) != cudaSuccess || cudaEventCreate(&h->e2) != cudaSuccess)
-        return bail(SDPB_ERR_CUDA, "stream / event creation failed");
+    auto bail = [&](int rc, std::string msg) { sdpb_reached_destroy(h); return ml_fail(rc, msg); };
+    if (h->mt.open(T, g_ml_error) != SDPB_OK) return bail(SDPB_ERR_CUDA, g_ml_error);
     std::vector<double> pg((size_t)T * nD);
     for (size_t i = 0; i < pg.size(); i++) pg[i] = m->p[i] * m->gamma;  // first product of p * gamma * V
     auto upload = [&](const void* src, size_t bytes) -> void* {
         void* p = nullptr;
         if (cudaMalloc(&p, bytes) != cudaSuccess) { cudaGetLastError(); return nullptr; }
         h->owned.push_back(p);
-        if (cudaMemcpyAsync(p, src, bytes, cudaMemcpyHostToDevice, h->stream) != cudaSuccess) return nullptr;
+        if (cudaMemcpyAsync(p, src, bytes, cudaMemcpyHostToDevice, h->mt.stream) != cudaSuccess) return nullptr;
         return p;
     };
     MLParams& P = h->P;
@@ -852,15 +712,12 @@ int sdpb_reached_open(const sdpb_reached_model* m, int device, int64_t scratch_b
     P.pg = (const double*)upload(pg.data(), tab); P.ovh = (const double*)upload(m->overhead_t, (size_t)T * sizeof(double));
     P.nDt = (const int*)upload(lens.data(), (size_t)T * sizeof(int));
     if (!P.d1 || !P.d2 || !P.p || !P.pg || !P.ovh || !P.nDt) return bail(SDPB_ERR_NOMEM, "allocation of the model tables failed");
-    if (cudaStreamSynchronize(h->stream) != cudaSuccess) return bail(SDPB_ERR_CUDA, "uploading the model tables failed");  // (pg, lens are locals)
+    if (cudaStreamSynchronize(h->mt.stream) != cudaSuccess) return bail(SDPB_ERR_CUDA, "uploading the model tables failed");  // (pg, lens are locals)
 
     std::vector<std::vector<MLKey>> roots((size_t)T);
     int rc = ml_root_keys(h, init_states, n, roots[0]);
     if (rc == SDPB_OK && n > 0) rc = ml_extend(h, 1, roots);
-    if (rc != SDPB_OK) {
-        const std::string msg = g_ml_error;
-        return bail(rc, msg);
-    }
+    if (rc != SDPB_OK) return bail(rc, g_ml_error);
     *out = h;
     return SDPB_OK;
 }
@@ -877,24 +734,10 @@ int sdpb_reached_value(sdpb_reached* h, int period, const double* states, int n,
         if (!ml_encode(h, states + (size_t)i * nd, keys[i]))
             return ml_fail(SDPB_ERR_UNSOLVED, "state " + std::to_string(i) + " was not reached in period " + std::to_string(period));
     cudaSetDevice(h->device);
-    DevBuf kq, vq, aq;
-    if (!kq.alloc(keys.size() * sizeof(MLKey)) || !vq.alloc((size_t)n * sizeof(double)) || !aq.alloc((size_t)n * sizeof(int)))
-        return ml_fail(SDPB_ERR_NOMEM, "allocation failed");
-    std::vector<double> vv((size_t)n);
-    std::vector<int> qi((size_t)n);
-    cudaStream_t st = h->stream;
-    if (cudaMemcpyAsync(kq.p, keys.data(), keys.size() * sizeof(MLKey), cudaMemcpyHostToDevice, st) != cudaSuccess)
-        return ml_fail(SDPB_ERR_CUDA, "cudaMemcpyAsync failed");
-    ml_query<<<(n + 127) / 128, 128, 0, st>>>(h->F[period - 1], h->nF[period - 1], h->V[period - 1], h->Qa[period - 1],
-                                               (const MLKey*)kq.p, n, (double*)vq.p, (int*)aq.p);
-    if (cudaGetLastError() != cudaSuccess ||
-        cudaMemcpyAsync(vv.data(), vq.p, (size_t)n * sizeof(double), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
-        cudaMemcpyAsync(qi.data(), aq.p, (size_t)n * sizeof(int), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
-        cudaStreamSynchronize(st) != cudaSuccess)
-        return ml_fail(SDPB_ERR_CUDA, std::string("query: ") + cudaGetErrorString(cudaGetLastError()));
-    for (int i = 0; i < n; i++)
-        if (qi[i] == -2)
-            return ml_fail(SDPB_ERR_UNSOLVED, "state " + std::to_string(i) + " was not reached in period " + std::to_string(period));
+    std::vector<double> vv;
+    std::vector<int> qi;
+    const int rc = memo::lookup(h->mt, period, keys, vv, qi, g_ml_error);
+    if (rc != SDPB_OK) return rc;
     for (int i = 0; i < n; i++) {
         double b1, b2;
         ml_reported_action(h->m.kind, h->P.Q2, ml_state(keys[i]), qi[i], vv[i], b1, b2);
@@ -920,54 +763,35 @@ int sdpb_reached_extend(sdpb_reached* h, int period, const double* states, int n
 int sdpb_reached_opt_table(sdpb_reached* h, double* rows, size_t* nrows) {
     g_ml_error.clear();
     if (!h || !nrows) return ml_fail(SDPB_ERR_ARG, "null argument");
-    size_t total = 0;
-    for (int t = 0; t < h->m.T; t++) total += (size_t)h->nF[t];
-    if (!rows) { *nrows = total; return SDPB_OK; }
-    if (*nrows < total) return ml_fail(SDPB_ERR_ARG, "rows holds fewer than the reached states");
     cudaSetDevice(h->device);
-    const int nd = h->n_int + 1, w = nd + 3;
-    size_t r = 0;
-    for (int t = 1; t <= h->m.T; t++) {  // the device order is the memo-map order: a straight copy
-        const long long n = h->nF[t - 1];
-        std::vector<MLKey> k((size_t)n);
-        std::vector<double> v((size_t)n);
-        std::vector<int> qi((size_t)n);
-        if (cudaMemcpyAsync(k.data(), h->F[t - 1], (size_t)n * sizeof(MLKey), cudaMemcpyDeviceToHost, h->stream) != cudaSuccess ||
-            cudaMemcpyAsync(v.data(), h->V[t - 1], (size_t)n * sizeof(double), cudaMemcpyDeviceToHost, h->stream) != cudaSuccess ||
-            cudaMemcpyAsync(qi.data(), h->Qa[t - 1], (size_t)n * sizeof(int), cudaMemcpyDeviceToHost, h->stream) != cudaSuccess ||
-            cudaStreamSynchronize(h->stream) != cudaSuccess)
-            return ml_fail(SDPB_ERR_CUDA, "cudaMemcpyAsync failed");
-        for (long long i = 0; i < n; i++, r++) {
-            const MLState s = ml_state(k[i]);
-            double* row = rows + r * w;
-            int c = 0;
-            row[c++] = t;
-            if (h->m.kind == SDPB_REACHED_CASH_ROUNDED) {
-                row[c++] = (double)s.x1 / h->P.sq;
-            } else {
-                row[c++] = s.x1;
-                row[c++] = s.x2;
-                if (h->m.kind == SDPB_REACHED_MULTILEAD) { row[c++] = s.q1; row[c++] = s.q2; }
-            }
-            row[c++] = s.cash;
-            ml_reported_action(h->m.kind, h->P.Q2, s, qi[i], v[i], row[c], row[c + 1]);
+    auto row = [h](int t, const MLKey& k, double v, int qi, double* row) {  // the device order is the memo-map order
+        const MLState s = ml_state(k);
+        int c = 0;
+        row[c++] = t;
+        if (h->m.kind == SDPB_REACHED_CASH_ROUNDED) {
+            row[c++] = (double)s.x1 / h->P.sq;
+        } else {
+            row[c++] = s.x1;
+            row[c++] = s.x2;
+            if (h->m.kind == SDPB_REACHED_MULTILEAD) { row[c++] = s.q1; row[c++] = s.q2; }
         }
-    }
-    *nrows = total;
-    return SDPB_OK;
+        row[c++] = s.cash;
+        ml_reported_action(h->m.kind, h->P.Q2, s, qi, v, row[c], row[c + 1]);
+    };
+    return memo::opt_table(h->mt, rows, nrows, h->n_int + 4, row, g_ml_error);
 }
 
 int sdpb_reached_states(const sdpb_reached* h, int64_t* n_states) {
     g_ml_error.clear();
     if (!h || !n_states) return ml_fail(SDPB_ERR_ARG, "null argument");
-    for (int t = 0; t < h->m.T; t++) n_states[t] = h->nF[t];
+    for (int t = 0; t < h->m.T; t++) n_states[t] = h->mt.nF[t];
     return SDPB_OK;
 }
 
 int sdpb_reached_stats(const sdpb_reached* h, sdpb_stats* s) {
     g_ml_error.clear();
     if (!h || !s) return ml_fail(SDPB_ERR_ARG, "null argument");
-    *s = h->stats;
+    *s = h->mt.stats;
     return SDPB_OK;
 }
 
@@ -985,95 +809,9 @@ int sdpb_reached_simulate(sdpb_reached* h, const double* init_state, const doubl
     std::vector<std::vector<MLKey>> roots((size_t)T);
     int rc = ml_root_keys(h, init_state, 1, roots[0]);
     if (rc != SDPB_OK) return rc;
-    const MLKey k0 = roots[0][0];
-    const auto w0 = std::chrono::steady_clock::now();
     cudaSetDevice(h->device);
-    rc = ml_extend(h, 1, roots);  // getExpectedValue(iniState) first
-    if (rc != SDPB_OK) return rc;
-
-    cudaStream_t st = h->stream;
-    std::vector<double> pw((size_t)T);
-    for (int t = 0; t < T; t++) pw[t] = std::pow(discount, (double)t);  // Math.pow(discountFactor, t)
-    std::vector<MLKey> key0(N, k0);
-    std::vector<int> per0(N, 1), act0(N);
-    for (int i = 0; i < n; i++) act0[i] = i;
-    DevBuf smp_b, pw_b, key_b, per_b, sum_b, val_b, act_b[2], st_b, sk_b, sn_b, tab_b;
-    if (!smp_b.alloc(N * T * nd * sizeof(double)) || !pw_b.alloc(T * sizeof(double)) || !key_b.alloc(N * sizeof(MLKey)) ||
-        !per_b.alloc(N * sizeof(int)) || !sum_b.alloc(N * sizeof(double)) || !val_b.alloc(N * sizeof(double)) ||
-        !act_b[0].alloc(N * sizeof(int)) || !act_b[1].alloc(N * sizeof(int)) || !st_b.alloc(N * sizeof(int)) ||
-        !sk_b.alloc(N * sizeof(MLKey)) || !sn_b.alloc(sizeof(int)) || !tab_b.alloc((size_t)T * 4 * 8))
-        return ml_fail(SDPB_ERR_NOMEM, "allocation of the roll-out buffers failed");
-    const MLKey** dF = (const MLKey**)tab_b.p;
-    const double** dV = (const double**)(dF + T);
-    const int** dQ = (const int**)(dV + T);
-    long long* dn = (long long*)(dQ + T);
-    if (cudaMemcpyAsync(smp_b.p, samples, N * T * nd * sizeof(double), cudaMemcpyHostToDevice, st) != cudaSuccess ||
-        cudaMemcpyAsync(pw_b.p, pw.data(), T * sizeof(double), cudaMemcpyHostToDevice, st) != cudaSuccess ||
-        cudaMemcpyAsync(key_b.p, key0.data(), N * sizeof(MLKey), cudaMemcpyHostToDevice, st) != cudaSuccess ||
-        cudaMemcpyAsync(per_b.p, per0.data(), N * sizeof(int), cudaMemcpyHostToDevice, st) != cudaSuccess ||
-        cudaMemcpyAsync(act_b[0].p, act0.data(), N * sizeof(int), cudaMemcpyHostToDevice, st) != cudaSuccess ||
-        cudaMemsetAsync(sum_b.p, 0, N * sizeof(double), st) != cudaSuccess)
-        return ml_fail(SDPB_ERR_CUDA, "cudaMemcpyAsync failed");
-    std::vector<const void*> tab((size_t)T * 4);
-    std::vector<int> stall_t;
-    std::vector<MLKey> stall_k;
-    float kern = 0;
-    int rounds = 0, na = n, cur = 0;
-    while (na > 0) {
-        // the tables move when an extension merges new states in: hand the kernel the current ones
-        for (int t = 0; t < T; t++) {
-            tab[t] = h->F[t];
-            tab[T + t] = h->V[t];
-            tab[2 * T + t] = h->Qa[t];
-            std::memcpy(&tab[3 * T + t], &h->nF[t], sizeof(long long));
-        }
-        int ns = 0;
-        if (cudaMemcpyAsync(tab_b.p, tab.data(), tab.size() * 8, cudaMemcpyHostToDevice, st) != cudaSuccess ||
-            cudaMemsetAsync(sn_b.p, 0, sizeof(int), st) != cudaSuccess || cudaEventRecord(h->e1, st) != cudaSuccess)
-            return ml_fail(SDPB_ERR_CUDA, "cudaMemcpyAsync failed");
-        ml_simulate<<<(na + 127) / 128, 128, 0, st>>>(h->P, dF, dV, dQ, dn, (const double*)smp_b.p, nd, (const double*)pw_b.p,
-                                                      (const int*)act_b[cur].p, na, (MLKey*)key_b.p, (int*)per_b.p,
-                                                      (double*)sum_b.p, (double*)val_b.p, (int*)sn_b.p,
-                                                      (int*)act_b[1 - cur].p, (int*)st_b.p, (MLKey*)sk_b.p);
-        if (cudaGetLastError() != cudaSuccess) return ml_fail(SDPB_ERR_CUDA, "ml_simulate launch failed");
-        if (cudaEventRecord(h->e2, st) != cudaSuccess ||
-            cudaMemcpyAsync(&ns, sn_b.p, sizeof(int), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
-            cudaStreamSynchronize(st) != cudaSuccess)
-            return ml_fail(SDPB_ERR_CUDA, std::string("roll-out: ") + cudaGetErrorString(cudaGetLastError()));
-        float ms = 0;
-        cudaEventElapsedTime(&ms, h->e1, h->e2);
-        kern += ms;
-        rounds++;
-        if (ns == 0) break;
-        // the states the stalled paths stand on become the roots of one extension (getExpectedValue(state))
-        stall_t.resize((size_t)ns);
-        stall_k.resize((size_t)ns);
-        if (cudaMemcpyAsync(stall_t.data(), st_b.p, (size_t)ns * sizeof(int), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
-            cudaMemcpyAsync(stall_k.data(), sk_b.p, (size_t)ns * sizeof(MLKey), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
-            cudaStreamSynchronize(st) != cudaSuccess)
-            return ml_fail(SDPB_ERR_CUDA, "cudaMemcpyAsync failed");
-        std::vector<std::vector<MLKey>> r((size_t)T);
-        int p = T;
-        for (int j = 0; j < ns; j++) {
-            r[stall_t[j] - 1].push_back(stall_k[j]);
-            p = std::min(p, stall_t[j]);
-        }
-        for (auto& v : r) {
-            std::sort(v.begin(), v.end(), MLKeyLess());
-            v.erase(std::unique(v.begin(), v.end(), MLKeyEq()), v.end());
-        }
-        rc = ml_extend(h, p, r);
-        if (rc != SDPB_OK) return rc;
-        na = ns;
-        cur = 1 - cur;
-    }
-    if (cudaMemcpyAsync(values, val_b.p, N * sizeof(double), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
-        cudaStreamSynchronize(st) != cudaSuccess)
-        return ml_fail(SDPB_ERR_CUDA, "cudaMemcpyAsync failed");
-    h->stats.solve_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - w0).count();
-    h->stats.kernel_ms = kern;
-    h->stats.launches = rounds;
-    return SDPB_OK;
+    auto extend = [h](int p, const std::vector<std::vector<MLKey>>& r) { return ml_extend(h, p, r); };
+    return memo::rollout(h->mt, MLStep{h->P}, roots[0][0], samples, n, nd, discount, extend, values, g_ml_error);
 }
 
 int sdpb_reached_solve(const sdpb_reached_model* m, int device, const double* init_state, double* value, double* action1,
@@ -1084,7 +822,7 @@ int sdpb_reached_solve(const sdpb_reached_model* m, int device, const double* in
     if (rc != SDPB_OK) return rc;
     rc = sdpb_reached_value(h, 1, init_state, 1, value, action1, action2);
     if (rc == SDPB_OK && n_states) sdpb_reached_states(h, n_states);
-    if (rc == SDPB_OK && solve_ms) *solve_ms = h->stats.solve_ms;
+    if (rc == SDPB_OK && solve_ms) *solve_ms = h->mt.stats.solve_ms;
     sdpb_reached_destroy(h);
     return rc;
 }

@@ -31,15 +31,12 @@
 #include <thrust/execution_policy.h>
 #include <thrust/merge.h>
 #include <thrust/remove.h>
-#include <thrust/iterator/zip_iterator.h>
 #include <thrust/scan.h>
 #include <thrust/set_operations.h>
-#include <thrust/tuple.h>
 #include <thrust/unique.h>
 
 #include <algorithm>
 #include <cfloat>
-#include <chrono>
 #include <cmath>
 #include <cstdint>
 #include <cstring>
@@ -49,6 +46,7 @@
 
 #include "../../include/sdpb200.h"
 #include "kernel_generic.cuh"
+#include "memo_tables.cuh"
 
 namespace {
 using namespace sdpb;
@@ -91,6 +89,7 @@ template <> struct TDDecomp<4> {
 };
 
 // order-preserving encoding of a double: set the sign bit of a non-negative value, flip every bit of a negative one
+// (a select: reached.cu's branch-free ml_enc, the same mapping, changes every td_* kernel here and was not timed)
 __host__ __device__ inline u64 td_enc(double v) {
     v += 0.0;  // -0.0 and +0.0 are one key (the memo map compares with ==)
     u64 b;
@@ -235,6 +234,15 @@ __device__ __forceinline__ long long td_find(const TDKey* __restrict__ F, long l
     return td_lower(F, max(b - step + 1, 0ll), b, k);
 }
 
+struct TDTraits {  // the key of the memo tables (memo_tables.cuh)
+    typedef TDKey Key;
+    typedef TDLess Less;
+    typedef TDEq Eq;
+    static __device__ __forceinline__ long long lower(const TDKey* __restrict__ F, long long n, const TDKey& k) {
+        return td_lower(F, 0, n, k);
+    }
+};
+
 // |A_t(s)| of every state; XR states whose order-up-to range was cut at max_order_idx + 1 are counted
 template <int KIND>
 __global__ void __launch_bounds__(256) td_count_actions(const __grid_constant__ TDModel P, const int t,
@@ -338,67 +346,25 @@ __global__ void __launch_bounds__(256) td_backward(const __grid_constant__ TDMod
     }
 }
 
-// queries: (V, action index) of each key, or action index -2 when the state was not reached
-__global__ void td_query(const TDKey* __restrict__ F, const long long n, const double* __restrict__ V,
-                         const int* __restrict__ Q, const TDKey* __restrict__ q, const int nq, double* __restrict__ v,
-                         int* __restrict__ qi) {
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= nq) return;
-    const TDKey k = q[i];
-    const long long at = td_lower(F, 0, n, k);
-    const bool hit = at < n && TDEq()(F[at], k);
-    v[i] = hit ? V[at] : 0.0;
-    qi[i] = hit ? Q[at] : -2;
-}
-
-// One thread per path of act[0, na): Simulation.java:59-70 from where the path stands (period per[i], state key[i],
-// partial sum sum[i]) -- Q = getAction(state), d = Math.round(sample), sum += discount^(t-1) c, state = f(s, Q, d) --
-// until it ends (values[i] = sum) or meets a state the handle has not reached.  There it writes (path, t, state) to
-// the next slot of the stall list, keeps its period, state and partial sum, and stops; the host extends the handle
-// with the stalled states and relaunches the stalled paths.  f is applied whatever the cash: a survival model's
-// roll-out goes on after a bankrupt period, as the reference's does.
+// One period of Simulation.java:59-70 for memo::memo_simulate: Q = getAction(state), d = Math.round(sample),
+// c = the immediate value, state = f(s, Q, d).  f is applied whatever the cash: a survival model's roll-out goes on after
+// a bankrupt period, as the reference's does.
 template <int KIND>
-__global__ void __launch_bounds__(128) td_simulate(const __grid_constant__ TDModel P, const TDKey* const* __restrict__ tF,
-                                                   const int* const* __restrict__ tQ, const long long* __restrict__ tn,
-                                                   const double* __restrict__ samples, const double* __restrict__ pw,
-                                                   const int* __restrict__ act, const int na, TDKey* __restrict__ key,
-                                                   int* __restrict__ per, double* __restrict__ sum,
-                                                   double* __restrict__ values, int* __restrict__ stall_n,
-                                                   int* __restrict__ stall_path, int* __restrict__ stall_t,
-                                                   TDKey* __restrict__ stall_key) {
-    const int k = blockIdx.x * blockDim.x + threadIdx.x;
-    if (k >= na) return;
-    const int i = act[k], T = P.M.T;
-    TDKey s = key[i];
-    double acc = sum[i];
-    for (int t = per[i]; t <= T; t++) {
-        const TDKey* __restrict__ F = tF[t - 1];
-        const long long n = tn[t - 1];
-        const long long at = td_lower(F, 0, n, s);
-        if (at >= n || !TDEq()(F[at], s)) {
-            key[i] = s;
-            per[i] = t;
-            sum[i] = acc;
-            const int slot = atomicAdd(stall_n, 1);
-            stall_path[slot] = i;
-            stall_t[slot] = t;
-            stall_key[slot] = s;
-            return;
-        }
-        int qi = tQ[t - 1][at];
+struct TDStep {
+    TDModel P;
+    __device__ __forceinline__ bool operator()(int t, TDKey& s, int qi, double, const double* smp, double& c) const {
         if (qi < 0) qi = 0;  // bestOrderQty stayed 0
         double q2;
         const StateCtx S = td_state<KIND>(P, t, s, q2);
         const ActionCtx A = prep_action<KIND>(P.M, S, qi);
-        const double d = (double)jround(samples[(size_t)i * T + (t - 1)]);  // Math.round(samples[i][t])
+        const double d = (double)jround(*smp);  // Math.round(samples[i][t])
         double after;
-        const double c = immediate<KIND>(P.M, S, A, d, after);
-        acc += pw[t - 1] * c;
+        c = immediate<KIND>(P.M, S, A, d, after);
         bool bankrupt;
-        if (t < T) s = td_next<KIND>(P, S, q2, A, d, c, after, bankrupt);
+        if (t < P.M.T) s = td_next<KIND>(P, S, q2, A, d, c, after, bankrupt);
+        return false;
     }
-    values[i] = acc;
-}
+};
 
 bool has_cash(const sdpb_model& m) { return m.cost_kind != SDPB_COST_BACKORDER; }
 
@@ -413,15 +379,9 @@ struct sdpb_topdown {
     int ndim = 1;
     unsigned allow = 0;
     long long scratch_bytes = 0;
-    cudaStream_t stream = nullptr;
-    cudaEvent_t e0 = nullptr, e1 = nullptr, e2 = nullptr;
     std::vector<int> pmf_len, pmf_off;
-    std::vector<void*> owned;                                 // model tables
-    std::vector<TDKey*> F;                                    // [T] reached states, sorted
-    std::vector<double*> V;                                   // [T]
-    std::vector<int*> Q;                                      // [T] action index, -1: none improved on the initial value
-    std::vector<long long> nF;
-    sdpb_stats stats{};
+    std::vector<void*> owned;   // model tables
+    memo::Tables<TDTraits> mt;  // action index -1: none improved on the initial value
     std::string err;
 };
 
@@ -430,16 +390,6 @@ namespace {
 int td_fail(sdpb_topdown* h, int rc, const std::string& msg) {
     if (h) h->err = msg; else g_td_error = msg;
     return rc;
-}
-
-void td_free_tables(sdpb_topdown* h) {
-    for (TDKey* p : h->F) cudaFree(p);
-    for (double* p : h->V) cudaFree(p);
-    for (int* p : h->Q) cudaFree(p);
-    h->F.assign(h->m.T, nullptr);
-    h->V.assign(h->m.T, nullptr);
-    h->Q.assign(h->m.T, nullptr);
-    h->nF.assign(h->m.T, 0);
 }
 
 template <int ND>
@@ -458,7 +408,7 @@ cudaError_t td_sort_nd(int nd, void* tmp, size_t& tmp_bytes, cub::DoubleBuffer<T
 template <int KIND>
 void launch_count(const sdpb_topdown* h, int t, const TDKey* F, long long n, long long* nA, unsigned long long* capped) {
     if (n == 0) return;
-    td_count_actions<KIND><<<(unsigned)((n + 255) / 256), 256, 0, h->stream>>>(h->P, t, F, n, nA, capped);
+    td_count_actions<KIND><<<(unsigned)((n + 255) / 256), 256, 0, h->mt.stream>>>(h->P, t, F, n, nA, capped);
 }
 template <int KIND>
 void launch_expand(const sdpb_topdown* h, int t, const TDKey* F, long long n, const long long* off, long long p0,
@@ -466,9 +416,9 @@ void launch_expand(const sdpb_topdown* h, int t, const TDKey* F, long long n, co
     const int D = h->pmf_len[t - 1], po = h->pmf_off[t - 1];
     const unsigned blocks = (unsigned)((np + 255) / 256);
     if (h->m.recursion == SDPB_REC_SURVIVAL)
-        td_expand<KIND, true><<<blocks, 256, 0, h->stream>>>(h->P, t, D, po, F, n, off, p0, np, out);
+        td_expand<KIND, true><<<blocks, 256, 0, h->mt.stream>>>(h->P, t, D, po, F, n, off, p0, np, out);
     else
-        td_expand<KIND, false><<<blocks, 256, 0, h->stream>>>(h->P, t, D, po, F, n, off, p0, np, out);
+        td_expand<KIND, false><<<blocks, 256, 0, h->mt.stream>>>(h->P, t, D, po, F, n, off, p0, np, out);
 }
 // V, Q of the n states F of period t, against the sorted (Fn, Vn) of period t + 1 (nn states; none when t == T)
 template <int KIND>
@@ -479,23 +429,13 @@ void launch_backward(const sdpb_topdown* h, int t, const TDKey* F, long long n, 
     const unsigned blocks = (unsigned)((n + 7) / 8);
     if (h->m.recursion == SDPB_REC_SURVIVAL) {
         if constexpr (KIND == SDPB_COST_CASH_DEPOSIT || KIND == SDPB_COST_CASH_OVERDRAFT)
-            td_backward<KIND, true, false><<<blocks, 256, 0, h->stream>>>(h->P, t, D, po, F, n, Fn, Vn, nn, V, Q);
+            td_backward<KIND, true, false><<<blocks, 256, 0, h->mt.stream>>>(h->P, t, D, po, F, n, Fn, Vn, nn, V, Q);
     } else if (h->m.direction == SDPB_MIN) {
-        td_backward<KIND, false, true><<<blocks, 256, 0, h->stream>>>(h->P, t, D, po, F, n, Fn, Vn, nn, V, Q);
+        td_backward<KIND, false, true><<<blocks, 256, 0, h->mt.stream>>>(h->P, t, D, po, F, n, Fn, Vn, nn, V, Q);
     } else {
-        td_backward<KIND, false, false><<<blocks, 256, 0, h->stream>>>(h->P, t, D, po, F, n, Fn, Vn, nn, V, Q);
+        td_backward<KIND, false, false><<<blocks, 256, 0, h->mt.stream>>>(h->P, t, D, po, F, n, Fn, Vn, nn, V, Q);
     }
 }
-template <int KIND>
-void launch_simulate(const sdpb_topdown* h, const TDKey* const* tF, const int* const* tQ, const long long* tn,
-                     const double* samples, const double* pw,
-                     const int* act, int na, TDKey* key, int* per, double* sum, double* values, int* stall_n,
-                     int* stall_path, int* stall_t, TDKey* stall_key) {
-    td_simulate<KIND><<<(na + 127) / 128, 128, 0, h->stream>>>(h->P, tF, tQ, tn, samples, pw, act, na, key, per, sum,
-                                                               values,
-                                                               stall_n, stall_path, stall_t, stall_key);
-}
-
 #define TD_DISPATCH(fn, ...)                                                                  \
     switch (h->m.cost_kind) {                                                                 \
     case SDPB_COST_BACKORDER: fn<SDPB_COST_BACKORDER>(__VA_ARGS__); break;                    \
@@ -506,42 +446,6 @@ void launch_simulate(const sdpb_topdown* h, const TDKey* const* tF, const int* c
     case SDPB_COST_CASH_OD_TESTING: fn<SDPB_COST_CASH_OD_TESTING>(__VA_ARGS__); break;        \
     default: fn<SDPB_COST_CASH_LOAN>(__VA_ARGS__); break;                                     \
     }
-
-struct DevBuf {  // a scratch allocation released when it goes out of scope
-    void* p = nullptr;
-    ~DevBuf() { if (p) cudaFree(p); }
-    bool alloc(size_t bytes) {
-        if (p) { cudaFree(p); p = nullptr; }
-        if (cudaMalloc(&p, bytes > 0 ? bytes : 16) != cudaSuccess) { cudaGetLastError(); p = nullptr; return false; }
-        return true;
-    }
-};
-
-template <class P>
-bool td_alloc(P*& p, long long n) {
-    if (cudaMalloc((void**)&p, (size_t)std::max(n, 1ll) * sizeof(P)) == cudaSuccess) return true;
-    cudaGetLastError();
-    p = nullptr;
-    return false;
-}
-
-// What one extension builds, owned here until it is committed to the handle: per period the new states N_t with their
-// V / Q, and the merged tables F_t u N_t.  Whatever is still owned when the stage goes out of scope is freed, so an
-// extension that fails leaves the handle as it found it.
-struct TDStage {
-    std::vector<TDKey*> N, MF;
-    std::vector<double*> VN, MV;
-    std::vector<int*> QN, MQ;
-    std::vector<long long> nN, nM;
-    explicit TDStage(int T)
-        : N(T, nullptr), MF(T, nullptr), VN(T, nullptr), MV(T, nullptr), QN(T, nullptr), MQ(T, nullptr), nN(T, 0),
-          nM(T, 0) {}
-    ~TDStage() {
-        for (size_t k = 0; k < N.size(); k++) {
-            cudaFree(N[k]); cudaFree(MF[k]); cudaFree(VN[k]); cudaFree(MV[k]); cudaFree(QN[k]); cudaFree(MQ[k]);
-        }
-    }
-};
 
 // N_t: the roots of period t and the successors of the n_src states `src` of period t - 1 (`off`: their action offsets,
 // `pairs` (state, action) pairs), minus the states the handle already holds in period t; sorted, into *out.
@@ -557,9 +461,9 @@ int td_new_states(sdpb_topdown* h, int t, const TDKey* src, long long n_src, con
     const long long nr = (long long)roots.size();
     if (pairs == 0 && nr == 0) return SDPB_OK;
     const int nd = h->P.nd(), D = t > 1 ? h->pmf_len[t - 2] : 1;
-    const TDKey* Fo = h->F[t - 1];
-    const long long no = h->nF[t - 1];
-    cudaStream_t st = h->stream;
+    const TDKey* Fo = h->mt.F[t - 1];
+    const long long no = h->mt.nF[t - 1];
+    cudaStream_t st = h->mt.stream;
     auto par = thrust::cuda::par.on(st);
     const long long cand = pairs * D + nr, key3 = 3 * (long long)sizeof(TDKey);
     const std::string per = "period " + std::to_string(t);
@@ -586,7 +490,7 @@ int td_new_states(sdpb_topdown* h, int t, const TDKey* src, long long n_src, con
                            " keys per buffer, at most half of them new states) can expand");
     };
     if (nr > cap) return too_many(nr);
-    DevBuf kb[3], tmp_b;
+    memo::DevBuf kb[3], tmp_b;
     for (auto& b : kb)
         if (!b.alloc((size_t)cap * sizeof(TDKey)))
             return td_fail(h, SDPB_ERR_NOMEM, "allocation of the expansion scratch failed (" + per + ")");
@@ -633,7 +537,7 @@ int td_new_states(sdpb_topdown* h, int t, const TDKey* src, long long n_src, con
         return td_fail(h, SDPB_ERR_CUDA, std::string("sort / merge: ") + ex.what());
     }
     if (nf == 0) return cudaStreamSynchronize(st) == cudaSuccess ? SDPB_OK : td_fail(h, SDPB_ERR_CUDA, "forward pass");
-    if (!td_alloc(*out, nf)) return td_fail(h, SDPB_ERR_NOMEM, "allocation of the states of " + per + " failed");
+    if (!memo::alloc(*out, nf)) return td_fail(h, SDPB_ERR_NOMEM, "allocation of the states of " + per + " failed");
     *n_out = nf;
     if (cudaMemcpyAsync(*out, front, (size_t)nf * sizeof(TDKey), cudaMemcpyDeviceToDevice, st) != cudaSuccess ||
         cudaStreamSynchronize(st) != cudaSuccess)
@@ -643,12 +547,12 @@ int td_new_states(sdpb_topdown* h, int t, const TDKey* src, long long n_src, con
 
 // The forward pass of an extension from period p: N_t for t = p .. T into the stage, and the evaluations and capped XR
 // action sets of the new states.
-int td_forward(sdpb_topdown* h, int p, const std::vector<std::vector<TDKey>>& roots, TDStage& sg, double& evals,
-               double& capped_total) {
+int td_forward(sdpb_topdown* h, int p, const std::vector<std::vector<TDKey>>& roots, memo::Stage<TDTraits>& sg,
+               double& evals, double& capped_total) {
     const int T = h->m.T;
-    cudaStream_t st = h->stream;
+    cudaStream_t st = h->mt.stream;
     auto par = thrust::cuda::par.on(st);
-    DevBuf cap_b, off_b;  // off_b: exclusive prefix sum of |A_t(s)| over N_t (n + 1 entries)
+    memo::DevBuf cap_b, off_b;  // off_b: exclusive prefix sum of |A_t(s)| over N_t (n + 1 entries)
     if (!cap_b.alloc(sizeof(unsigned long long))) return td_fail(h, SDPB_ERR_NOMEM, "allocation failed");
     unsigned long long* d_capped = (unsigned long long*)cap_b.p;
     long long pairs = 0;
@@ -686,76 +590,28 @@ int td_forward(sdpb_topdown* h, int p, const std::vector<std::vector<TDKey>>& ro
 // t < p): the forward pass builds the states no earlier call reached, the backward pass solves only those against the
 // merged tables of the next period, and the merged tables of every touched period replace the handle's at the end.
 int td_extend(sdpb_topdown* h, int p, const std::vector<std::vector<TDKey>>& roots) {
-    const int T = h->m.T;
-    cudaStream_t st = h->stream;
-    auto par = thrust::cuda::par.on(st);
-    TDStage sg(T);
-    if (cudaEventRecord(h->e0, st) != cudaSuccess) return td_fail(h, SDPB_ERR_CUDA, "cudaEventRecord failed");
+    memo::Stage<TDTraits> sg(h->m.T);
+    if (cudaEventRecord(h->mt.e0, h->mt.stream) != cudaSuccess) return td_fail(h, SDPB_ERR_CUDA, "cudaEventRecord failed");
     double evals = 0, capped = 0;
-    int rc = td_forward(h, p, roots, sg, evals, capped);
+    const int rc = td_forward(h, p, roots, sg, evals, capped);
     if (rc != SDPB_OK) return rc;
     if (capped > 0 && !(h->allow & SDPB_ALLOW_CAPPED_ACTIONS))
         return td_fail(h, SDPB_ERR_OFFGRID,
                        std::to_string((long long)capped) +
                            " reached XR states have an order-up-to range longer than max_order_idx + 1 "
                            "(allow SDPB_ALLOW_CAPPED_ACTIONS to cut it there)");
-    if (cudaEventRecord(h->e1, st) != cudaSuccess) return td_fail(h, SDPB_ERR_CUDA, "cudaEventRecord failed");
-    int launches = 0;
-    for (int t = T; t >= p; t--) {
-        const int k = t - 1;
-        const long long n = sg.nN[k], no = h->nF[k];
-        if (n == 0) continue;
-        if (!td_alloc(sg.VN[k], n) || !td_alloc(sg.QN[k], n))
-            return td_fail(h, SDPB_ERR_NOMEM, "allocation of the value tables failed");
-        const bool nxt = t < T, nxt_new = nxt && sg.nN[k + 1] > 0;
-        TD_DISPATCH(launch_backward, h, t, sg.N[k], n, nxt ? (nxt_new ? sg.MF[k + 1] : h->F[k + 1]) : nullptr,
-                    nxt ? (nxt_new ? sg.MV[k + 1] : h->V[k + 1]) : nullptr,
-                    nxt ? (nxt_new ? sg.nM[k + 1] : h->nF[k + 1]) : 0, sg.VN[k], sg.QN[k])
-        launches++;
-        if (cudaGetLastError() != cudaSuccess) return td_fail(h, SDPB_ERR_CUDA, "td_backward launch failed");
-        sg.nM[k] = no + n;
-        if (no == 0) {  // nothing to merge with: the new tables are the merged ones
-            std::swap(sg.MF[k], sg.N[k]);
-            std::swap(sg.MV[k], sg.VN[k]);
-            std::swap(sg.MQ[k], sg.QN[k]);
-            continue;
-        }
-        if (!td_alloc(sg.MF[k], no + n) || !td_alloc(sg.MV[k], no + n) || !td_alloc(sg.MQ[k], no + n))
-            return td_fail(h, SDPB_ERR_NOMEM, "allocation of the merged tables of period " + std::to_string(t) + " failed");
-        try {  // the two key sets are disjoint: a merge by key keeps every row
-            thrust::merge_by_key(par, h->F[k], h->F[k] + no, sg.N[k], sg.N[k] + n,
-                                 thrust::make_zip_iterator(thrust::make_tuple(h->V[k], h->Q[k])),
-                                 thrust::make_zip_iterator(thrust::make_tuple(sg.VN[k], sg.QN[k])), sg.MF[k],
-                                 thrust::make_zip_iterator(thrust::make_tuple(sg.MV[k], sg.MQ[k])), TDLess());
-        } catch (const std::exception& ex) {
-            return td_fail(h, SDPB_ERR_CUDA, std::string("merge: ") + ex.what());
-        }
-    }
-    if (cudaEventRecord(h->e2, st) != cudaSuccess || cudaEventSynchronize(h->e2) != cudaSuccess)
-        return td_fail(h, SDPB_ERR_CUDA, std::string("backward pass: ") + cudaGetErrorString(cudaGetLastError()));
-    for (int k = p - 1; k < T; k++) {  // commit
-        if (sg.nN[k] == 0) continue;
-        cudaFree(h->F[k]);
-        cudaFree(h->V[k]);
-        cudaFree(h->Q[k]);
-        h->F[k] = sg.MF[k];
-        h->V[k] = sg.MV[k];
-        h->Q[k] = sg.MQ[k];
-        sg.MF[k] = nullptr;
-        sg.MV[k] = nullptr;
-        sg.MQ[k] = nullptr;
-        h->nF[k] = sg.nM[k];
-    }
-    float solve = 0, kern = 0;
-    cudaEventElapsedTime(&solve, h->e0, h->e2);
-    cudaEventElapsedTime(&kern, h->e1, h->e2);
-    h->stats.evals += evals;
-    h->stats.evals_executed += evals;
-    h->stats.capped_action_sets += capped;
-    h->stats.solve_ms = solve;
-    h->stats.kernel_ms = kern;
-    h->stats.launches = launches;
-    return SDPB_OK;
+    auto backward = [h](int t, const TDKey* F, long long n, const TDKey* Fn, const double* Vn, long long nn, double* V,
+                        int* Q) {
+        TD_DISPATCH(launch_backward, h, t, F, n, Fn, Vn, nn, V, Q)
+        return 1;
+    };
+    return memo::commit(h->mt, sg, p, evals, capped, backward, h->err);
+}
+
+template <int KIND>
+int td_rollout(sdpb_topdown* h, const TDKey& k0, const double* samples, int n, double discount, double* values) {
+    auto extend = [h](int p, const std::vector<std::vector<TDKey>>& r) { return td_extend(h, p, r); };
+    return memo::rollout(h->mt, TDStep<KIND>{h->P}, k0, samples, n, 1, discount, extend, values, h->err);
 }
 
 // The key of one API-order state
@@ -776,22 +632,15 @@ int td_root_keys(sdpb_topdown* h, const double* states, int n, std::vector<TDKey
             if (!std::isfinite(s[k])) return td_fail(h, SDPB_ERR_ARG, "a state is not finite");
         out[i] = td_key_of(h, s);
     }
-    std::sort(out.begin(), out.end(), TDLess());
-    out.erase(std::unique(out.begin(), out.end(), TDEq()), out.end());
+    memo::canonical<TDTraits>(out);
     return SDPB_OK;
 }
 
 void td_destroy(sdpb_topdown* h) {
     if (!h) return;
     if (h->device >= 0) cudaSetDevice(h->device);
-    td_free_tables(h);
     for (void* p : h->owned) cudaFree(p);
-    if (h->e0) cudaEventDestroy(h->e0);
-    if (h->e1) cudaEventDestroy(h->e1);
-    if (h->e2) cudaEventDestroy(h->e2);
-    if (h->stream) cudaStreamDestroy(h->stream);
-    cudaGetLastError();
-    delete h;
+    delete h;  // and its memo tables
 }
 
 }  // namespace
@@ -864,11 +713,8 @@ int sdpb_topdown_solve(const sdpb_model* m, const sdpb_topdown_options* opt, con
     h->pmf_len = len;
     h->pmf_off = poff;
     h->ndim = 1 + (has_cash(*m) ? 1 : 0) + m->lead_time;
-    auto bail = [&](int rc, const std::string& msg) { td_destroy(h); return td_fail(nullptr, rc, msg); };
-    if (cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking) != cudaSuccess || cudaEventCreate(&h->e0) != cudaSuccess ||
-        cudaEventCreate(&h->e1) != cudaSuccess || cudaEventCreate(&h->e2) != cudaSuccess)
-        return bail(SDPB_ERR_CUDA, "stream / event creation failed");
-    td_free_tables(h);
+    auto bail = [&](int rc, std::string msg) { td_destroy(h); return td_fail(nullptr, rc, msg); };
+    if (h->mt.open(T, h->err) != SDPB_OK) return bail(SDPB_ERR_CUDA, h->err);
 
     // device model: the scalars the lambdas read, per-period tables expanded to T entries
     const int NP = poff[T];
@@ -885,7 +731,7 @@ int sdpb_topdown_solve(const sdpb_model* m, const sdpb_topdown_options* opt, con
         void* p = nullptr;
         if (cudaMalloc(&p, v.size() * sizeof(double)) != cudaSuccess) { cudaGetLastError(); return nullptr; }
         h->owned.push_back(p);
-        if (cudaMemcpyAsync(p, v.data(), v.size() * sizeof(double), cudaMemcpyHostToDevice, h->stream) != cudaSuccess) return nullptr;
+        if (cudaMemcpyAsync(p, v.data(), v.size() * sizeof(double), cudaMemcpyHostToDevice, h->mt.stream) != cudaSuccess) return nullptr;
         return (const double*)p;
     };
     DevModel& d = h->P.M;
@@ -936,23 +782,20 @@ int sdpb_topdown_solve(const sdpb_model* m, const sdpb_topdown_options* opt, con
     std::vector<std::vector<TDKey>> roots((size_t)T);
     int rc = td_root_keys(h, init_states, n, roots[0]);
     if (rc == SDPB_OK) rc = td_extend(h, 1, roots);
-    if (rc != SDPB_OK) {
-        const std::string msg = h->err;
-        return bail(rc, msg);
-    }
+    if (rc != SDPB_OK) return bail(rc, h->err);
     *out = h;
     return SDPB_OK;
 }
 
 int sdpb_topdown_states(const sdpb_topdown* h, int64_t* n_states) {
     if (!h || !n_states) return SDPB_ERR_ARG;
-    for (int t = 0; t < h->m.T; t++) n_states[t] = h->nF[t];
+    for (int t = 0; t < h->m.T; t++) n_states[t] = h->mt.nF[t];
     return SDPB_OK;
 }
 
 int sdpb_topdown_stats(const sdpb_topdown* h, sdpb_stats* s) {
     if (!h || !s) return SDPB_ERR_ARG;
-    *s = h->stats;
+    *s = h->mt.stats;
     return SDPB_OK;
 }
 
@@ -963,23 +806,10 @@ int sdpb_topdown_value(sdpb_topdown* h, int period, const double* states, int n,
     cudaSetDevice(h->device);
     std::vector<TDKey> keys((size_t)n);
     for (int i = 0; i < n; i++) keys[i] = td_key_of(h, states + (size_t)i * h->ndim);
-    DevBuf kq, vq, aq;
-    if (!kq.alloc(keys.size() * sizeof(TDKey)) || !vq.alloc((size_t)n * sizeof(double)) || !aq.alloc((size_t)n * sizeof(int)))
-        return td_fail(h, SDPB_ERR_NOMEM, "allocation failed");
-    std::vector<double> vv((size_t)n);
-    std::vector<int> qi((size_t)n);
-    cudaStream_t st = h->stream;
-    if (cudaMemcpyAsync(kq.p, keys.data(), keys.size() * sizeof(TDKey), cudaMemcpyHostToDevice, st) != cudaSuccess)
-        return td_fail(h, SDPB_ERR_CUDA, "cudaMemcpyAsync failed");
-    td_query<<<(n + 127) / 128, 128, 0, st>>>(h->F[period - 1], h->nF[period - 1], h->V[period - 1], h->Q[period - 1],
-                                               (const TDKey*)kq.p, n, (double*)vq.p, (int*)aq.p);
-    if (cudaMemcpyAsync(vv.data(), vq.p, (size_t)n * sizeof(double), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
-        cudaMemcpyAsync(qi.data(), aq.p, (size_t)n * sizeof(int), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
-        cudaStreamSynchronize(st) != cudaSuccess)
-        return td_fail(h, SDPB_ERR_CUDA, std::string("query: ") + cudaGetErrorString(cudaGetLastError()));
-    for (int i = 0; i < n; i++)
-        if (qi[i] == -2)
-            return td_fail(h, SDPB_ERR_UNSOLVED, "state " + std::to_string(i) + " was not reached in period " + std::to_string(period));
+    std::vector<double> vv;
+    std::vector<int> qi;
+    const int rc = memo::lookup(h->mt, period, keys, vv, qi, h->err);
+    if (rc != SDPB_OK) return rc;
     for (int i = 0; i < n; i++) {
         if (v) v[i] = vv[i];
         // bestOrderQty stays 0 when no action improves on the initial value; XR reports the order-up-to level
@@ -991,37 +821,20 @@ int sdpb_topdown_value(sdpb_topdown* h, int period, const double* states, int n,
 
 int sdpb_topdown_opt_table(sdpb_topdown* h, double* rows, size_t* nrows) {
     if (!h || !nrows) return td_fail(h, SDPB_ERR_ARG, "null argument");
-    size_t total = 0;
-    for (int t = 0; t < h->m.T; t++) total += (size_t)h->nF[t];
-    if (!rows) { *nrows = total; return SDPB_OK; }
-    if (*nrows < total) return td_fail(h, SDPB_ERR_ARG, "rows holds fewer than the reached states");
     cudaSetDevice(h->device);
-    const int w = h->ndim + 2;
-    size_t r = 0;
-    for (int t = 1; t <= h->m.T; t++) {
-        const long long n = h->nF[t - 1];
-        std::vector<TDKey> k((size_t)n);
-        std::vector<int> qi((size_t)n);
-        if (cudaMemcpyAsync(k.data(), h->F[t - 1], (size_t)n * sizeof(TDKey), cudaMemcpyDeviceToHost, h->stream) != cudaSuccess ||
-            cudaMemcpyAsync(qi.data(), h->Q[t - 1], (size_t)n * sizeof(int), cudaMemcpyDeviceToHost, h->stream) != cudaSuccess ||
-            cudaStreamSynchronize(h->stream) != cudaSuccess)
-            return td_fail(h, SDPB_ERR_CUDA, "cudaMemcpyAsync failed");
-        for (long long i = 0; i < n; i++, r++) {
-            double x, q1, q2, cw;
-            td_unpack(h->P, k[i], x, q1, q2, cw);
-            double* row = rows + r * w;
-            int c = 0;
-            row[c++] = t;
-            row[c++] = x;
-            if (h->P.cash) row[c++] = cw;
-            if (h->P.lead >= 1) row[c++] = q1;
-            if (h->P.lead >= 2) row[c++] = q2;
-            const double a = qi[i] < 0 ? 0.0 : qi[i] * h->m.step;
-            row[c] = (qi[i] >= 0 && h->m.cost_kind == SDPB_COST_CASH_XR) ? x + a : a;
-        }
-    }
-    *nrows = total;
-    return SDPB_OK;
+    auto row = [h](int t, const TDKey& k, double, int qi, double* row) {
+        double x, q1, q2, cw;
+        td_unpack(h->P, k, x, q1, q2, cw);
+        int c = 0;
+        row[c++] = t;
+        row[c++] = x;
+        if (h->P.cash) row[c++] = cw;
+        if (h->P.lead >= 1) row[c++] = q1;
+        if (h->P.lead >= 2) row[c++] = q2;
+        const double a = qi < 0 ? 0.0 : qi * h->m.step;
+        row[c] = (qi >= 0 && h->m.cost_kind == SDPB_COST_CASH_XR) ? x + a : a;
+    };
+    return memo::opt_table(h->mt, rows, nrows, h->ndim + 2, row, h->err);
 }
 
 int sdpb_topdown_extend(sdpb_topdown* h, int period, const double* states, int n) {
@@ -1045,93 +858,9 @@ int sdpb_topdown_simulate(sdpb_topdown* h, const double* init_state, const doubl
     std::vector<std::vector<TDKey>> roots((size_t)T);
     int rc = td_root_keys(h, init_state, 1, roots[0]);
     if (rc != SDPB_OK) return rc;
-    const TDKey k0 = roots[0][0];
-    const auto w0 = std::chrono::steady_clock::now();
     cudaSetDevice(h->device);
-    rc = td_extend(h, 1, roots);  // Simulation.java:62 asks for getExpectedValue(iniState) first
-    if (rc != SDPB_OK) return rc;
-
-    cudaStream_t st = h->stream;
-    std::vector<double> pw((size_t)T);
-    for (int t = 0; t < T; t++) pw[t] = std::pow(discount, (double)t);  // Math.pow(discountFactor, t)
-    std::vector<TDKey> key0((size_t)n, k0);
-    std::vector<int> per0((size_t)n, 1), act0((size_t)n);
-    for (int i = 0; i < n; i++) act0[i] = i;
-    DevBuf smp_b, pw_b, key_b, per_b, sum_b, val_b, act_b[2], st_b, sk_b, sn_b, tab_b;
-    const size_t N = (size_t)n;
-    if (!smp_b.alloc(N * T * sizeof(double)) || !pw_b.alloc(T * sizeof(double)) || !key_b.alloc(N * sizeof(TDKey)) ||
-        !per_b.alloc(N * sizeof(int)) || !sum_b.alloc(N * sizeof(double)) || !val_b.alloc(N * sizeof(double)) ||
-        !act_b[0].alloc(N * sizeof(int)) || !act_b[1].alloc(N * sizeof(int)) || !st_b.alloc(N * sizeof(int)) ||
-        !sk_b.alloc(N * sizeof(TDKey)) || !sn_b.alloc(sizeof(int)) || !tab_b.alloc((size_t)T * 3 * 8))
-        return td_fail(h, SDPB_ERR_NOMEM, "allocation of the roll-out buffers failed");
-    const TDKey** dF = (const TDKey**)tab_b.p;
-    const int** dQ = (const int**)(dF + T);
-    long long* dn = (long long*)(dQ + T);
-    if (cudaMemcpyAsync(smp_b.p, samples, N * T * sizeof(double), cudaMemcpyHostToDevice, st) != cudaSuccess ||
-        cudaMemcpyAsync(pw_b.p, pw.data(), T * sizeof(double), cudaMemcpyHostToDevice, st) != cudaSuccess ||
-        cudaMemcpyAsync(key_b.p, key0.data(), N * sizeof(TDKey), cudaMemcpyHostToDevice, st) != cudaSuccess ||
-        cudaMemcpyAsync(per_b.p, per0.data(), N * sizeof(int), cudaMemcpyHostToDevice, st) != cudaSuccess ||
-        cudaMemcpyAsync(act_b[0].p, act0.data(), N * sizeof(int), cudaMemcpyHostToDevice, st) != cudaSuccess ||
-        cudaMemsetAsync(sum_b.p, 0, N * sizeof(double), st) != cudaSuccess)
-        return td_fail(h, SDPB_ERR_CUDA, "cudaMemcpyAsync failed");
-    std::vector<const void*> tab((size_t)T * 3);
-    std::vector<int> stall_t;
-    std::vector<TDKey> stall_k;
-    float kern = 0;
-    int rounds = 0, na = n, cur = 0;
-    while (na > 0) {
-        // the tables move when an extension merges new states in: hand the kernel the current ones
-        for (int t = 0; t < T; t++) {
-            tab[t] = h->F[t];
-            tab[T + t] = h->Q[t];
-            std::memcpy(&tab[2 * T + t], &h->nF[t], sizeof(long long));
-        }
-        int ns = 0;
-        if (cudaMemcpyAsync(tab_b.p, tab.data(), tab.size() * 8, cudaMemcpyHostToDevice, st) != cudaSuccess ||
-            cudaMemsetAsync(sn_b.p, 0, sizeof(int), st) != cudaSuccess || cudaEventRecord(h->e1, st) != cudaSuccess)
-            return td_fail(h, SDPB_ERR_CUDA, "cudaMemcpyAsync failed");
-        TD_DISPATCH(launch_simulate, h, dF, dQ, dn, (const double*)smp_b.p, (const double*)pw_b.p,
-                    (const int*)act_b[cur].p, na, (TDKey*)key_b.p, (int*)per_b.p, (double*)sum_b.p, (double*)val_b.p,
-                    (int*)sn_b.p, (int*)act_b[1 - cur].p, (int*)st_b.p, (TDKey*)sk_b.p)
-        if (cudaGetLastError() != cudaSuccess) return td_fail(h, SDPB_ERR_CUDA, "td_simulate launch failed");
-        if (cudaEventRecord(h->e2, st) != cudaSuccess ||
-            cudaMemcpyAsync(&ns, sn_b.p, sizeof(int), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
-            cudaStreamSynchronize(st) != cudaSuccess)
-            return td_fail(h, SDPB_ERR_CUDA, std::string("roll-out: ") + cudaGetErrorString(cudaGetLastError()));
-        float ms = 0;
-        cudaEventElapsedTime(&ms, h->e1, h->e2);
-        kern += ms;
-        rounds++;
-        if (ns == 0) break;
-        // the states the stalled paths stand on become roots of one extension (Simulation.java:62: getExpectedValue)
-        stall_t.resize((size_t)ns);
-        stall_k.resize((size_t)ns);
-        if (cudaMemcpyAsync(stall_t.data(), st_b.p, (size_t)ns * sizeof(int), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
-            cudaMemcpyAsync(stall_k.data(), sk_b.p, (size_t)ns * sizeof(TDKey), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
-            cudaStreamSynchronize(st) != cudaSuccess)
-            return td_fail(h, SDPB_ERR_CUDA, "cudaMemcpyAsync failed");
-        std::vector<std::vector<TDKey>> r((size_t)T);
-        int p = T;
-        for (int j = 0; j < ns; j++) {
-            r[stall_t[j] - 1].push_back(stall_k[j]);
-            p = std::min(p, stall_t[j]);
-        }
-        for (auto& v : r) {
-            std::sort(v.begin(), v.end(), TDLess());
-            v.erase(std::unique(v.begin(), v.end(), TDEq()), v.end());
-        }
-        rc = td_extend(h, p, r);
-        if (rc != SDPB_OK) return rc;
-        na = ns;
-        cur = 1 - cur;
-    }
-    if (cudaMemcpyAsync(values, val_b.p, N * sizeof(double), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
-        cudaStreamSynchronize(st) != cudaSuccess)
-        return td_fail(h, SDPB_ERR_CUDA, "cudaMemcpyAsync failed");
-    h->stats.solve_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - w0).count();
-    h->stats.kernel_ms = kern;
-    h->stats.launches = rounds;
-    return SDPB_OK;
+    TD_DISPATCH(rc = td_rollout, h, roots[0][0], samples, n, discount, values)
+    return rc;
 }
 
 }  // extern "C"
