@@ -656,7 +656,8 @@ bi_cash_row(const __grid_constant__ DevModel M, const int t, const int D, const 
     const long long idx = ixl * M.nW + iw;
     const bool valid = seg * 128 + (int)threadIdx.x < M.nW && idx >= lo && idx < hi;
     const StateCtx S = decode_state<KIND>(M, t, idx);
-    // the richest lane of the CTA has the longest action list (the cash bound of CashConstraint.java:96-99 grows with w)
+    // the richest lane of the CTA has the longest action list: the cash bound of CashConstraint.java:96-99 grows with w
+    // for a unit cost without its sign bit, which the host requires (cash_bound_grows_with_w)
     const StateCtx Stop = decode_state<KIND>(M, t, ixl * M.nW + min(seg * 128 + 127, M.nW - 1));
     const int nA_cta = Stop.nA;
     const double2* __restrict__ rec = M.pmf_rec + 2 * (size_t)pmf_off;
@@ -767,7 +768,7 @@ bi_cash_tail(const __grid_constant__ DevModel M, const int t, const int D, const
     const long long idx = ixl * M.nW + iw;
     const bool valid = seg * 128 + (int)threadIdx.x < M.nW && idx >= lo && idx < hi;
     const StateCtx S = decode_state<KIND>(M, t, idx);
-    const StateCtx Stop = decode_state<KIND>(M, t, ixl * M.nW + min(seg * 128 + 127, M.nW - 1));  // longest action list
+    const StateCtx Stop = decode_state<KIND>(M, t, ixl * M.nW + min(seg * 128 + 127, M.nW - 1));  // longest action list (bi_cash_row)
     const int nA_cta = Stop.nA;
     const double2* __restrict__ rec = M.pmf_rec + 2 * (size_t)pmf_off;
     // constants of the tail, in registers
@@ -866,6 +867,16 @@ bi_cash_tail(const __grid_constant__ DevModel M, const int t, const int D, const
 
 struct CashTailPlan { bool ok = false, div = false; int kk_lo = 0, kk_hi = 0; };
 
+// The row kernels give every lane of a CTA the action count of its richest lane.  The cash-limited bound
+// max(0, ((w - reserve) - reserve2) / v) grows with w for v > 0 and v = +0.0 (inf above the reserve, NaN on it), and
+// falls for v < 0 and v = -0.0, where the poorer lanes would lose actions: such models go to the generic kernel.
+inline bool cash_bound_grows_with_w(const sdpb_model& m) {
+    if (!(m.flags & SDPB_F_CASH_LIMITED_ACTIONS)) return true;
+    for (int t = 0; t < m.T; t++)
+        if (std::signbit(m.vari_cost_t ? m.vari_cost_t[t] : m.vari_cost)) return false;
+    return true;
+}
+
 // Both row-shared kinds, expectation recursion, no lead time, a rounding quantiser, 32-bit grid; every w' * q the
 // kernel can form must stay below 2^30 in magnitude (jround32's low-word read and the integer clamp).
 inline CashTailPlan plan_cash_tail(const sdpb_model& m, const DevModel& d, int D, const double* pmf_d, int n_pmf) {
@@ -873,7 +884,7 @@ inline CashTailPlan plan_cash_tail(const sdpb_model& m, const DevModel& d, int D
     if (!(m.cost_kind == SDPB_COST_CASH_DEPOSIT || m.cost_kind == SDPB_COST_CASH_OVERDRAFT ||
           m.cost_kind == SDPB_COST_CASH_OD_LIMIT || m.cost_kind == SDPB_COST_CASH_OD_TESTING)) return P;
     if (m.recursion != SDPB_REC_EXPECT || m.lead_time != 0 || d.small == 0 || m.quantiser == SDPB_Q_TRUNC) return P;
-    if ((size_t)D * sizeof(CashTailEntry) > 96 * 1024) return P;
+    if ((size_t)D * sizeof(CashTailEntry) > 96 * 1024 || !cash_bound_grows_with_w(m)) return P;
     if (m.cost_kind == SDPB_COST_CASH_DEPOSIT && !(1.0 - m.overhead_rate >= 0.0)) return P;
     double price = std::fabs(m.price), v = std::fabs(m.vari_cost), ovh = std::fabs(m.overhead), dmax = 0;
     for (int t = 0; t < m.T; t++) {
@@ -938,10 +949,11 @@ inline int launch_cash_tail(const CashTailPlan& P, const sdpb_model& m, const De
     return SDPB_OK;
 }
 
-// CASH_DEPOSIT kind without lead time on a grid whose indices fit 32 bits (DevModel::small).
+// CASH_DEPOSIT kind without lead time on a grid whose indices fit 32 bits (DevModel::small), with a cash bound that
+// grows with w.
 inline bool cash_row_ok(const sdpb_model& m, const DevModel& d, int D) {
     return m.cost_kind == SDPB_COST_CASH_DEPOSIT && m.lead_time == 0 && d.small != 0 &&
-           (size_t)D * sizeof(CashRowEntry) <= 96 * 1024;
+           (size_t)D * sizeof(CashRowEntry) <= 96 * 1024 && cash_bound_grows_with_w(m);
 }
 
 inline int launch_cash_row(const sdpb_model& m, const DevModel& dm, int t, int D, int pmf_off, const double* Vn,

@@ -272,6 +272,31 @@ def case_D_terminal():
     return spec, init
 
 
+def case_DL_terminal():
+    spec, init = case_DL_small()
+    spec.terminal_value = spec.tabulate(lambda x, w: w + 0.75 * x - 0.25 * np.maximum(-w, 0.0))
+    spec.name = "DL_terminal"
+    return spec, init
+
+
+def case_DT_terminal():
+    spec, init = case_DT_small()
+    spec.terminal_value = spec.tabulate(lambda x, w: np.minimum(w, 60.0) + 0.5 * x)
+    spec.name = "DT_terminal"
+    return spec, init
+
+
+def case_C_pen_div_terminal():
+    # bankruptcy penalty and the round(w*10)/10 quantiser with long division (CashOverdraft.java:116's idiom) on the
+    # cash-constraint lambdas
+    spec = S.cash_constraint_model(pmf([4, 5, 4]), price=6, vari_cost=2, fixed_cost=2, hold_cost=0.5, salvage=0.0,
+                                   overhead=1.5, penalty_cost=0.5, max_order=8, inv_min=0, inv_max=14, cash_min=-15,
+                                   cash_max=60, quantiser=A.Q_LONGDIV, q_mul=10.0, q_div=10.0,
+                                   name="C_pen_div_terminal")
+    spec.terminal_value = spec.tabulate(lambda x, w: w + 0.5 * x)
+    return spec, [[0.0, 10.0], [3.0, -4.0]]
+
+
 def case_E_terminal():
     spec, init = case_E_small()
     spec.terminal_value = spec.tabulate(lambda x, w, q: w + 0.5 * (x + q))
@@ -329,7 +354,8 @@ def case_CLSP_main():
 NOLAST = [case_A_nolast, case_B2_nolast, case_C_int_nolast]
 
 TERMINAL = [case_A_terminal, case_A_terminal_big, case_B1_terminal, case_B2_terminal, case_C_terminal,
-            case_C_terminal_frac, case_D_terminal, case_E_terminal, case_M2_terminal, case_W_terminal]
+            case_C_terminal_frac, case_D_terminal, case_DL_terminal, case_DT_terminal, case_C_pen_div_terminal,
+            case_E_terminal, case_M2_terminal, case_W_terminal]
 
 ALL = [case_A_small, case_A_max, case_A_gy, case_A_twopoint, case_A_halfstep, case_A_sparse_pmf,
        case_A_degenerate, case_A_one_state, case_B1_ref, case_B1_fixed,
