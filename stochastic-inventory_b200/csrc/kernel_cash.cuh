@@ -262,7 +262,9 @@ inline void plan_cash(CashPlan& P, const sdpb_model& m, const DevModel& d, const
 }
 
 // Shape of a bi_cash_int launch over [lo, hi): R = 16 cash levels per thread in the last period when the grid is large
-// enough, and the action range cut into slices when the launch would otherwise leave the GPU short of CTAs.
+// enough, and the action range cut into slices when the launch would otherwise leave the GPU short of CTAs.  gridDim.y
+// = ceil(nW / tile) stays far below CUDA's 65535: plan_cash keeps |cash_min| and |cash_max| below 2^20, so nW < 2^21
+// and the y dimension is at most 8192.
 struct CashIntShape { bool wide; int tile, parts; dim3 grid; };
 
 inline CashIntShape cash_int_shape(const sdpb_model& m, const DevModel& dm, int t, long long lo, long long hi, int sm_count) {
@@ -575,10 +577,12 @@ inline int cash_diag_parts(const sdpb_model& m, const DevModel& dm, const CashPe
 
 inline size_t cash_diag_smem(int D) { return (((size_t)D * 24 + 15) & ~(size_t)15) + 16; }
 
-// Whether bi_cash_diag can solve a period (t < T) whose integer plan is cp.
+// Whether bi_cash_diag can solve a period (t < T) whose integer plan is cp.  The launch puts the 8-row tiles on
+// gridDim.y, which CUDA caps at 65535: a whole-grid bound, since no shard has more rows than the grid.
 inline bool cash_diag_ok(const CashPeriod& cp, const sdpb_model& m, const DevModel& dm, int D) {
     return cp.price > 0 && cp.price * (kDiagYT - 1) <= dm.nW &&  // the diagonal must stay on the cash axis
            (long long)(dm.nI + D + std::abs(cp.d0) + 2 * kDiagYT + m.max_order_idx) * dm.nW < 0x7fffffffLL &&  // 32-bit row offsets
+           (dm.nI + kDiagYT - 1) / kDiagYT <= 65535 &&
            cash_diag_smem(D) <= 200 * 1024;
 }
 

@@ -899,7 +899,8 @@ int solve_period(sdpb_handle* h, int t) {
 //   request COLLAPSED or GENERIC: that kernel
 //   backorder, lead 0, clamp: TILED (tiled / tiled2 at launch) if the period has a plan and is not plain
 //   integer-exact deposit models, any request, periods with a plan, not plain or term_T, a non-empty shard:
-//     CASH_DIAG if t < T, the request is not CASH_INT and cash_diag_ok;  CASH_INT if its tables fit
+//     CASH_DIAG if t < T, the request is not CASH_INT and cash_diag_ok (which includes at most 65535 tiles of 8
+//     inventory rows);  CASH_INT if its tables fit
 //   backorder, lead >= 1, not plain: LEAD_Q2 (q2 / q2m at launch) if dVT exists (lead 2, unfolded, request AUTO or
 //     LEAD_Q2) and plan_q2 holds;  LEAD_COL if the request is neither STAGED nor LEAD_SLAB and plan_col holds;
 //     LEAD_SLAB if the request is not STAGED and plan_lead holds
